@@ -19,6 +19,9 @@ EVERY strip boundary — are read with their (16 + 2k)^2 light cones (state + ST
 lattice steps k = 12 more timesteps, and the oracle steps the same patches; last_firing_time must be bit-equal, float state equal
 to 1e-4.  The line carries `"parity": {"checked": n, "ok": true, ...}`; a mismatch exits non-zero.  At N > 1 the same line also
 carries `"strong"`: the SAME 3163-row lattice split over the N GPUs (strong scaling), timed and parity-checked the same way.
+
+`--dump-outputs DIR` (one GPU) writes, right after the timed steps, a seeded sample of the lattice state and weights those steps
+left as DIR/<field>.npy (see dump_outputs), so that the outputs of two builds can be compared.
 """
 import argparse
 import json
@@ -55,6 +58,8 @@ def parse_args():
     ap.add_argument("--no-strong", action="store_true", help="N > 1, weak mode: skip the extra strong-scaling leg")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--parity-steps", type=int, default=12)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the lattice state and STDP weights to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -96,6 +101,27 @@ def configure(be, fields):
     be.set_option(0, 1)      # electrical_synapse
     be.set_option(1, 1)      # chemical_synapse
     be.set_option(2, 1, 0)   # do_plasticity (STDP defaults 2, 2, 4.5, 4.5, dt 0.1)
+
+
+DUMP_SAMPLE = 1 << 20   # neurons and edges kept by --dump-outputs: 44 MB of .npy files in all
+
+
+def dump_outputs(np, be, out_dir):
+    """Write what the timed run_lattice calls left in the lattice, as a caller reads it back: every STATE_FIELDS array and the
+    STDP-learned in-edge weights (CSR order).  The whole state of the default workload is about 0.64 GB, so a fixed seeded sample
+    of neurons and of edges is kept; the inputs are seeded too, so two builds run with the same arguments compare array for
+    array.  Floating-point fields stay float32, integer fields are written as float64 (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0xD1FF)
+    n = be.size()
+    cells = np.sort(rng.choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    for nm in STATE_FIELDS:
+        a = be.get_field(0, nm).reshape(n, -1)[cells]
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        np.save(os.path.join(out_dir, nm.replace("$", ".") + ".npy"), a if nm in PER3 else a[:, 0])
+    w = be.get_connection_csr()[2]
+    edges = np.sort(rng.choice(w.size, size=min(w.size, DUMP_SAMPLE), replace=False))
+    np.save(os.path.join(out_dir, "weights.npy"), w[edges])
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -428,6 +454,8 @@ def measure_lattice(args, np, torch, dist, K, rows_g, rank, world, local_rank, s
     out = {"be": be, "fields": fields, "n_local": n_local, "dev_ms": dev_ms_max, "wall_ms": wall_ms_max, "launches": launches,
            "clocks": clocks, "spiked_fraction": spikes / max(1, n_local), "rows_global": rows_g,
            "total_neurons": rows_g * cols, "edges_total": 8 * rows_g * cols - 6 * (rows_g + cols) + 4}
+    if args.dump_outputs:
+        dump_outputs(np, be, args.dump_outputs)
 
     # ---- parity vs the CPU oracle on the live lattice (outside every timed region)
     if not args.no_parity:
@@ -472,6 +500,9 @@ def measure_lattice(args, np, torch, dist, K, rows_g, rank, world, local_rank, s
 
 def main():
     args = parse_args()
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        raise SystemExit("--dump-outputs writes the lattice of the single-GPU CUDA path: one process, --impl ours")
     if args.impl == "reference":
         return reference_arm(args)
 

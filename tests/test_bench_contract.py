@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -21,6 +23,66 @@ def test_reference_arm_prints_one_contract_line():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"] and d["vs_baseline"] is None and d["gpu_launches"] == 0
+
+
+def test_dump_outputs_writes_a_seeded_sample(tmp_path, monkeypatch):
+    """bench.dump_outputs on an oracle lattice (same protocol as CudaLatticeBackend): one float32/float64 .npy per state field plus
+    the weights, the values of a fixed sample of neurons and edges, identical on a second call, and within 64 MB at the full
+    sample size."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import bench
+    from oracle_api import OracleBackend
+    rows = cols = 20
+    n = rows * cols
+    ob = OracleBackend(4, 0, 0, rows=rows, cols=cols)
+    f = bench.init_fields(np, n, 3)
+    f["c_m"] = np.full(n, 4.0, np.float32)
+    for name, arr in f.items():
+        if name not in ("v_init", "w_init"):
+            ob.set_field(0, name, arr)
+    ob.connect_grid(0, 1, 1.0)
+    ob.set_option(0, 1); ob.set_option(1, 1); ob.set_option(2, 1, 0)
+    ob.run(30)
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 100)
+    bench.dump_outputs(np, ob, str(tmp_path / "a"))
+    bench.dump_outputs(np, ob, str(tmp_path / "b"))
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted([nm.replace("$", ".") + ".npy" for nm in bench.STATE_FIELDS] + ["weights.npy"])
+    total = 0
+    for nm in names:
+        a, b = np.load(tmp_path / "a" / nm), np.load(tmp_path / "b" / nm)
+        assert a.dtype in (np.float32, np.float64) and a.shape[0] == 100 and np.array_equal(a, b), nm
+        total += a.nbytes
+    assert total * (1 << 20) // 100 <= 64 << 20
+    lft = ob.get_field(0, "last_firing_time")
+    got = np.load(tmp_path / "a" / "last_firing_time.npy")
+    assert (got >= 0).any() and np.isin(got, lft.astype(np.float64)).all()
+    w = ob.get_connection_csr()[2]
+    assert (w != 1.0).any() and np.isin(np.load(tmp_path / "a" / "weights.npy"), w).all()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_follow_the_timed_steps(tmp_path):
+    """The GPU arm at 264 x 256 (large enough for the bench's window kernel): the same arguments dump the same arrays, and one
+    timed step fewer dumps different ones, so the dump is what the last of `--steps` timed steps left."""
+    import numpy as np
+
+    def run(tag, steps):
+        out = tmp_path / tag
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--iters", "20",
+                            "--rows", "264", "--cols", "256", "--no-cpu-baseline", "--no-configs", "--no-e2e", "--no-parity",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-4000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        return {p.name: np.load(p) for p in sorted(out.iterdir())}
+
+    a, b, c = run("a", 2), run("b", 2), run("c", 1)
+    assert len(a) == 7 and a.keys() == b.keys() == c.keys()
+    assert all(np.array_equal(a[k], b[k], equal_nan=True) for k in a)
+    assert not np.array_equal(a["current_voltage.npy"], c["current_voltage.npy"])
+    assert (a["last_firing_time.npy"] >= 0).any()
 
 
 def test_gpu_arm_fails_loudly_without_a_device():
