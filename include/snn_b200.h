@@ -159,8 +159,12 @@ typedef enum snn_option {
     SNN_OPT_GENERAL_PARTITION = 12,   /* partitioned handles: the next snn_lattice_set_graph_csr builds gather-list ghosts (general-graph
                                          partition) even if this rank's edges happen to stay inside the strip halo — set it on EVERY
                                          rank when any rank's graph reaches further (the mode must be the same on all ranks) */
-    SNN_OPT_HALO_TIMEOUT_MS = 11      /* partitioned handles: bound of one in-kernel wait for a neighbouring strip (default 30000);
+    SNN_OPT_HALO_TIMEOUT_MS = 11,     /* partitioned handles: bound of one in-kernel wait for a neighbouring strip (default 30000);
                                          run() first meets the neighbours on the host (4x this bound) before any step is enqueued */
+    SNN_OPT_UPDATE_GRAPH_HISTORY = 13,  /* default 0 (per lattice): Graph::update_history of the lattice's own graph (graph/mod.rs:278-284),
+                                           one record per step, read with snn_lattice_get_graph_history / snn_network_get_graph_history */
+    SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY = 14  /* default 0 (network-wide): LatticeNetwork::update_connecting_graph_history, one
+                                                     record per step of every connecting block (pre_id != post_id) */
 } snn_option_t;
 
 /* STDP, backend/src/neuron/plasticity/mod.rs:14-39 (defaults 2, 2, 4.5, 4.5, 0.1) */
@@ -335,6 +339,15 @@ SNN_API int32_t snn_lattice_get_spike_aggregate(snn_lattice_t *h, int64_t *out, 
 SNN_API int32_t snn_lattice_set_eeg_parameters(snn_lattice_t *h, float reference_voltage, float distance, float conductivity);
 SNN_API int32_t snn_lattice_get_eeg_history(snn_lattice_t *h, float *out, uint64_t capacity_floats);
 SNN_API int32_t snn_lattice_reset_history(snn_lattice_t *h);
+/* graph history (SNN_OPT_UPDATE_GRAPH_HISTORY): `steps` records of `nnz` f32 weights each, every record in the edge order of
+ * snn_lattice_get_graph_csr.  Record k holds the weights after step k's plasticity (Lattice::iterate pushes the history at the
+ * end of the step, neuron/mod.rs:973-979), so with STDP the last record equals snn_lattice_get_graph_csr after the run.  Recorded
+ * on the device and drained between history chunks; while it is on, every timestep is its own launch (SNN_OPT_STEPS_PER_GRAPH = 1).
+ * Cleared by reset_history (not by reset_timing).  SNN_UNSUPPORTED from run: partitioned handles and reward-modulated lattices
+ * (TraceRSTDP weights); from set_graph_* and edge-adding/removing edit_weight: while the history holds records, since the
+ * records assume one adjacency (edit_weight of an existing edge is allowed; reset_history lifts the restriction). */
+SNN_API int32_t snn_lattice_graph_history_len(snn_lattice_t *h, uint64_t *steps, uint64_t *nnz);
+SNN_API int32_t snn_lattice_get_graph_history(snn_lattice_t *h, float *out, uint64_t capacity_floats);
 
 /* ---- multi-GPU row strips (one process per GPU; plumbing by the caller, e.g. torch.distributed) */
 /* first global row of `rank`'s strip; rank == world gives `rows` */
@@ -428,10 +441,10 @@ SNN_API int32_t snn_network_lookup_weight(snn_network_t *h, uint64_t pre_id, uin
 SNN_API int32_t snn_network_edit_weight(snn_network_t *h, uint64_t pre_id, uint64_t post_id, uint64_t pre, uint64_t post,
                                         int32_t connected, float weight);
 
-/* network-wide: ELECTRICAL_SYNAPSE, CHEMICAL_SYNAPSE, INTERNAL_CLOCK, RNG_SEED, PARALLEL */
+/* network-wide: ELECTRICAL_SYNAPSE, CHEMICAL_SYNAPSE, INTERNAL_CLOCK, RNG_SEED, PARALLEL, UPDATE_CONNECTING_GRAPH_HISTORY */
 SNN_API int32_t snn_network_set_option(snn_network_t *h, int32_t option, int64_t value);
 SNN_API int32_t snn_network_get_option(const snn_network_t *h, int32_t option, int64_t *value);
-/* per lattice: DO_PLASTICITY, UPDATE_GRID_HISTORY, UPDATE_SPIKE_HISTORY, INTERNAL_CLOCK (spike-train lattices) */
+/* per lattice: DO_PLASTICITY, UPDATE_GRID_HISTORY, UPDATE_SPIKE_HISTORY, UPDATE_GRAPH_HISTORY, INTERNAL_CLOCK (spike-train lattices) */
 SNN_API int32_t snn_network_set_lattice_option(snn_network_t *h, uint64_t id, int32_t option, int64_t value);
 SNN_API int32_t snn_network_get_lattice_option(const snn_network_t *h, uint64_t id, int32_t option, int64_t *value);
 SNN_API int32_t snn_network_set_plasticity(snn_network_t *h, uint64_t id, const snn_stdp_t *stdp);
@@ -477,6 +490,13 @@ SNN_API int32_t snn_network_get_average_history(snn_network_t *h, uint64_t id, f
 SNN_API int32_t snn_network_set_eeg_parameters(snn_network_t *h, uint64_t id, float reference_voltage, float distance, float conductivity);
 SNN_API int32_t snn_network_get_eeg_history(snn_network_t *h, uint64_t id, float *out, uint64_t capacity_floats);
 SNN_API int32_t snn_network_reset_history(snn_network_t *h);
+/* graph history of the block pre_id -> post_id: a lattice's own graph (pre_id == post_id, SNN_OPT_UPDATE_GRAPH_HISTORY through
+ * snn_network_set_lattice_option) or a connecting block (SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY).  Record k holds the weights
+ * step k's input gather used: LatticeNetwork::iterate pushes the histories before that step's STDP (neuron/mod.rs:2565-2576), so
+ * record 0 is the weights before the run.  Edge order of snn_network_get_connection_csr(pre_id, post_id); a block never recorded
+ * (or without edges) reports steps = nnz = 0.  Same restrictions as the lattice calls (reward-modulated networks: SNN_UNSUPPORTED). */
+SNN_API int32_t snn_network_graph_history_len(snn_network_t *h, uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz);
+SNN_API int32_t snn_network_get_graph_history(snn_network_t *h, uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity_floats);
 
 #ifdef __cplusplus
 }

@@ -70,6 +70,13 @@ inline Csr evaluate(std::size_t pre_rows, std::size_t pre_cols, std::size_t post
 }
 }  // namespace detail
 
+// Graph::update_history records (graph/mod.rs:278-284): `steps` records of `nnz` weights, each in the edge order of the graph's CSR
+// (snn_lattice_get_graph_csr / snn_network_get_connection_csr), record k at weights[k * nnz]
+struct GraphHistory {
+    std::size_t steps = 0, nnz = 0;
+    std::vector<float> weights;
+};
+
 // ----------------------------------------------------------------------------------------------------------------------------
 // Lattice<T, AdjacencyMatrix, GridVoltageHistory, STDP, N>  (neuron/mod.rs:556-1220) on one B200
 // ----------------------------------------------------------------------------------------------------------------------------
@@ -78,6 +85,7 @@ public:
     // public fields of the reference struct (neuron/mod.rs:556-587)
     bool electrical_synapse = true, chemical_synapse = false, do_plasticity = false;
     bool update_grid_history = false, update_spike_history = false, parallel = false;
+    bool update_graph_history = false;   // records after each step's plasticity (Lattice::iterate, neuron/mod.rs:973-979)
     STDP plasticity;
 
     Lattice() = default;
@@ -165,6 +173,15 @@ public:
         return v;
     }
     void reset_history() { ck(snn_lattice_reset_history(need())); }
+    GraphHistory graph_history() {
+        GraphHistory g;
+        uint64_t steps = 0, nnz = 0;
+        ck(snn_lattice_graph_history_len(need(), &steps, &nnz));
+        g.steps = steps; g.nnz = nnz;
+        g.weights.resize(steps * nnz);
+        ck(snn_lattice_get_graph_history(h_, g.weights.data(), g.weights.size()));
+        return g;
+    }
 
     snn_lattice_t *handle() { return h_; }
 
@@ -182,6 +199,7 @@ protected:
         ck(snn_lattice_set_option(h_, SNN_OPT_DO_PLASTICITY, do_plasticity));
         ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_GRID_HISTORY, update_grid_history));
         ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_SPIKE_HISTORY, update_spike_history));
+        ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_GRAPH_HISTORY, update_graph_history));
         ck(snn_lattice_set_option(h_, SNN_OPT_PARALLEL, parallel));
         const snn_stdp_t s{plasticity.a_plus, plasticity.a_minus, plasticity.tau_plus, plasticity.tau_minus, plasticity.dt};
         ck(snn_lattice_set_plasticity(h_, &s));
@@ -230,6 +248,9 @@ protected:
 class LatticeNetwork {
 public:
     bool electrical_synapse = true, chemical_synapse = false;
+    // records of every connecting block before each step's STDP (neuron/mod.rs:2565-2576); a lattice's own graph is recorded with
+    // set_lattice_option(id, SNN_OPT_UPDATE_GRAPH_HISTORY, 1)
+    bool update_connecting_graph_history = false;
 
     explicit LatticeNetwork(snn_model_t model = SNN_MODEL_IZHIKEVICH, snn_spike_train_t spike_train = SNN_TRAIN_POISSON,
                             snn_nt_kinetics_t ntk = SNN_NT_APPROXIMATE, snn_receptor_kinetics_t rck = SNN_RC_APPROXIMATE,
@@ -280,7 +301,18 @@ public:
     void run_lattices(std::size_t iterations) {
         ck(snn_network_set_option(h_, SNN_OPT_ELECTRICAL_SYNAPSE, electrical_synapse));
         ck(snn_network_set_option(h_, SNN_OPT_CHEMICAL_SYNAPSE, chemical_synapse));
+        ck(snn_network_set_option(h_, SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY, update_connecting_graph_history));
         ck(snn_network_run(h_, iterations));
+    }
+    // the records of the block pre_id -> post_id (pre_id == post_id: the lattice's own graph)
+    GraphHistory graph_history(std::size_t pre_id, std::size_t post_id) {
+        GraphHistory g;
+        uint64_t steps = 0, nnz = 0;
+        ck(snn_network_graph_history_len(h_, pre_id, post_id, &steps, &nnz));
+        g.steps = steps; g.nnz = nnz;
+        g.weights.resize(steps * nnz);
+        ck(snn_network_get_graph_history(h_, pre_id, post_id, g.weights.data(), g.weights.size()));
+        return g;
     }
     std::vector<uint8_t> spike_history(std::size_t id) {
         uint64_t steps = 0, n = 0;
@@ -371,6 +403,7 @@ public:
     void run_lattices_with_reward(float reward) {
         ck(snn_network_set_option(h_, SNN_OPT_ELECTRICAL_SYNAPSE, electrical_synapse));
         ck(snn_network_set_option(h_, SNN_OPT_CHEMICAL_SYNAPSE, chemical_synapse));
+        ck(snn_network_set_option(h_, SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY, update_connecting_graph_history));
         ck(snn_network_run_with_rewards(h_, &reward, 1));
     }
     std::vector<float> connection_weights(std::size_t pre_id, std::size_t post_id) {

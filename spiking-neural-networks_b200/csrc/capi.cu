@@ -231,6 +231,8 @@ static int32_t engine_set_option(Engine *e, bool have_id, uint64_t id, int32_t o
     case SNN_OPT_UPDATE_SPIKE_HISTORY: if (!L) break; L->spike_hist = value != 0; return SNN_OK;
     case SNN_OPT_UPDATE_AVERAGE_HISTORY: if (!L || L->is_train) break; L->avg_hist = value != 0; return SNN_OK;
     case SNN_OPT_UPDATE_EEG_HISTORY: if (!L || L->is_train) break; L->eeg_hist = value != 0; return SNN_OK;
+    case SNN_OPT_UPDATE_GRAPH_HISTORY: if (!L || L->is_train) break; L->graph_hist = value != 0; return SNN_OK;
+    case SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY: if (L || !e->is_network) break; e->conn_graph_hist = value != 0; return SNN_OK;
     }
     return e->fail(SNN_INVALID_ARGUMENT, "unknown option or missing lattice id");
 }
@@ -252,6 +254,8 @@ static int32_t engine_get_option(const Engine *e, bool have_id, uint64_t id, int
     case SNN_OPT_UPDATE_SPIKE_HISTORY: if (!L) break; *value = L->spike_hist; return SNN_OK;
     case SNN_OPT_UPDATE_AVERAGE_HISTORY: if (!L) break; *value = L->avg_hist; return SNN_OK;
     case SNN_OPT_UPDATE_EEG_HISTORY: if (!L) break; *value = L->eeg_hist; return SNN_OK;
+    case SNN_OPT_UPDATE_GRAPH_HISTORY: if (!L) break; *value = L->graph_hist; return SNN_OK;
+    case SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY: if (L || !e->is_network) break; *value = e->conn_graph_hist; return SNN_OK;
     }
     return SNN_INVALID_ARGUMENT;
 }
@@ -345,6 +349,14 @@ int32_t snn_lattice_reset_history(snn_lattice_t *h) {
     if (!h) return SNN_INVALID_ARGUMENT;
     return h->e->reset_history();
 }
+int32_t snn_lattice_graph_history_len(snn_lattice_t *h, uint64_t *steps, uint64_t *nnz) {
+    if (!h || !steps || !nnz) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->graph_history_len(kLatticeId, kLatticeId, steps, nnz); SNN_CATCH(h)
+}
+int32_t snn_lattice_get_graph_history(snn_lattice_t *h, float *out, uint64_t capacity_floats) {
+    if (!h) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->get_graph_history(kLatticeId, kLatticeId, out, capacity_floats); SNN_CATCH(h)
+}
 
 uint32_t snn_lattice_ipc_blob_size(void) { return (uint32_t)sizeof(snn::IpcBlob); }
 int32_t snn_lattice_ipc_export(snn_lattice_t *h, void *blob) {
@@ -389,6 +401,7 @@ int32_t snn_network_create(const snn_network_desc_t *desc, snn_network_t **out) 
         Engine *e = new Engine(desc->model, desc->nt_kinetics, desc->receptor_kinetics, desc->spike_train, desc->refractoriness, desc->device);
         int r = e->init();
         if (r) { g_create_error = e->last_error; delete e; return r; }
+        e->is_network = true;
         *out = new snn_network{e};
         return SNN_OK;
     } catch (...) { g_create_error = "allocation failed"; return SNN_GPU_BUFFER_CREATE_ERROR; }
@@ -589,6 +602,14 @@ int32_t snn_network_get_spike_history(snn_network_t *h, uint64_t id, uint8_t *ou
 int32_t snn_network_reset_history(snn_network_t *h) {
     if (!h) return SNN_INVALID_ARGUMENT;
     return h->e->reset_history();
+}
+int32_t snn_network_graph_history_len(snn_network_t *h, uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz) {
+    if (!h || !steps || !nnz) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->graph_history_len(pre_id, post_id, steps, nnz); SNN_CATCH(h)
+}
+int32_t snn_network_get_graph_history(snn_network_t *h, uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity_floats) {
+    if (!h) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->get_graph_history(pre_id, post_id, out, capacity_floats); SNN_CATCH(h)
 }
 
 }  // extern "C"

@@ -394,5 +394,10 @@ cudaError_t launch_bits_from_u32(const uint32_t *src, uint32_t *words, uint64_t 
 cudaError_t launch_u32_from_bits(const uint32_t *words, uint32_t *dst, uint64_t n, uint64_t bit0, cudaStream_t s);
 cudaError_t launch_transpose_in(const float *src_nm, float *dst_tm, uint64_t n, uint64_t stride, cudaStream_t s);
 cudaError_t launch_transpose_out(const float *src_tm, float *dst_nm, uint64_t n, uint64_t stride, cudaStream_t s);
+// graph history (graph_history.cu): row_off[0 .. 32 n_slices] = exclusive prefix sum of the valid entries per table row, and one
+// record of every table weight in canonical CSR order written to out[0 .. row_off[32 n_slices]); max_width = widest slice in k-rows
+cudaError_t launch_graph_row_offsets(const uint32_t *col, const uint32_t *slice_off, uint32_t n_slices, uint32_t *row_off, cudaStream_t s);
+cudaError_t launch_graph_record(const float *wgt, const uint32_t *slice_off, const uint32_t *row_off, uint32_t n_slices,
+                                uint32_t max_width, float *out, cudaStream_t s);
 
 }  // namespace snn

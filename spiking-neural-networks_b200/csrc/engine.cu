@@ -71,6 +71,7 @@ Engine::~Engine() {
     if (rnet_tab_) cudaFree(rnet_tab_);
     if (wide_scratch_) cudaFree(wide_scratch_);
     if (scratch_) cudaFree(scratch_);
+    if (ghist_row_off_) cudaFree(ghist_row_off_);
     if (ev0_) cudaEventDestroy(ev0_);
     if (ev1_) cudaEventDestroy(ev1_);
     if (stream_) cudaStreamDestroy(stream_);
@@ -924,6 +925,7 @@ int Engine::connect_dense(uint64_t pre_id, uint64_t post_id, const uint32_t *con
     if (r) return r;
     if (n_pre != A->n || n_post != B->n) return fail(SNN_GRAPH_DIMENSIONS_DO_NOT_MATCH, "Dimensions do not match");
     if (n_pre != 0 && n_post != 0 && (!connections || !weights)) return fail(SNN_INVALID_ARGUMENT, "null graph pointers");
+    if ((r = refuse_if_graph_history("connect"))) return r;
     if (part_world > 1) return fail(SNN_UNSUPPORTED, "dense graphs are not supported on partitioned handles");
     if (itp) {
         if (pre_id != post_id) return fail(SNN_INVALID_ARGUMENT, "index_to_position only applies to an internal graph");
@@ -969,6 +971,7 @@ int Engine::connect_csr(uint64_t pre_id, uint64_t post_id, const uint64_t *row_p
         if (pre[k] >= pre_limit) return fail(SNN_GRAPH_PRESYNAPTIC_NOT_FOUND, "Presynaptic position not found, position: " + std::to_string(pre[k]));
     for (uint64_t q = 0; q < n_post; ++q)
         if (row_ptr[q + 1] < row_ptr[q]) return fail(SNN_INVALID_ARGUMENT, "row_ptr must be non-decreasing");
+    if ((r = refuse_if_graph_history("connect"))) return r;
     if (dev_weights_newer_) { r = sync_weights_to_host(); if (r) return r; }
     Block b;
     b.kind = Block::CSR;
@@ -1007,6 +1010,7 @@ int Engine::connect_grid(uint64_t id, uint32_t radius, float weight) {
     int r = check_connect(*this, id, id, &A, &B);
     if (r) return r;
     if (radius > 7) return fail(SNN_UNSUPPORTED, "stencil radius too large");
+    if ((r = refuse_if_graph_history("connect"))) return r;
     if (part_world > 1) {
         const uint32_t need = radius * A->cols;
         if (need > A->n && A->n) return fail(SNN_UNSUPPORTED, "strip is thinner than the stencil radius");
@@ -1091,6 +1095,7 @@ uint32_t Engine::rc_used() const { refresh_flag_cache(); return rc_used_; }
 
 int Engine::finalize_graph() {
     if (!graph_dirty_) return SNN_OK;
+    ghist_off_valid_ = false;   // the canonical order of the new table is counted again by the next run that records it
     free_reward_arrays();   // a rebuilt graph starts from TraceRSTDP::default traces
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
     // the stencil fast path re-generates the table in place when its size is unchanged (set_graph_grid called again,
@@ -1668,6 +1673,7 @@ int Engine::edit_weight(uint64_t pre_id, uint64_t post_id, uint64_t pre, uint64_
         return SNN_OK;
     }
     if (e < 0 && !has) return SNN_OK;   // None over None
+    if ((r = refuse_if_graph_history("adding or removing an edge"))) return r;
     // the adjacency changes (None -> Some, Some -> None): edit the host CSR of the block and rebuild the device table lazily
     if (part_world > 1) return fail(SNN_UNSUPPORTED, "adding or removing edges is not supported on partitioned handles (weights of existing edges are)");
     dev_weights_newer_ = true;   // the device holds the live weights (STDP, earlier in-place edits)
@@ -1735,6 +1741,41 @@ int Engine::reset_timing() {
 
 int Engine::reset_history() {
     for (auto &L : lats_) { L.grid_history.clear(); L.spike_history.clear(); L.spike_agg.clear(); L.average_history.clear(); L.eeg_history.clear(); L.hist_len = 0; }
+    graph_hist_.clear();
+    return SNN_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// graph history (Graph::update_history, graph/mod.rs:278-284)
+// ------------------------------------------------------------------------------------------------
+bool Engine::graph_history_nonempty() const {
+    for (auto &kv : graph_hist_) if (kv.second.steps) return true;
+    return false;
+}
+
+// a record is the block's weights in a fixed edge order: the adjacency stays put until reset_history clears the records
+int Engine::refuse_if_graph_history(const char *what) {
+    if (!graph_history_nonempty()) return SNN_OK;
+    return fail(SNN_UNSUPPORTED, std::string(what) + ": the adjacency cannot change while a graph history holds records (reset_history first)");
+}
+
+int Engine::graph_history_len(uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz) {
+    const Lat *A = find(pre_id), *B = find(post_id);
+    if (!A || !B || B->is_train) return fail(SNN_NET_ID_NOT_FOUND_IN_LATTICES, "Id not present in lattices");
+    auto it = graph_hist_.find({pre_id, post_id});
+    if (steps) *steps = it == graph_hist_.end() ? 0 : it->second.steps;
+    if (nnz) *nnz = it == graph_hist_.end() ? 0 : it->second.nnz;
+    return SNN_OK;
+}
+
+int Engine::get_graph_history(uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity) {
+    const Lat *A = find(pre_id), *B = find(post_id);
+    if (!A || !B || B->is_train) return fail(SNN_NET_ID_NOT_FOUND_IN_LATTICES, "Id not present in lattices");
+    auto it = graph_hist_.find({pre_id, post_id});
+    if (it == graph_hist_.end() || it->second.w.empty()) return SNN_OK;
+    if (capacity < it->second.w.size()) return fail(SNN_SIZE_MISMATCH, "graph history buffer too small");
+    if (!out) return fail(SNN_INVALID_ARGUMENT, "null argument");
+    memcpy(out, it->second.w.data(), it->second.w.size() * 4);
     return SNN_OK;
 }
 
@@ -2039,6 +2080,16 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
     if (iterations == 0 || (n_neurons == 0 && n_trains == 0)) return SNN_OK;
     if (!electrical && !chemical) return SNN_OK;
     if (internal_clock + iterations > 0x7FFFFFF0ull) return fail(SNN_UNSUPPORTED, "internal clock would overflow the i32 last_firing_time");
+    // graph history: the blocks whose records this run appends to (a lattice's own graph; every non-empty connecting block)
+    std::vector<std::pair<uint64_t, uint64_t>> gh_keys;
+    for (auto &L : lats_) if (!L.is_train && L.graph_hist) gh_keys.emplace_back(L.id, L.id);
+    if (conn_graph_hist)
+        for (auto &kv : blocks_)
+            if (kv.first.first != kv.first.second && (kv.second.kind == Block::GRID || !kv.second.pre.empty())) gh_keys.push_back(kv.first);
+    const bool ghist_on = !gh_keys.empty();
+    if (ghist_on && part_world > 1) return fail(SNN_UNSUPPORTED, "graph history: whole-GPU handles only (not row strips or general-graph partitions)");
+    if (ghist_on && (reward_mode || has_reward_lattices()))
+        return fail(SNN_UNSUPPORTED, "graph history: not recorded for reward-modulated lattices and networks (TraceRSTDP weights)");
     if (part_world > 1 && !gpart_) {
         if ((part_rank > 0 && !halo_dir_[0].active) || (part_rank < part_world - 1 && !halo_dir_[1].active))
             return fail(SNN_INVALID_ARGUMENT, "partitioned handle: neighbouring strips are not attached");
@@ -2051,6 +2102,63 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
     r = upload_lat_table();
     if (r) return r;
     if (gpart_) { r = gpart_build_device(); if (r) return r; }
+    // graph history: per-row offsets of the table's canonical order (once per graph build), then how each requested block is cut
+    // out of a record: the whole record (the table holds that block only) or one contiguous range per postsynaptic row
+    struct GhPlan { GraphHist *h; bool whole; const Block *b; std::vector<uint64_t> src; };
+    std::vector<GhPlan> gh_plans;
+    if (ghist_on) {
+        if (!ghist_off_valid_) {
+            if (ghist_row_off_) cudaFree(ghist_row_off_);
+            ghist_row_off_ = nullptr;
+            CK(dev_alloc(&ghist_row_off_, (size_t)n_slices_ * 32 + 1), SNN_GPU_BUFFER_CREATE_ERROR);
+            CK(launch_graph_row_offsets(col_, slice_off_, n_slices_, ghist_row_off_, stream_), SNN_GPU_QUEUE_FAILURE);
+            uint32_t tot = 0;
+            CK(cudaMemcpyAsync(&tot, ghist_row_off_ + (size_t)n_slices_ * 32, 4, cudaMemcpyDeviceToHost, stream_), SNN_GPU_BUFFER_READ_ERROR);
+            CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
+            ghist_nnz_ = tot;
+            std::vector<uint32_t> so((size_t)n_slices_ + 1);
+            CK(cudaMemcpy(so.data(), slice_off_, so.size() * 4, cudaMemcpyDeviceToHost), SNN_GPU_BUFFER_READ_ERROR);
+            ghist_max_width_ = 0;
+            for (uint32_t sl = 0; sl < n_slices_; ++sl) ghist_max_width_ = std::max(ghist_max_width_, so[sl + 1] - so[sl]);
+            ghist_off_valid_ = true;
+        }
+        std::vector<uint64_t> roff;   // canonical row offsets of the table from the host blocks (several blocks only)
+        for (auto &key : gh_keys) {
+            GhPlan pl{&graph_hist_[key], false, nullptr, {}};
+            auto it = blocks_.find(key);
+            if (it != blocks_.end() && blocks_.size() == 1) {
+                pl.whole = true;
+                pl.h->nnz = ghist_nnz_;
+            } else if (it != blocks_.end()) {
+                // finalize_graph's general path: every block is host CSR; rows hold the blocks into their lattice ordered by the
+                // presynaptic lattice's node offset (sync_weights_to_host walks them the same way)
+                if (roff.empty()) {
+                    roff.assign(n_neurons + 1, 0);
+                    for (auto &kv : blocks_) {
+                        const Lat *B = find(kv.first.second);
+                        for (uint64_t q = 0; q < B->n; ++q) roff[B->off + q + 1] += kv.second.row_ptr[q + 1] - kv.second.row_ptr[q];
+                    }
+                    for (uint64_t i = 0; i < n_neurons; ++i) roff[i + 1] += roff[i];
+                    if (roff[n_neurons] != ghist_nnz_) return fail(SNN_GPU_BUFFER_READ_ERROR, "graph history: host and device tables disagree");
+                }
+                const Lat *A = find(key.first), *B = find(key.second);
+                std::vector<const Block *> before;
+                for (auto &kv : blocks_)
+                    if (kv.first.second == key.second && kv.first != key && node_off(*find(kv.first.first)) < node_off(*A)) before.push_back(&kv.second);
+                pl.b = &it->second;
+                pl.src.resize(B->n);
+                for (uint64_t q = 0; q < B->n; ++q) {
+                    uint64_t o = roff[B->off + q];
+                    for (const Block *o_b : before) o += o_b->row_ptr[q + 1] - o_b->row_ptr[q];
+                    pl.src[q] = o;
+                }
+                pl.h->nnz = it->second.pre.size();
+            } else {
+                pl.h->nnz = 0;   // a lattice without an internal graph: empty records
+            }
+            gh_plans.push_back(std::move(pl));
+        }
+    }
 
     bool stdp = false, want_grid = false, want_spk = false, want_tgrid = false, want_tspk = false, want_red = false;
     for (auto &L : lats_) {
@@ -2240,6 +2348,7 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
         }
     }
 
+    uint64_t n_launch = 0;
     // history staging: chunks of steps recorded on the device, drained to the host between chunks
     const uint64_t n_words = (n_neurons + 31) / 32, t_words = (n_trains + 31) / 32;
     uint64_t per_step_bytes = 0;
@@ -2250,6 +2359,7 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
     if (want_spk) per_step_bytes += n_words * 4;
     if (want_tgrid) per_step_bytes += n_trains * 4;
     if (want_tspk) per_step_bytes += t_words * 4;
+    if (ghist_on) per_step_bytes += std::max<uint64_t>(ghist_nnz_, 1) * 4;
     uint64_t chunk = iterations;
     if (per_step_bytes) chunk = std::max<uint64_t>(1, std::min<uint64_t>(iterations, (256ull << 20) / per_step_bytes));
     float *d_grid = nullptr, *d_tgrid = nullptr; uint32_t *d_spk = nullptr, *d_tspk = nullptr;
@@ -2272,9 +2382,20 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
         CK(dev_alloc(&d_red_lat, 3 * nl), SNN_GPU_BUFFER_CREATE_ERROR);
         CK(h2d_sync(d_red_lat, meta.data(), meta.size() * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     }
-    auto free_hist = [&]() { cudaFree(d_grid); cudaFree(d_spk); cudaFree(d_tgrid); cudaFree(d_tspk); cudaFree(d_red); cudaFree(d_red_lat); };
+    // graph records of a chunk: one per step, plus the final one of a Lattice with STDP (taken after the end-of-run flush)
+    float *d_ghist = nullptr;
+    if (ghist_on && ghist_nnz_) CK(dev_alloc(&d_ghist, (chunk + 1) * ghist_nnz_), SNN_GPU_BUFFER_CREATE_ERROR);
+    uint64_t gh_recs = 0;
+    // Lattice::iterate records after the step's plasticity (neuron/mod.rs:973-979); lazily applied STDP lands in the table with the
+    // next step kernel (or the end-of-run flush), so a Lattice with STDP records step k after step kernel k + 1.  LatticeNetwork
+    // records before the step's STDP (neuron/mod.rs:2565-2576): the table after step kernel k.  BCM is applied right after the step.
+    auto record_graph = [&]() -> cudaError_t {
+        cudaError_t e = ghist_nnz_ ? launch_graph_record(wgt_, slice_off_, ghist_row_off_, n_slices_, ghist_max_width_, d_ghist + gh_recs * ghist_nnz_, stream_) : cudaSuccess;
+        if (e == cudaSuccess) { ++gh_recs; if (ghist_nnz_) n_launch++; }
+        return e;
+    };
+    auto free_hist = [&]() { cudaFree(d_grid); cudaFree(d_spk); cudaFree(d_tgrid); cudaFree(d_tspk); cudaFree(d_red); cudaFree(d_red_lat); cudaFree(d_ghist); };
 
-    uint64_t n_launch = 0;
     float total_ms = 0.f;
     int status = SNN_OK;
     auto bail = [&](cudaError_t e, int st, const char *what) { status = cuda_fail(e, st, what); };
@@ -2320,7 +2441,7 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
     // small lattices / networks (everything the staged kernels do not take): a whole chunk of timesteps per cooperative launch
     // (step_multi.cu).  SNN_OPT_STEPS_PER_GRAPH: 0 = as many as the history chunk holds, 1 = one launch per timestep, k = at most k.
     bool multi = part_world == 1 && n_neurons > 0 && !win_ok && !tma_ok && !bcm_on && !reward_mode && !net_reward && steps_per_graph != 1 &&
-                 !getenv("SNN_DEBUG_TIMING");
+                 !ghist_on && !getenv("SNN_DEBUG_TIMING");   // graph records are taken between launches: one launch per timestep
     if (wide && wide_split) multi = false;   // the two-pass wide kernels are one-launch-per-step kernels
     if (const char *e = getenv("SNN_B200_MULTI")) multi = multi && atoi(e) != 0;
     if (multi) {
@@ -2481,6 +2602,10 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
                 }
                 for (auto &L : lats_) if (L.is_train) L.clock += 1;
             }
+            if (ghist_on && (is_network || !stdp || sp.apply_pending)) {
+                cudaError_t e = record_graph();
+                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record"); break; }
+            }
             internal_clock += 1;
             cur_ = out;
             if (lft_pp) lft_loc_ ^= 1;
@@ -2499,6 +2624,10 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
             cudaError_t e = launch_flush_stdp(fp, stream_);
             if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "flush_stdp"); break; }
             n_launch++;
+            if (ghist_on && !is_network) {
+                e = record_graph();
+                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record"); break; }
+            }
         }
         cudaEventRecord(ev1_, stream_);
         const auto host_t1 = std::chrono::steady_clock::now();
@@ -2533,6 +2662,37 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
         float ms = 0.f;
         cudaEventElapsedTime(&ms, ev0_, ev1_);
         total_ms += ms;
+        // drain the graph records: each requested block's weights cut out of the canonical order
+        if (ghist_on && gh_recs) {
+            const uint64_t nz = ghist_nnz_;
+            if (nz && gh_plans.size() == 1 && gh_plans[0].whole) {
+                std::vector<float> &w = gh_plans[0].h->w;   // straight into the block's record vector
+                const size_t o = w.size();
+                w.resize(o + gh_recs * nz);
+                e = cudaMemcpy(w.data() + o, d_ghist, gh_recs * nz * 4, cudaMemcpyDeviceToHost);
+            } else if (nz) {
+                std::vector<float> hr(gh_recs * nz);
+                e = cudaMemcpy(hr.data(), d_ghist, hr.size() * 4, cudaMemcpyDeviceToHost);
+                for (auto &pl : gh_plans) {
+                    if (e != cudaSuccess || pl.h->nnz == 0) continue;
+                    std::vector<float> &w = pl.h->w;
+                    for (uint64_t k = 0; k < gh_recs; ++k) {
+                        const float *rec = hr.data() + k * nz;
+                        if (pl.whole) { w.insert(w.end(), rec, rec + nz); continue; }
+                        const size_t o = w.size();
+                        w.resize(o + pl.h->nnz);
+                        const uint64_t n_post = pl.src.size();
+                        for (uint64_t q = 0; q < n_post; ++q) {
+                            const uint64_t a = pl.b->row_ptr[q], c = pl.b->row_ptr[q + 1] - a;
+                            if (c) memcpy(w.data() + o + a, rec + pl.src[q], c * 4);
+                        }
+                    }
+                }
+            }
+            if (e != cudaSuccess) { bail(e, SNN_GPU_BUFFER_READ_ERROR, "graph history drain"); break; }
+            for (auto &pl : gh_plans) pl.h->steps += gh_recs;
+            gh_recs = 0;
+        }
         // drain histories
         if (per_step_bytes) {
             std::vector<float> hg, htg; std::vector<uint32_t> hs, hts;

@@ -25,6 +25,7 @@ struct Lat {
     uint64_t off = 0;  // offset inside its domain (local neuron number / local train number)
     bool do_plasticity = false, grid_hist = false, spike_hist = false;
     bool avg_hist = false, eeg_hist = false;        // AverageVoltageHistory / EEGHistory (neuron/mod.rs:231-322)
+    bool graph_hist = false;                        // update_graph_history: records of this lattice's own graph (graph/mod.rs:278-284)
     float eeg_ref = 0.007f, eeg_dist = 0.8f, eeg_cond = 251.f;   // EEGHistory::default, neuron/mod.rs:243-252
     std::vector<float> average_history, eeg_history;
     snn_stdp_t stdp{2.f, 2.f, 4.5f, 4.5f, 0.1f};  // STDP::default, plasticity/mod.rs:29-39
@@ -136,6 +137,11 @@ public:
     int get_spike_aggregate(uint64_t id, int64_t *out, uint64_t capacity);   // SpikeHistory::aggregate, neuron/mod.rs:335-359
     int get_reduced_history(uint64_t id, bool eeg, float *out, uint64_t capacity);
     int set_eeg_parameters(uint64_t id, float reference_voltage, float distance, float conductivity);
+    // graph history: one record per timestep of the block pre_id -> post_id (pre_id == post_id: a lattice's own graph), nnz f32
+    // weights in the order of get_connection_csr
+    int graph_history_len(uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz);
+    int get_graph_history(uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity);
+    bool graph_history_nonempty() const;
 
     // multi-GPU
     int ipc_export(IpcBlob *blob);
@@ -150,6 +156,10 @@ public:
 
     // public knobs (Lattice / LatticeNetwork pub fields, neuron/mod.rs:556-587, 1554-1563)
     bool electrical = true, chemical = false, parallel = false;
+    // a LatticeNetwork handle (snn_network_create) rather than a Lattice: the two take their graph history records at different
+    // points of the step (Lattice::iterate after the step's plasticity, LatticeNetwork::iterate before it)
+    bool is_network = false;
+    bool conn_graph_hist = false;   // LatticeNetwork::update_connecting_graph_history: records of every connecting block
     uint64_t internal_clock = 0;
     uint64_t seed;                  // Philox key of the Poisson trains: distinct per handle unless SNN_OPT_RNG_SEED sets it
     uint64_t train_draws = 0;       // Philox counter word: one per spike-train step of this handle, never reset (reset_timing
@@ -241,6 +251,15 @@ private:
     uint64_t node_to_global(uint32_t node) const;
     // scratch
     void *scratch_ = nullptr; size_t scratch_bytes_ = 0;
+    // graph history: host records per requested block, and the per-row offsets of the canonical CSR order of the device table
+    // (32 * n_slices_ + 1 entries, rebuilt after each finalize_graph while some graph history is on)
+    struct GraphHist { uint64_t steps = 0, nnz = 0; std::vector<float> w; };
+    std::map<std::pair<uint64_t, uint64_t>, GraphHist> graph_hist_;
+    uint32_t *ghist_row_off_ = nullptr;
+    uint64_t ghist_nnz_ = 0;
+    uint32_t ghist_max_width_ = 0;   // widest slice of the table, in k-rows
+    bool ghist_off_valid_ = false;
+    int refuse_if_graph_history(const char *what);
 
     int ipc_export_layout(IpcBlob *blob);
     int attach_view(int direction, const IpcBlob *blob, void *slab, void *flags);

@@ -5,7 +5,7 @@ The CUDA library is the product; this package holds no compute and no CPU fallba
 from . import _capi
 from ._capi import SnnError, load_library
 from .backend import CudaLatticeBackend, CudaNetworkBackend
-from .lattice import (AverageVoltageHistory, EEGHistory, GridVoltageHistory, Lattice, LatticeNetwork,
+from .lattice import (AverageVoltageHistory, EEGHistory, GraphHistory, GridVoltageHistory, Lattice, LatticeNetwork,
                       RewardModulatedConnection, RewardModulatedLattice, RewardModulatedLatticeNetwork, SpikeHistory,
                       SpikeTrainLattice, TraceRSTDP)
 from .neurons import *  # noqa: F401,F403

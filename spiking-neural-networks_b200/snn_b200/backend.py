@@ -272,6 +272,14 @@ class CudaLatticeBackend(_CudaBase):
     def reset_history(self):
         self._ck(self.lib.snn_lattice_reset_history(self.h))
 
+    def graph_history(self, pre_id=0, post_id=0):
+        """Graph::update_history records of the lattice's graph: steps x nnz f32, edge order of get_connection_csr."""
+        steps, nnz = C.c_uint64(), C.c_uint64()
+        self._ck(self.lib.snn_lattice_graph_history_len(self.h, C.byref(steps), C.byref(nnz)))
+        out = np.zeros(max(steps.value * nnz.value, 1), np.float32)
+        self._ck(self.lib.snn_lattice_get_graph_history(self.h, _ptr(out), out.size))
+        return out[:steps.value * nnz.value].reshape(steps.value, nnz.value)
+
     # multi-GPU plumbing
     def ipc_export(self) -> bytes:
         buf = C.create_string_buffer(self.lib.snn_lattice_ipc_blob_size())
@@ -478,3 +486,12 @@ class CudaNetworkBackend(_CudaBase):
 
     def reset_history(self):
         self._ck(self.lib.snn_network_reset_history(self.h))
+
+    def graph_history(self, pre_id, post_id):
+        """Records of the block pre_id -> post_id (a lattice's own graph when equal): steps x nnz f32, edge order of
+        get_connection_csr(pre_id, post_id)."""
+        steps, nnz = C.c_uint64(), C.c_uint64()
+        self._ck(self.lib.snn_network_graph_history_len(self.h, pre_id, post_id, C.byref(steps), C.byref(nnz)))
+        out = np.zeros(max(steps.value * nnz.value, 1), np.float32)
+        self._ck(self.lib.snn_network_get_graph_history(self.h, pre_id, post_id, _ptr(out), out.size))
+        return out[:steps.value * nnz.value].reshape(steps.value, nnz.value)

@@ -42,6 +42,15 @@ def _default_network_backend(model, ntk, rck, train_kind, refract):
     return CudaNetworkBackend(model, ntk, rck, train_kind, refract)
 
 
+def _push_flag(owner, be, option, value, id=None):
+    """Set an option that back ends without the feature need not know: only when it is on, or to switch it off again on the
+    back end it was switched on for."""
+    key = ("_flag_on", option)
+    if value or owner.__dict__.get(key) is be:
+        be.set_option(option, value, id)
+    owner.__dict__[key] = be if value else None
+
+
 def _enc(v):
     if v is None:
         return -1
@@ -99,6 +108,46 @@ class EEGHistory(GridVoltageHistory):
     @property
     def history(self):
         return self._o._be.eeg_history(self._o._bid)
+
+
+class GraphHistory:
+    """Graph::update_history (graph/mod.rs:278-284) of one graph: a lattice's own graph or one block of a network's connecting
+    graph.  `.history[step]` holds every edge weight in the order of `row_ptr` / `pre` (CSR by postsynaptic cell, presynaptic
+    cells ascending); `dense(step)` expands one record to the (connections, weights) layout of get_graph_dense.  A Lattice
+    records after each step's plasticity, a LatticeNetwork before it (record 0 = the weights the first step read)."""
+
+    def __init__(self, target):
+        self._target = target   # () -> (back end, presynaptic id, postsynaptic id)
+
+    @property
+    def history(self):
+        be, a, b = self._target()
+        return be.graph_history(a, b)
+
+    def _csr(self):
+        be, a, b = self._target()
+        return be.get_connection_csr(a, b)
+
+    @property
+    def row_ptr(self):
+        return self._csr()[0]
+
+    @property
+    def pre(self):
+        return self._csr()[1]
+
+    def dense(self, step):
+        be, a, b = self._target()
+        rp, pre, _ = be.get_connection_csr(a, b)
+        n_pre, n_post = be.size(a), be.size(b)
+        post = np.repeat(np.arange(n_post), np.diff(rp.astype(np.int64)))
+        conn, weights = np.zeros((n_pre, n_post), np.uint32), np.zeros((n_pre, n_post), np.float32)
+        conn[pre, post] = 1
+        weights[pre, post] = self.history[step]
+        return conn, weights
+
+    def reset(self):
+        self._target()[0].reset_history()
 
 
 class _CellLattice:
@@ -192,6 +241,8 @@ class Lattice(_CellLattice):
         self.do_plasticity = False
         self.plasticity = STDP()
         self.parallel = False
+        self.update_graph_history = False
+        self.graph_history = GraphHistory(lambda: (self._be, self._bid, self._bid))
         self._in_network = None
         self._graph_spec = None  # remembered so that a lattice can be moved into a network
 
@@ -433,6 +484,7 @@ class Lattice(_CellLattice):
             be.set_eeg_parameters(i, gh.reference_voltage, gh.distance, gh.conductivity)
         be.set_option(gh.option, self.update_grid_history, i)
         be.set_option(K.OPT_UPDATE_SPIKE_HISTORY, self.update_spike_history, i)
+        _push_flag(self, be, K.OPT_UPDATE_GRAPH_HISTORY, self.update_graph_history, i)
         p = self.plasticity
         if isinstance(p, BCM):   # Lattice<BCMIzhikevichNeuron, ..., BCM, ...>
             be.set_bcm_plasticity(i, True, p.decay, p.average_scalar, p.dt)
@@ -461,7 +513,6 @@ class RewardModulatedLattice(Lattice):
         super().__init__(neuron_type, id, backend_factory, history_type)
         self.do_modulation = True                      # RewardModulatedLattice::default, neuron/mod.rs:2762-2777
         self.reward_modulator = RewardModulatedSTDP()
-        self.update_graph_history = False
 
     def _push_options(self):
         self.do_plasticity = False
@@ -651,10 +702,15 @@ class LatticeNetwork:
         self.electrical_synapse = True
         self.chemical_synapse = False
         self.parallel = False
+        self.update_connecting_graph_history = False
 
     @classmethod
     def default_impl(cls, **kw):
         return cls(**kw)
+
+    def connecting_graph_history(self, presynaptic_id, postsynaptic_id):
+        """Records of the connecting block presynaptic_id -> postsynaptic_id (update_connecting_graph_history)."""
+        return GraphHistory(lambda: (self._be, presynaptic_id, postsynaptic_id))
 
     @classmethod
     def generate_network(cls, lattices, spike_train_lattices=(), backend_factory=None):
@@ -811,6 +867,7 @@ class LatticeNetwork:
             return
         self._be.set_option(K.OPT_ELECTRICAL_SYNAPSE, self.electrical_synapse)
         self._be.set_option(K.OPT_CHEMICAL_SYNAPSE, self.chemical_synapse)
+        _push_flag(self, self._be, K.OPT_UPDATE_CONNECTING_GRAPH_HISTORY, self.update_connecting_graph_history)
         for lat in self._lattices.values():
             lat._push_options()
         for st in self._spike_train_lattices.values():
@@ -985,6 +1042,7 @@ class RewardModulatedLatticeNetwork(LatticeNetwork):
     def _push_all(self):
         self._be.set_option(K.OPT_ELECTRICAL_SYNAPSE, self.electrical_synapse)
         self._be.set_option(K.OPT_CHEMICAL_SYNAPSE, self.chemical_synapse)
+        _push_flag(self, self._be, K.OPT_UPDATE_CONNECTING_GRAPH_HISTORY, self.update_connecting_graph_history)
         for lat in list(self._lattices.values()) + list(self._reward_modulated_lattices.values()):
             lat._push_options()
         for st in self._spike_train_lattices.values():
