@@ -14,32 +14,27 @@ namespace snn {
 // Programmatic dependent launch: a kernel launched through launch_pdl may be scheduled while its predecessor in the stream is
 // still draining (its CTAs take the SMs the predecessor's CTAs leave); it must execute pdl_wait() before it touches anything the
 // predecessor wrote — that returns once the predecessor grid has completed and its writes are visible.  Hides the launch latency
-// and the prologue (barrier initialisation, parameter loads) behind the predecessor's tail.  SNN_B200_PDL=0 switches it off.
+// and the prologue (barrier initialisation, parameter loads) behind the predecessor's tail.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 }
 #endif
-// SNN_B200_PDL is a mask of these.  Measured (profiles/README.md, round 2): step kernels gain 2.5-3 us per launch (1000 x 1000
-// lattice 26.5 -> 23.4 us per step, wide-row network 30.6 -> 28.0 us); the persistent per-edge reward kernel LOSES 90 us per
-// step as a dependent launch (its three CTAs per SM arrive one by one as the step kernel's CTAs drain) and stays a plain launch.
-enum PdlKind : unsigned { PDL_STEP = 1u, PDL_TRAINS = 2u, PDL_EDGES = 4u };
-inline unsigned pdl_mask() {
-    static const unsigned m = getenv("SNN_B200_PDL") ? (unsigned)atoi(getenv("SNN_B200_PDL")) : (PDL_STEP | PDL_TRAINS);
-    return m;
-}
-// `allow` = false launches plainly: row strips and general-graph partitions (measured: the same 10^7-neuron lattice over 4 GPUs takes
-// 83.8 us per step with dependent launches and 79.8 us without — the early CTAs of the next step only add to the neighbour
-// handshake's critical path).
-template <unsigned KIND, typename... KArgs, typename... Args>
+// Measured (profiles/README.md, round 2): step kernels gain 2.5-3 us per launch (1000 x 1000 lattice 26.5 -> 23.4 us per step,
+// wide-row network 30.6 -> 28.0 us); the persistent per-edge reward kernel LOSES 90 us per step as a dependent launch (its three
+// CTAs per SM arrive one by one as the step kernel's CTAs drain).  `allow` = false launches plainly: the per-edge kernels, and
+// every kernel of row strips and general-graph partitions (measured: the same 10^7-neuron lattice over 4 GPUs takes 83.8 us per
+// step with dependent launches and 79.8 us without — the early CTAs of the next step only add to the neighbour handshake's
+// critical path).
+template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(bool allow, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args &&...args) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = (allow && (pdl_mask() & KIND)) ? 1u : 0u;
+    cfg.attrs = at; cfg.numAttrs = allow ? 1u : 0u;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -160,7 +155,10 @@ struct StepParams {
     uint32_t n_gslices;
     uint32_t reverse;                // window kernel: sweep the tiles back to front (alternates per step: the tail of the
                                      // arrays that the previous step left in L2 is what this step reads first)
-    unsigned long long *dbg;         // SNN_DEBUG_TIMING: {clock64, globaltimer} at the start and end of CTA 0 (else null)
+    // window kernel: {clock64, globaltimer} of CTA 0 at its start and end, when non-null.  The engine leaves it null; the stamps
+    // stay because the window kernel compiled without them took 1.0 us longer per step on the 10^7-neuron bench lattice (296.3 vs
+    // 295.3 us, B200 at 1000 W)
+    unsigned long long *dbg;
 };
 
 struct TrainParams {
@@ -308,13 +306,8 @@ struct WinParams {
 };
 
 // groups of 8 consumer warps per CTA (register budget: 65536 / ((groups * 8 + 1) * 32))
-#ifndef SNN_WIN_GROUPS
-#define SNN_WIN_GROUPS 3
-#endif
-#ifndef SNN_WIN_GROUPS_WIDE
-#define SNN_WIN_GROUPS_WIDE 2   // models with wide operand sets (Hodgkin-Huxley, three neurotransmitter types): fewer, fatter stages
-#endif
-__host__ __device__ constexpr int win_groups(int model, int chemg) { return (model == SNN_MODEL_HODGKIN_HUXLEY || chemg == 3) ? SNN_WIN_GROUPS_WIDE : SNN_WIN_GROUPS; }
+// models with wide operand sets (Hodgkin-Huxley, three neurotransmitter types): fewer, fatter stages
+__host__ __device__ constexpr int win_groups(int model, int chemg) { return (model == SNN_MODEL_HODGKIN_HUXLEY || chemg == 3) ? 2 : 3; }
 
 cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, int model, int chemg, bool ntrel, bool stdp, unsigned grid,
                             cudaStream_t s);

@@ -67,8 +67,7 @@ Engine::~Engine() {
     if (flags_) cudaFree(flags_);
     if (halo_done_) cudaFree(halo_done_);
     if (multi_barrier_) cudaFree(multi_barrier_);
-    if (rs_tab_) cudaFree(rs_tab_);
-    if (rnet_tab_) cudaFree(rnet_tab_);
+    if (stdp_tab_) cudaFree(stdp_tab_);
     if (wide_scratch_) cudaFree(wide_scratch_);
     if (scratch_) cudaFree(scratch_);
     if (ghist_row_off_) cudaFree(ghist_row_off_);
@@ -104,7 +103,7 @@ int Engine::init() {
     CK(dev_alloc(&flags_, 8 + kMaxRanks), SNN_GPU_BUFFER_CREATE_ERROR);
     CK(cudaMemsetAsync(flags_, 0, (8 + kMaxRanks) * sizeof(unsigned long long), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     CK(dev_alloc(&multi_barrier_, 1), SNN_GPU_BUFFER_CREATE_ERROR);
-    CK(dev_alloc(&halo_done_, 8), SNN_GPU_BUFFER_CREATE_ERROR);  // [4] ns / 16 spent in halo waits, [5] waits that spun (diagnostics); [0],[1] completion counters, [2] halo time-out flag, [3] per-edge kernel CTAs done
+    CK(dev_alloc(&halo_done_, 8), SNN_GPU_BUFFER_CREATE_ERROR);  // [0],[1] completion counters, [2] halo time-out flag, [3] per-edge kernel CTAs done, [4],[5] halo wait counters, [6] general-partition slices done
     CK(cudaMemsetAsync(halo_done_, 0, 8 * sizeof(unsigned int), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
     return SNN_OK;
@@ -292,9 +291,7 @@ struct LatSnap { uint64_t id; std::vector<FieldSnap> fields; };
 int Engine::add_lattice(uint64_t id, uint32_t rows, uint32_t cols, bool is_train, bool is_reward) {
     // LatticeNetwork::add_lattice / add_spike_train_lattice, neuron/mod.rs:1663-1698
     if (find(id)) return fail(SNN_NET_GRAPH_ID_ALREADY_PRESENT, "Graph id already present in network, id: " + std::to_string(id));
-    int n_neuron_lat = 0;
-    for (auto &L : lats_) if (!L.is_train) n_neuron_lat++;
-    if (!is_train && n_neuron_lat >= kMaxLattices) return fail(SNN_UNSUPPORTED, "too many lattices");
+    if (!is_train && n_neuron_lattices() >= kMaxLattices) return fail(SNN_UNSUPPORTED, "too many lattices");
     if (part_world > 1 && (!lats_.empty() || is_train)) return fail(SNN_UNSUPPORTED, "a partitioned handle holds exactly one neuron lattice");
     if (is_reward && (is_train || part_world > 1 || reward_mode || bcm_mode))
         return fail(SNN_UNSUPPORTED, "reward-modulated lattices of a network: single-GPU network handles only");
@@ -1128,9 +1125,8 @@ int Engine::finalize_graph() {
         CK(h2d_sync(node_flags_, h_node_flags_.data(), node_cap_, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
         flags_cache_valid_ = false;
     }
-    int n_neuron_lat = 0;
-    const Lat *only = nullptr;
-    for (auto &L : lats_) if (!L.is_train) { n_neuron_lat++; only = &L; }
+    const int n_neuron_lat = n_neuron_lattices();
+    const Lat *only = n_neuron_lat == 1 ? &lats_[0] : nullptr;   // neuron lattices come first in lats_
     // fast path: one lattice whose only block is a grid stencil -> built directly in sliced-ELL form on the device
     if (n_neuron_lat == 1 && blocks_.size() == 1 && blocks_.begin()->second.kind == Block::GRID &&
         blocks_.begin()->first == std::make_pair(only->id, only->id)) {
@@ -1155,6 +1151,7 @@ int Engine::finalize_graph() {
         CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
         grid_fast_ = true;
         uniform_width_ = width;
+        max_slice_width_ = n_slices_ ? width : 0;
         graph_dirty_ = false;
         dev_weights_newer_ = false;
         return SNN_OK;
@@ -1228,6 +1225,8 @@ int Engine::finalize_graph() {
             sell_krows_ = (uint64_t)n_slices_ * stencil_width;
         }
     }
+    max_slice_width_ = 0;
+    for (uint32_t s = 0; s < n_slices_; ++s) max_slice_width_ = std::max(max_slice_width_, slice_off[s + 1] - slice_off[s]);
     const uint64_t alloc_krows = stencil_width ? round_up(n_slices_, kTmaConsumerWarps) * stencil_width : sell_krows_;
     CK(dev_alloc(&col_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
     CK(dev_alloc(&wgt_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
@@ -1266,18 +1265,14 @@ int Engine::finalize_graph() {
 // ------------------------------------------------------------------------------------------------
 int Engine::set_bcm_plasticity(bool enable, const snn_bcm_t *b) {
     if (enable && model != SNN_MODEL_BCM_IZHIKEVICH) return fail(SNN_INVALID_ARGUMENT, "BCM plasticity needs neurons with BCMActivity (SNN_MODEL_BCM_IZHIKEVICH)");
-    int n_neuron_lat = 0;
-    for (auto &L : lats_) if (!L.is_train) n_neuron_lat++;
-    if (enable && (part_world > 1 || n_neuron_lat > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "BCM plasticity: single-GPU Lattice handles only");
+    if (enable && (part_world > 1 || n_neuron_lattices() > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "BCM plasticity: single-GPU Lattice handles only");
     bcm_mode = enable;
     if (b) bcm = *b;
     return SNN_OK;
 }
 
 int Engine::set_reward_modulator(bool enable, bool modulate, const snn_rstdp_t *m) {
-    int n_neuron_lat = 0;
-    for (auto &L : lats_) if (!L.is_train) n_neuron_lat++;
-    if (enable && (n_neuron_lat > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "snn_lattice_set_reward_modulator is for single-lattice handles; networks add reward-modulated lattices with snn_network_add_reward_modulated_lattice");
+    if (enable && (n_neuron_lattices() > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "snn_lattice_set_reward_modulator is for single-lattice handles; networks add reward-modulated lattices with snn_network_add_reward_modulated_lattice");
     reward_mode = enable; do_modulation = modulate;
     if (m) rstdp = *m;
     if (!enable) free_reward_arrays();
@@ -1868,9 +1863,7 @@ void Engine::fill_step_params(StepParams &p) {
     p.train0 = train0_; p.n_trains = (uint32_t)n_trains;
     for (int s = 0; s < TF_COUNT; ++s) p.tf[s] = TF_[s];
     p.lat = d_lat_;
-    int nl = 0;
-    for (auto &L : lats_) if (!L.is_train) nl++;
-    p.n_lat = std::max(nl, 1);
+    p.n_lat = std::max(n_neuron_lattices(), 1);
     p.halo[0] = halo_dir_[0]; p.halo[1] = halo_dir_[1];
     p.halo_done = halo_done_;
     p.halo_timeout_ns = halo_timeout_ms * 1000000ull;
@@ -1881,14 +1874,9 @@ void Engine::fill_step_params(StepParams &p) {
 }
 
 // Operand streams of the TMA-staged kernel for the current configuration; false = not eligible (use the general kernel).
-bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp, unsigned *grid) {
+bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid) {
     memset(&tp, 0xFF, sizeof tp);
     if (!grid_fast_ || !uniform_width_ || n_neurons == 0) return false;
-    int mode = use_tma;
-    if (mode < 0) {
-        const char *e = getenv("SNN_B200_TMA");
-        mode = e ? atoi(e) : 1;
-    }
     if (mode == 0) return false;
     // tiny lattices are launch-latency bound: the persistent kernel only pays off with at least a few tiles per SM
     if (mode < 2 && n_neurons < 64 * 1024) return false;
@@ -1937,7 +1925,6 @@ bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp,
         }
     }
     if (n >= (uint32_t)kMaxTmaStreams) return false;
-    if (const char *ek = getenv("SNN_B200_TMA_EXPERIMENT_KEEP")) n = std::min<uint32_t>(n, (uint32_t)atoi(ek));  // timing experiment only: results are wrong
     tp.n_streams = n;
     tp.stage_bytes = off;
     tp.tx_bytes = 0;
@@ -1948,12 +1935,9 @@ bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp,
     const uint32_t budget = 220 * 1024;
     uint32_t ctas = 3, stages = (budget / ctas) / off;
     if (stages < 2) { ctas = 2; stages = (budget / ctas) / off; }
-    const char *es = getenv("SNN_B200_TMA_STAGES"), *ec = getenv("SNN_B200_TMA_CTAS");
-    if (ec) { ctas = (uint32_t)std::max(1, atoi(ec)); stages = (budget / ctas) / off; }
     if (stages < 2) { ctas = 1; stages = budget / off; }
     if (stages < 2) return false;
     stages = std::min<uint32_t>(stages, 4);
-    if (es) stages = (uint32_t)std::max(2, atoi(es));
     if ((uint64_t)stages * off + 64 > 227 * 1024) return false;
     tp.stages = stages;
     int sms = 148;
@@ -1963,16 +1947,10 @@ bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp,
 }
 
 // Operand streams of the window-staged kernel (step_win.cu): radius-1 stencil lattices.  false = not eligible.
-bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, unsigned *grid) {
+bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid) {
     memset(&wp, 0xFF, sizeof wp);
     if (!grid_fast_ || uniform_width_ != kWinWidth || n_neurons == 0) return false;
-    int mode = use_tma;
-    if (mode < 0) {
-        const char *e = getenv("SNN_B200_TMA");
-        mode = e ? atoi(e) : 1;
-    }
     if (mode == 0) return false;
-    if (const char *e = getenv("SNN_B200_WIN")) if (atoi(e) == 0) return false;
     // tiny lattices are launch-latency bound: the persistent kernel only pays off with at least a few tiles per SM
     if (mode < 2 && n_neurons < 64 * 1024) return false;
     uint32_t cols = 0;
@@ -2041,11 +2019,9 @@ bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, b
         }
         wp.bnd_lo = wp.first_lo; wp.bnd_hi = wp.first_hi;
         if (wp.first_lo + wp.first_hi > wp.n_tiles) wp.first_lo = wp.first_hi = 0;   // a strip of a few rows: every tile is a boundary tile
-        if (const char *e = getenv("SNN_B200_BOUNDARY_FIRST")) if (atoi(e) == 0) wp.first_lo = wp.first_hi = 0;
     }
     const uint32_t G = (uint32_t)win_groups(model, chemg);
     uint32_t stages = (224u * 1024u) / (off + 16u);
-    if (const char *es = getenv("SNN_B200_WIN_STAGES")) stages = std::min<uint32_t>(stages, (uint32_t)std::max(1, atoi(es)));
     stages = std::min<uint32_t>(stages, 8);
     if (stages < G) return false;   // the consumer groups need a stage each
     wp.stages = stages;
@@ -2073,22 +2049,400 @@ void Engine::wait_local_peers_launched(unsigned long long need, bool second) {
     }
 }
 
-int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, const float *rewards) {
-    if (elapsed_ms) *elapsed_ms = 0.f;
-    if (launches) *launches = 0;
-    // gpu_lattices/mod.rs:1089-1091: empty lattice or zero iterations -> Ok(()); neuron/mod.rs:1217: both flags off -> Ok(())
-    if (iterations == 0 || (n_neurons == 0 && n_trains == 0)) return SNN_OK;
-    if (!electrical && !chemical) return SNN_OK;
-    if (internal_clock + iterations > 0x7FFFFFF0ull) return fail(SNN_UNSUPPORTED, "internal clock would overflow the i32 last_firing_time");
-    // graph history: the blocks whose records this run appends to (a lattice's own graph; every non-empty connecting block)
-    std::vector<std::pair<uint64_t, uint64_t>> gh_keys;
-    for (auto &L : lats_) if (!L.is_train && L.graph_hist) gh_keys.emplace_back(L.id, L.id);
+// The step path of a run: which kernel steps the neurons of one timestep.
+enum class StepPath {
+    Win,         // window-staged persistent kernel (step_win.cu): radius-1 stencil lattices
+    Tma,         // TMA-staged persistent kernel (step_tma.cu): other uniform-width stencil lattices
+    Wide,        // one CTA per slice (step_wide.cu): wide rows
+    WideSplit,   // two passes, per-edge terms then ordered sums (step_wide.cu): very wide rows
+    General      // one thread per neuron (kernels.cu)
+};
+
+// Decisions fixed for a whole run(), taken once by plan_run.
+struct Engine::RunPlan {
+    // kernel specialisation: ntrel = neurotransmitter / receptor state must be stepped; chemg = how the chemical gather reads
+    // presynaptic types (0 none, 1 a single type in the whole node array, 3 per-edge masks); net = several lattices and/or spike
+    // trains share the node array
+    bool stdp = false, ntrel = false, net = false;
+    int chemg = 0;
+    bool rmod = false, rmod_part = false;          // reward-modulated lattice (rmod_part: a row strip of one)
+    bool bcm_on = false;                           // BCM rule instead of STDP
+    bool net_reward = false, net_rmod = false;     // reward-modulated lattices in a network (net_rmod: one of them modulates)
+    bool lft_pp = false;                           // last_firing_time is ping-ponged
+    // histories: grid (including the grid record the reductions read), its host copy, spikes, train grid / spikes, reductions
+    bool want_grid = false, copy_grid = false, want_spk = false, want_tgrid = false, want_tspk = false, want_red = false;
+    bool ghist_on = false;
+    std::vector<std::pair<uint64_t, uint64_t>> gh_keys;   // blocks whose graph records this run appends to
+    StepPath path = StepPath::General;
+    bool multi = false;          // a chunk of timesteps per cooperative launch (step_multi.cu)
+    bool trains_fused = false;   // WideSplit: the spike trains ride in extra CTAs of the sum pass
+    unsigned grid = 0;           // Win / Tma: persistent grid size
+    uint32_t wide_chunks_cap = 0;   // WideSplit: chunk buffers per slice
+    int tma_iv = -1, tma_il = -1, tma_it[kNT] = {-1, -1, -1};   // Tma: streams whose source ping-pongs (patched every step)
+};
+
+// The kernel parameter blocks of a run and its counters.  The step functions patch the per-step fields.
+struct Engine::LaunchArgs {
+    StepParams sp{};
+    TrainParams tp{};
+    WinParams win{};
+    TmaParams tma{};
+    RstdpParams rsp{};   // reward-modulated lattice: dopamine is patched every step
+    RnetParams rnp{};    // reward-modulated network: the lattices' dopamine is patched every step
+    uint64_t launches = 0;
+    float total_ms = 0.f;
+};
+
+// History staging: chunks of timesteps are recorded on the device and drained to the host between chunks.  Owns the staging
+// buffers of one run().
+struct Engine::HistStage {
+    Engine &e;
+    const RunPlan &pl;
+    const uint64_t n_words, t_words;
+    uint64_t per_step_bytes = 0;   // staged bytes per timestep (0: nothing is recorded)
+    uint64_t chunk = 0;            // timesteps per chunk
+    float *grid = nullptr, *tgrid = nullptr;
+    uint32_t *spk = nullptr, *tspk = nullptr;
+    double *red = nullptr;
+    uint32_t *red_lat = nullptr;
+    std::vector<Lat *> red_lats;   // AverageVoltageHistory / EEGHistory lattices (lats_ is not resized inside run())
+    // graph records of a chunk: one per step, plus the final one of a Lattice with STDP (taken after the end-of-run flush)
+    float *ghist = nullptr;
+    uint64_t gh_recs = 0;
+    // how each requested block is cut out of a record: the whole record (the table holds that block only) or one contiguous range
+    // per postsynaptic row
+    struct GhPlan { GraphHist *h; bool whole; const Block *b; std::vector<uint64_t> src; };
+    std::vector<GhPlan> gh_plans;
+
+    HistStage(Engine &eng, const RunPlan &plan)
+        : e(eng), pl(plan), n_words((eng.n_neurons + 31) / 32), t_words((eng.n_trains + 31) / 32) {}
+    ~HistStage() { cudaFree(grid); cudaFree(spk); cudaFree(tgrid); cudaFree(tspk); cudaFree(red); cudaFree(red_lat); cudaFree(ghist); }
+    int cuda_fail(cudaError_t x, int status, const char *what) { return e.cuda_fail(x, status, what); }
+
+    int init(uint64_t iterations);
+    int plan_graph_history();
+    // the records of step s of the chunk
+    void point(StepParams &sp, uint64_t s) const {
+        sp.grid_hist = pl.want_grid ? grid + s * e.n_neurons : nullptr;
+        sp.spike_hist = pl.want_spk ? spk + s * n_words : nullptr;
+    }
+    void point(TrainParams &tp, uint64_t s) const {
+        tp.grid_hist = pl.want_tgrid ? tgrid + s * e.n_trains : nullptr;
+        tp.spike_hist = pl.want_tspk ? tspk + s * t_words : nullptr;
+    }
+    void point(MultiParams &mp, uint64_t s) const {
+        mp.grid_hist = pl.want_grid ? grid + s * e.n_neurons : nullptr;
+        mp.spike_hist = pl.want_spk ? spk + s * n_words : nullptr;
+        mp.tgrid_hist = pl.want_tgrid ? tgrid + s * e.n_trains : nullptr;
+        mp.tspike_hist = pl.want_tspk ? tspk + s * t_words : nullptr;
+    }
+    // Lattice::iterate records after the step's plasticity (neuron/mod.rs:973-979); lazily applied STDP lands in the table with
+    // the next step kernel (or the end-of-run flush), so a Lattice with STDP records step k after step kernel k + 1.
+    // LatticeNetwork records before the step's STDP (neuron/mod.rs:2565-2576): the table after step kernel k.  BCM is applied
+    // right after the step.
+    cudaError_t record_graph(uint64_t &launches) {
+        if (!e.ghist_nnz_) { ++gh_recs; return cudaSuccess; }
+        cudaError_t x = launch_graph_record(e.wgt_, e.slice_off_, e.ghist_row_off_, e.n_slices_, e.max_slice_width_,
+                                            ghist + gh_recs * e.ghist_nnz_, e.stream_);
+        if (x == cudaSuccess) { ++gh_recs; ++launches; }
+        return x;
+    }
+    int drain(uint64_t steps);
+    int drain_graph();
+};
+
+int Engine::HistStage::init(uint64_t iterations) {
+    if (pl.ghist_on) { int r = plan_graph_history(); if (r) return r; }
+    if (pl.want_grid) per_step_bytes += e.n_neurons * 4;
+    if (pl.want_spk) per_step_bytes += n_words * 4;
+    if (pl.want_tgrid) per_step_bytes += e.n_trains * 4;
+    if (pl.want_tspk) per_step_bytes += t_words * 4;
+    if (pl.ghist_on) per_step_bytes += std::max<uint64_t>(e.ghist_nnz_, 1) * 4;
+    chunk = iterations;
+    if (per_step_bytes) chunk = std::max<uint64_t>(1, std::min<uint64_t>(iterations, (256ull << 20) / per_step_bytes));
+    if (pl.want_grid) CK(dev_alloc(&grid, chunk * e.n_neurons), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (pl.want_spk) CK(dev_alloc(&spk, chunk * n_words), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (pl.want_tgrid) CK(dev_alloc(&tgrid, chunk * e.n_trains), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (pl.want_tspk) CK(dev_alloc(&tspk, chunk * t_words), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (pl.want_red) {
+        for (auto &L : e.lats_) if (!L.is_train && (L.avg_hist || L.eeg_hist)) red_lats.push_back(&L);
+        const size_t nl = red_lats.size();
+        std::vector<uint32_t> meta(3 * nl);
+        for (size_t k = 0; k < nl; ++k) {
+            meta[k] = (uint32_t)red_lats[k]->off; meta[nl + k] = (uint32_t)red_lats[k]->n;
+            memcpy(&meta[2 * nl + k], &red_lats[k]->eeg_ref, 4);
+        }
+        CK(dev_alloc(&red, chunk * nl * 2), SNN_GPU_BUFFER_CREATE_ERROR);
+        CK(dev_alloc(&red_lat, 3 * nl), SNN_GPU_BUFFER_CREATE_ERROR);
+        CK(h2d_sync(red_lat, meta.data(), meta.size() * 4, e.stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    }
+    if (pl.ghist_on && e.ghist_nnz_) CK(dev_alloc(&ghist, (chunk + 1) * e.ghist_nnz_), SNN_GPU_BUFFER_CREATE_ERROR);
+    return SNN_OK;
+}
+
+// Per-row offsets of the table's canonical order (once per graph build), then how each requested block is cut out of a record.
+int Engine::HistStage::plan_graph_history() {
+    if (!e.ghist_off_valid_) {
+        if (e.ghist_row_off_) cudaFree(e.ghist_row_off_);
+        e.ghist_row_off_ = nullptr;
+        CK(dev_alloc(&e.ghist_row_off_, (size_t)e.n_slices_ * 32 + 1), SNN_GPU_BUFFER_CREATE_ERROR);
+        CK(launch_graph_row_offsets(e.col_, e.slice_off_, e.n_slices_, e.ghist_row_off_, e.stream_), SNN_GPU_QUEUE_FAILURE);
+        uint32_t tot = 0;
+        CK(cudaMemcpyAsync(&tot, e.ghist_row_off_ + (size_t)e.n_slices_ * 32, 4, cudaMemcpyDeviceToHost, e.stream_), SNN_GPU_BUFFER_READ_ERROR);
+        CK(cudaStreamSynchronize(e.stream_), SNN_GPU_WAIT_ERROR);
+        e.ghist_nnz_ = tot;
+        e.ghist_off_valid_ = true;
+    }
+    std::vector<uint64_t> roff;   // canonical row offsets of the table from the host blocks (several blocks only)
+    for (auto &key : pl.gh_keys) {
+        GhPlan gp{&e.graph_hist_[key], false, nullptr, {}};
+        auto it = e.blocks_.find(key);
+        if (it != e.blocks_.end() && e.blocks_.size() == 1) {
+            gp.whole = true;
+            gp.h->nnz = e.ghist_nnz_;
+        } else if (it != e.blocks_.end()) {
+            // finalize_graph's general path: every block is host CSR; rows hold the blocks into their lattice ordered by the
+            // presynaptic lattice's node offset (sync_weights_to_host walks them the same way)
+            if (roff.empty()) {
+                roff.assign(e.n_neurons + 1, 0);
+                for (auto &kv : e.blocks_) {
+                    const Lat *B = e.find(kv.first.second);
+                    for (uint64_t q = 0; q < B->n; ++q) roff[B->off + q + 1] += kv.second.row_ptr[q + 1] - kv.second.row_ptr[q];
+                }
+                for (uint64_t i = 0; i < e.n_neurons; ++i) roff[i + 1] += roff[i];
+                if (roff[e.n_neurons] != e.ghist_nnz_) return e.fail(SNN_GPU_BUFFER_READ_ERROR, "graph history: host and device tables disagree");
+            }
+            const Lat *A = e.find(key.first), *B = e.find(key.second);
+            std::vector<const Block *> before;
+            for (auto &kv : e.blocks_)
+                if (kv.first.second == key.second && kv.first != key && e.node_off(*e.find(kv.first.first)) < e.node_off(*A)) before.push_back(&kv.second);
+            gp.b = &it->second;
+            gp.src.resize(B->n);
+            for (uint64_t q = 0; q < B->n; ++q) {
+                uint64_t o = roff[B->off + q];
+                for (const Block *o_b : before) o += o_b->row_ptr[q + 1] - o_b->row_ptr[q];
+                gp.src[q] = o;
+            }
+            gp.h->nnz = it->second.pre.size();
+        } else {
+            gp.h->nnz = 0;   // a lattice without an internal graph: empty records
+        }
+        gh_plans.push_back(std::move(gp));
+    }
+    return SNN_OK;
+}
+
+// The graph records of the chunk: each requested block's weights cut out of the canonical order.
+int Engine::HistStage::drain_graph() {
+    const uint64_t nz = e.ghist_nnz_;
+    cudaError_t x = cudaSuccess;
+    if (nz && gh_plans.size() == 1 && gh_plans[0].whole) {
+        std::vector<float> &w = gh_plans[0].h->w;   // straight into the block's record vector
+        const size_t o = w.size();
+        w.resize(o + gh_recs * nz);
+        x = cudaMemcpy(w.data() + o, ghist, gh_recs * nz * 4, cudaMemcpyDeviceToHost);
+    } else if (nz) {
+        std::vector<float> hr(gh_recs * nz);
+        x = cudaMemcpy(hr.data(), ghist, hr.size() * 4, cudaMemcpyDeviceToHost);
+        for (auto &gp : gh_plans) {
+            if (x != cudaSuccess || gp.h->nnz == 0) continue;
+            std::vector<float> &w = gp.h->w;
+            for (uint64_t k = 0; k < gh_recs; ++k) {
+                const float *rec = hr.data() + k * nz;
+                if (gp.whole) { w.insert(w.end(), rec, rec + nz); continue; }
+                const size_t o = w.size();
+                w.resize(o + gp.h->nnz);
+                const uint64_t n_post = gp.src.size();
+                for (uint64_t q = 0; q < n_post; ++q) {
+                    const uint64_t a = gp.b->row_ptr[q], c = gp.b->row_ptr[q + 1] - a;
+                    if (c) memcpy(w.data() + o + a, rec + gp.src[q], c * 4);
+                }
+            }
+        }
+    }
+    if (x != cudaSuccess) return cuda_fail(x, SNN_GPU_BUFFER_READ_ERROR, "graph history drain");
+    for (auto &gp : gh_plans) gp.h->steps += gh_recs;
+    gh_recs = 0;
+    return SNN_OK;
+}
+
+// The records of the chunk's `steps` timesteps, appended to the lattices' host histories.
+int Engine::HistStage::drain(uint64_t steps) {
+    if (pl.ghist_on && gh_recs) { int r = drain_graph(); if (r) return r; }
+    if (!per_step_bytes) return SNN_OK;
+    const uint64_t n_neurons = e.n_neurons, n_trains = e.n_trains;
+    std::vector<float> hg, htg; std::vector<uint32_t> hs, hts;
+    cudaError_t he = cudaSuccess;
+    if (pl.copy_grid) { hg.resize(steps * n_neurons); he = cudaMemcpy(hg.data(), grid, hg.size() * 4, cudaMemcpyDeviceToHost); }
+    if (he != cudaSuccess) return cuda_fail(he, SNN_GPU_BUFFER_READ_ERROR, "grid history drain");
+    if (pl.want_red) {
+        const size_t nl = red_lats.size();
+        cudaError_t re = launch_history_reduce(grid, n_neurons, (uint32_t)steps, red_lat, red_lat + nl, (const float *)(red_lat + 2 * nl),
+                                               (int)nl, red, e.stream_);
+        std::vector<double> hr(steps * nl * 2);
+        // stream_ is non-blocking: a copy on the legacy stream would not wait for the reduction
+        if (re == cudaSuccess) re = cudaMemcpyAsync(hr.data(), red, hr.size() * 8, cudaMemcpyDeviceToHost, e.stream_);
+        if (re == cudaSuccess) re = cudaStreamSynchronize(e.stream_);
+        if (re != cudaSuccess) return cuda_fail(re, SNN_GPU_BUFFER_READ_ERROR, "history reduce");
+        for (size_t k = 0; k < nl; ++k) {
+            Lat &L = *red_lats[k];
+            for (uint64_t s = 0; s < steps; ++s) {
+                const double sum_v = hr[(s * nl + k) * 2], sum_dv = hr[(s * nl + k) * 2 + 1];
+                // AverageVoltageHistory::update, neuron/mod.rs:310-316: sum / len as f32
+                if (L.avg_hist) L.average_history.push_back((float)sum_v / (float)L.n);
+                // EEGHistory::update, neuron/mod.rs:266-279: (1 / (4 pi sigma d)) * total_current
+                if (L.eeg_hist) L.eeg_history.push_back((1.f / (4.f * 3.14159274101257324f * L.eeg_cond * L.eeg_dist)) * (float)sum_dv);
+            }
+            if (!L.grid_hist && !L.spike_hist) L.hist_len += steps;
+        }
+    }
+    if (pl.want_spk) { hs.resize(steps * n_words); he = cudaMemcpy(hs.data(), spk, hs.size() * 4, cudaMemcpyDeviceToHost); }
+    if (he == cudaSuccess && pl.want_tgrid) { htg.resize(steps * n_trains); he = cudaMemcpy(htg.data(), tgrid, htg.size() * 4, cudaMemcpyDeviceToHost); }
+    if (he == cudaSuccess && pl.want_tspk) { hts.resize(steps * t_words); he = cudaMemcpy(hts.data(), tspk, hts.size() * 4, cudaMemcpyDeviceToHost); }
+    if (he != cudaSuccess) return cuda_fail(he, SNN_GPU_BUFFER_READ_ERROR, "history drain");
+    // SpikeHistory::aggregate (neuron/mod.rs:335-359): the sum over the chunk's steps is taken on the device from the staged
+    // raster; the host only adds one count per neuron and chunk
+    std::vector<uint32_t> cnt_n, cnt_t;
+    for (int dom = 0; dom < 2 && he == cudaSuccess; ++dom) {
+        const bool on = dom ? pl.want_tspk : pl.want_spk;
+        const uint64_t dn = dom ? n_trains : n_neurons, dw = dom ? t_words : n_words;
+        if (!on || dn == 0) continue;
+        std::vector<uint32_t> &cnt = dom ? cnt_t : cnt_n;
+        cnt.resize(dn);
+        if (e.ensure_scratch(dn * 4)) { he = cudaErrorMemoryAllocation; break; }
+        he = launch_spike_count(dom ? tspk : spk, (uint32_t)steps, dw, dn, (uint32_t *)e.scratch_, e.stream_);
+        if (he == cudaSuccess) he = cudaMemcpyAsync(cnt.data(), e.scratch_, dn * 4, cudaMemcpyDeviceToHost, e.stream_);
+        if (he == cudaSuccess) he = cudaStreamSynchronize(e.stream_);
+    }
+    if (he != cudaSuccess) return cuda_fail(he, SNN_GPU_BUFFER_READ_ERROR, "spike aggregate");
+    for (auto &L : e.lats_) {
+        if (!L.grid_hist && !L.spike_hist) continue;
+        const uint64_t dom_n = L.is_train ? n_trains : n_neurons, dom_w = L.is_train ? t_words : n_words;
+        const std::vector<float> &G = L.is_train ? htg : hg;
+        const std::vector<uint32_t> &S = L.is_train ? hts : hs;
+        if (L.spike_hist) {
+            const std::vector<uint32_t> &cnt = L.is_train ? cnt_t : cnt_n;
+            if (L.spike_agg.size() != L.n) L.spike_agg.assign(L.n, 0);
+            for (uint64_t j = 0; j < L.n; ++j) L.spike_agg[j] += cnt[L.off + j];
+        }
+        for (uint64_t s = 0; s < steps; ++s) {
+            if (L.grid_hist) L.grid_history.insert(L.grid_history.end(), G.begin() + s * dom_n + L.off, G.begin() + s * dom_n + L.off + L.n);
+            if (L.spike_hist) {
+                const size_t o = L.spike_history.size();
+                L.spike_history.resize(o + L.n);
+                for (uint64_t j = 0; j < L.n; ++j) {
+                    const uint64_t b = L.off + j;
+                    L.spike_history[o + j] = (uint8_t)((S[s * dom_w + (b >> 5)] >> (b & 31)) & 1u);
+                }
+            }
+        }
+        L.hist_len += steps;
+    }
+    return SNN_OK;
+}
+
+// Difference tables of the STDP term, one per lattice (lattice l at tab + l * 2 * tab_n, the layout of RstdpParams::tab), long
+// enough for every exponential to have underflowed to zero at its end.  Only a, tau and dt of each entry are read.  *tab stays
+// null when a time constant is out of range: the kernels evaluate the formula then.
+int Engine::build_stdp_tables(const std::vector<RstdpParams> &lat, const float **tab, uint32_t *tab_n) {
+    double reach = 0.0;
+    bool ok = true;
+    for (const RstdpParams &q : lat) {
+        ok = ok && q.tau_plus > 0.f && q.tau_minus > 0.f && q.dt > 0.f;
+        reach = std::max(reach, 110.0 * std::max((double)q.tau_plus, (double)q.tau_minus) / std::max((double)q.dt, 1e-30));
+    }
+    if (!ok || !(reach > 0 && reach < 60000.0)) return SNN_OK;
+    const uint32_t n = (uint32_t)reach + 8u;
+    const size_t need = lat.size() * 2u * n;
+    if (stdp_tab_elems_ != need) {
+        if (stdp_tab_) cudaFree(stdp_tab_);
+        stdp_tab_ = nullptr; stdp_tab_elems_ = 0;
+        CK(dev_alloc(&stdp_tab_, need), SNN_GPU_BUFFER_CREATE_ERROR);
+        stdp_tab_elems_ = need;
+    }
+    for (size_t l = 0; l < lat.size(); ++l)   // the parameters may have changed since the last run
+        CK(launch_rstdp_table(lat[l], stdp_tab_ + l * 2u * n, n, stream_), SNN_GPU_QUEUE_FAILURE);
+    *tab = stdp_tab_; *tab_n = n;
+    return SNN_OK;
+}
+
+// RewardModulatedLatticeNetwork: reward-modulated lattices next to plain lattices and spike trains.  Refuses the configurations
+// the reference cannot run itself.
+int Engine::build_rnet_params(RnetParams &rnp, bool *net_rmod) {
+    if (part_world > 1 || reward_mode || bcm_mode) return fail(SNN_UNSUPPORTED, "reward-modulated lattice networks run on single-GPU network handles");
+    // update_weights_from_neurons_across_(reward_)lattices looks the OUTGOING connecting edges up with the end points swapped and
+    // unwraps the result (neuron/mod.rs:4760-4763, 4931-4934), and its incoming arms unwrap lattice kinds that need not be there
+    // (:4727-4731, 4741-4747)
+    for (auto &kv : blocks_) {
+        if (kv.first.first == kv.first.second) continue;
+        if (kv.second.kind != Block::GRID && kv.second.pre.empty()) continue;
+        const Lat *A = find(kv.first.first), *B = find(kv.first.second);
+        if (!A || !B) continue;
+        if (A->is_reward && A->do_modulation)
+            return fail(SNN_UNSUPPORTED, "connecting edges out of a reward-modulated lattice with do_modulation: the reference panics on them (neuron/mod.rs:4931-4934)");
+        if (!A->is_train && !A->is_reward && A->do_plasticity)
+            return fail(SNN_UNSUPPORTED, "connecting edges out of a plastic lattice of a reward-modulated network: the reference panics on them (neuron/mod.rs:4760-4763)");
+        if (!B->is_reward && kv.second.reward_conn)
+            return fail(SNN_UNSUPPORTED, "RewardModulatedWeight connections must end in a reward-modulated lattice");
+        if (!B->is_reward && B->do_plasticity && A->is_reward)
+            return fail(SNN_UNSUPPORTED, "a plastic lattice fed by a reward-modulated lattice: the reference panics on it (neuron/mod.rs:4727-4731)");
+    }
+    *net_rmod = false;
+    std::map<uint64_t, int> cls;   // lattice id -> presynaptic class of RnetParams::kinds
+    std::vector<const Lat *> nl;
+    int kn = 0, kt = 0;
+    for (auto &L : lats_) {
+        if (L.is_train) { rnp.tl_base[kt] = (uint32_t)L.off; cls[L.id] = kMaxLattices + kt; ++kt; continue; }
+        RnetLat &R = rnp.lat[kn];
+        R.dopamine = L.rstdp.dopamine; R.tau_c = L.rstdp.tau_c; R.a_plus = L.rstdp.a_plus; R.a_minus = L.rstdp.a_minus;
+        R.tau_plus = L.rstdp.tau_plus; R.tau_minus = L.rstdp.tau_minus; R.dt = L.rstdp.dt;
+        R.flags = (L.is_reward ? 1u : 0u) | (L.is_reward && L.do_modulation ? 2u : 0u);
+        *net_rmod |= L.is_reward && L.do_modulation && L.n > 0;
+        rnp.nbase[kn] = (uint32_t)L.off;
+        nl.push_back(&L);
+        cls[L.id] = kn++;
+    }
+    rnp.n_lat = (uint32_t)kn; rnp.nbase[kn] = (uint32_t)n_neurons;
+    rnp.n_tl = (uint32_t)kt; rnp.tl_base[kt] = (uint32_t)n_trains; rnp.train0 = train0_;
+    for (int post = 0; post < kn; ++post) {
+        if (!nl[post]->is_reward) continue;
+        uint64_t k = 1ull << (2 * post);                                 // own graph
+        for (int pre = 0; pre < kn; ++pre)
+            if (pre != post && !nl[pre]->is_reward) k |= 3ull << (2 * pre);   // Weight block fed by a plain lattice (the default kind)
+        rnp.kinds[post] = k;
+    }
+    for (auto &kv : blocks_)
+        if (kv.second.reward_conn && kv.first.first != kv.first.second && cls.count(kv.first.first) && cls.count(kv.first.second)) {
+            uint64_t &k = rnp.kinds[cls[kv.first.second]];
+            const int q = cls[kv.first.first];
+            k = (k & ~(3ull << (2 * q))) | (2ull << (2 * q));
+        }
+    if (!*net_rmod) return SNN_OK;
+    int r = ensure_reward_arrays();
+    if (r) return r;
+    rnp.counter = rs_counter_; rnp.dw = rs_dw_; rnp.c = rs_c_;
+    rnp.canonical = rs_canonical_ ? 1u : 0u;
+    // one table per neuron lattice: the modulator's STDP term for a reward-modulated lattice, the lattice's own STDP for a plain
+    // one (what Weight edges out of it use)
+    std::vector<RstdpParams> tl(nl.size(), RstdpParams{});
+    for (size_t l = 0; l < nl.size(); ++l) {
+        const Lat &L = *nl[l];
+        RstdpParams &q = tl[l];
+        if (L.is_reward) { q.a_plus = L.rstdp.a_plus; q.a_minus = L.rstdp.a_minus; q.tau_plus = L.rstdp.tau_plus; q.tau_minus = L.rstdp.tau_minus; q.dt = L.rstdp.dt; }
+        else { q.a_plus = L.stdp.a_plus; q.a_minus = L.stdp.a_minus; q.tau_plus = L.stdp.tau_plus; q.tau_minus = L.stdp.tau_minus; q.dt = L.stdp.dt; }
+    }
+    return build_stdp_tables(tl, &rnp.tab, &rnp.tab_n);
+}
+
+// Refusals, the device graph, and every decision fixed for the whole run, with the kernel parameter blocks it selects.
+int Engine::plan_run(RunPlan &pl, LaunchArgs &a) {
+    for (auto &L : lats_) if (!L.is_train && L.graph_hist) pl.gh_keys.emplace_back(L.id, L.id);
     if (conn_graph_hist)
         for (auto &kv : blocks_)
-            if (kv.first.first != kv.first.second && (kv.second.kind == Block::GRID || !kv.second.pre.empty())) gh_keys.push_back(kv.first);
-    const bool ghist_on = !gh_keys.empty();
-    if (ghist_on && part_world > 1) return fail(SNN_UNSUPPORTED, "graph history: whole-GPU handles only (not row strips or general-graph partitions)");
-    if (ghist_on && (reward_mode || has_reward_lattices()))
+            if (kv.first.first != kv.first.second && (kv.second.kind == Block::GRID || !kv.second.pre.empty())) pl.gh_keys.push_back(kv.first);
+    pl.ghist_on = !pl.gh_keys.empty();
+    if (pl.ghist_on && part_world > 1) return fail(SNN_UNSUPPORTED, "graph history: whole-GPU handles only (not row strips or general-graph partitions)");
+    if (pl.ghist_on && (reward_mode || has_reward_lattices()))
         return fail(SNN_UNSUPPORTED, "graph history: not recorded for reward-modulated lattices and networks (TraceRSTDP weights)");
     if (part_world > 1 && !gpart_) {
         if ((part_rank > 0 && !halo_dir_[0].active) || (part_rank < part_world - 1 && !halo_dir_[1].active))
@@ -2102,679 +2456,319 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
     r = upload_lat_table();
     if (r) return r;
     if (gpart_) { r = gpart_build_device(); if (r) return r; }
-    // graph history: per-row offsets of the table's canonical order (once per graph build), then how each requested block is cut
-    // out of a record: the whole record (the table holds that block only) or one contiguous range per postsynaptic row
-    struct GhPlan { GraphHist *h; bool whole; const Block *b; std::vector<uint64_t> src; };
-    std::vector<GhPlan> gh_plans;
-    if (ghist_on) {
-        if (!ghist_off_valid_) {
-            if (ghist_row_off_) cudaFree(ghist_row_off_);
-            ghist_row_off_ = nullptr;
-            CK(dev_alloc(&ghist_row_off_, (size_t)n_slices_ * 32 + 1), SNN_GPU_BUFFER_CREATE_ERROR);
-            CK(launch_graph_row_offsets(col_, slice_off_, n_slices_, ghist_row_off_, stream_), SNN_GPU_QUEUE_FAILURE);
-            uint32_t tot = 0;
-            CK(cudaMemcpyAsync(&tot, ghist_row_off_ + (size_t)n_slices_ * 32, 4, cudaMemcpyDeviceToHost, stream_), SNN_GPU_BUFFER_READ_ERROR);
-            CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
-            ghist_nnz_ = tot;
-            std::vector<uint32_t> so((size_t)n_slices_ + 1);
-            CK(cudaMemcpy(so.data(), slice_off_, so.size() * 4, cudaMemcpyDeviceToHost), SNN_GPU_BUFFER_READ_ERROR);
-            ghist_max_width_ = 0;
-            for (uint32_t sl = 0; sl < n_slices_; ++sl) ghist_max_width_ = std::max(ghist_max_width_, so[sl + 1] - so[sl]);
-            ghist_off_valid_ = true;
-        }
-        std::vector<uint64_t> roff;   // canonical row offsets of the table from the host blocks (several blocks only)
-        for (auto &key : gh_keys) {
-            GhPlan pl{&graph_hist_[key], false, nullptr, {}};
-            auto it = blocks_.find(key);
-            if (it != blocks_.end() && blocks_.size() == 1) {
-                pl.whole = true;
-                pl.h->nnz = ghist_nnz_;
-            } else if (it != blocks_.end()) {
-                // finalize_graph's general path: every block is host CSR; rows hold the blocks into their lattice ordered by the
-                // presynaptic lattice's node offset (sync_weights_to_host walks them the same way)
-                if (roff.empty()) {
-                    roff.assign(n_neurons + 1, 0);
-                    for (auto &kv : blocks_) {
-                        const Lat *B = find(kv.first.second);
-                        for (uint64_t q = 0; q < B->n; ++q) roff[B->off + q + 1] += kv.second.row_ptr[q + 1] - kv.second.row_ptr[q];
-                    }
-                    for (uint64_t i = 0; i < n_neurons; ++i) roff[i + 1] += roff[i];
-                    if (roff[n_neurons] != ghist_nnz_) return fail(SNN_GPU_BUFFER_READ_ERROR, "graph history: host and device tables disagree");
-                }
-                const Lat *A = find(key.first), *B = find(key.second);
-                std::vector<const Block *> before;
-                for (auto &kv : blocks_)
-                    if (kv.first.second == key.second && kv.first != key && node_off(*find(kv.first.first)) < node_off(*A)) before.push_back(&kv.second);
-                pl.b = &it->second;
-                pl.src.resize(B->n);
-                for (uint64_t q = 0; q < B->n; ++q) {
-                    uint64_t o = roff[B->off + q];
-                    for (const Block *o_b : before) o += o_b->row_ptr[q + 1] - o_b->row_ptr[q];
-                    pl.src[q] = o;
-                }
-                pl.h->nnz = it->second.pre.size();
-            } else {
-                pl.h->nnz = 0;   // a lattice without an internal graph: empty records
-            }
-            gh_plans.push_back(std::move(pl));
-        }
-    }
 
-    bool stdp = false, want_grid = false, want_spk = false, want_tgrid = false, want_tspk = false, want_red = false;
     for (auto &L : lats_) {
-        if (!L.is_train) { stdp |= L.do_plasticity && !L.is_reward; want_grid |= L.grid_hist; want_spk |= L.spike_hist; want_red |= L.avg_hist || L.eeg_hist; }
-        else { want_tgrid |= L.grid_hist; want_tspk |= L.spike_hist; }
+        if (!L.is_train) { pl.stdp |= L.do_plasticity && !L.is_reward; pl.want_grid |= L.grid_hist; pl.want_spk |= L.spike_hist; pl.want_red |= L.avg_hist || L.eeg_hist; }
+        else { pl.want_tgrid |= L.grid_hist; pl.want_tspk |= L.spike_hist; }
     }
-    // kernel specialisation: ntrel = neurotransmitter / receptor state must be stepped; chemg = how the chemical gather
-    // reads presynaptic types (0 none, 1 a single type in the whole node array, 3 per-edge masks); net = several
-    // lattices and/or spike trains share the node array
-    const bool ntrel = chem_alloc_ && (chemical || nt_used() != 0 || (model == SNN_MODEL_HODGKIN_HUXLEY && rc_used() != 0));
-    int n_neuron_lat = 0;
-    for (auto &L : lats_) if (!L.is_train) n_neuron_lat++;
-    const bool net = n_neuron_lat > 1 || n_trains > 0;
-    int chemg = 0;
-    if (chemical && ntrel && nt_used() != 0) chemg = (!net && __builtin_popcount(nt_used()) == 1) ? 1 : 3;
+    // AverageVoltageHistory / EEGHistory are reductions of the staged grid record (it stays on the device for them)
+    pl.copy_grid = pl.want_grid;
+    pl.want_grid = pl.want_grid || pl.want_red;
+    pl.ntrel = chem_alloc_ && (chemical || nt_used() != 0 || (model == SNN_MODEL_HODGKIN_HUXLEY && rc_used() != 0));
+    pl.net = n_neuron_lattices() > 1 || n_trains > 0;
+    if (chemical && pl.ntrel && nt_used() != 0) pl.chemg = (!pl.net && __builtin_popcount(nt_used()) == 1) ? 1 : 3;
     // reward-modulated lattice: the modulator replaces the plasticity rule and needs last_firing_time before and after a step
-    const bool rmod = reward_mode && do_modulation && n_neurons > 0;
+    pl.rmod = reward_mode && do_modulation && n_neurons > 0;
     // BCM rule instead of STDP: applied by its own per-edge kernel right after each step (it reads the activities the step wrote)
-    const bool bcm_on = bcm_mode && stdp && !reward_mode && n_neurons > 0;
-    if (reward_mode || bcm_mode) stdp = false;
-    if (rmod) { int rr = ensure_reward_arrays(); if (rr) return rr; }
-    RstdpParams rsp{rstdp.dopamine, rstdp.tau_c, rstdp.a_plus, rstdp.a_minus, rstdp.tau_plus, rstdp.tau_minus, rstdp.dt,
-                    rs_counter_, rs_dw_, rs_c_, rs_canonical_ ? 1u : 0u, nullptr, 0u};
-    if (rmod && !getenv("SNN_B200_RSTDP_NOTAB")) {
-        // difference table of the STDP term: long enough for the exponential to have underflowed to zero at its end
-        const double reach = 110.0 * std::max((double)rstdp.tau_plus, (double)rstdp.tau_minus) / std::max((double)rstdp.dt, 1e-30);
-        if (reach > 0 && reach < 60000.0 && rstdp.tau_plus > 0.f && rstdp.tau_minus > 0.f && rstdp.dt > 0.f) {
-            const uint32_t tab_n = (uint32_t)reach + 8u;
-            if (rs_tab_n_ != tab_n) {
-                if (rs_tab_) cudaFree(rs_tab_);
-                rs_tab_ = nullptr; rs_tab_n_ = 0;
-                CK(dev_alloc(&rs_tab_, (size_t)tab_n * 2), SNN_GPU_BUFFER_CREATE_ERROR);
-                rs_tab_n_ = tab_n;
-            }
-            CK(launch_rstdp_table(rsp, rs_tab_, tab_n, stream_), SNN_GPU_QUEUE_FAILURE);   // the parameters may have changed since the last run
-            rsp.tab = rs_tab_; rsp.tab_n = tab_n;
-        }
-    }
-    // RewardModulatedLatticeNetwork: reward-modulated lattices next to plain lattices and spike trains
-    const bool net_reward = has_reward_lattices();
-    bool net_rmod = false;
-    RnetParams rnp;
-    memset(&rnp, 0, sizeof rnp);
-    if (net_reward) {
-        if (part_world > 1 || reward_mode || bcm_mode) return fail(SNN_UNSUPPORTED, "reward-modulated lattice networks run on single-GPU network handles");
-        // the configurations the reference cannot run itself: update_weights_from_neurons_across_(reward_)lattices looks the OUTGOING
-        // connecting edges up with the end points swapped and unwraps the result (neuron/mod.rs:4760-4763, 4931-4934), and its
-        // incoming arms unwrap lattice kinds that need not be there (:4727-4731, 4741-4747)
-        for (auto &kv : blocks_) {
-            if (kv.first.first == kv.first.second) continue;
-            if (kv.second.kind != Block::GRID && kv.second.pre.empty()) continue;
-            const Lat *A = find(kv.first.first), *B = find(kv.first.second);
-            if (!A || !B) continue;
-            if (A->is_reward && A->do_modulation)
-                return fail(SNN_UNSUPPORTED, "connecting edges out of a reward-modulated lattice with do_modulation: the reference panics on them (neuron/mod.rs:4931-4934)");
-            if (!A->is_train && !A->is_reward && A->do_plasticity)
-                return fail(SNN_UNSUPPORTED, "connecting edges out of a plastic lattice of a reward-modulated network: the reference panics on them (neuron/mod.rs:4760-4763)");
-            if (!B->is_reward && kv.second.reward_conn)
-                return fail(SNN_UNSUPPORTED, "RewardModulatedWeight connections must end in a reward-modulated lattice");
-            if (!B->is_reward && B->do_plasticity && A->is_reward)
-                return fail(SNN_UNSUPPORTED, "a plastic lattice fed by a reward-modulated lattice: the reference panics on it (neuron/mod.rs:4727-4731)");
-        }
-        std::map<uint64_t, int> cls;   // lattice id -> presynaptic class of RnetParams::kinds
-        std::vector<const Lat *> nl;
-        int kn = 0, kt = 0;
-        for (auto &L : lats_) {
-            if (L.is_train) { rnp.tl_base[kt] = (uint32_t)L.off; cls[L.id] = kMaxLattices + kt; ++kt; continue; }
-            RnetLat &R = rnp.lat[kn];
-            R.dopamine = L.rstdp.dopamine; R.tau_c = L.rstdp.tau_c; R.a_plus = L.rstdp.a_plus; R.a_minus = L.rstdp.a_minus;
-            R.tau_plus = L.rstdp.tau_plus; R.tau_minus = L.rstdp.tau_minus; R.dt = L.rstdp.dt;
-            R.flags = (L.is_reward ? 1u : 0u) | (L.is_reward && L.do_modulation ? 2u : 0u);
-            net_rmod |= L.is_reward && L.do_modulation && L.n > 0;
-            rnp.nbase[kn] = (uint32_t)L.off;
-            nl.push_back(&L);
-            cls[L.id] = kn++;
-        }
-        rnp.n_lat = (uint32_t)kn; rnp.nbase[kn] = (uint32_t)n_neurons;
-        rnp.n_tl = (uint32_t)kt; rnp.tl_base[kt] = (uint32_t)n_trains; rnp.train0 = train0_;
-        for (int post = 0; post < kn; ++post) {
-            if (!nl[post]->is_reward) continue;
-            uint64_t k = 1ull << (2 * post);                                 // own graph
-            for (int pre = 0; pre < kn; ++pre)
-                if (pre != post && !nl[pre]->is_reward) k |= 3ull << (2 * pre);   // Weight block fed by a plain lattice (the default kind)
-            rnp.kinds[post] = k;
-        }
-        for (auto &kv : blocks_)
-            if (kv.second.reward_conn && kv.first.first != kv.first.second && cls.count(kv.first.first) && cls.count(kv.first.second)) {
-                uint64_t &k = rnp.kinds[cls[kv.first.second]];
-                const int q = cls[kv.first.first];
-                k = (k & ~(3ull << (2 * q))) | (2ull << (2 * q));
-            }
-        if (net_rmod) { int rr = ensure_reward_arrays(); if (rr) return rr; }
-        rnp.counter = rs_counter_; rnp.dw = rs_dw_; rnp.c = rs_c_;
-        rnp.canonical = (rs_canonical_ && !getenv("SNN_B200_RNET_NOCANON")) ? 1u : 0u;
-        if (net_rmod && !getenv("SNN_B200_RSTDP_NOTAB")) {
-            // one difference table per neuron lattice: the modulator's STDP term for a reward-modulated lattice, the lattice's own
-            // STDP for a plain one (what Weight edges out of it use); long enough for every exponential to have underflowed
-            double reach = 0.0;
-            bool ok = true;
-            for (const Lat *L : nl) {
-                const float tp_ = L->is_reward ? L->rstdp.tau_plus : L->stdp.tau_plus, tm_ = L->is_reward ? L->rstdp.tau_minus : L->stdp.tau_minus;
-                const float dt_ = L->is_reward ? L->rstdp.dt : L->stdp.dt;
-                ok = ok && tp_ > 0.f && tm_ > 0.f && dt_ > 0.f;
-                reach = std::max(reach, 110.0 * std::max((double)tp_, (double)tm_) / std::max((double)dt_, 1e-30));
-            }
-            if (ok && reach > 0 && reach < 60000.0) {
-                const uint32_t tab_n = (uint32_t)reach + 8u;
-                const size_t need = (size_t)kn * 2u * tab_n;
-                if (rnet_tab_elems_ != need) {
-                    if (rnet_tab_) cudaFree(rnet_tab_);
-                    rnet_tab_ = nullptr; rnet_tab_elems_ = 0;
-                    CK(dev_alloc(&rnet_tab_, need), SNN_GPU_BUFFER_CREATE_ERROR);
-                    rnet_tab_elems_ = need;
-                }
-                for (int l = 0; l < kn; ++l) {   // the parameters may have changed since the last run
-                    const Lat &L = *nl[l];
-                    RstdpParams tpar{};
-                    if (L.is_reward) { tpar.a_plus = L.rstdp.a_plus; tpar.a_minus = L.rstdp.a_minus; tpar.tau_plus = L.rstdp.tau_plus; tpar.tau_minus = L.rstdp.tau_minus; tpar.dt = L.rstdp.dt; }
-                    else { tpar.a_plus = L.stdp.a_plus; tpar.a_minus = L.stdp.a_minus; tpar.tau_plus = L.stdp.tau_plus; tpar.tau_minus = L.stdp.tau_minus; tpar.dt = L.stdp.dt; }
-                    CK(launch_rstdp_table(tpar, rnet_tab_ + (size_t)l * 2u * tab_n, tab_n, stream_), SNN_GPU_QUEUE_FAILURE);
-                }
-                rnp.tab = rnet_tab_; rnp.tab_n = tab_n;
-            }
-        }
-    }
-    const bool lft_pp = stdp || rmod || net_rmod || (n_trains && electrical) || part_world > 1;
-    const bool rmod_part = rmod && part_world > 1;
+    pl.bcm_on = bcm_mode && pl.stdp && !reward_mode && n_neurons > 0;
+    if (reward_mode || bcm_mode) pl.stdp = false;
+    if (pl.rmod) { r = ensure_reward_arrays(); if (r) return r; }
+    a.rsp = RstdpParams{rstdp.dopamine, rstdp.tau_c, rstdp.a_plus, rstdp.a_minus, rstdp.tau_plus, rstdp.tau_minus, rstdp.dt,
+                        rs_counter_, rs_dw_, rs_c_, rs_canonical_ ? 1u : 0u, nullptr, 0u};
+    if (pl.rmod) { r = build_stdp_tables({a.rsp}, &a.rsp.tab, &a.rsp.tab_n); if (r) return r; }
+    pl.net_reward = has_reward_lattices();
+    if (pl.net_reward) { r = build_rnet_params(a.rnp, &pl.net_rmod); if (r) return r; }
+    pl.lft_pp = pl.stdp || pl.rmod || pl.net_rmod || (n_trains && electrical) || part_world > 1;
+    pl.rmod_part = pl.rmod && part_world > 1;
 
-    StepParams sp;
-    fill_step_params(sp);
-    sp.lft_pp = lft_pp;
-    if (rmod_part)   // step s + 1 overwrites ghost slots that the neighbour's per-edge kernel of step s still reads: wait for that one
-        for (int d = 0; d < 2; ++d) sp.halo[d].my_flag = halo_dir_[d].my_flag2;
-    TmaParams tma;
-    unsigned tma_grid = 0;
-    WinParams win;
-    unsigned win_grid = 0;
-    const bool win_ok = !net && build_win_params(win, chemg, ntrel, stdp, lft_pp, &win_grid);
-    const bool tma_ok = !win_ok && !net && build_tma_params(tma, ntrel, stdp, lft_pp, &tma_grid);
-    // wide rows (hundreds of in-edges per neuron, e.g. all-to-all spike-train input): one CTA per slice
-    bool wide = !win_ok && !tma_ok && part_world == 1 && n_slices_ > 0 && sell_krows_ / n_slices_ >= kWideMinWidth;
-    if (const char *e = getenv("SNN_B200_WIDE")) wide = wide && atoi(e) != 0;
-    // very wide slices (hundreds of k-rows): one SM per slice cannot issue the per-edge instructions fast enough — two passes, the
-    // per-edge terms of every (slice, chunk) on its own CTA, then the ordered sums (step_wide.cu)
-    bool wide_split = false;
-    uint32_t wide_chunks_cap = 0;
-    if (wide) {
-        const uint64_t mean = sell_krows_ / n_slices_;
-        wide_split = mean >= 2 * wide_chunk_krows();
-        if (const char *e = getenv("SNN_B200_WIDE_SPLIT")) wide_split = atoi(e) != 0;
-        if (wide_split) {
-            std::vector<uint32_t> so((size_t)n_slices_ + 1);
-            CK(cudaMemcpy(so.data(), slice_off_, so.size() * 4, cudaMemcpyDeviceToHost), SNN_GPU_BUFFER_READ_ERROR);
-            uint32_t mx = 0;
-            for (uint32_t sl = 0; sl < n_slices_; ++sl) mx = std::max(mx, so[sl + 1] - so[sl]);
-            wide_chunks_cap = (mx + wide_chunk_krows() - 1) / wide_chunk_krows();
-            const size_t need = (size_t)n_slices_ * wide_chunks_cap * wide_chunk_bytes(chemg) + (size_t)n_slices_ * wide_part_bytes();
-            if (need != wide_scratch_bytes_) {
-                if (wide_scratch_) cudaFree(wide_scratch_);
-                wide_scratch_ = nullptr; wide_scratch_bytes_ = 0;
-                CK(cudaMalloc((void **)&wide_scratch_, need), SNN_GPU_BUFFER_CREATE_ERROR);
-                wide_scratch_bytes_ = need;
-            }
-            // the arrival counters of the sum pass start at zero (they reset themselves after every timestep)
-            CK(cudaMemsetAsync(wide_scratch_ + (size_t)n_slices_ * wide_chunks_cap * wide_chunk_bytes(chemg), 0, (size_t)n_slices_ * wide_part_bytes(), stream_),
-               SNN_GPU_BUFFER_WRITE_ERROR);
-        }
-    }
-    // indices of the ping-ponged streams, patched every step
-    int tma_iv = -1, tma_il = -1, tma_it[kNT] = {-1, -1, -1};
-    if (tma_ok) {
-        for (uint32_t k = 0; k < tma.n_streams; ++k) {
-            if (tma.st[k].smem_off == tma.o_v) tma_iv = (int)k;
-            if ((stdp || lft_pp) && tma.st[k].smem_off == tma.o_lft) tma_il = (int)k;
-            for (int ty = 0; ty < kNT; ++ty) if (tma.o_t[ty] != 0xFFFFFFFFu && tma.st[k].smem_off == tma.o_t[ty]) tma_it[ty] = (int)k;
-        }
-    }
-    TrainParams tp;
-    memset(&tp, 0, sizeof tp);
+    fill_step_params(a.sp);
+    a.sp.lft_pp = pl.lft_pp;
+    if (pl.rmod_part)   // step s + 1 overwrites ghost slots that the neighbour's per-edge kernel of step s still reads: wait for that one
+        for (int d = 0; d < 2; ++d) a.sp.halo[d].my_flag = halo_dir_[d].my_flag2;
     if (n_trains) {
+        TrainParams &tp = a.tp;
         tp.train0 = train0_; tp.n_trains = (uint32_t)n_trains; tp.kind = train_kind; tp.ntk = ntk; tp.seed = seed;
         tp.t_stride = node_cap_; tp.node_flags = node_flags_; tp.nt_stride = node_cap_;
         for (int s = 0; s < NTF_COUNT; ++s) tp.nt[s] = NT_[s];
         for (int s = 0; s < TF_COUNT; ++s) tp.tf[s] = TF_[s];
-        tp.ft_off = ft_off_; tp.ft = ft_; tp.lft_pp = lft_pp;
-        if (!chem_alloc_) {  // train kernel reads node_flags only; nt pointers unused when no types are present
-        }
+        tp.ft_off = ft_off_; tp.ft = ft_; tp.lft_pp = pl.lft_pp;
     }
+    return plan_step_path(pl, a);
+}
 
-    uint64_t n_launch = 0;
-    // history staging: chunks of steps recorded on the device, drained to the host between chunks
-    const uint64_t n_words = (n_neurons + 31) / 32, t_words = (n_trains + 31) / 32;
-    uint64_t per_step_bytes = 0;
-    // AverageVoltageHistory / EEGHistory are reductions of the staged grid record (it stays on the device for them)
-    const bool copy_grid = want_grid;
-    want_grid = want_grid || want_red;
-    if (want_grid) per_step_bytes += n_neurons * 4;
-    if (want_spk) per_step_bytes += n_words * 4;
-    if (want_tgrid) per_step_bytes += n_trains * 4;
-    if (want_tspk) per_step_bytes += t_words * 4;
-    if (ghist_on) per_step_bytes += std::max<uint64_t>(ghist_nnz_, 1) * 4;
-    uint64_t chunk = iterations;
-    if (per_step_bytes) chunk = std::max<uint64_t>(1, std::min<uint64_t>(iterations, (256ull << 20) / per_step_bytes));
-    float *d_grid = nullptr, *d_tgrid = nullptr; uint32_t *d_spk = nullptr, *d_tspk = nullptr;
-    if (want_grid) CK(dev_alloc(&d_grid, chunk * n_neurons), SNN_GPU_BUFFER_CREATE_ERROR);
-    if (want_spk) CK(dev_alloc(&d_spk, chunk * n_words), SNN_GPU_BUFFER_CREATE_ERROR);
-    if (want_tgrid) CK(dev_alloc(&d_tgrid, chunk * n_trains), SNN_GPU_BUFFER_CREATE_ERROR);
-    if (want_tspk) CK(dev_alloc(&d_tspk, chunk * t_words), SNN_GPU_BUFFER_CREATE_ERROR);
-    double *d_red = nullptr; uint32_t *d_red_lat = nullptr;
-    std::vector<Lat *> red_lats;
-    if (want_red) {
-        std::vector<uint32_t> meta;
-        for (auto &L : lats_) if (!L.is_train && (L.avg_hist || L.eeg_hist)) red_lats.push_back(&L);   // lats_ is not resized inside run()
-        const size_t nl = red_lats.size();
-        meta.resize(3 * nl);
-        for (size_t k = 0; k < nl; ++k) {
-            meta[k] = (uint32_t)red_lats[k]->off; meta[nl + k] = (uint32_t)red_lats[k]->n;
-            memcpy(&meta[2 * nl + k], &red_lats[k]->eeg_ref, 4);
+// The step path, and whether a whole chunk of timesteps goes into one launch.
+int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
+    // SNN_B200_TMA: 0 never takes the staged kernels, 2 takes them at any lattice size (the tests cover them at small sizes);
+    // SNN_B200_WIN=0 leaves the window kernel out
+    const char *tma_env = getenv("SNN_B200_TMA"), *win_env = getenv("SNN_B200_WIN");
+    const int tma_mode = tma_env ? atoi(tma_env) : 1;
+    const int win_mode = (win_env && atoi(win_env) == 0) ? 0 : tma_mode;
+    if (!pl.net && build_win_params(a.win, pl.chemg, pl.ntrel, pl.stdp, pl.lft_pp, win_mode, &pl.grid)) {
+        pl.path = StepPath::Win;
+    } else if (!pl.net && build_tma_params(a.tma, pl.ntrel, pl.stdp, pl.lft_pp, tma_mode, &pl.grid)) {
+        pl.path = StepPath::Tma;
+        for (uint32_t k = 0; k < a.tma.n_streams; ++k) {
+            if (a.tma.st[k].smem_off == a.tma.o_v) pl.tma_iv = (int)k;
+            if ((pl.stdp || pl.lft_pp) && a.tma.st[k].smem_off == a.tma.o_lft) pl.tma_il = (int)k;
+            for (int ty = 0; ty < kNT; ++ty) if (a.tma.o_t[ty] != 0xFFFFFFFFu && a.tma.st[k].smem_off == a.tma.o_t[ty]) pl.tma_it[ty] = (int)k;
         }
-        CK(dev_alloc(&d_red, chunk * nl * 2), SNN_GPU_BUFFER_CREATE_ERROR);
-        CK(dev_alloc(&d_red_lat, 3 * nl), SNN_GPU_BUFFER_CREATE_ERROR);
-        CK(h2d_sync(d_red_lat, meta.data(), meta.size() * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    } else if (part_world == 1 && n_slices_ > 0 && sell_krows_ / n_slices_ >= kWideMinWidth) {
+        // wide rows (hundreds of in-edges per neuron, e.g. all-to-all spike-train input): one CTA per slice.  Very wide slices
+        // (hundreds of k-rows): one SM per slice cannot issue the per-edge instructions fast enough — two passes, the per-edge
+        // terms of every (slice, chunk) on its own CTA, then the ordered sums (step_wide.cu)
+        pl.path = sell_krows_ / n_slices_ >= 2 * wide_chunk_krows() ? StepPath::WideSplit : StepPath::Wide;
     }
-    // graph records of a chunk: one per step, plus the final one of a Lattice with STDP (taken after the end-of-run flush)
-    float *d_ghist = nullptr;
-    if (ghist_on && ghist_nnz_) CK(dev_alloc(&d_ghist, (chunk + 1) * ghist_nnz_), SNN_GPU_BUFFER_CREATE_ERROR);
-    uint64_t gh_recs = 0;
-    // Lattice::iterate records after the step's plasticity (neuron/mod.rs:973-979); lazily applied STDP lands in the table with the
-    // next step kernel (or the end-of-run flush), so a Lattice with STDP records step k after step kernel k + 1.  LatticeNetwork
-    // records before the step's STDP (neuron/mod.rs:2565-2576): the table after step kernel k.  BCM is applied right after the step.
-    auto record_graph = [&]() -> cudaError_t {
-        cudaError_t e = ghist_nnz_ ? launch_graph_record(wgt_, slice_off_, ghist_row_off_, n_slices_, ghist_max_width_, d_ghist + gh_recs * ghist_nnz_, stream_) : cudaSuccess;
-        if (e == cudaSuccess) { ++gh_recs; if (ghist_nnz_) n_launch++; }
-        return e;
-    };
-    auto free_hist = [&]() { cudaFree(d_grid); cudaFree(d_spk); cudaFree(d_tgrid); cudaFree(d_tspk); cudaFree(d_red); cudaFree(d_red_lat); cudaFree(d_ghist); };
-
-    float total_ms = 0.f;
-    int status = SNN_OK;
-    auto bail = [&](cudaError_t e, int st, const char *what) { status = cuda_fail(e, st, what); };
-
-    // multi-GPU: push the current boundary state into the neighbours' ghost slots
-    if (part_world > 1) {
-        StepParams hp = sp;
-        hp.v_in = V_[cur_]; hp.lft_in = LFT_[lft_loc_]; hp.t_in = T_[cur_]; hp.out_par = (uint32_t)cur_;
-        hp.halo_epoch = halo_epoch_;
-        if (lft_loc_ != cur_) {  // keep lft parity aligned with the V parity on partitioned handles
-            cudaMemcpyAsync(LFT_[cur_], LFT_[lft_loc_], node_cap_ * 4, cudaMemcpyDeviceToDevice, stream_);
-            lft_loc_ = cur_; hp.lft_in = LFT_[lft_loc_];
+    if (pl.path == StepPath::WideSplit) {
+        pl.wide_chunks_cap = (max_slice_width_ + wide_chunk_krows() - 1) / wide_chunk_krows();
+        const size_t chunks_bytes = (size_t)n_slices_ * pl.wide_chunks_cap * wide_chunk_bytes(pl.chemg);
+        const size_t need = chunks_bytes + (size_t)n_slices_ * wide_part_bytes();
+        if (need != wide_scratch_bytes_) {
+            if (wide_scratch_) cudaFree(wide_scratch_);
+            wide_scratch_ = nullptr; wide_scratch_bytes_ = 0;
+            CK(cudaMalloc((void **)&wide_scratch_, need), SNN_GPU_BUFFER_CREATE_ERROR);
+            wide_scratch_bytes_ = need;
         }
-        cudaError_t e = gpart_ ? launch_gpart_push(hp, stream_) : launch_halo_push(hp, stream_);
-        if (e != cudaSuccess) { free_hist(); return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "halo_push"); }
-        halo_epoch_ += 1;
-        launched_pub_.store(halo_epoch_, std::memory_order_release);
-        launched_pub2_.store(halo_epoch_, std::memory_order_release);
-        n_launch++;
-        // rendez-vous before any step kernel is enqueued: the in-kernel waits are bounded, so ordinary host-side skew between
-        // the ranks (Python work, history drains, allocation) must be absorbed here, where nothing has been computed yet
-        e = cudaStreamSynchronize(stream_);
-        if (e != cudaSuccess) { free_hist(); return cuda_fail(e, SNN_GPU_WAIT_ERROR, "halo_push"); }
-        const auto t_wait0 = std::chrono::steady_clock::now();
-        for (;;) {
-            unsigned long long f[8 + kMaxRanks];
-            e = cudaMemcpy(f, flags_, sizeof f, cudaMemcpyDeviceToHost);
-            if (e != cudaSuccess) { free_hist(); return cuda_fail(e, SNN_GPU_BUFFER_READ_ERROR, "halo rendez-vous"); }
-            bool ready = true;
-            for (int d = 0; d < 2; ++d) if (halo_dir_[d].active && f[d] < halo_epoch_) ready = false;
-            for (auto &G : gpeers_) if (f[8 + G.rank] < halo_epoch_) ready = false;
-            if (ready) break;
-            if (std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_wait0).count() > 4.0 * (double)halo_timeout_ms) {
-                free_hist();
-                return fail(SNN_GPU_WAIT_ERROR, "timed out waiting for the neighbouring strips to enter run() (is every rank calling run with the same number of steps?)");
-            }
-            std::this_thread::sleep_for(std::chrono::microseconds(20));
-        }
+        // the arrival counters of the sum pass start at zero (they reset themselves after every timestep)
+        CK(cudaMemsetAsync(wide_scratch_ + chunks_bytes, 0, (size_t)n_slices_ * wide_part_bytes(), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+        // the spike trains ride in extra CTAs of the sum pass (nothing in that pass reads train state; the terms pass, which
+        // does, has completed) — one launch and one launch gap less per timestep
+        pl.trains_fused = n_neurons && n_trains > 0;
     }
-
-    static const bool halo_nowait = getenv("SNN_B200_HALO_NOWAIT") != nullptr;
-    static const bool win_reverse = !(getenv("SNN_B200_WIN_REVERSE") && atoi(getenv("SNN_B200_WIN_REVERSE")) == 0);
     // small lattices / networks (everything the staged kernels do not take): a whole chunk of timesteps per cooperative launch
-    // (step_multi.cu).  SNN_OPT_STEPS_PER_GRAPH: 0 = as many as the history chunk holds, 1 = one launch per timestep, k = at most k.
-    bool multi = part_world == 1 && n_neurons > 0 && !win_ok && !tma_ok && !bcm_on && !reward_mode && !net_reward && steps_per_graph != 1 &&
-                 !ghist_on && !getenv("SNN_DEBUG_TIMING");   // graph records are taken between launches: one launch per timestep
-    if (wide && wide_split) multi = false;   // the two-pass wide kernels are one-launch-per-step kernels
-    if (const char *e = getenv("SNN_B200_MULTI")) multi = multi && atoi(e) != 0;
-    if (multi) {
-        StepParams probe = sp;
-        TrainParams tprobe = tp;
-        MultiParams mprobe{};
-        mprobe.wide_stage = (wide && n_nodes_ <= 4096) ? 1u : 0u;
-        multi = launch_step_multi(probe, tprobe, mprobe, model, chemg, ntrel, stdp, net, wide, device, true, stream_) == cudaSuccess;
+    // (step_multi.cu).  SNN_OPT_STEPS_PER_GRAPH: 0 = as many as the history chunk holds, 1 = one launch per timestep, k = at most
+    // k.  Graph records are taken between launches, and the two-pass wide kernels are one-launch-per-step kernels.
+    pl.multi = part_world == 1 && n_neurons > 0 && (pl.path == StepPath::Wide || pl.path == StepPath::General) && !pl.bcm_on &&
+               !reward_mode && !pl.net_reward && steps_per_graph != 1 && !pl.ghist_on;
+    if (pl.multi) {
+        MultiParams probe{};
+        probe.wide_stage = (pl.path == StepPath::Wide && n_nodes_ <= 4096) ? 1u : 0u;
+        pl.multi = launch_step_multi(a.sp, a.tp, probe, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, pl.path == StepPath::Wide, device,
+                                     true, stream_) == cudaSuccess;
         cudaGetLastError();
     }
-    uint64_t done = 0;
-    bool first_step = true;
-    while (done < iterations && status == SNN_OK) {
-        const uint64_t steps = std::min(chunk, iterations - done);
-        cudaEventRecord(ev0_, stream_);
-        const auto host_t0 = std::chrono::steady_clock::now();
-        static const bool dbg_timing = getenv("SNN_DEBUG_TIMING") != nullptr;
-        std::vector<cudaEvent_t> dbg_ev;
-        unsigned long long *dbg_clk = nullptr;
-        if (dbg_timing && steps <= 32) { cudaMalloc(&dbg_clk, 32 * 4 * sizeof(unsigned long long)); cudaMemsetAsync(dbg_clk, 0, 32 * 4 * sizeof(unsigned long long), stream_); }
-        for (uint64_t s0 = 0; multi && s0 < steps;) {
-            const uint64_t k = steps_per_graph ? std::min<uint64_t>(steps_per_graph, steps - s0) : steps - s0;
-            sp.clock = (uint32_t)internal_clock;
-            sp.dbg = nullptr; sp.reverse = 0u;
-            if (n_trains) {
-                tp.n_tl = 0;
-                for (auto &L : lats_)
-                    if (L.is_train) { tp.tl_base[tp.n_tl] = (uint32_t)L.off; tp.tl_clock[tp.n_tl] = (uint32_t)L.clock; tp.n_tl++; }
-                tp.tl_base[tp.n_tl] = (uint32_t)n_trains;
-                tp.draw = train_draws;
-            }
-            MultiParams mp{};
-            mp.steps = (uint32_t)k; mp.first_pending = first_step ? 0u : 1u;
-            mp.cur = (uint32_t)cur_; mp.lft_loc = (uint32_t)lft_loc_; mp.lft_pp = lft_pp ? 1u : 0u;
-            mp.train_sync = (stdp && n_trains) ? 1u : 0u;
-            for (int q = 0; q < 2; ++q) { mp.v[q] = V_[q]; mp.lft[q] = LFT_[q]; mp.spk[q] = SPK_[q]; mp.t[q] = T_[q]; }
-            mp.grid_hist = want_grid ? d_grid + s0 * n_neurons : nullptr;
-            mp.spike_hist = want_spk ? d_spk + s0 * n_words : nullptr;
-            mp.tgrid_hist = want_tgrid ? d_tgrid + s0 * n_trains : nullptr;
-            mp.tspike_hist = want_tspk ? d_tspk + s0 * t_words : nullptr;
-            mp.n_neurons = n_neurons; mp.n_words = n_words; mp.n_trains = n_trains; mp.t_words = t_words;
-            mp.barrier = multi_barrier_;
-            mp.cache_rows = (!stdp && !getenv("SNN_B200_MULTI_NOCACHE")) ? 1u : 0u;
-            mp.wide_stage = (wide && n_nodes_ <= 4096 && !(getenv("SNN_B200_WIDE_STAGE") && atoi(getenv("SNN_B200_WIDE_STAGE")) == 0)) ? 1u : 0u;
-            cudaError_t e = cudaMemsetAsync(multi_barrier_, 0, sizeof(unsigned int), stream_);
-            if (e == cudaSuccess) e = launch_step_multi(sp, tp, mp, model, chemg, ntrel, stdp, net, wide, device, false, stream_);
-            if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_step_multi"); break; }
-            n_launch++;
-            // the host mirrors what the launch did to the ping-pong state and the clocks
-            internal_clock += k;
-            if (k & 1ull) { cur_ ^= 1; if (lft_pp) lft_loc_ ^= 1; }
-            if (n_trains) { train_draws += k; for (auto &L : lats_) if (L.is_train) L.clock += k; }
-            first_step = false;
-            s0 += k;
+    return SNN_OK;
+}
+
+// Multi-GPU: push the current boundary state into the neighbours' ghost slots, then meet the neighbours on the host before any
+// step kernel is enqueued: the in-kernel waits are bounded, so ordinary host-side skew between the ranks (Python work, history
+// drains, allocation) must be absorbed here, where nothing has been computed yet.
+int Engine::halo_rendezvous(const StepParams &sp, uint64_t &launches) {
+    StepParams hp = sp;
+    hp.v_in = V_[cur_]; hp.lft_in = LFT_[lft_loc_]; hp.t_in = T_[cur_]; hp.out_par = (uint32_t)cur_;
+    hp.halo_epoch = halo_epoch_;
+    if (lft_loc_ != cur_) {  // keep lft parity aligned with the V parity on partitioned handles
+        cudaMemcpyAsync(LFT_[cur_], LFT_[lft_loc_], node_cap_ * 4, cudaMemcpyDeviceToDevice, stream_);
+        lft_loc_ = cur_; hp.lft_in = LFT_[lft_loc_];
+    }
+    cudaError_t e = gpart_ ? launch_gpart_push(hp, stream_) : launch_halo_push(hp, stream_);
+    if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "halo_push");
+    halo_epoch_ += 1;
+    launched_pub_.store(halo_epoch_, std::memory_order_release);
+    launched_pub2_.store(halo_epoch_, std::memory_order_release);
+    launches++;
+    e = cudaStreamSynchronize(stream_);
+    if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_WAIT_ERROR, "halo_push");
+    const auto t_wait0 = std::chrono::steady_clock::now();
+    for (;;) {
+        unsigned long long f[8 + kMaxRanks];
+        e = cudaMemcpy(f, flags_, sizeof f, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_BUFFER_READ_ERROR, "halo rendez-vous");
+        bool ready = true;
+        for (int d = 0; d < 2; ++d) if (halo_dir_[d].active && f[d] < halo_epoch_) ready = false;
+        for (auto &G : gpeers_) if (f[8 + G.rank] < halo_epoch_) ready = false;
+        if (ready) return SNN_OK;
+        if (std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_wait0).count() > 4.0 * (double)halo_timeout_ms)
+            return fail(SNN_GPU_WAIT_ERROR, "timed out waiting for the neighbouring strips to enter run() (is every rank calling run with the same number of steps?)");
+        std::this_thread::sleep_for(std::chrono::microseconds(20));
+    }
+}
+
+// The clock of every spike-train lattice: lattice l covers trains [tl_base[l], tl_base[l + 1]) and stamps tl_clock[l].
+void Engine::fill_train_clocks(TrainParams &tp) const {
+    tp.n_tl = 0;
+    for (auto &L : lats_)
+        if (L.is_train) { tp.tl_base[tp.n_tl] = (uint32_t)L.off; tp.tl_clock[tp.n_tl] = (uint32_t)L.clock; tp.n_tl++; }
+    tp.tl_base[tp.n_tl] = (uint32_t)n_trains;
+}
+
+// `steps` timesteps in cooperative launches of up to steps_per_graph timesteps each (step_multi.cu).
+int Engine::run_multi_chunk(const RunPlan &pl, LaunchArgs &a, const HistStage &hist, uint64_t steps, bool first_chunk) {
+    StepParams &sp = a.sp;
+    TrainParams &tp = a.tp;
+    const bool wide = pl.path == StepPath::Wide;
+    for (uint64_t s0 = 0; s0 < steps;) {
+        const uint64_t k = steps_per_graph ? std::min<uint64_t>(steps_per_graph, steps - s0) : steps - s0;
+        sp.clock = (uint32_t)internal_clock;
+        sp.reverse = 0u;
+        if (n_trains) {
+            fill_train_clocks(tp);
+            tp.draw = train_draws;
         }
-        for (uint64_t s = 0; !multi && s < steps; ++s) {
-            if (dbg_timing && steps <= 32) { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, stream_); dbg_ev.push_back(ev); }
-            const int in = cur_, out = cur_ ^ 1;
-            sp.clock = (uint32_t)internal_clock;
-            sp.dbg = dbg_clk ? dbg_clk + 4 * s : nullptr;
-            sp.reverse = (win_reverse && (internal_clock & 1ull)) ? 1u : 0u;
-            sp.apply_pending = (stdp && !first_step) ? 1u : 0u;
-            sp.v_in = V_[in]; sp.v_out = V_[out];
-            sp.spk_in = SPK_[in]; sp.spk_out = SPK_[out];
-            sp.t_in = T_[in]; sp.t_out = T_[out];
-            if (lft_pp) { sp.lft_in = LFT_[lft_loc_]; sp.lft_out = LFT_[lft_loc_ ^ 1]; }
-            else { sp.lft_in = LFT_[lft_loc_]; sp.lft_out = LFT_[lft_loc_]; }
-            sp.grid_hist = want_grid ? d_grid + s * n_neurons : nullptr;
-            sp.spike_hist = want_spk ? d_spk + s * n_words : nullptr;
-            sp.out_par = (uint32_t)out;
-            sp.halo_epoch = halo_nowait ? 0ull : halo_epoch_;   // timing experiment only (SNN_B200_HALO_NOWAIT): results are wrong
-            if (!local_peers_.empty()) wait_local_peers_launched(halo_epoch_, rmod_part);
-            // spike-train parameters of this timestep (the trains step after the neurons, with their own clocks)
-            auto fill_train_step = [&](uint64_t step_in_chunk) {
-                tp.v_in = V_[in]; tp.v_out = V_[out]; tp.spk_in = SPK_[in]; tp.spk_out = SPK_[out];
-                tp.t_in = T_[in]; tp.t_out = T_[out];
-                tp.lft_in = sp.lft_in; tp.lft_out = sp.lft_out;
-                tp.n_tl = 0;
-                for (auto &L : lats_)
-                    if (L.is_train) { tp.tl_base[tp.n_tl] = (uint32_t)L.off; tp.tl_clock[tp.n_tl] = (uint32_t)L.clock; tp.n_tl++; }
-                tp.tl_base[tp.n_tl] = (uint32_t)n_trains;
-                tp.draw = train_draws++;
-                tp.grid_hist = want_tgrid ? d_tgrid + step_in_chunk * n_trains : nullptr;
-                tp.spike_hist = want_tspk ? d_tspk + step_in_chunk * t_words : nullptr;
-            };
-            // two-pass wide kernels: the spike trains ride in extra CTAs of the sum pass (nothing in that pass reads train state; the
-            // terms pass, which does, has completed) — one launch and one launch gap less per timestep
-            const bool trains_fused = n_neurons && !win_ok && !tma_ok && wide && wide_split && n_trains > 0;
-            if (trains_fused) fill_train_step(s);
-            if (n_neurons && win_ok) {
-                cudaError_t e = launch_step_win(sp, win, model, chemg, ntrel, stdp, win_grid, stream_);
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_step_win"); break; }
-                n_launch++;
-            } else if (n_neurons && tma_ok) {
-                tma.st[tma_iv].src = (const unsigned char *)(sp.v_in + own0_);
-                if (tma_il >= 0) tma.st[tma_il].src = (const unsigned char *)(sp.lft_in + own0_);
-                for (int ty = 0; ty < kNT; ++ty)
-                    if (tma_it[ty] >= 0) tma.st[tma_it[ty]].src = (const unsigned char *)(sp.t_in + (size_t)ty * node_cap_ + own0_);
-                cudaError_t e = launch_step_tma(sp, tma, model, chemg, ntrel, stdp, tma_grid, stream_);
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_step_tma"); break; }
-                n_launch++;
-            } else if (n_neurons) {
-                cudaError_t e = wide ? launch_step_wide(sp, model, chemg, ntrel, stdp, net, wide_split ? wide_scratch_ : nullptr, wide_chunks_cap, trains_fused ? &tp : nullptr, stream_)
-                                     : launch_step(sp, model, chemg, ntrel, stdp, net, stream_);
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_step"); break; }
-                n_launch += (wide && wide_split) ? 2 : 1;   // terms pass + sum pass
-            }
-            if (reward_mode && rewards) {
-                // RewardModulatedSTDP::update, plasticity/mod.rs:193-195 (run_lattice_with_reward, neuron/mod.rs:3160-3172)
-                rstdp.dopamine = rstdp.dopamine * expf(-rstdp.dt / rstdp.tau_d) + rstdp.tau_d * rewards[done + s];
-            }
-            if (net_reward) {
-                // RewardModulatedLatticeNetwork::run_lattices_with_reward (neuron/mod.rs:5280-5297): every reward-modulated lattice's
-                // modulator takes the reward before iterate; then post_neuron_update_step's pass over their rows
-                int kn = 0;
-                for (auto &L : lats_) {
-                    if (L.is_train) continue;
-                    if (L.is_reward && rewards) L.rstdp.dopamine = L.rstdp.dopamine * expf(-L.rstdp.dt / L.rstdp.tau_d) + L.rstdp.tau_d * rewards[done + s];
-                    rnp.lat[kn++].dopamine = L.rstdp.dopamine;
-                }
-                if (net_rmod) {
-                    cudaError_t e = launch_rstdp_net_edges(sp, rnp, stream_);
-                    if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_rstdp_net_edges"); break; }
-                    n_launch++;
-                }
-            }
-            if (bcm_on) {
-                cudaError_t e = launch_bcm_edges(sp, BcmParams{bcm.decay, bcm.average_scalar, bcm.dt}, stream_);
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_bcm_edges"); break; }
-                n_launch++;
-            }
-            if (rmod) {
-                rsp.dopamine = rstdp.dopamine;
-                StepParams ep = sp;
-                if (rmod_part) {
-                    // the kernel needs the neighbours' step-s exports (their last_firing_time of this step in my ghost slots)
-                    for (int d = 0; d < 2; ++d) ep.halo[d].my_flag = halo_dir_[d].my_flag;
-                    ep.halo_epoch = halo_epoch_ + 1;
-                }
-                if (rmod_part && !local_peers_.empty()) {
-                    launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);   // my step kernel of this timestep is in the queue
-                    wait_local_peers_launched(halo_epoch_ + 1, false);
-                }
-                cudaError_t e = launch_rstdp_edges(ep, rsp, stream_);
-                if (rmod_part) launched_pub2_.store(halo_epoch_ + 1, std::memory_order_release);
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_rstdp_edges"); break; }
-                n_launch++;
-            }
-            if (part_world > 1) { halo_epoch_ += 1; launched_pub_.store(halo_epoch_, std::memory_order_release); }
-            // LatticeNetwork::iterate: clock += 1, then the spike trains step with their own clocks
-            // (neuron/mod.rs:2582-2591)
-            if (n_trains) {
-                if (!trains_fused) {
-                    fill_train_step(s);
-                    cudaError_t e = launch_trains(tp, stream_);
-                    if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_trains"); break; }
-                    n_launch++;
-                }
-                for (auto &L : lats_) if (L.is_train) L.clock += 1;
-            }
-            if (ghist_on && (is_network || !stdp || sp.apply_pending)) {
-                cudaError_t e = record_graph();
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record"); break; }
-            }
-            internal_clock += 1;
-            cur_ = out;
-            if (lft_pp) lft_loc_ ^= 1;
-            first_step = false;
+        MultiParams mp{};
+        mp.steps = (uint32_t)k; mp.first_pending = (first_chunk && s0 == 0) ? 0u : 1u;
+        mp.cur = (uint32_t)cur_; mp.lft_loc = (uint32_t)lft_loc_; mp.lft_pp = pl.lft_pp ? 1u : 0u;
+        mp.train_sync = (pl.stdp && n_trains) ? 1u : 0u;
+        for (int q = 0; q < 2; ++q) { mp.v[q] = V_[q]; mp.lft[q] = LFT_[q]; mp.spk[q] = SPK_[q]; mp.t[q] = T_[q]; }
+        hist.point(mp, s0);
+        mp.n_neurons = n_neurons; mp.n_words = hist.n_words; mp.n_trains = n_trains; mp.t_words = hist.t_words;
+        mp.barrier = multi_barrier_;
+        mp.cache_rows = !pl.stdp ? 1u : 0u;
+        mp.wide_stage = (wide && n_nodes_ <= 4096) ? 1u : 0u;
+        cudaError_t e = cudaMemsetAsync(multi_barrier_, 0, sizeof(unsigned int), stream_);
+        if (e == cudaSuccess) e = launch_step_multi(sp, tp, mp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, wide, device, false, stream_);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_step_multi");
+        a.launches++;
+        // the host mirrors what the launch did to the ping-pong state and the clocks
+        internal_clock += k;
+        if (k & 1ull) { cur_ ^= 1; if (pl.lft_pp) lft_loc_ ^= 1; }
+        if (n_trains) { train_draws += k; for (auto &L : lats_) if (L.is_train) L.clock += k; }
+        s0 += k;
+    }
+    return SNN_OK;
+}
+
+// Timestep s of the chunk: the step kernel, the per-edge plasticity pass, the spike trains and the graph record, in the order
+// the reference applies them.  The host-side launch publications of in-process strips keep this order (wait_local_peers_launched).
+int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t s, bool first, const float *reward) {
+    StepParams &sp = a.sp;
+    TrainParams &tp = a.tp;
+    const int in = cur_, out = cur_ ^ 1;
+    sp.clock = (uint32_t)internal_clock;
+    // window kernel: sweep the tiles back to front every other step (the tail the previous step left in L2 is read first)
+    sp.reverse = (internal_clock & 1ull) ? 1u : 0u;
+    sp.apply_pending = (pl.stdp && !first) ? 1u : 0u;
+    sp.v_in = V_[in]; sp.v_out = V_[out];
+    sp.spk_in = SPK_[in]; sp.spk_out = SPK_[out];
+    sp.t_in = T_[in]; sp.t_out = T_[out];
+    sp.lft_in = LFT_[lft_loc_]; sp.lft_out = LFT_[pl.lft_pp ? lft_loc_ ^ 1 : lft_loc_];
+    hist.point(sp, s);
+    sp.out_par = (uint32_t)out;
+    sp.halo_epoch = halo_epoch_;
+    if (!local_peers_.empty()) wait_local_peers_launched(halo_epoch_, pl.rmod_part);
+    // spike-train parameters of this timestep (the trains step after the neurons, with their own clocks)
+    auto fill_train_step = [&]() {
+        tp.v_in = V_[in]; tp.v_out = V_[out]; tp.spk_in = SPK_[in]; tp.spk_out = SPK_[out];
+        tp.t_in = T_[in]; tp.t_out = T_[out];
+        tp.lft_in = sp.lft_in; tp.lft_out = sp.lft_out;
+        fill_train_clocks(tp);
+        tp.draw = train_draws++;
+        hist.point(tp, s);
+    };
+    if (pl.trains_fused) fill_train_step();
+    if (n_neurons) {
+        cudaError_t e = cudaSuccess;
+        const char *what = "launch_step";
+        switch (pl.path) {
+        case StepPath::Win:
+            e = launch_step_win(sp, a.win, model, pl.chemg, pl.ntrel, pl.stdp, pl.grid, stream_);
+            what = "launch_step_win";
+            break;
+        case StepPath::Tma:
+            a.tma.st[pl.tma_iv].src = (const unsigned char *)(sp.v_in + own0_);
+            if (pl.tma_il >= 0) a.tma.st[pl.tma_il].src = (const unsigned char *)(sp.lft_in + own0_);
+            for (int ty = 0; ty < kNT; ++ty)
+                if (pl.tma_it[ty] >= 0) a.tma.st[pl.tma_it[ty]].src = (const unsigned char *)(sp.t_in + (size_t)ty * node_cap_ + own0_);
+            e = launch_step_tma(sp, a.tma, model, pl.chemg, pl.ntrel, pl.stdp, pl.grid, stream_);
+            what = "launch_step_tma";
+            break;
+        case StepPath::Wide:
+            e = launch_step_wide(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, nullptr, 0u, nullptr, stream_);
+            break;
+        case StepPath::WideSplit:
+            e = launch_step_wide(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, wide_scratch_, pl.wide_chunks_cap,
+                                 pl.trains_fused ? &tp : nullptr, stream_);
+            break;
+        case StepPath::General:
+            e = launch_step(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, stream_);
+            break;
         }
-        if (status != SNN_OK) break;
-        done += steps;
-        if (done == iterations && stdp) {
-            // the last step's STDP is still pending: apply it now so that weights are final at the API boundary
-            StepParams fp = sp;
-            fp.clock = (uint32_t)internal_clock;
-            fp.lft_in = LFT_[lft_loc_];
-            fp.lft_out = LFT_[lft_loc_ ^ 1];  // spike trains: last_firing_time from before their last iterate
-            fp.halo_epoch = halo_epoch_;
-            if (!local_peers_.empty()) wait_local_peers_launched(halo_epoch_, false);
-            cudaError_t e = launch_flush_stdp(fp, stream_);
-            if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "flush_stdp"); break; }
-            n_launch++;
-            if (ghist_on && !is_network) {
-                e = record_graph();
-                if (e != cudaSuccess) { bail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record"); break; }
-            }
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, what);
+        a.launches += pl.path == StepPath::WideSplit ? 2 : 1;   // terms pass + sum pass
+    }
+    if (reward_mode && reward) {
+        // RewardModulatedSTDP::update, plasticity/mod.rs:193-195 (run_lattice_with_reward, neuron/mod.rs:3160-3172)
+        rstdp.dopamine = rstdp.dopamine * expf(-rstdp.dt / rstdp.tau_d) + rstdp.tau_d * *reward;
+    }
+    if (pl.net_reward) {
+        // RewardModulatedLatticeNetwork::run_lattices_with_reward (neuron/mod.rs:5280-5297): every reward-modulated lattice's
+        // modulator takes the reward before iterate; then post_neuron_update_step's pass over their rows
+        int kn = 0;
+        for (auto &L : lats_) {
+            if (L.is_train) continue;
+            if (L.is_reward && reward) L.rstdp.dopamine = L.rstdp.dopamine * expf(-L.rstdp.dt / L.rstdp.tau_d) + L.rstdp.tau_d * *reward;
+            a.rnp.lat[kn++].dopamine = L.rstdp.dopamine;
         }
-        cudaEventRecord(ev1_, stream_);
-        const auto host_t1 = std::chrono::steady_clock::now();
-        cudaError_t e = cudaStreamSynchronize(stream_);
-        if (e != cudaSuccess) { bail(e, SNN_GPU_WAIT_ERROR, "cudaStreamSynchronize(step loop)"); break; }
-        if (dbg_timing && !dbg_ev.empty()) {
-            fprintf(stderr, "[snn] per-step device us:");
-            for (size_t k = 0; k < dbg_ev.size(); ++k) {
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, dbg_ev[k], k + 1 < dbg_ev.size() ? dbg_ev[k + 1] : ev1_);
-                fprintf(stderr, " %.0f", ms * 1e3f);
-                cudaEventDestroy(dbg_ev[k]);
-            }
-            fprintf(stderr, "\n");
-            if (dbg_clk) {
-                unsigned long long h[32 * 4];
-                cudaMemcpy(h, dbg_clk, sizeof h, cudaMemcpyDeviceToHost);
-                fprintf(stderr, "[snn] effective SM MHz of CTA 0 per step:");
-                for (uint64_t k = 0; k < steps; ++k)
-                    if (h[4 * k + 3] > h[4 * k + 1]) fprintf(stderr, " %.0f", (double)(h[4 * k + 2] - h[4 * k]) * 1e3 / (double)(h[4 * k + 3] - h[4 * k + 1]));
-                fprintf(stderr, "\n");
-                cudaFree(dbg_clk);
-            }
-        }
-        sp.dbg = nullptr;
-        if (dbg_timing) {
-            const auto host_t2 = std::chrono::steady_clock::now();
-            fprintf(stderr, "[snn] %llu steps: enqueue %.1f us/step on the host, then waited %.1f us/step\n", (unsigned long long)steps,
-                    std::chrono::duration<double, std::micro>(host_t1 - host_t0).count() / steps,
-                    std::chrono::duration<double, std::micro>(host_t2 - host_t1).count() / steps);
-        }
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, ev0_, ev1_);
-        total_ms += ms;
-        // drain the graph records: each requested block's weights cut out of the canonical order
-        if (ghist_on && gh_recs) {
-            const uint64_t nz = ghist_nnz_;
-            if (nz && gh_plans.size() == 1 && gh_plans[0].whole) {
-                std::vector<float> &w = gh_plans[0].h->w;   // straight into the block's record vector
-                const size_t o = w.size();
-                w.resize(o + gh_recs * nz);
-                e = cudaMemcpy(w.data() + o, d_ghist, gh_recs * nz * 4, cudaMemcpyDeviceToHost);
-            } else if (nz) {
-                std::vector<float> hr(gh_recs * nz);
-                e = cudaMemcpy(hr.data(), d_ghist, hr.size() * 4, cudaMemcpyDeviceToHost);
-                for (auto &pl : gh_plans) {
-                    if (e != cudaSuccess || pl.h->nnz == 0) continue;
-                    std::vector<float> &w = pl.h->w;
-                    for (uint64_t k = 0; k < gh_recs; ++k) {
-                        const float *rec = hr.data() + k * nz;
-                        if (pl.whole) { w.insert(w.end(), rec, rec + nz); continue; }
-                        const size_t o = w.size();
-                        w.resize(o + pl.h->nnz);
-                        const uint64_t n_post = pl.src.size();
-                        for (uint64_t q = 0; q < n_post; ++q) {
-                            const uint64_t a = pl.b->row_ptr[q], c = pl.b->row_ptr[q + 1] - a;
-                            if (c) memcpy(w.data() + o + a, rec + pl.src[q], c * 4);
-                        }
-                    }
-                }
-            }
-            if (e != cudaSuccess) { bail(e, SNN_GPU_BUFFER_READ_ERROR, "graph history drain"); break; }
-            for (auto &pl : gh_plans) pl.h->steps += gh_recs;
-            gh_recs = 0;
-        }
-        // drain histories
-        if (per_step_bytes) {
-            std::vector<float> hg, htg; std::vector<uint32_t> hs, hts;
-            cudaError_t he = cudaSuccess;
-            if (copy_grid) { hg.resize(steps * n_neurons); he = cudaMemcpy(hg.data(), d_grid, hg.size() * 4, cudaMemcpyDeviceToHost); }
-            if (he != cudaSuccess) { bail(he, SNN_GPU_BUFFER_READ_ERROR, "grid history drain"); break; }
-            if (want_red) {
-                const size_t nl = red_lats.size();
-                cudaError_t re = launch_history_reduce(d_grid, n_neurons, (uint32_t)steps, d_red_lat, d_red_lat + nl,
-                                                       (const float *)(d_red_lat + 2 * nl), (int)nl, d_red, stream_);
-                std::vector<double> hr(steps * nl * 2);
-                // stream_ is non-blocking: a copy on the legacy stream would not wait for the reduction
-                if (re == cudaSuccess) re = cudaMemcpyAsync(hr.data(), d_red, hr.size() * 8, cudaMemcpyDeviceToHost, stream_);
-                if (re == cudaSuccess) re = cudaStreamSynchronize(stream_);
-                if (re != cudaSuccess) { bail(re, SNN_GPU_BUFFER_READ_ERROR, "history reduce"); break; }
-                for (size_t k = 0; k < nl; ++k) {
-                    Lat &L = *red_lats[k];
-                    for (uint64_t s = 0; s < steps; ++s) {
-                        const double sum_v = hr[(s * nl + k) * 2], sum_dv = hr[(s * nl + k) * 2 + 1];
-                        // AverageVoltageHistory::update, neuron/mod.rs:310-316: sum / len as f32
-                        if (L.avg_hist) L.average_history.push_back((float)sum_v / (float)L.n);
-                        // EEGHistory::update, neuron/mod.rs:266-279: (1 / (4 pi sigma d)) * total_current
-                        if (L.eeg_hist) L.eeg_history.push_back((1.f / (4.f * 3.14159274101257324f * L.eeg_cond * L.eeg_dist)) * (float)sum_dv);
-                    }
-                    if (!L.grid_hist && !L.spike_hist) L.hist_len += steps;
-                }
-            }
-            if (want_spk) { hs.resize(steps * n_words); he = cudaMemcpy(hs.data(), d_spk, hs.size() * 4, cudaMemcpyDeviceToHost); }
-            if (he == cudaSuccess && want_tgrid) { htg.resize(steps * n_trains); he = cudaMemcpy(htg.data(), d_tgrid, htg.size() * 4, cudaMemcpyDeviceToHost); }
-            if (he == cudaSuccess && want_tspk) { hts.resize(steps * t_words); he = cudaMemcpy(hts.data(), d_tspk, hts.size() * 4, cudaMemcpyDeviceToHost); }
-            if (he != cudaSuccess) { bail(he, SNN_GPU_BUFFER_READ_ERROR, "history drain"); break; }
-            // SpikeHistory::aggregate (neuron/mod.rs:335-359): the sum over the chunk's steps is taken on the device from the
-            // staged raster; the host only adds one count per neuron and chunk
-            std::vector<uint32_t> cnt_n, cnt_t;
-            for (int dom = 0; dom < 2 && he == cudaSuccess; ++dom) {
-                const bool on = dom ? want_tspk : want_spk;
-                const uint64_t dn = dom ? n_trains : n_neurons, dw = dom ? t_words : n_words;
-                if (!on || dn == 0) continue;
-                std::vector<uint32_t> &cnt = dom ? cnt_t : cnt_n;
-                cnt.resize(dn);
-                if (ensure_scratch(dn * 4)) { he = cudaErrorMemoryAllocation; break; }
-                he = launch_spike_count(dom ? d_tspk : d_spk, (uint32_t)steps, dw, dn, (uint32_t *)scratch_, stream_);
-                if (he == cudaSuccess) he = cudaMemcpyAsync(cnt.data(), scratch_, dn * 4, cudaMemcpyDeviceToHost, stream_);
-                if (he == cudaSuccess) he = cudaStreamSynchronize(stream_);
-            }
-            if (he != cudaSuccess) { bail(he, SNN_GPU_BUFFER_READ_ERROR, "spike aggregate"); break; }
-            for (auto &L : lats_) {
-                if (!L.grid_hist && !L.spike_hist) continue;
-                const uint64_t dom_n = L.is_train ? n_trains : n_neurons, dom_w = L.is_train ? t_words : n_words;
-                const std::vector<float> &G = L.is_train ? htg : hg;
-                const std::vector<uint32_t> &S = L.is_train ? hts : hs;
-                if (L.spike_hist) {
-                    const std::vector<uint32_t> &cnt = L.is_train ? cnt_t : cnt_n;
-                    if (L.spike_agg.size() != L.n) L.spike_agg.assign(L.n, 0);
-                    for (uint64_t j = 0; j < L.n; ++j) L.spike_agg[j] += cnt[L.off + j];
-                }
-                for (uint64_t s = 0; s < steps; ++s) {
-                    if (L.grid_hist) L.grid_history.insert(L.grid_history.end(), G.begin() + s * dom_n + L.off, G.begin() + s * dom_n + L.off + L.n);
-                    if (L.spike_hist) {
-                        const size_t o = L.spike_history.size();
-                        L.spike_history.resize(o + L.n);
-                        for (uint64_t j = 0; j < L.n; ++j) {
-                            const uint64_t b = L.off + j;
-                            L.spike_history[o + j] = (uint8_t)((S[s * dom_w + (b >> 5)] >> (b & 31)) & 1u);
-                        }
-                    }
-                }
-                L.hist_len += steps;
-            }
+        if (pl.net_rmod) {
+            cudaError_t e = launch_rstdp_net_edges(sp, a.rnp, stream_);
+            if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_rstdp_net_edges");
+            a.launches++;
         }
     }
-    free_hist();
-    if (status != SNN_OK) return status;
-    if (part_world > 1) {
-        if (getenv("SNN_DEBUG_HALO")) {
-            unsigned int d[8];
-            cudaMemcpy(d, halo_done_, sizeof d, cudaMemcpyDeviceToHost);
-            fprintf(stderr, "[snn rank %d] %llu steps: %u halo waits spun, %.1f us waited in total (%.2f us per step)\n", part_rank,
-                    (unsigned long long)iterations, d[5], d[4] * 16e-3, d[4] * 16e-3 / (double)iterations);
-            cudaMemsetAsync(halo_done_ + 4, 0, 8, stream_);
-            cudaStreamSynchronize(stream_);
+    if (pl.bcm_on) {
+        cudaError_t e = launch_bcm_edges(sp, BcmParams{bcm.decay, bcm.average_scalar, bcm.dt}, stream_);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_bcm_edges");
+        a.launches++;
+    }
+    if (pl.rmod) {
+        a.rsp.dopamine = rstdp.dopamine;
+        StepParams ep = sp;
+        if (pl.rmod_part) {
+            // the kernel needs the neighbours' step-s exports (their last_firing_time of this step in my ghost slots)
+            for (int d = 0; d < 2; ++d) ep.halo[d].my_flag = halo_dir_[d].my_flag;
+            ep.halo_epoch = halo_epoch_ + 1;
         }
+        if (pl.rmod_part && !local_peers_.empty()) {
+            launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);   // my step kernel of this timestep is in the queue
+            wait_local_peers_launched(halo_epoch_ + 1, false);
+        }
+        cudaError_t e = launch_rstdp_edges(ep, a.rsp, stream_);
+        if (pl.rmod_part) launched_pub2_.store(halo_epoch_ + 1, std::memory_order_release);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_rstdp_edges");
+        a.launches++;
+    }
+    if (part_world > 1) { halo_epoch_ += 1; launched_pub_.store(halo_epoch_, std::memory_order_release); }
+    // LatticeNetwork::iterate: clock += 1, then the spike trains step with their own clocks (neuron/mod.rs:2582-2591)
+    if (n_trains) {
+        if (!pl.trains_fused) {
+            fill_train_step();
+            cudaError_t e = launch_trains(tp, stream_);
+            if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_trains");
+            a.launches++;
+        }
+        for (auto &L : lats_) if (L.is_train) L.clock += 1;
+    }
+    if (pl.ghist_on && (is_network || !pl.stdp || sp.apply_pending)) {
+        cudaError_t e = hist.record_graph(a.launches);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record");
+    }
+    internal_clock += 1;
+    cur_ = out;
+    if (pl.lft_pp) lft_loc_ ^= 1;
+    return SNN_OK;
+}
+
+// The last step's STDP is still pending after the last step kernel: apply it so that weights are final at the API boundary.
+int Engine::flush_stdp(const RunPlan &pl, LaunchArgs &a, HistStage &hist) {
+    StepParams fp = a.sp;
+    fp.clock = (uint32_t)internal_clock;
+    fp.lft_in = LFT_[lft_loc_];
+    fp.lft_out = LFT_[lft_loc_ ^ 1];  // spike trains: last_firing_time from before their last iterate
+    fp.halo_epoch = halo_epoch_;
+    if (!local_peers_.empty()) wait_local_peers_launched(halo_epoch_, false);
+    cudaError_t e = launch_flush_stdp(fp, stream_);
+    if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "flush_stdp");
+    a.launches++;
+    if (pl.ghist_on && !is_network) {
+        e = hist.record_graph(a.launches);
+        if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record");
+    }
+    return SNN_OK;
+}
+
+// After the last step: a neighbour's halo time-out, and the derived fields (receptor currents, HH gate rates / channel currents)
+// from the retained pre-update V.
+int Engine::finish_run(const RunPlan &pl, const StepParams &sp) {
+    if (part_world > 1) {
         unsigned int err = 0;
         CK(cudaMemcpy(&err, halo_done_ + 2, 4, cudaMemcpyDeviceToHost), SNN_GPU_BUFFER_READ_ERROR);
         if (err) {
@@ -2783,16 +2777,53 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
             return fail(SNN_GPU_WAIT_ERROR, "timed out waiting for a neighbouring strip's halo (is every rank running the same number of steps?)");
         }
     }
-    if (stdp || rmod || net_rmod || bcm_on) dev_weights_newer_ = true;
-    // derived fields (receptor currents, HH gate rates / channel currents) from the retained pre-update V
+    if (pl.stdp || pl.rmod || pl.net_rmod || pl.bcm_on) dev_weights_newer_ = true;
     if ((chemical && chem_alloc_) || model == SNN_MODEL_HODGKIN_HUXLEY) {
         StepParams fp = sp;
         fp.chemical = chemical && chem_alloc_;
         CK(launch_finalize(fp, model, V_[cur_ ^ 1], stream_), SNN_GPU_QUEUE_FAILURE);
         CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
     }
-    if (elapsed_ms) *elapsed_ms = total_ms;
-    if (launches) *launches = n_launch;
+    return SNN_OK;
+}
+
+int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, const float *rewards) {
+    if (elapsed_ms) *elapsed_ms = 0.f;
+    if (launches) *launches = 0;
+    // gpu_lattices/mod.rs:1089-1091: empty lattice or zero iterations -> Ok(()); neuron/mod.rs:1217: both flags off -> Ok(())
+    if (iterations == 0 || (n_neurons == 0 && n_trains == 0)) return SNN_OK;
+    if (!electrical && !chemical) return SNN_OK;
+    if (internal_clock + iterations > 0x7FFFFFF0ull) return fail(SNN_UNSUPPORTED, "internal clock would overflow the i32 last_firing_time");
+    RunPlan pl;
+    LaunchArgs a;
+    int r = plan_run(pl, a);
+    if (r) return r;
+    {
+        HistStage hist(*this, pl);
+        r = hist.init(iterations);
+        if (!r && part_world > 1) r = halo_rendezvous(a.sp, a.launches);
+        for (uint64_t done = 0; !r && done < iterations;) {
+            const uint64_t steps = std::min(hist.chunk, iterations - done);
+            cudaEventRecord(ev0_, stream_);
+            if (pl.multi) r = run_multi_chunk(pl, a, hist, steps, done == 0);
+            for (uint64_t s = 0; !pl.multi && !r && s < steps; ++s)
+                r = run_step(pl, a, hist, s, done == 0 && s == 0, rewards ? rewards + done + s : nullptr);
+            done += steps;
+            if (!r && done == iterations && pl.stdp) r = flush_stdp(pl, a, hist);
+            if (r) break;
+            cudaEventRecord(ev1_, stream_);
+            cudaError_t e = cudaStreamSynchronize(stream_);
+            if (e != cudaSuccess) { r = cuda_fail(e, SNN_GPU_WAIT_ERROR, "cudaStreamSynchronize(step loop)"); break; }
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, ev0_, ev1_);
+            a.total_ms += ms;
+            r = hist.drain(steps);
+        }
+    }   // the history staging buffers are freed here
+    if (!r) r = finish_run(pl, a.sp);
+    if (r) return r;
+    if (elapsed_ms) *elapsed_ms = a.total_ms;
+    if (launches) *launches = a.launches;
     return SNN_OK;
 }
 

@@ -167,7 +167,6 @@ public:
     uint32_t steps_per_graph = 0;
     bool force_gpart = false;           // SNN_OPT_GENERAL_PARTITION: CSR graphs of a partitioned handle always use gather-list ghosts
     uint64_t halo_timeout_ms = 30000;   // multi-GPU: how long a step may wait for a neighbouring strip before SNN_GPU_WAIT_ERROR
-    int use_tma = -1;   // -1 auto (env SNN_B200_TMA), 0 never, 1 whenever eligible
     std::string last_error;
 
     int model, ntk, rck, train_kind, refract, device;
@@ -214,12 +213,15 @@ private:
     uint32_t *slice_off_ = nullptr, *col_ = nullptr; float *wgt_ = nullptr;
     // TraceRSTDP members next to wgt_ (same sliced-ELL positions), allocated on the first reward-modulated run
     uint8_t *rs_counter_ = nullptr; float *rs_dw_ = nullptr, *rs_c_ = nullptr; uint64_t rs_elems_ = 0;
-    float *rnet_tab_ = nullptr; size_t rnet_tab_elems_ = 0;   // per-lattice difference tables of a reward-modulated network (RnetParams::tab)
-    float *rs_tab_ = nullptr; uint32_t rs_tab_n_ = 0;   // difference table of the reward-modulated STDP term (RstdpParams::tab)
+    // difference tables of the STDP term (RstdpParams::tab of a reward-modulated lattice, RnetParams::tab of a network)
+    float *stdp_tab_ = nullptr; size_t stdp_tab_elems_ = 0;
+    int build_stdp_tables(const std::vector<RstdpParams> &lat, const float **tab, uint32_t *tab_n);
+    int build_rnet_params(RnetParams &rnp, bool *net_rmod);
     bool rs_canonical_ = true;   // counter == 0 and dw == 0 on every edge (TraceRSTDP::default, kept by two calls per timestep)
     int ensure_reward_arrays();
     void free_reward_arrays();
     uint64_t sell_krows_ = 0, sell_alloc_krows_ = 0; uint32_t n_slices_ = 0, uniform_width_ = 0;
+    uint32_t max_slice_width_ = 0;   // widest slice of the table, in k-rows
     // halo
     unsigned long long *flags_ = nullptr;  // [0] arrivals from rank-1, [1] arrivals from rank+1
     unsigned int *halo_done_ = nullptr;
@@ -257,7 +259,6 @@ private:
     std::map<std::pair<uint64_t, uint64_t>, GraphHist> graph_hist_;
     uint32_t *ghist_row_off_ = nullptr;
     uint64_t ghist_nnz_ = 0;
-    uint32_t ghist_max_width_ = 0;   // widest slice of the table, in k-rows
     bool ghist_off_valid_ = false;
     int refuse_if_graph_history(const char *what);
 
@@ -276,6 +277,7 @@ private:
     int relayout_add(const Lat &nl);
     void compute_layout();
     uint32_t node_off(const Lat &L) const { return (L.is_train ? train0_ : own0_) + (uint32_t)L.off; }
+    int n_neuron_lattices() const { int n = 0; for (auto &L : lats_) n += !L.is_train; return n; }
     int lookup_field(const Lat &L, const char *name, FieldDef *out) const;
     int field_io(Lat &L, const FieldDef &fd, void *data, uint64_t count, bool set);
     int set_bits(uint32_t *words, const uint32_t *host_u32, uint64_t n, uint64_t bit0);
@@ -291,9 +293,23 @@ private:
     mutable bool flags_cache_valid_ = false;
     mutable uint32_t nt_used_ = 0, rc_used_ = 0;
     void fill_step_params(StepParams &p);
+    void fill_train_clocks(TrainParams &tp) const;
     int upload_lat_table();
-    bool build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp, unsigned *grid);
-    bool build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, unsigned *grid);
+    // mode (SNN_B200_TMA): 0 not eligible, 1 lattices of at least 64 Ki neurons, 2 any size
+    bool build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid);
+    bool build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid);
+
+    // run(), phase by phase (engine.cu)
+    struct RunPlan;      // decisions fixed for the whole run
+    struct LaunchArgs;   // kernel parameter blocks and launch count
+    struct HistStage;    // device staging of the recorded histories
+    int plan_run(RunPlan &pl, LaunchArgs &a);
+    int plan_step_path(RunPlan &pl, LaunchArgs &a);
+    int halo_rendezvous(const StepParams &sp, uint64_t &launches);
+    int run_multi_chunk(const RunPlan &pl, LaunchArgs &a, const HistStage &hist, uint64_t steps, bool first_chunk);
+    int run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t s, bool first, const float *reward);
+    int flush_stdp(const RunPlan &pl, LaunchArgs &a, HistStage &hist);
+    int finish_run(const RunPlan &pl, const StepParams &sp);
 };
 
 }  // namespace snn

@@ -596,12 +596,11 @@ template <int MODEL, int CHEMG, bool NTREL, bool NET>
 static cudaError_t launch_step_3(const StepParams &p, bool stdp, cudaStream_t s) {
     const unsigned grid = blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256);
     if constexpr (NET && !NTREL && MODEL != SNN_MODEL_HODGKIN_HUXLEY) {
-        if (stdp) return launch_pdl<PDL_STEP>(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, true>, dim3(grid), dim3(256), 0, s, p);
-        return launch_pdl<PDL_STEP>(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, false>, dim3(grid), dim3(256), 0, s, p);
+        if (stdp) return launch_pdl(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, true>, dim3(grid), dim3(256), 0, s, p);
+        return launch_pdl(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, false>, dim3(grid), dim3(256), 0, s, p);
     }
-    if (stdp) return launch_pdl<PDL_STEP>(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, true, NET>, dim3(grid), dim3(256), 0, s, p);
-    return launch_pdl<PDL_STEP>(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, false, NET>, dim3(grid), dim3(256), 0, s, p);
-    return cudaGetLastError();
+    if (stdp) return launch_pdl(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, true, NET>, dim3(grid), dim3(256), 0, s, p);
+    return launch_pdl(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, false, NET>, dim3(grid), dim3(256), 0, s, p);
 }
 
 template <int MODEL>
@@ -636,8 +635,7 @@ cudaError_t launch_step(const StepParams &p, int model, int chemg, bool ntrel, b
 
 cudaError_t launch_trains(const TrainParams &p, cudaStream_t s) {
     if (p.n_trains == 0) return cudaSuccess;
-    return launch_pdl<PDL_TRAINS>(pdl_ok(p), train_kernel, dim3(blocks_for((uint64_t)((p.n_trains + 31u) / 32u) * 32u, 256)), dim3(256), 0, s, p);
-    return cudaGetLastError();
+    return launch_pdl(pdl_ok(p), train_kernel, dim3(blocks_for((uint64_t)((p.n_trains + 31u) / 32u) * 32u, 256)), dim3(256), 0, s, p);
 }
 
 cudaError_t launch_halo_push(const StepParams &p, cudaStream_t s) {
@@ -655,8 +653,7 @@ cudaError_t launch_gpart_push(const StepParams &p, cudaStream_t s) {
 
 cudaError_t launch_bcm_edges(const StepParams &p, const BcmParams &b, cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
-    return launch_pdl<PDL_EDGES>(pdl_ok(p), bcm_edge_kernel, dim3(blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256)), dim3(256), 0, s, p, b);
-    return cudaGetLastError();
+    return launch_pdl(false, bcm_edge_kernel, dim3(blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256)), dim3(256), 0, s, p, b);
 }
 
 cudaError_t launch_rstdp_edges(const StepParams &p, const RstdpParams &r, cudaStream_t s) {
@@ -665,18 +662,17 @@ cudaError_t launch_rstdp_edges(const StepParams &p, const RstdpParams &r, cudaSt
     const unsigned grid = (n_slices + kRsSlices - 1) / kRsSlices;
     // the table stands for the formula while every spike time is exact in f32 (clock < 2^24)
     const bool tab = r.tab != nullptr && p.clock < (1u << 24);
-    static const bool pipe_env = !(getenv("SNN_B200_RSTDP_PIPE") && atoi(getenv("SNN_B200_RSTDP_PIPE")) == 0);
-    if (pipe_env && p.uniform_width == 8u && !(p.halo[0].active | p.halo[1].active) && grid > 512u) {
+    if (p.uniform_width == 8u && !(p.halo[0].active | p.halo[1].active) && grid > 512u) {
         // whole lattices with radius-1 stencil tables, large enough to fill the persistent grid
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         const unsigned pg = (unsigned)sms * (unsigned)SNN_RS_CTAS;
-        if (r.canonical) return tab ? launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge8_kernel<true, true>, dim3(pg), dim3(256), 0, s, p, r) : launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge8_kernel<true, false>, dim3(pg), dim3(256), 0, s, p, r);
-        return tab ? launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge8_kernel<false, true>, dim3(pg), dim3(256), 0, s, p, r) : launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge8_kernel<false, false>, dim3(pg), dim3(256), 0, s, p, r);
+        if (r.canonical) return tab ? launch_pdl(false, rstdp_edge8_kernel<true, true>, dim3(pg), dim3(256), 0, s, p, r) : launch_pdl(false, rstdp_edge8_kernel<true, false>, dim3(pg), dim3(256), 0, s, p, r);
+        return tab ? launch_pdl(false, rstdp_edge8_kernel<false, true>, dim3(pg), dim3(256), 0, s, p, r) : launch_pdl(false, rstdp_edge8_kernel<false, false>, dim3(pg), dim3(256), 0, s, p, r);
     }
-    if (r.canonical) return tab ? launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge_kernel<true, true>, dim3(grid), dim3(256), 0, s, p, r) : launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge_kernel<true, false>, dim3(grid), dim3(256), 0, s, p, r);
-    return tab ? launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge_kernel<false, true>, dim3(grid), dim3(256), 0, s, p, r) : launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_edge_kernel<false, false>, dim3(grid), dim3(256), 0, s, p, r);
+    if (r.canonical) return tab ? launch_pdl(false, rstdp_edge_kernel<true, true>, dim3(grid), dim3(256), 0, s, p, r) : launch_pdl(false, rstdp_edge_kernel<true, false>, dim3(grid), dim3(256), 0, s, p, r);
+    return tab ? launch_pdl(false, rstdp_edge_kernel<false, true>, dim3(grid), dim3(256), 0, s, p, r) : launch_pdl(false, rstdp_edge_kernel<false, false>, dim3(grid), dim3(256), 0, s, p, r);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -692,7 +688,8 @@ cudaError_t launch_rstdp_edges(const StepParams &p, const RstdpParams &r, cudaSt
 // Connecting edges OUT of such a lattice are refused by Engine::run (the reference looks them up with swapped end points and
 // panics).  One CTA per 32-row slice, one thread per edge, no ordering between edges.
 // U k-rows per thread and round: all col words first, then the spike-time gathers and trace loads they address, then the
-// arithmetic — U independent chains per thread hide the dependent round trips per edge.  The pass is instruction-bound before it
+// arithmetic — U independent chains per thread hide the dependent round trips per edge.  Only U = 1 is launched: more k-rows per
+// thread lose more in occupancy than they gain in memory-level parallelism (DESIGN.md, 144 / 162 / 199 us for 1 / 2 / 4).  The pass is instruction-bound before it
 // is bandwidth-bound (ncu, profiles/r2_rstdp_net_edge_v2_full.txt: 186 warp instructions per k-row with the exponentials
 // evaluated in place), hence:
 //  - TAB: the STDP term through per-lattice difference tables (RnetParams::tab, filled by rstdp_table_kernel with the very
@@ -799,11 +796,7 @@ __global__ void __launch_bounds__(256) rstdp_net_edge_kernel(const __grid_consta
 
 template <bool CANON, bool TAB>
 static cudaError_t launch_rnet_2(const StepParams &p, const RnetParams &r, cudaStream_t s) {
-    static const int u = getenv("SNN_B200_RNET_U") ? atoi(getenv("SNN_B200_RNET_U")) : 1;
-    const dim3 grid((p.n_neurons + 31u) / 32u);
-    if (u == 2) return launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_net_edge_kernel<CANON, TAB, 2>, grid, dim3(256), 0, s, p, r);
-    if (u == 1) return launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_net_edge_kernel<CANON, TAB, 1>, grid, dim3(256), 0, s, p, r);
-    return launch_pdl<PDL_EDGES>(pdl_ok(p), rstdp_net_edge_kernel<CANON, TAB, 4>, grid, dim3(256), 0, s, p, r);
+    return launch_pdl(false, rstdp_net_edge_kernel<CANON, TAB, 1>, dim3((p.n_neurons + 31u) / 32u), dim3(256), 0, s, p, r);
 }
 
 cudaError_t launch_rstdp_net_edges(const StepParams &p, const RnetParams &r, cudaStream_t s) {

@@ -194,9 +194,8 @@ static cudaError_t launch_multi_5(const StepParams &p, const TrainParams &t, con
     cudaError_t e;
     if constexpr (!WIDE) {
         // small enough for one cluster: every slice (and spike-train warp) gets its own warp in 16 CTAs of 640 threads
-        static const bool cluster_on = !(getenv("SNN_B200_MULTI_CLUSTER") && atoi(getenv("SNN_B200_MULTI_CLUSTER")) == 0);
         const uint32_t warps = kClusterCtas * (kClusterThreads / 32);
-        if (cluster_on && n_slices <= warps && n_twarps <= warps) {
+        if (n_slices <= warps && n_twarps <= warps) {
             auto kc = step_multi_kernel<MODEL, CHEMG, NTREL, STDP, NET, false, true>;
             static thread_local int cluster_ok = -1;   // per instantiation
             if (cluster_ok < 0) {
@@ -212,7 +211,6 @@ static cudaError_t launch_multi_5(const StepParams &p, const TrainParams &t, con
                 }
                 cudaGetLastError();
             }
-            if (getenv("SNN_B200_MULTI_DEBUG") && !dry) fprintf(stderr, "[snn] multi-step launch: cluster path %s (%u slices)\n", cluster_ok == 1 ? "ON" : "unavailable", n_slices);
             if (cluster_ok == 1) {
                 if (dry) return cudaSuccess;
                 cudaLaunchConfig_t cfg{};

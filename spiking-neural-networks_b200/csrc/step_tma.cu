@@ -141,12 +141,12 @@ static cudaError_t launch_tma_3(const StepParams &p, const TmaParams &tp, bool s
         auto k = step_tma_kernel<MODEL, CHEMG, NTREL, true>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        return launch_pdl<PDL_STEP>(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
+        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
     } else {
         auto k = step_tma_kernel<MODEL, CHEMG, NTREL, false>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        return launch_pdl<PDL_STEP>(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
+        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
     }
     return cudaGetLastError();
 }

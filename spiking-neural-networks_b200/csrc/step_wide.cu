@@ -49,7 +49,7 @@ static cudaError_t launch_wide_3(const StepParams &p, bool stdp, unsigned char *
     static const TrainParams no_trains{};
     auto launch = [&](auto k, dim3 g, size_t smem, uint32_t stage, WideSplit sp) -> cudaError_t {
         if (smem > 48u * 1024u) { cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); if (e != cudaSuccess) return e; }
-        return launch_pdl<PDL_STEP>(pdl_ok(p), k, g, dim3(kWideWarps * 32), smem, s, p, stage, sp, (sp.mode == 2u && trains) ? *trains : no_trains);
+        return launch_pdl(pdl_ok(p), k, g, dim3(kWideWarps * 32), smem, s, p, stage, sp, (sp.mode == 2u && trains) ? *trains : no_trains);
     };
     auto both = [&](dim3 g, size_t smem, uint32_t stage, WideSplit sp) -> cudaError_t {
         if (stdp) return launch(step_wide_kernel<MODEL, CHEMG, NTREL, true, NET>, g, smem, stage, sp);
@@ -65,9 +65,8 @@ static cudaError_t launch_wide_3(const StepParams &p, bool stdp, unsigned char *
         return both(dim3(grid + train_ctas, n_acc), kWideSumBufs * (kWideChunk * 32u * 4u + 128u), 0u, WideSplit{2u, scratch, chunks_cap, grid});
     }
     // small networks: the node state rides in shared memory next to the chunk buffers (WideStage, step_body.cuh)
-    static const bool stage_env = !(getenv("SNN_B200_WIDE_STAGE") && atoi(getenv("SNN_B200_WIDE_STAGE")) == 0);
     const uint32_t sb = wide_stage_bytes(p.n_nodes, NET ? p.n_trains : 0u);
-    const bool stage = stage_env && p.n_nodes <= kWideStageMaxNodes && 2u * wide_buf_bytes(CHEMG) + sb <= 200u * 1024u;
+    const bool stage = p.n_nodes <= kWideStageMaxNodes && 2u * wide_buf_bytes(CHEMG) + sb <= 200u * 1024u;
     return both(dim3(grid), 2u * wide_buf_bytes(CHEMG) + (stage ? sb : 0u), stage ? 1u : 0u, WideSplit{0u, nullptr, 0u, grid});
 }
 

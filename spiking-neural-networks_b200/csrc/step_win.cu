@@ -125,10 +125,7 @@ __device__ __forceinline__ uint32_t win_tile_of(const StepParams &p, const WinPa
     return wp.first_lo + (p.reverse ? n_int - 1u - k : k);
 }
 
-#ifndef SNN_WIN_PRODUCERS
-#define SNN_WIN_PRODUCERS 4
-#endif
-constexpr int kWinProducers = SNN_WIN_PRODUCERS;   // producer warps per CTA; together they issue the copies of every tile
+constexpr int kWinProducers = 4;   // producer warps per CTA; together they issue the copies of every tile
 template <int G> constexpr int win_threads() { return (G * 8 + kWinProducers) * 32; }
 
 template <int MODEL, int CHEMG, bool NTREL, bool STDP, int G>
@@ -300,12 +297,12 @@ static cudaError_t launch_win_3(const StepParams &p, const WinParams &wp, bool s
         auto k = step_win_kernel<MODEL, CHEMG, NTREL, true, G>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        return launch_pdl<PDL_STEP>(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
+        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
     } else {
         auto k = step_win_kernel<MODEL, CHEMG, NTREL, false, G>;
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        return launch_pdl<PDL_STEP>(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
+        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
     }
     return cudaGetLastError();
 }

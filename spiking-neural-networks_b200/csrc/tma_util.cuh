@@ -2,16 +2,6 @@
 #pragma once
 #include <cstdint>
 
-#ifndef SNN_WIN_PROD_SLEEP
-#define SNN_WIN_PROD_SLEEP 256   // ns between probes of a producer waiting for a free stage
-#endif
-#ifndef SNN_WIN_CONS_HINT
-#define SNN_WIN_CONS_HINT 0      // ns a consumer's try_wait may stay suspended (0 = no hint)
-#endif
-#ifndef SNN_WIN_PROD_HINT
-#define SNN_WIN_PROD_HINT 0      // ns a producer's try_wait may stay suspended (0 = no hint: probe + nanosleep)
-#endif
-
 namespace snn {
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -25,35 +15,8 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *bar, uint32_t by
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-#ifndef SNN_WIN_CONS_SLEEP
-#define SNN_WIN_CONS_SLEEP 0     // ns a consumer sleeps between probes of a barrier that is not ready (0 = spin)
-#endif
+// consumer-side wait: spin (a sleep or a suspend-time hint changes neither the power draw nor the time, DESIGN.md §2)
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-#if SNN_WIN_CONS_SLEEP
-    uint32_t done = 0;
-    while (true) {
-        asm volatile(
-            "{\n"
-            ".reg .pred P1;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, P1;\n"
-            "}\n" : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(SNN_WIN_CONS_SLEEP);
-    }
-    return;
-#endif
-#if SNN_WIN_CONS_HINT
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1, %2;\n"
-        "@P1 bra DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)SNN_WIN_CONS_HINT) : "memory");
-#else
     asm volatile(
         "{\n"
         ".reg .pred P1;\n"
@@ -63,22 +26,9 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
         "bra WAIT_LOOP;\n"
         "DONE:\n"
         "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-#endif
 }
-// producer-side wait: back off between probes so that the spinning lane does not eat issue slots of the consumers
+// producer-side wait: back off 256 ns between probes so that the spinning lane does not eat issue slots of the consumers
 __device__ __forceinline__ void mbar_wait_backoff(uint64_t *bar, uint32_t parity) {
-#if SNN_WIN_PROD_HINT
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1, %2;\n"
-        "@P1 bra DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)SNN_WIN_PROD_HINT) : "memory");
-    return;
-#endif
     uint32_t done = 0;
     while (true) {
         asm volatile(
@@ -88,7 +38,7 @@ __device__ __forceinline__ void mbar_wait_backoff(uint64_t *bar, uint32_t parity
             "selp.u32 %0, 1, 0, P1;\n"
             "}\n" : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
         if (done) break;
-        if (SNN_WIN_PROD_SLEEP) __nanosleep(SNN_WIN_PROD_SLEEP);
+        __nanosleep(256);
     }
 }
 // TMA bulk copy global -> shared, completion counted in bytes on an mbarrier (SASS: UBLKCP)

@@ -1,7 +1,6 @@
 """2-rank experiment (torchrun): where do the extra microseconds per step of a partitioned run come from?
   A: two INDEPENDENT whole lattices, one per GPU, stepped at the same time (no coupling)
-  B: the row-strip pair (halo exchange + waits)
-  C: the row-strip pair with the waits disabled (SNN_B200_HALO_NOWAIT: exports and publishes only; results wrong)"""
+  B: the row-strip pair (halo exchange + waits)"""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "spiking-neural-networks_b200"))
