@@ -305,7 +305,10 @@ SNN_API int32_t snn_lattice_run_timed(snn_lattice_t *h, uint64_t iterations, flo
 
 /* Lattice<BCMIzhikevichNeuron, ..., BCM, ...>: the plasticity rule of the lattice becomes BCM (plasticity/mod.rs:99-111, triggered
  * by spiking neurons like STDP: every in-edge and out-edge of a neuron that spiked, using the BCMActivity values of both
- * ends).  SNN_OPT_DO_PLASTICITY keeps switching plasticity on and off.  SNN_MODEL_BCM_IZHIKEVICH, single-GPU `Lattice` handles. */
+ * ends).  SNN_OPT_DO_PLASTICITY keeps switching plasticity on and off.  SNN_MODEL_BCM_IZHIKEVICH `Lattice` handles: whole lattices,
+ * row strips and general-graph partitions (an edge whose presynaptic neuron lives on another rank is updated by the rank that owns
+ * its postsynaptic row, from that neuron's spike time and current_activity exported after every step).  May be called before or
+ * after the partition is attached.  A reward modulator, when enabled, takes precedence. */
 SNN_API int32_t snn_lattice_set_bcm_plasticity(snn_lattice_t *h, int32_t enable, const snn_bcm_t *bcm);
 
 /* RewardModulatedLattice (neuron/mod.rs:2717-3416).  set_reward_modulator(enable = 1) turns the handle into a reward-modulated

@@ -136,7 +136,7 @@ struct StepParams {
     float *rc[RCF_COUNT]; uint64_t rc_stride;   // per neuron
     // spike trains (nodes [train0, train0+n_trains))
     uint32_t train0, n_trains;
-    const float *tf[TF_COUNT];
+    const float *tf[TF_COUNT];   // on BCM Izhikevich partitions: the activity exchange (BcmSlot)
     // lattices
     const LatInfo *lat; int n_lat;
     // histories: this step's record
@@ -160,6 +160,25 @@ struct StepParams {
     // 295.3 us, B200 at 1000 W)
     unsigned long long *dbg;
 };
+
+// BCM Izhikevich partitions: current_activity travels to the neighbours next to V and last_firing_time, into node-indexed
+// ping-pong buffers of their slabs.  A partitioned handle holds one neuron lattice and no spike trains, so the pointers ride in
+// the spike-train slots StepParams::tf (null on every other handle).  New members of HaloDir, GPeer or StepParams would move the
+// parameters, and with them change the code, of every other kernel.
+enum BcmSlot : int {
+    TFB_HALO_ACT = 0,    // tf[TFB_HALO_ACT + 2 * direction + parity]: the neighbour's activity buffer (addressed like HaloDir::peer_v)
+    TFB_GPEER_ACT = 4,   // a float *const * table, [2 * peer slot + parity]: the same for general-graph peers (addressed like GPeer::v)
+    TFB_ACT_GHOST = 5,   // my own buffer of parity out_par: the ghosts' activity after this step (BCM edge kernel)
+};
+static_assert((int)TFB_ACT_GHOST < (int)TF_COUNT, "the BCM activity pointers must fit into StepParams::tf");
+#ifdef __CUDACC__
+__device__ __forceinline__ float *bcm_halo_act(const StepParams &p, uint32_t d, uint32_t par) {
+    return const_cast<float *>(p.tf[TFB_HALO_ACT + 2u * d + par]);
+}
+__device__ __forceinline__ float *bcm_gpeer_act(const StepParams &p, uint32_t q, uint32_t par) {
+    return reinterpret_cast<float *const *>(p.tf[TFB_GPEER_ACT])[2u * q + par];
+}
+#endif
 
 struct TrainParams {
     uint32_t train0, n_trains, clock; int kind; int ntk;
@@ -332,7 +351,8 @@ cudaError_t launch_trains(const TrainParams &p, cudaStream_t s);
 cudaError_t launch_flush_stdp(const StepParams &p, cudaStream_t s);
 // RewardModulatedSTDP::update_weight on every edge, both calls of the timestep (p.lft_in = last_firing_time before the step,
 // p.lft_out = after it)
-// BCM::update_weight on the edges of the neurons that spiked in the step just computed (p.spk_out)
+// BCM::update_weight on the edges of the neurons that spiked in the step just computed (p.spk_out).  On partitioned handles
+// (p.halo active or p.n_gpeers != 0) p.halo_epoch is the value the neighbours' step kernels of this timestep publish.
 struct BcmParams { float decay, average_scalar, dt; };
 cudaError_t launch_bcm_edges(const StepParams &p, const BcmParams &b, cudaStream_t s);
 struct RstdpParams {

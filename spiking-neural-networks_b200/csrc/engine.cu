@@ -63,6 +63,7 @@ Engine::~Engine() {
     if (d_gexp_off_) cudaFree(d_gexp_off_);
     if (d_gexp_ent_) cudaFree(d_gexp_ent_);
     if (d_gslice_) cudaFree(d_gslice_);
+    if (d_gact_) cudaFree(d_gact_);
     free_device();
     if (flags_) cudaFree(flags_);
     if (halo_done_) cudaFree(halo_done_);
@@ -160,7 +161,7 @@ void Engine::free_device() {
     auto fr = [](auto *&p) { if (p) cudaFree(p); p = nullptr; };
     if (slab_) cudaFree(slab_);
     slab_ = nullptr;
-    V_[0] = V_[1] = nullptr; LFT_[0] = LFT_[1] = nullptr; T_[0] = T_[1] = nullptr;
+    V_[0] = V_[1] = nullptr; LFT_[0] = LFT_[1] = nullptr; T_[0] = T_[1] = nullptr; ACT_[0] = ACT_[1] = nullptr;
     fr(SPK_[0]); fr(SPK_[1]); fr(was_inc_);
     node_flags_ = nullptr;   // lives in the slab
     for (auto &p : NT_) fr(p);
@@ -189,13 +190,21 @@ int Engine::alloc_device() {
     // node flags ride in the slab too: a neighbouring strip reads the neurotransmitter type sets of my boundary rows at attach time
     const size_t fbytes = round_up(node_cap_, 256);
     slab_off_flags_ = 4 * vb;
-    slab_off_t_[0] = 4 * vb + fbytes; slab_off_t_[1] = slab_off_t_[0] + round_up(node_cap_ * 4 * kNT, 256);
-    slab_bytes_ = 4 * vb + fbytes;  // T appended by ensure_chem (which reallocates the slab)
+    // BCM Izhikevich strips and partitions: ACT[2] after the flags (the model is fixed at create time, so BCM plasticity may be
+    // switched on at any point before run; no other handle carries these bytes)
+    const bool act = model == SNN_MODEL_BCM_IZHIKEVICH && part_world > 1;
+    slab_off_act_[0] = act ? 4 * vb + fbytes : 0; slab_off_act_[1] = act ? 5 * vb + fbytes : 0;
+    slab_off_t_[0] = (act ? 6 * vb : 4 * vb) + fbytes; slab_off_t_[1] = slab_off_t_[0] + round_up(node_cap_ * 4 * kNT, 256);
+    slab_bytes_ = slab_off_t_[0];  // T appended by ensure_chem (which reallocates the slab)
     CK(cudaMalloc(&slab_, slab_bytes_), SNN_GPU_BUFFER_CREATE_ERROR);
     node_flags_ = (uint8_t *)slab_ + slab_off_flags_;
     for (int k = 0; k < 2; ++k) {
         V_[k] = (float *)((char *)slab_ + slab_off_v_[k]);
         LFT_[k] = (int *)((char *)slab_ + slab_off_lft_[k]);
+        if (act) {
+            ACT_[k] = (float *)((char *)slab_ + slab_off_act_[k]);
+            CK(fill_f32(ACT_[k], 0.f, node_cap_, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+        }
         CK(fill_f32(V_[k], 0.f, node_cap_, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
         CK(launch_fill_u32((uint32_t *)LFT_[k], 0xFFFFFFFFu, node_cap_, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
         CK(dev_alloc(&SPK_[k], node_cap_ / 32 + 1), SNN_GPU_BUFFER_CREATE_ERROR);
@@ -260,6 +269,7 @@ int Engine::ensure_chem() {
         V_[k] = (float *)((char *)slab_ + slab_off_v_[k]);
         LFT_[k] = (int *)((char *)slab_ + slab_off_lft_[k]);
         T_[k] = (float *)((char *)slab_ + slab_off_t_[k]);
+        if (ACT_[k]) ACT_[k] = (float *)((char *)slab_ + slab_off_act_[k]);
     }
     node_flags_ = (uint8_t *)slab_ + slab_off_flags_;
     for (int s = 0; s < NTF_COUNT; ++s) {
@@ -814,6 +824,7 @@ int Engine::gpart_attach(int peer, const IpcBlob *blob_in, Engine *local_peer) {
     }
     if (blob.rank != peer || blob.world != part_world) return fail(SNN_INVALID_ARGUMENT, "ipc blob is not from that rank");
     if ((blob.chem != 0) != chem_alloc_) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on chemistry");
+    if ((blob.off_act[0] != 0) != (ACT_[0] != nullptr)) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on the neuron model");
     G->view = blob;
     G->attached = true;
     layout_frozen_ = true;
@@ -846,9 +857,10 @@ int Engine::gpart_attach(int peer, const IpcBlob *blob_in, Engine *local_peer) {
 int Engine::gpart_build_device() {
     if (!gpart_dirty_) return SNN_OK;
     auto fr = [](auto *&p) { if (p) cudaFree(p); p = nullptr; };
-    fr(d_gpeers_); fr(d_gexp_off_); fr(d_gexp_ent_); fr(d_gslice_);
+    fr(d_gpeers_); fr(d_gexp_off_); fr(d_gexp_ent_); fr(d_gslice_); fr(d_gact_);
     if (gpeers_.size() > 15) return fail(SNN_UNSUPPORTED, "too many peers");
     std::vector<GPeer> hp(std::max<size_t>(gpeers_.size(), 1));
+    std::vector<float *> act(2 * hp.size(), nullptr);
     std::vector<std::vector<uint32_t>> per(n_neurons);
     for (size_t q = 0; q < gpeers_.size(); ++q) {
         GPeerHost &G = gpeers_[q];
@@ -858,6 +870,7 @@ int Engine::gpart_build_device() {
             D.v[k] = (float *)((char *)G.slab + G.view.off_v[k]);
             D.lft[k] = (int *)((char *)G.slab + G.view.off_lft[k]);
             D.t[k] = (float *)((char *)G.slab + G.view.off_t[k]);
+            if (ACT_[0]) act[2 * q + k] = (float *)((char *)G.slab + G.view.off_act[k]);
         }
         D.t_stride = G.view.t_stride;
         D.peer_flag = (unsigned long long *)G.flags + 8 + part_rank;
@@ -881,6 +894,10 @@ int Engine::gpart_build_device() {
     CK(h2d_sync(d_gexp_off_, off.data(), off.size() * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     CK(h2d_sync(d_gexp_ent_, ent.data(), ent.size() * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     CK(h2d_sync(d_gslice_, gs.data(), gs.size(), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    if (ACT_[0]) {
+        CK(dev_alloc(&d_gact_, act.size()), SNN_GPU_BUFFER_CREATE_ERROR);
+        CK(h2d_sync(d_gact_, act.data(), act.size() * sizeof(float *), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    }
     gpart_dirty_ = false;
     return SNN_OK;
 }
@@ -1265,7 +1282,7 @@ int Engine::finalize_graph() {
 // ------------------------------------------------------------------------------------------------
 int Engine::set_bcm_plasticity(bool enable, const snn_bcm_t *b) {
     if (enable && model != SNN_MODEL_BCM_IZHIKEVICH) return fail(SNN_INVALID_ARGUMENT, "BCM plasticity needs neurons with BCMActivity (SNN_MODEL_BCM_IZHIKEVICH)");
-    if (enable && (part_world > 1 || n_neuron_lattices() > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "BCM plasticity: single-GPU Lattice handles only");
+    if (enable && (n_neuron_lattices() > 1 || n_trains > 0)) return fail(SNN_UNSUPPORTED, "BCM plasticity: Lattice handles only (whole, row-strip or general-graph partitioned)");
     bcm_mode = enable;
     if (b) bcm = *b;
     return SNN_OK;
@@ -1871,6 +1888,11 @@ void Engine::fill_step_params(StepParams &p) {
         p.gpeers = d_gpeers_; p.n_gpeers = (uint32_t)gpeers_.size();
         p.gexp_off = d_gexp_off_; p.gexp_ent = d_gexp_ent_; p.gslice = d_gslice_; p.n_gslices = n_slices_;
     }
+    if (ACT_[0]) {   // a BCM Izhikevich partition (no spike trains): the train slots carry the activity exchange (BcmSlot)
+        for (int d = 0; d < 2; ++d)
+            for (int k = 0; k < 2; ++k) p.tf[TFB_HALO_ACT + 2 * d + k] = halo_act_[d][k];
+        p.tf[TFB_GPEER_ACT] = reinterpret_cast<const float *>(d_gact_);
+    }
 }
 
 // Operand streams of the TMA-staged kernel for the current configuration; false = not eligible (use the general kernel).
@@ -2448,7 +2470,7 @@ int Engine::plan_run(RunPlan &pl, LaunchArgs &a) {
         if ((part_rank > 0 && !halo_dir_[0].active) || (part_rank < part_world - 1 && !halo_dir_[1].active))
             return fail(SNN_INVALID_ARGUMENT, "partitioned handle: neighbouring strips are not attached");
     }
-    if (gpart_ && (reward_mode || bcm_mode)) return fail(SNN_UNSUPPORTED, "general-graph partitions step plain and STDP lattices");
+    if (gpart_ && reward_mode) return fail(SNN_UNSUPPORTED, "general-graph partitions step plain, STDP and BCM lattices");
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
     if (chemical) { int r = ensure_chem(); if (r) return r; }
     int r = finalize_graph();
@@ -2705,7 +2727,18 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
         }
     }
     if (pl.bcm_on) {
-        cudaError_t e = launch_bcm_edges(sp, BcmParams{bcm.decay, bcm.average_scalar, bcm.dt}, stream_);
+        StepParams ep = sp;
+        if (part_world > 1) {
+            // the kernel reads the neighbours' step-s exports: their last_firing_time and current_activity of this step in my
+            // ghost slots (see bcm_edge_body for why no second handshake is needed)
+            ep.halo_epoch = halo_epoch_ + 1;
+            ep.tf[TFB_ACT_GHOST] = ACT_[out];
+            if (!local_peers_.empty()) {
+                launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);   // my step kernel of this timestep is in the queue
+                wait_local_peers_launched(halo_epoch_ + 1, false);
+            }
+        }
+        cudaError_t e = launch_bcm_edges(ep, BcmParams{bcm.decay, bcm.average_scalar, bcm.dt}, stream_);
         if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_bcm_edges");
         a.launches++;
     }
@@ -2844,7 +2877,10 @@ int Engine::ipc_export_layout(IpcBlob *blob) {
     if (part_world <= 1) return fail(SNN_INVALID_ARGUMENT, "handle is not partitioned");
     memset(blob, 0, sizeof *blob);
     blob->magic = 0x534E4E42u; blob->version = SNN_B200_ABI_VERSION;
-    for (int k = 0; k < 2; ++k) { blob->off_v[k] = slab_off_v_[k]; blob->off_lft[k] = slab_off_lft_[k]; blob->off_t[k] = slab_off_t_[k]; }
+    for (int k = 0; k < 2; ++k) {
+        blob->off_v[k] = slab_off_v_[k]; blob->off_lft[k] = slab_off_lft_[k]; blob->off_t[k] = slab_off_t_[k];
+        blob->off_act[k] = slab_off_act_[k];
+    }
     blob->off_flags = slab_off_flags_;
     blob->t_stride = node_cap_;
     blob->own0 = own0_; blob->n_neurons = (uint32_t)n_neurons; blob->ghost_hi0 = ghost_hi0_; blob->halo = halo_;
@@ -2906,6 +2942,7 @@ int Engine::attach_view(int direction, const IpcBlob *blob, void *slab, void *fl
     if (blob->rank != part_rank + direction || blob->world != part_world) return fail(SNN_INVALID_ARGUMENT, "ipc blob is not from the neighbouring rank");
     if (blob->halo != halo_ || (blob->chem != 0) != chem_alloc_) return fail(SNN_INVALID_ARGUMENT, "neighbouring strips disagree on halo width / chemistry");
     if (halo_ > n_neurons || halo_ > blob->n_neurons) return fail(SNN_UNSUPPORTED, "strip thinner than the halo");
+    if ((blob->off_act[0] != 0) != (ACT_[0] != nullptr)) return fail(SNN_INVALID_ARGUMENT, "neighbouring strips disagree on the neuron model");
     const int d = direction < 0 ? 0 : 1;
     HaloDir &H = halo_dir_[d];
     memset(&H, 0, sizeof H);
@@ -2919,6 +2956,7 @@ int Engine::attach_view(int direction, const IpcBlob *blob, void *slab, void *fl
         H.peer_v[k] = (float *)((char *)slab + blob->off_v[k]);
         H.peer_lft[k] = (int *)((char *)slab + blob->off_lft[k]);
         H.peer_t[k] = (float *)((char *)slab + blob->off_t[k]);
+        halo_act_[d][k] = ACT_[0] ? (float *)((char *)slab + blob->off_act[k]) : nullptr;
     }
     H.peer_t_stride = blob->t_stride;
     // the neighbour's arrival counter for data coming from me: I am its rank+1 when d == 0 (slot 1), its rank-1 when d == 1 (slot 0)

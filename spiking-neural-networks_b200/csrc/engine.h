@@ -61,6 +61,7 @@ struct IpcBlob {  // exchanged between neighbouring ranks by the caller (e.g. to
     uint32_t magic, version;
     cudaIpcMemHandle_t slab, flags;
     uint64_t off_v[2], off_lft[2], off_t[2], off_flags;
+    uint64_t off_act[2];   // current_activity ping-pong of a BCM Izhikevich strip; 0 = the slab has none
     uint64_t t_stride;
     uint32_t own0, n_neurons, ghost_hi0, halo, cols, chem;
     int32_t rank, world;
@@ -190,6 +191,11 @@ private:
     int *LFT_[2] = {nullptr, nullptr};
     float *T_[2] = {nullptr, nullptr};
     uint64_t slab_off_v_[2] = {0, 0}, slab_off_lft_[2] = {0, 0}, slab_off_t_[2] = {0, 0}, slab_off_flags_ = 0;
+    // BCM Izhikevich partitions only: node-indexed current_activity ping-pong, of which the ghost slots are filled by the
+    // neighbours (the partitioned BCM edge kernel reads a ghost's activity there)
+    float *ACT_[2] = {nullptr, nullptr};
+    uint64_t slab_off_act_[2] = {0, 0};
+    float *halo_act_[2][2] = {};   // the neighbours' buffers, [direction][parity] (BcmSlot TFB_HALO_ACT)
     bool ghost_flags_from_peer_[2] = {false, false};
     uint32_t *SPK_[2] = {nullptr, nullptr};
     uint8_t *node_flags_ = nullptr;
@@ -245,6 +251,7 @@ private:
     std::vector<GPeerHost> gpeers_;        // ascending rank
     std::vector<uint8_t> h_gslice_;        // per slice: bit 0 = a row of the slice reads a ghost
     GPeer *d_gpeers_ = nullptr; uint32_t *d_gexp_off_ = nullptr, *d_gexp_ent_ = nullptr; uint8_t *d_gslice_ = nullptr;
+    float **d_gact_ = nullptr;             // BCM Izhikevich: the peers' activity buffers (BcmSlot TFB_GPEER_ACT), else null
     GPeerHost *gpeer(int rank, bool create);
     int gpart_build_device();
     int gpart_enable(const std::vector<uint32_t> &remote_sorted_unique);

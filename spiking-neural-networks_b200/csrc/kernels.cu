@@ -57,7 +57,7 @@ __device__ __forceinline__ void step_kernel_body(const StepParams &p) {
     const GlobalSrc src{p, lnc, p.own0 + lnc, lane, k0, k1, t0};
     neuron_step<MODEL, CHEMG, NTREL, STDP, NET>(p, src, warp_global, lane, ln, lnc, valid, export_lo, export_hi);
     if (!NET) halo_publish(p, warp_global, lane);
-    if (!NET) gpart_export_publish(p, warp_global, lane, ln, valid);
+    if (!NET) gpart_export_publish<MODEL == SNN_MODEL_BCM_IZHIKEVICH>(p, warp_global, lane, ln, valid);
 }
 
 // (single lattices keep the compiler's choice of 64 registers: bounded to five / six resident CTAs the general-graph lattices of
@@ -190,12 +190,41 @@ __global__ void __launch_bounds__(256) flush_stdp_kernel(const __grid_constant__
 // that spiked is updated with the same function of (weight, presynaptic activity, postsynaptic activity / average), so an edge
 // whose two ends both spiked is simply updated twice.  Runs after the step kernel (deferred, canonicalisation (3)): the raster
 // word of the step tells who spiked, the activities are the ones the step just wrote.
-__global__ void __launch_bounds__(256) bcm_edge_kernel(const __grid_constant__ StepParams p, const __grid_constant__ BcmParams b) {
+//
+// PART: row strips and general-graph partitions.  The rank that owns an edge's postsynaptic row applies both of its updates, so an
+// out-edge of a neuron on another rank is updated here as an in-edge whose presynaptic node is a ghost.  A ghost has no raster bit
+// in this rank's spk_out; it spiked in this step iff its last_firing_time (ping-ponged on every partitioned handle, exported each
+// step into the ghost slot of parity out_par) equals the step's clock.  Its current_activity comes from the node-indexed ghost
+// buffer tf[TFB_ACT_GHOST], exported next to it.  A warp whose slice reads ghosts first waits until every neighbour / peer has published
+// this step (p.halo_epoch).  No second handshake is needed: the neighbour overwrites this parity of the ghost slots in its step
+// s + 2, whose boundary warps first wait for this rank's step s + 1, and that kernel starts only after this one has finished
+// (same stream, plain launches on partitioned handles).
+template <bool PART>
+__device__ __forceinline__ void bcm_edge_body(const StepParams &p, const BcmParams &b) {
     pdl_wait();   // launch_pdl
+    if (PART && halo_failed(p)) return;
     const uint32_t warp_global = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t ln = warp_global * 32u + lane;
     if (warp_global * 32u >= p.n_neurons) return;
+    if constexpr (PART) {
+        // slices that read ghosts: the first / last halo rows of a strip (the predicates of halo_import), bit 0 of gslice on a
+        // general-graph partition; interior slices start at once
+        const uint32_t w0 = warp_global * 32u, w1 = min(w0 + 32u, p.n_neurons);
+        const bool near_lo = p.halo[0].active && w0 < p.halo[0].first + p.halo[0].count;
+        const bool near_hi = p.halo[1].active && w1 > p.halo[1].first;
+        const bool gwait = p.n_gpeers && (p.gslice[warp_global] & 1u);
+        if (near_lo | near_hi | gwait) {
+            if (lane == 0) {
+                if (near_lo) halo_wait(p.halo[0].my_flag, p.halo_epoch, p.halo_done + 2, p.halo_timeout_ns);
+                if (near_hi) halo_wait(p.halo[1].my_flag, p.halo_epoch, p.halo_done + 2, p.halo_timeout_ns);
+                if (gwait)
+                    for (uint32_t q = 0; q < p.n_gpeers; ++q)
+                        if (!halo_wait(p.gpeers[q].my_flag, p.halo_epoch, p.halo_done + 2, p.halo_timeout_ns)) break;
+            }
+            __syncwarp();
+        }
+    }
     const uint32_t k0 = p.uniform_width ? warp_global * p.uniform_width : __ldg(p.slice_off + warp_global);
     const uint32_t k1 = p.uniform_width ? k0 + p.uniform_width : __ldg(p.slice_off + warp_global + 1);
     const uint32_t word0 = p.own0 >> 5;
@@ -206,11 +235,17 @@ __global__ void __launch_bounds__(256) bcm_edge_kernel(const __grid_constant__ S
         const uint32_t c = valid ? __ldg(p.col + e) : kColPad;
         if (c == kColPad) continue;
         const uint32_t j = c & kColIdxMask;
-        const bool pre_spk = (p.spk_out[j >> 5] >> (j & 31u)) & 1u;
+        bool ghost = false, pre_spk;
+        if constexpr (PART) {
+            ghost = j - p.own0 >= p.n_neurons;   // below or above this rank's own nodes
+            pre_spk = ghost ? p.lft_out[j] == (int)p.clock : ((p.spk_out[j >> 5] >> (j & 31u)) & 1u);
+        } else {
+            pre_spk = (p.spk_out[j >> 5] >> (j & 31u)) & 1u;
+        }
         const int n_upd = (post_spk ? 1 : 0) + (pre_spk ? 1 : 0);
         if (n_upd == 0) continue;
         const uint32_t jl = j - p.own0;
-        const float act_post = p.f[F_CUR_ACT][ln], avg_post = p.f[F_AVG_ACT][ln], act_pre = p.f[F_CUR_ACT][jl];
+        const float act_post = p.f[F_CUR_ACT][ln], avg_post = p.f[F_AVG_ACT][ln], act_pre = ghost ? p.tf[TFB_ACT_GHOST][j] : p.f[F_CUR_ACT][jl];
         const float sliding_threshold = avg_post / b.average_scalar;
         const float activity_term = act_post * (act_post - sliding_threshold);
         float w = p.wgt[e];
@@ -220,6 +255,13 @@ __global__ void __launch_bounds__(256) bcm_edge_kernel(const __grid_constant__ S
         }
         p.wgt[e] = w;
     }
+}
+
+__global__ void __launch_bounds__(256) bcm_edge_kernel(const __grid_constant__ StepParams p, const __grid_constant__ BcmParams b) {
+    bcm_edge_body<false>(p, b);
+}
+__global__ void __launch_bounds__(256) bcm_part_edge_kernel(const __grid_constant__ StepParams p, const __grid_constant__ BcmParams b) {
+    bcm_edge_body<true>(p, b);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -653,7 +695,9 @@ cudaError_t launch_gpart_push(const StepParams &p, cudaStream_t s) {
 
 cudaError_t launch_bcm_edges(const StepParams &p, const BcmParams &b, cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
-    return launch_pdl(false, bcm_edge_kernel, dim3(blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256)), dim3(256), 0, s, p, b);
+    const bool part = (p.halo[0].active | p.halo[1].active) || p.n_gpeers;
+    return launch_pdl(false, part ? bcm_part_edge_kernel : bcm_edge_kernel, dim3(blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256)),
+                      dim3(256), 0, s, p, b);
 }
 
 cudaError_t launch_rstdp_edges(const StepParams &p, const RstdpParams &r, cudaStream_t s) {

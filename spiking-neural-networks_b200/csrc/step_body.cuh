@@ -171,7 +171,9 @@ __device__ __forceinline__ void gpart_wait(const StepParams &p, uint32_t slice, 
 }
 
 // after neuron_step: copy this neuron's new state into the ghost slots of every peer that lists it, then count the warp as done;
-// the last warp of the step raises every peer's completion counter
+// the last warp of the step raises every peer's completion counter.  BCM: BCM Izhikevich neurons, whose current_activity is
+// exported too (the peers' BCM edge kernels read it)
+template <bool BCM>
 __device__ __forceinline__ void gpart_export_publish(const StepParams &p, uint32_t slice, uint32_t lane, uint32_t ln, bool valid) {
     if (!p.n_gpeers) return;
     const bool exports = (p.gslice[slice] & 2u) != 0u;
@@ -184,6 +186,7 @@ __device__ __forceinline__ void gpart_export_publish(const StepParams &p, uint32
             G.lft[p.out_par][dst] = p.lft_out[i];
             for (int ty = 0; ty < kNT; ++ty)
                 if (p.nt_used & (1u << ty)) G.t[p.out_par][(size_t)ty * G.t_stride + dst] = p.t_out[(size_t)ty * p.t_stride + i];
+            if constexpr (BCM) bcm_gpeer_act(p, ent >> 28, p.out_par)[dst] = p.f[F_CUR_ACT][ln];
         }
     }
     __syncwarp();
@@ -1208,12 +1211,14 @@ __device__ __forceinline__ void neuron_step(const StepParams &p, const SRC &src,
             const uint32_t dst = H.peer_node0 + (ln - H.first);
             H.peer_v[p.out_par][dst] = v;
             if (p.lft_pp) H.peer_lft[p.out_par][dst] = lft_new;
+            if constexpr (BCM) bcm_halo_act(p, 0, p.out_par)[dst] = p.f[F_CUR_ACT][lnc];   // read by the neighbour's BCM edge kernel
         }
         if (part && export_hi) {
             const HaloDir &H = p.halo[1];
             const uint32_t dst = H.peer_node0 + (ln - H.first);
             H.peer_v[p.out_par][dst] = v;
             if (p.lft_pp) H.peer_lft[p.out_par][dst] = lft_new;
+            if constexpr (BCM) bcm_halo_act(p, 1, p.out_par)[dst] = p.f[F_CUR_ACT][lnc];
         }
     }
 }
