@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/snn_b200.h"
+#include "step_spec.h"
 
 #include <cstdlib>
 #include <utility>
@@ -212,8 +213,8 @@ struct MultiParams {
     uint32_t cache_rows;      // the stencil rows and parameters may live in registers for the whole launch (nothing rewrites them)
 };
 // dry = only report whether the configuration is eligible (cudaSuccess) without launching
-cudaError_t launch_step_multi(const StepParams &p, const TrainParams &t, const MultiParams &m, int model, int chemg, bool ntrel, bool stdp,
-                              bool net, bool wide, int device, bool dry, cudaStream_t s);
+cudaError_t launch_step_multi(const StepParams &p, const TrainParams &t, const MultiParams &m, const StepSpec &spec, bool wide, int device,
+                              bool dry, cudaStream_t s);
 
 // ---- TMA-staged step kernel (step_tma.cu) -----------------------------------------------------
 constexpr int kTmaTile = 256;            // neurons per tile
@@ -238,8 +239,7 @@ struct TmaParams {
     uint32_t o_rc[RCF_COUNT][kNT];
 };
 
-cudaError_t launch_step_tma(const StepParams &p, const TmaParams &tp, int model, int chemg, bool ntrel, bool stdp, unsigned grid,
-                            cudaStream_t s);
+cudaError_t launch_step_tma(const StepParams &p, const TmaParams &tp, const StepSpec &spec, unsigned grid, cudaStream_t s);
 
 // ---- window-staged step kernel (step_win.cu): radius-1 stencil lattices ----------------------
 // One persistent CTA per SM; every operand of a 256-neuron tile, INCLUDING the three neighbour row windows of the node
@@ -328,20 +328,17 @@ struct WinParams {
 // models with wide operand sets (Hodgkin-Huxley, three neurotransmitter types): fewer, fatter stages
 __host__ __device__ constexpr int win_groups(int model, int chemg) { return (model == SNN_MODEL_HODGKIN_HUXLEY || chemg == 3) ? 2 : 3; }
 
-cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, int model, int chemg, bool ntrel, bool stdp, unsigned grid,
-                            cudaStream_t s);
+cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const StepSpec &spec, unsigned grid, cudaStream_t s);
 
 // ---- kernel launchers (kernels.cu) ------------------------------------------------------------
-// chemg: 0 no chemical gather, 1 one neurotransmitter type in the whole node array, 3 general; ntrel: neurotransmitter /
-// receptor state is present and must be stepped; net: several lattices and/or spike trains share the node array
-cudaError_t launch_step(const StepParams &p, int model, int chemg, bool ntrel, bool stdp, bool net, cudaStream_t s);
+cudaError_t launch_step(const StepParams &p, const StepSpec &spec, cudaStream_t s);
 // same contract as launch_step, one CTA per slice (step_wide.cu): graphs with wide rows, single-GPU handles only
 constexpr uint32_t kWideMinWidth = 48;   // mean k-rows per slice from which the wide kernel is used
 // scratch != nullptr: two passes (per-edge terms of every slice chunk on its own CTA, parked in `scratch`: chunks_cap buffers of
 // wide_chunk_bytes(chemg) per slice; then the ordered sums) — very wide slices, where one SM per slice is issue-bound
 // trains != nullptr (two-pass mode only): the spike trains of the timestep are stepped by extra CTAs of the sum pass
-cudaError_t launch_step_wide(const StepParams &p, int model, int chemg, bool ntrel, bool stdp, bool net, unsigned char *scratch, uint32_t chunks_cap,
-                             const TrainParams *trains, cudaStream_t s);
+cudaError_t launch_step_wide(const StepParams &p, const StepSpec &spec, unsigned char *scratch, uint32_t chunks_cap, const TrainParams *trains,
+                             cudaStream_t s);
 uint32_t wide_chunk_bytes(int chemg);
 uint32_t wide_chunk_krows();
 size_t wide_part_bytes();   // per slice, after the chunk buffers: partial sums, counts and the arrival counter of the sum pass (zeroed once)

@@ -2082,11 +2082,7 @@ enum class StepPath {
 
 // Decisions fixed for a whole run(), taken once by plan_run.
 struct Engine::RunPlan {
-    // kernel specialisation: ntrel = neurotransmitter / receptor state must be stepped; chemg = how the chemical gather reads
-    // presynaptic types (0 none, 1 a single type in the whole node array, 3 per-edge masks); net = several lattices and/or spike
-    // trains share the node array
-    bool stdp = false, ntrel = false, net = false;
-    int chemg = 0;
+    StepSpec spec;                                 // kernel specialisation (step_spec.h)
     bool rmod = false, rmod_part = false;          // reward-modulated lattice (rmod_part: a row strip of one)
     bool bcm_on = false;                           // BCM rule instead of STDP
     bool net_reward = false, net_rmod = false;     // reward-modulated lattices in a network (net_rmod: one of them modulates)
@@ -2480,27 +2476,28 @@ int Engine::plan_run(RunPlan &pl, LaunchArgs &a) {
     if (gpart_) { r = gpart_build_device(); if (r) return r; }
 
     for (auto &L : lats_) {
-        if (!L.is_train) { pl.stdp |= L.do_plasticity && !L.is_reward; pl.want_grid |= L.grid_hist; pl.want_spk |= L.spike_hist; pl.want_red |= L.avg_hist || L.eeg_hist; }
+        if (!L.is_train) { pl.spec.stdp |= L.do_plasticity && !L.is_reward; pl.want_grid |= L.grid_hist; pl.want_spk |= L.spike_hist; pl.want_red |= L.avg_hist || L.eeg_hist; }
         else { pl.want_tgrid |= L.grid_hist; pl.want_tspk |= L.spike_hist; }
     }
     // AverageVoltageHistory / EEGHistory are reductions of the staged grid record (it stays on the device for them)
     pl.copy_grid = pl.want_grid;
     pl.want_grid = pl.want_grid || pl.want_red;
-    pl.ntrel = chem_alloc_ && (chemical || nt_used() != 0 || (model == SNN_MODEL_HODGKIN_HUXLEY && rc_used() != 0));
-    pl.net = n_neuron_lattices() > 1 || n_trains > 0;
-    if (chemical && pl.ntrel && nt_used() != 0) pl.chemg = (!pl.net && __builtin_popcount(nt_used()) == 1) ? 1 : 3;
+    pl.spec.model = model;
+    pl.spec.ntrel = chem_alloc_ &&(chemical || nt_used() != 0 || (model == SNN_MODEL_HODGKIN_HUXLEY && rc_used() != 0));
+    pl.spec.net = n_neuron_lattices() > 1 || n_trains > 0;
+    if (chemical && pl.spec.ntrel && nt_used() != 0) pl.spec.chemg = (!pl.spec.net && __builtin_popcount(nt_used()) == 1) ? 1 : 3;
     // reward-modulated lattice: the modulator replaces the plasticity rule and needs last_firing_time before and after a step
     pl.rmod = reward_mode && do_modulation && n_neurons > 0;
     // BCM rule instead of STDP: applied by its own per-edge kernel right after each step (it reads the activities the step wrote)
-    pl.bcm_on = bcm_mode && pl.stdp && !reward_mode && n_neurons > 0;
-    if (reward_mode || bcm_mode) pl.stdp = false;
+    pl.bcm_on = bcm_mode && pl.spec.stdp && !reward_mode && n_neurons > 0;
+    if (reward_mode || bcm_mode) pl.spec.stdp = false;
     if (pl.rmod) { r = ensure_reward_arrays(); if (r) return r; }
     a.rsp = RstdpParams{rstdp.dopamine, rstdp.tau_c, rstdp.a_plus, rstdp.a_minus, rstdp.tau_plus, rstdp.tau_minus, rstdp.dt,
                         rs_counter_, rs_dw_, rs_c_, rs_canonical_ ? 1u : 0u, nullptr, 0u};
     if (pl.rmod) { r = build_stdp_tables({a.rsp}, &a.rsp.tab, &a.rsp.tab_n); if (r) return r; }
     pl.net_reward = has_reward_lattices();
     if (pl.net_reward) { r = build_rnet_params(a.rnp, &pl.net_rmod); if (r) return r; }
-    pl.lft_pp = pl.stdp || pl.rmod || pl.net_rmod || (n_trains && electrical) || part_world > 1;
+    pl.lft_pp = pl.spec.stdp || pl.rmod || pl.net_rmod || (n_trains && electrical) || part_world > 1;
     pl.rmod_part = pl.rmod && part_world > 1;
 
     fill_step_params(a.sp);
@@ -2525,13 +2522,13 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
     const char *tma_env = getenv("SNN_B200_TMA"), *win_env = getenv("SNN_B200_WIN");
     const int tma_mode = tma_env ? atoi(tma_env) : 1;
     const int win_mode = (win_env && atoi(win_env) == 0) ? 0 : tma_mode;
-    if (!pl.net && build_win_params(a.win, pl.chemg, pl.ntrel, pl.stdp, pl.lft_pp, win_mode, &pl.grid)) {
+    if (!pl.spec.net && build_win_params(a.win, pl.spec.chemg, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, win_mode, &pl.grid)) {
         pl.path = StepPath::Win;
-    } else if (!pl.net && build_tma_params(a.tma, pl.ntrel, pl.stdp, pl.lft_pp, tma_mode, &pl.grid)) {
+    } else if (!pl.spec.net && build_tma_params(a.tma, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, tma_mode, &pl.grid)) {
         pl.path = StepPath::Tma;
         for (uint32_t k = 0; k < a.tma.n_streams; ++k) {
             if (a.tma.st[k].smem_off == a.tma.o_v) pl.tma_iv = (int)k;
-            if ((pl.stdp || pl.lft_pp) && a.tma.st[k].smem_off == a.tma.o_lft) pl.tma_il = (int)k;
+            if ((pl.spec.stdp || pl.lft_pp) && a.tma.st[k].smem_off == a.tma.o_lft) pl.tma_il = (int)k;
             for (int ty = 0; ty < kNT; ++ty) if (a.tma.o_t[ty] != 0xFFFFFFFFu && a.tma.st[k].smem_off == a.tma.o_t[ty]) pl.tma_it[ty] = (int)k;
         }
     } else if (part_world == 1 && n_slices_ > 0 && sell_krows_ / n_slices_ >= kWideMinWidth) {
@@ -2542,7 +2539,7 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
     }
     if (pl.path == StepPath::WideSplit) {
         pl.wide_chunks_cap = (max_slice_width_ + wide_chunk_krows() - 1) / wide_chunk_krows();
-        const size_t chunks_bytes = (size_t)n_slices_ * pl.wide_chunks_cap * wide_chunk_bytes(pl.chemg);
+        const size_t chunks_bytes = (size_t)n_slices_ * pl.wide_chunks_cap * wide_chunk_bytes(pl.spec.chemg);
         const size_t need = chunks_bytes + (size_t)n_slices_ * wide_part_bytes();
         if (need != wide_scratch_bytes_) {
             if (wide_scratch_) cudaFree(wide_scratch_);
@@ -2564,8 +2561,7 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
     if (pl.multi) {
         MultiParams probe{};
         probe.wide_stage = (pl.path == StepPath::Wide && n_nodes_ <= 4096) ? 1u : 0u;
-        pl.multi = launch_step_multi(a.sp, a.tp, probe, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, pl.path == StepPath::Wide, device,
-                                     true, stream_) == cudaSuccess;
+        pl.multi = launch_step_multi(a.sp, a.tp, probe, pl.spec, pl.path == StepPath::Wide, device, true, stream_) == cudaSuccess;
         cudaGetLastError();
     }
     return SNN_OK;
@@ -2629,15 +2625,15 @@ int Engine::run_multi_chunk(const RunPlan &pl, LaunchArgs &a, const HistStage &h
         MultiParams mp{};
         mp.steps = (uint32_t)k; mp.first_pending = (first_chunk && s0 == 0) ? 0u : 1u;
         mp.cur = (uint32_t)cur_; mp.lft_loc = (uint32_t)lft_loc_; mp.lft_pp = pl.lft_pp ? 1u : 0u;
-        mp.train_sync = (pl.stdp && n_trains) ? 1u : 0u;
+        mp.train_sync = (pl.spec.stdp && n_trains) ? 1u : 0u;
         for (int q = 0; q < 2; ++q) { mp.v[q] = V_[q]; mp.lft[q] = LFT_[q]; mp.spk[q] = SPK_[q]; mp.t[q] = T_[q]; }
         hist.point(mp, s0);
         mp.n_neurons = n_neurons; mp.n_words = hist.n_words; mp.n_trains = n_trains; mp.t_words = hist.t_words;
         mp.barrier = multi_barrier_;
-        mp.cache_rows = !pl.stdp ? 1u : 0u;
+        mp.cache_rows = !pl.spec.stdp ? 1u : 0u;
         mp.wide_stage = (wide && n_nodes_ <= 4096) ? 1u : 0u;
         cudaError_t e = cudaMemsetAsync(multi_barrier_, 0, sizeof(unsigned int), stream_);
-        if (e == cudaSuccess) e = launch_step_multi(sp, tp, mp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, wide, device, false, stream_);
+        if (e == cudaSuccess) e = launch_step_multi(sp, tp, mp, pl.spec, wide, device, false, stream_);
         if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_step_multi");
         a.launches++;
         // the host mirrors what the launch did to the ping-pong state and the clocks
@@ -2658,7 +2654,7 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
     sp.clock = (uint32_t)internal_clock;
     // window kernel: sweep the tiles back to front every other step (the tail the previous step left in L2 is read first)
     sp.reverse = (internal_clock & 1ull) ? 1u : 0u;
-    sp.apply_pending = (pl.stdp && !first) ? 1u : 0u;
+    sp.apply_pending = (pl.spec.stdp && !first) ? 1u : 0u;
     sp.v_in = V_[in]; sp.v_out = V_[out];
     sp.spk_in = SPK_[in]; sp.spk_out = SPK_[out];
     sp.t_in = T_[in]; sp.t_out = T_[out];
@@ -2682,7 +2678,7 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
         const char *what = "launch_step";
         switch (pl.path) {
         case StepPath::Win:
-            e = launch_step_win(sp, a.win, model, pl.chemg, pl.ntrel, pl.stdp, pl.grid, stream_);
+            e = launch_step_win(sp, a.win, pl.spec, pl.grid, stream_);
             what = "launch_step_win";
             break;
         case StepPath::Tma:
@@ -2690,18 +2686,17 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
             if (pl.tma_il >= 0) a.tma.st[pl.tma_il].src = (const unsigned char *)(sp.lft_in + own0_);
             for (int ty = 0; ty < kNT; ++ty)
                 if (pl.tma_it[ty] >= 0) a.tma.st[pl.tma_it[ty]].src = (const unsigned char *)(sp.t_in + (size_t)ty * node_cap_ + own0_);
-            e = launch_step_tma(sp, a.tma, model, pl.chemg, pl.ntrel, pl.stdp, pl.grid, stream_);
+            e = launch_step_tma(sp, a.tma, pl.spec, pl.grid, stream_);
             what = "launch_step_tma";
             break;
         case StepPath::Wide:
-            e = launch_step_wide(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, nullptr, 0u, nullptr, stream_);
+            e = launch_step_wide(sp, pl.spec, nullptr, 0u, nullptr, stream_);
             break;
         case StepPath::WideSplit:
-            e = launch_step_wide(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, wide_scratch_, pl.wide_chunks_cap,
-                                 pl.trains_fused ? &tp : nullptr, stream_);
+            e = launch_step_wide(sp, pl.spec, wide_scratch_, pl.wide_chunks_cap, pl.trains_fused ? &tp : nullptr, stream_);
             break;
         case StepPath::General:
-            e = launch_step(sp, model, pl.chemg, pl.ntrel, pl.stdp, pl.net, stream_);
+            e = launch_step(sp, pl.spec, stream_);
             break;
         }
         if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, what);
@@ -2770,7 +2765,7 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
         }
         for (auto &L : lats_) if (L.is_train) L.clock += 1;
     }
-    if (pl.ghist_on && (is_network || !pl.stdp || sp.apply_pending)) {
+    if (pl.ghist_on && (is_network || !pl.spec.stdp || sp.apply_pending)) {
         cudaError_t e = hist.record_graph(a.launches);
         if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_graph_record");
     }
@@ -2810,7 +2805,7 @@ int Engine::finish_run(const RunPlan &pl, const StepParams &sp) {
             return fail(SNN_GPU_WAIT_ERROR, "timed out waiting for a neighbouring strip's halo (is every rank running the same number of steps?)");
         }
     }
-    if (pl.stdp || pl.rmod || pl.net_rmod || pl.bcm_on) dev_weights_newer_ = true;
+    if (pl.spec.stdp || pl.rmod || pl.net_rmod || pl.bcm_on) dev_weights_newer_ = true;
     if ((chemical && chem_alloc_) || model == SNN_MODEL_HODGKIN_HUXLEY) {
         StepParams fp = sp;
         fp.chemical = chemical && chem_alloc_;
@@ -2842,7 +2837,7 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
             for (uint64_t s = 0; !pl.multi && !r && s < steps; ++s)
                 r = run_step(pl, a, hist, s, done == 0 && s == 0, rewards ? rewards + done + s : nullptr);
             done += steps;
-            if (!r && done == iterations && pl.stdp) r = flush_stdp(pl, a, hist);
+            if (!r && done == iterations && pl.spec.stdp) r = flush_stdp(pl, a, hist);
             if (r) break;
             cudaEventRecord(ev1_, stream_);
             cudaError_t e = cudaStreamSynchronize(stream_);

@@ -634,45 +634,16 @@ __global__ void transpose_out_kernel(const float *src_tm, float *dst_nm, uint64_
 // ------------------------------------------------------------------------------------------------
 static inline unsigned blocks_for(uint64_t n, unsigned bs) { return (unsigned)((n + bs - 1) / bs); }
 
-template <int MODEL, int CHEMG, bool NTREL, bool NET>
-static cudaError_t launch_step_3(const StepParams &p, bool stdp, cudaStream_t s) {
-    const unsigned grid = blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256);
-    if constexpr (NET && !NTREL && MODEL != SNN_MODEL_HODGKIN_HUXLEY) {
-        if (stdp) return launch_pdl(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, true>, dim3(grid), dim3(256), 0, s, p);
-        return launch_pdl(pdl_ok(p), step_net5_kernel<MODEL, CHEMG, NTREL, false>, dim3(grid), dim3(256), 0, s, p);
-    }
-    if (stdp) return launch_pdl(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, true, NET>, dim3(grid), dim3(256), 0, s, p);
-    return launch_pdl(pdl_ok(p), step_kernel<MODEL, CHEMG, NTREL, false, NET>, dim3(grid), dim3(256), 0, s, p);
-}
-
-template <int MODEL>
-static cudaError_t launch_step_model(const StepParams &p, int chemg, bool ntrel, bool stdp, bool net, cudaStream_t s) {
-    if (net) {
-        // several lattices and/or spike trains: general per-edge type masks
-        if (chemg) return launch_step_3<MODEL, 3, true, true>(p, stdp, s);
-        if (ntrel) return launch_step_3<MODEL, 0, true, true>(p, stdp, s);
-        return launch_step_3<MODEL, 0, false, true>(p, stdp, s);
-    }
-    if (chemg == 1) return launch_step_3<MODEL, 1, true, false>(p, stdp, s);
-    if (chemg == 3) return launch_step_3<MODEL, 3, true, false>(p, stdp, s);
-    if (ntrel) return launch_step_3<MODEL, 0, true, false>(p, stdp, s);
-    return launch_step_3<MODEL, 0, false, false>(p, stdp, s);
-}
-
-cudaError_t launch_step(const StepParams &p, int model, int chemg, bool ntrel, bool stdp, bool net, cudaStream_t s) {
+cudaError_t launch_step(const StepParams &p, const StepSpec &spec, cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
-    switch (model) {
-    case SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE: return launch_step_model<SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE: return launch_step_model<SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE: return launch_step_model<SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE: return launch_step_model<SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_IZHIKEVICH: return launch_step_model<SNN_MODEL_IZHIKEVICH>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_LEAKY_IZHIKEVICH: return launch_step_model<SNN_MODEL_LEAKY_IZHIKEVICH>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE: return launch_step_model<SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_HODGKIN_HUXLEY: return launch_step_model<SNN_MODEL_HODGKIN_HUXLEY>(p, chemg, ntrel, stdp, net, s);
-    case SNN_MODEL_BCM_IZHIKEVICH: return launch_step_model<SNN_MODEL_BCM_IZHIKEVICH>(p, chemg, ntrel, stdp, net, s);
-    }
-    return cudaErrorInvalidValue;
+    const unsigned grid = blocks_for((uint64_t)((p.n_neurons + 31u) / 32u) * 32u, 256);
+    return dispatch_step(spec, cudaErrorInvalidValue, [&](auto k) {
+        using K = decltype(k);
+        if constexpr (K::NET && !K::NTREL && K::MODEL != SNN_MODEL_HODGKIN_HUXLEY)
+            return launch_pdl(pdl_ok(p), step_net5_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP>, dim3(grid), dim3(256), 0, s, p);
+        else
+            return launch_pdl(pdl_ok(p), step_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, K::NET>, dim3(grid), dim3(256), 0, s, p);
+    });
 }
 
 cudaError_t launch_trains(const TrainParams &p, cudaStream_t s) {

@@ -188,15 +188,15 @@ step_multi_kernel(const __grid_constant__ StepParams p0, const __grid_constant__
 // ------------------------------------------------------------------------------------------------
 // launcher
 // ------------------------------------------------------------------------------------------------
-template <int MODEL, int CHEMG, bool NTREL, bool STDP, bool NET, bool WIDE>
-static cudaError_t launch_multi_5(const StepParams &p, const TrainParams &t, const MultiParams &m, int device, bool dry, cudaStream_t s) {
+template <class K, bool WIDE>
+static cudaError_t launch_multi(const StepParams &p, const TrainParams &t, const MultiParams &m, int device, bool dry, cudaStream_t s) {
     const uint32_t n_slices = (p.n_neurons + 31u) / 32u, n_twarps = (t.n_trains + 31u) / 32u;
     cudaError_t e;
     if constexpr (!WIDE) {
         // small enough for one cluster: every slice (and spike-train warp) gets its own warp in 16 CTAs of 640 threads
         const uint32_t warps = kClusterCtas * (kClusterThreads / 32);
         if (n_slices <= warps && n_twarps <= warps) {
-            auto kc = step_multi_kernel<MODEL, CHEMG, NTREL, STDP, NET, false, true>;
+            auto kc = step_multi_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, K::NET, false, true>;
             static thread_local int cluster_ok = -1;   // per instantiation
             if (cluster_ok < 0) {
                 cluster_ok = 0;
@@ -222,9 +222,9 @@ static cudaError_t launch_multi_5(const StepParams &p, const TrainParams &t, con
             }
         }
     }
-    auto k = step_multi_kernel<MODEL, CHEMG, NTREL, STDP, NET, WIDE, false>;
+    auto k = step_multi_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, K::NET, WIDE, false>;
     const int threads = WIDE ? kWideWarps * 32 : 256;
-    const size_t smem = WIDE ? 2u * wide_buf_bytes(CHEMG) + (m.wide_stage ? wide_stage_bytes(p.n_nodes, NET ? p.n_trains : 0u) : 0u) : 0u;
+    const size_t smem = WIDE ? 2u * wide_buf_bytes(K::CHEMG) + (m.wide_stage ? wide_stage_bytes(p.n_nodes, K::NET ? p.n_trains : 0u) : 0u) : 0u;
     if (smem > 40u * 1024u) { e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); if (e != cudaSuccess) return e; }
     int per_sm = 0, sms = 0;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem);
@@ -243,43 +243,12 @@ static cudaError_t launch_multi_5(const StepParams &p, const TrainParams &t, con
     return cudaLaunchCooperativeKernel((const void *)k, dim3(grid), dim3(threads), args, smem, s);
 }
 
-template <int MODEL, int CHEMG, bool NTREL, bool NET>
-static cudaError_t launch_multi_3(const StepParams &p, const TrainParams &t, const MultiParams &m, bool stdp, bool wide, int device, bool dry,
-                                  cudaStream_t s) {
-    if (stdp) return wide ? launch_multi_5<MODEL, CHEMG, NTREL, true, NET, true>(p, t, m, device, dry, s)
-                          : launch_multi_5<MODEL, CHEMG, NTREL, true, NET, false>(p, t, m, device, dry, s);
-    return wide ? launch_multi_5<MODEL, CHEMG, NTREL, false, NET, true>(p, t, m, device, dry, s)
-                : launch_multi_5<MODEL, CHEMG, NTREL, false, NET, false>(p, t, m, device, dry, s);
-}
-
-template <int MODEL>
-static cudaError_t launch_multi_model(const StepParams &p, const TrainParams &t, const MultiParams &m, int chemg, bool ntrel, bool stdp, bool net,
-                                      bool wide, int device, bool dry, cudaStream_t s) {
-    if (net) {
-        if (chemg) return launch_multi_3<MODEL, 3, true, true>(p, t, m, stdp, wide, device, dry, s);
-        if (ntrel) return launch_multi_3<MODEL, 0, true, true>(p, t, m, stdp, wide, device, dry, s);
-        return launch_multi_3<MODEL, 0, false, true>(p, t, m, stdp, wide, device, dry, s);
-    }
-    if (chemg == 1) return launch_multi_3<MODEL, 1, true, false>(p, t, m, stdp, wide, device, dry, s);
-    if (chemg == 3) return launch_multi_3<MODEL, 3, true, false>(p, t, m, stdp, wide, device, dry, s);
-    if (ntrel) return launch_multi_3<MODEL, 0, true, false>(p, t, m, stdp, wide, device, dry, s);
-    return launch_multi_3<MODEL, 0, false, false>(p, t, m, stdp, wide, device, dry, s);
-}
-
-cudaError_t launch_step_multi(const StepParams &p, const TrainParams &t, const MultiParams &m, int model, int chemg, bool ntrel, bool stdp,
-                              bool net, bool wide, int device, bool dry, cudaStream_t s) {
-    switch (model) {
-    case SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE: return launch_multi_model<SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE: return launch_multi_model<SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE: return launch_multi_model<SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE: return launch_multi_model<SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_IZHIKEVICH: return launch_multi_model<SNN_MODEL_IZHIKEVICH>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_LEAKY_IZHIKEVICH: return launch_multi_model<SNN_MODEL_LEAKY_IZHIKEVICH>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE: return launch_multi_model<SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_HODGKIN_HUXLEY: return launch_multi_model<SNN_MODEL_HODGKIN_HUXLEY>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    case SNN_MODEL_BCM_IZHIKEVICH: return launch_multi_model<SNN_MODEL_BCM_IZHIKEVICH>(p, t, m, chemg, ntrel, stdp, net, wide, device, dry, s);
-    }
-    return cudaErrorInvalidValue;
+cudaError_t launch_step_multi(const StepParams &p, const TrainParams &t, const MultiParams &m, const StepSpec &spec, bool wide, int device,
+                              bool dry, cudaStream_t s) {
+    return dispatch_step(spec, cudaErrorInvalidValue, [&](auto k) {
+        using K = decltype(k);
+        return wide ? launch_multi<K, true>(p, t, m, device, dry, s) : launch_multi<K, false>(p, t, m, device, dry, s);
+    });
 }
 
 }  // namespace snn

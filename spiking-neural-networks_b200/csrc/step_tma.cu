@@ -135,47 +135,20 @@ __global__ void __launch_bounds__(kTmaThreads, tma_min_ctas<MODEL, CHEMG>()) ste
 // ------------------------------------------------------------------------------------------------
 // launcher
 // ------------------------------------------------------------------------------------------------
-template <int MODEL, int CHEMG, bool NTREL>
-static cudaError_t launch_tma_3(const StepParams &p, const TmaParams &tp, bool stdp, unsigned grid, size_t smem, cudaStream_t s) {
-    if (stdp) {
-        auto k = step_tma_kernel<MODEL, CHEMG, NTREL, true>;
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
-    } else {
-        auto k = step_tma_kernel<MODEL, CHEMG, NTREL, false>;
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
-    }
-    return cudaGetLastError();
-}
-
-template <int MODEL>
-static cudaError_t launch_tma_model(const StepParams &p, const TmaParams &tp, int chemg, bool ntrel, bool stdp, unsigned grid,
-                                    size_t smem, cudaStream_t s) {
-    if (chemg == 1) return launch_tma_3<MODEL, 1, true>(p, tp, stdp, grid, smem, s);
-    if (chemg == 3) return launch_tma_3<MODEL, 3, true>(p, tp, stdp, grid, smem, s);
-    if (ntrel) return launch_tma_3<MODEL, 0, true>(p, tp, stdp, grid, smem, s);
-    return launch_tma_3<MODEL, 0, false>(p, tp, stdp, grid, smem, s);
-}
-
-cudaError_t launch_step_tma(const StepParams &p, const TmaParams &tp, int model, int chemg, bool ntrel, bool stdp, unsigned grid,
-                            cudaStream_t s) {
+cudaError_t launch_step_tma(const StepParams &p, const TmaParams &tp, const StepSpec &spec, unsigned grid, cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
     const size_t smem = (size_t)tp.stages * tp.stage_bytes + 2 * tp.stages * sizeof(uint64_t);
-    switch (model) {
-    case SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE: return launch_tma_model<SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE: return launch_tma_model<SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE: return launch_tma_model<SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE: return launch_tma_model<SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_IZHIKEVICH: return launch_tma_model<SNN_MODEL_IZHIKEVICH>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_LEAKY_IZHIKEVICH: return launch_tma_model<SNN_MODEL_LEAKY_IZHIKEVICH>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE: return launch_tma_model<SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_HODGKIN_HUXLEY: return launch_tma_model<SNN_MODEL_HODGKIN_HUXLEY>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_BCM_IZHIKEVICH: return launch_tma_model<SNN_MODEL_BCM_IZHIKEVICH>(p, tp, chemg, ntrel, stdp, grid, smem, s);
-    }
-    return cudaErrorInvalidValue;
+    return dispatch_step(spec, cudaErrorInvalidValue, [&](auto k) {
+        using K = decltype(k);
+        if constexpr (K::NET) {
+            return cudaErrorInvalidValue;   // single lattices only
+        } else {
+            auto kern = step_tma_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP>;
+            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+            return launch_pdl(pdl_ok(p), kern, dim3(grid), dim3(kTmaThreads), smem, s, p, tp);
+        }
+    });
 }
 
 }  // namespace snn

@@ -43,66 +43,36 @@ __global__ void __launch_bounds__(kWideWarps * 32) step_wide_kernel(const __grid
     neuron_step<MODEL, CHEMG, NTREL, STDP, NET>(p, src, warp_global, lane, ln, lnc, valid, false, false);
 }
 
-template <int MODEL, int CHEMG, bool NTREL, bool NET>
-static cudaError_t launch_wide_3(const StepParams &p, bool stdp, unsigned char *scratch, uint32_t chunks_cap, const TrainParams *trains, cudaStream_t s) {
-    const unsigned grid = (p.n_neurons + 31u) / 32u;
-    static const TrainParams no_trains{};
-    auto launch = [&](auto k, dim3 g, size_t smem, uint32_t stage, WideSplit sp) -> cudaError_t {
-        if (smem > 48u * 1024u) { cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); if (e != cudaSuccess) return e; }
-        return launch_pdl(pdl_ok(p), k, g, dim3(kWideWarps * 32), smem, s, p, stage, sp, (sp.mode == 2u && trains) ? *trains : no_trains);
-    };
-    auto both = [&](dim3 g, size_t smem, uint32_t stage, WideSplit sp) -> cudaError_t {
-        if (stdp) return launch(step_wide_kernel<MODEL, CHEMG, NTREL, true, NET>, g, smem, stage, sp);
-        return launch(step_wide_kernel<MODEL, CHEMG, NTREL, false, NET>, g, smem, stage, sp);
-    };
-    if (scratch && chunks_cap) {
-        // the per-edge work of every (slice, chunk) pair on its own CTA — all SMs — then one CTA per slice for the ordered additions
-        // and the neuron update; the terms travel through L2
-        cudaError_t e = both(dim3(grid, chunks_cap), 0, 0u, WideSplit{1u, scratch, chunks_cap, grid});
-        if (e != cudaSuccess) return e;
-        constexpr uint32_t n_acc = 1u + (CHEMG == 3 ? (uint32_t)kNT : (CHEMG == 1 ? 1u : 0u));
-        const unsigned train_ctas = (NET && trains) ? ((trains->n_trains + 31u) / 32u + kWideWarps - 1u) / kWideWarps : 0u;
-        return both(dim3(grid + train_ctas, n_acc), kWideSumBufs * (kWideChunk * 32u * 4u + 128u), 0u, WideSplit{2u, scratch, chunks_cap, grid});
-    }
-    // small networks: the node state rides in shared memory next to the chunk buffers (WideStage, step_body.cuh)
-    const uint32_t sb = wide_stage_bytes(p.n_nodes, NET ? p.n_trains : 0u);
-    const bool stage = p.n_nodes <= kWideStageMaxNodes && 2u * wide_buf_bytes(CHEMG) + sb <= 200u * 1024u;
-    return both(dim3(grid), 2u * wide_buf_bytes(CHEMG) + (stage ? sb : 0u), stage ? 1u : 0u, WideSplit{0u, nullptr, 0u, grid});
-}
-
-template <int MODEL>
-static cudaError_t launch_wide_model(const StepParams &p, int chemg, bool ntrel, bool stdp, bool net, unsigned char *scratch, uint32_t chunks_cap,
-                                     const TrainParams *trains, cudaStream_t s) {
-    if (net) {
-        if (chemg) return launch_wide_3<MODEL, 3, true, true>(p, stdp, scratch, chunks_cap, trains, s);
-        if (ntrel) return launch_wide_3<MODEL, 0, true, true>(p, stdp, scratch, chunks_cap, trains, s);
-        return launch_wide_3<MODEL, 0, false, true>(p, stdp, scratch, chunks_cap, trains, s);
-    }
-    if (chemg == 1) return launch_wide_3<MODEL, 1, true, false>(p, stdp, scratch, chunks_cap, trains, s);
-    if (chemg == 3) return launch_wide_3<MODEL, 3, true, false>(p, stdp, scratch, chunks_cap, trains, s);
-    if (ntrel) return launch_wide_3<MODEL, 0, true, false>(p, stdp, scratch, chunks_cap, trains, s);
-    return launch_wide_3<MODEL, 0, false, false>(p, stdp, scratch, chunks_cap, trains, s);
-}
-
 uint32_t wide_chunk_bytes(int chemg) { return wide_buf_bytes(chemg); }
 uint32_t wide_chunk_krows() { return kWideChunk; }
 size_t wide_part_bytes() { return wide_part_bytes_per_slice(); }
 
-cudaError_t launch_step_wide(const StepParams &p, int model, int chemg, bool ntrel, bool stdp, bool net, unsigned char *scratch, uint32_t chunks_cap,
-                             const TrainParams *trains, cudaStream_t s) {
+cudaError_t launch_step_wide(const StepParams &p, const StepSpec &spec, unsigned char *scratch, uint32_t chunks_cap, const TrainParams *trains,
+                             cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
-    switch (model) {
-    case SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE: return launch_wide_model<SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE: return launch_wide_model<SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE: return launch_wide_model<SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE: return launch_wide_model<SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_IZHIKEVICH: return launch_wide_model<SNN_MODEL_IZHIKEVICH>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_LEAKY_IZHIKEVICH: return launch_wide_model<SNN_MODEL_LEAKY_IZHIKEVICH>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE: return launch_wide_model<SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_HODGKIN_HUXLEY: return launch_wide_model<SNN_MODEL_HODGKIN_HUXLEY>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    case SNN_MODEL_BCM_IZHIKEVICH: return launch_wide_model<SNN_MODEL_BCM_IZHIKEVICH>(p, chemg, ntrel, stdp, net, scratch, chunks_cap, trains, s);
-    }
-    return cudaErrorInvalidValue;
+    const unsigned grid = (p.n_neurons + 31u) / 32u;
+    static const TrainParams no_trains{};
+    return dispatch_step(spec, cudaErrorInvalidValue, [&](auto k) {
+        using K = decltype(k);
+        auto launch = [&](dim3 g, size_t smem, uint32_t stage, WideSplit sp) -> cudaError_t {
+            auto kern = step_wide_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, K::NET>;
+            if (smem > 48u * 1024u) { cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); if (e != cudaSuccess) return e; }
+            return launch_pdl(pdl_ok(p), kern, g, dim3(kWideWarps * 32), smem, s, p, stage, sp, (sp.mode == 2u && trains) ? *trains : no_trains);
+        };
+        if (scratch && chunks_cap) {
+            // the per-edge work of every (slice, chunk) pair on its own CTA — all SMs — then one CTA per slice for the ordered additions
+            // and the neuron update; the terms travel through L2
+            cudaError_t e = launch(dim3(grid, chunks_cap), 0, 0u, WideSplit{1u, scratch, chunks_cap, grid});
+            if (e != cudaSuccess) return e;
+            constexpr uint32_t n_acc = 1u + (K::CHEMG == 3 ? (uint32_t)kNT : (K::CHEMG == 1 ? 1u : 0u));
+            const unsigned train_ctas = (K::NET && trains) ? ((trains->n_trains + 31u) / 32u + kWideWarps - 1u) / kWideWarps : 0u;
+            return launch(dim3(grid + train_ctas, n_acc), kWideSumBufs * (kWideChunk * 32u * 4u + 128u), 0u, WideSplit{2u, scratch, chunks_cap, grid});
+        }
+        // small networks: the node state rides in shared memory next to the chunk buffers (WideStage, step_body.cuh)
+        const uint32_t sb = wide_stage_bytes(p.n_nodes, K::NET ? p.n_trains : 0u);
+        const bool stage = p.n_nodes <= kWideStageMaxNodes && 2u * wide_buf_bytes(K::CHEMG) + sb <= 200u * 1024u;
+        return launch(dim3(grid), 2u * wide_buf_bytes(K::CHEMG) + (stage ? sb : 0u), stage ? 1u : 0u, WideSplit{0u, nullptr, 0u, grid});
+    });
 }
 
 }  // namespace snn

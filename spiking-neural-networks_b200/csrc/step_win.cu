@@ -290,48 +290,21 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
 // ------------------------------------------------------------------------------------------------
 // launcher
 // ------------------------------------------------------------------------------------------------
-template <int MODEL, int CHEMG, bool NTREL>
-static cudaError_t launch_win_3(const StepParams &p, const WinParams &wp, bool stdp, unsigned grid, size_t smem, cudaStream_t s) {
-    constexpr int G = win_groups(MODEL, CHEMG);
-    if (stdp) {
-        auto k = step_win_kernel<MODEL, CHEMG, NTREL, true, G>;
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
-    } else {
-        auto k = step_win_kernel<MODEL, CHEMG, NTREL, false, G>;
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        return launch_pdl(pdl_ok(p), k, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
-    }
-    return cudaGetLastError();
-}
-
-template <int MODEL>
-static cudaError_t launch_win_model(const StepParams &p, const WinParams &wp, int chemg, bool ntrel, bool stdp, unsigned grid,
-                                    size_t smem, cudaStream_t s) {
-    if (chemg == 1) return launch_win_3<MODEL, 1, true>(p, wp, stdp, grid, smem, s);
-    if (chemg == 3) return launch_win_3<MODEL, 3, true>(p, wp, stdp, grid, smem, s);
-    if (ntrel) return launch_win_3<MODEL, 0, true>(p, wp, stdp, grid, smem, s);
-    return launch_win_3<MODEL, 0, false>(p, wp, stdp, grid, smem, s);
-}
-
-cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, int model, int chemg, bool ntrel, bool stdp, unsigned grid,
-                            cudaStream_t s) {
+cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const StepSpec &spec, unsigned grid, cudaStream_t s) {
     if (p.n_neurons == 0) return cudaSuccess;
     const size_t smem = (size_t)wp.stages * wp.stage_bytes + 2 * wp.stages * sizeof(uint64_t);
-    switch (model) {
-    case SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE: return launch_win_model<SNN_MODEL_LEAKY_INTEGRATE_AND_FIRE>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE: return launch_win_model<SNN_MODEL_QUADRATIC_INTEGRATE_AND_FIRE>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE: return launch_win_model<SNN_MODEL_ADAPTIVE_LEAKY_INTEGRATE_AND_FIRE>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE: return launch_win_model<SNN_MODEL_ADAPTIVE_EXP_LEAKY_INTEGRATE_AND_FIRE>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_IZHIKEVICH: return launch_win_model<SNN_MODEL_IZHIKEVICH>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_LEAKY_IZHIKEVICH: return launch_win_model<SNN_MODEL_LEAKY_IZHIKEVICH>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE: return launch_win_model<SNN_MODEL_SIMPLE_LEAKY_INTEGRATE_AND_FIRE>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_HODGKIN_HUXLEY: return launch_win_model<SNN_MODEL_HODGKIN_HUXLEY>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    case SNN_MODEL_BCM_IZHIKEVICH: return launch_win_model<SNN_MODEL_BCM_IZHIKEVICH>(p, wp, chemg, ntrel, stdp, grid, smem, s);
-    }
-    return cudaErrorInvalidValue;
+    return dispatch_step(spec, cudaErrorInvalidValue, [&](auto k) {
+        using K = decltype(k);
+        if constexpr (K::NET) {
+            return cudaErrorInvalidValue;   // single lattices only
+        } else {
+            constexpr int G = win_groups(K::MODEL, K::CHEMG);
+            auto kern = step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G>;
+            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+            return launch_pdl(pdl_ok(p), kern, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
+        }
+    });
 }
 
 }  // namespace snn
