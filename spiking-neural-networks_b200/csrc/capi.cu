@@ -365,11 +365,11 @@ int32_t snn_lattice_ipc_export(snn_lattice_t *h, void *blob) {
 }
 int32_t snn_lattice_ipc_attach(snn_lattice_t *h, int32_t direction, const void *blob) {
     if (!h || !blob) return SNN_INVALID_ARGUMENT;
-    SNN_TRY return h->e->ipc_attach(direction, (const snn::IpcBlob *)blob); SNN_CATCH(h)
+    SNN_TRY return h->e->attach_strip(direction, (const snn::IpcBlob *)blob, nullptr); SNN_CATCH(h)
 }
 int32_t snn_lattice_attach_local(snn_lattice_t *h, int32_t direction, snn_lattice_t *neighbour) {
     if (!h || !neighbour) return SNN_INVALID_ARGUMENT;
-    SNN_TRY return h->e->attach_local(direction, neighbour->e); SNN_CATCH(h)
+    SNN_TRY return h->e->attach_strip(direction, nullptr, neighbour->e); SNN_CATCH(h)
 }
 int32_t snn_lattice_gpart_wants(snn_lattice_t *h, int32_t peer, uint32_t *global_idx, uint64_t capacity, uint64_t *n, uint32_t *first_slot) {
     if (!h) return SNN_INVALID_ARGUMENT;

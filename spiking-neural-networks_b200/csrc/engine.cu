@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstring>
 #include <functional>
+#include <numeric>
 
 namespace snn {
 
@@ -51,14 +52,15 @@ Engine::Engine(int model_, int ntk_, int rck_, int train_kind_, int refract_, in
     seed = splitmix64(0x5EED5EEDull + serial.fetch_add(1));
 }
 
+static void unmap_peer(PeerMap &m) {
+    if (m.ipc) { cudaIpcCloseMemHandle(m.slab); cudaIpcCloseMemHandle(m.flags); }
+    m = PeerMap{};
+}
+
 Engine::~Engine() {
     if (device >= 0) cudaSetDevice(device);
-    for (int d = 0; d < 2; ++d) {
-        if (peer_slab_[d]) cudaIpcCloseMemHandle(peer_slab_[d]);
-        if (peer_flags_[d]) cudaIpcCloseMemHandle(peer_flags_[d]);
-    }
-    for (auto &G : gpeers_)
-        if (G.ipc) { if (G.slab) cudaIpcCloseMemHandle(G.slab); if (G.flags) cudaIpcCloseMemHandle(G.flags); }
+    for (auto &m : strip_map_) unmap_peer(m);
+    for (auto &G : gpeers_) unmap_peer(G.map);
     if (d_gpeers_) cudaFree(d_gpeers_);
     if (d_gexp_off_) cudaFree(d_gexp_off_);
     if (d_gexp_ent_) cudaFree(d_gexp_ent_);
@@ -253,7 +255,7 @@ int Engine::alloc_device() {
 
 int Engine::ensure_chem() {
     if (chem_alloc_) return SNN_OK;
-    if (peer_slab_[0] || peer_slab_[1] || layout_frozen_) return fail(SNN_UNSUPPORTED, "chemical fields must be set before the halo slab is exported");
+    if (layout_frozen_) return fail(SNN_UNSUPPORTED, "chemical fields must be set before the halo slab is exported");
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
     // grow the slab to hold T[2]
     const size_t tb = round_up(node_cap_ * 4 * kNT, 256);
@@ -295,9 +297,6 @@ int Engine::set_partition(uint32_t rows_g, uint32_t cols, int rank, int world) {
     return SNN_OK;
 }
 
-struct FieldSnap { std::string name; int dtype; std::vector<uint8_t> data; uint64_t count; };
-struct LatSnap { uint64_t id; std::vector<FieldSnap> fields; };
-
 int Engine::add_lattice(uint64_t id, uint32_t rows, uint32_t cols, bool is_train, bool is_reward) {
     // LatticeNetwork::add_lattice / add_spike_train_lattice, neuron/mod.rs:1663-1698
     if (find(id)) return fail(SNN_NET_GRAPH_ID_ALREADY_PRESENT, "Graph id already present in network, id: " + std::to_string(id));
@@ -310,17 +309,18 @@ int Engine::add_lattice(uint64_t id, uint32_t rows, uint32_t cols, bool is_train
     nl.id = id; nl.rows = rows; nl.cols = cols; nl.n = (uint64_t)rows * cols; nl.is_train = is_train;
     if ((is_train ? n_trains : n_neurons) + nl.n + 64ull * (part_world > 1 ? cols : 0) > kMaxNodes)
         return fail(SNN_UNSUPPORTED, "lattice too large for one device (node index is 28 bits)");
-    return relayout_add(nl);
+    // lattices are added at set-up time; the single-lattice (large) case never has anything to snapshot
+    if (dev_weights_newer_) { int r = sync_weights_to_host(); if (r) return r; }
+    return relayout([&]() { lats_.push_back(nl); });
 }
 
-int Engine::relayout_add(const Lat &nl) {
-    // snapshot every existing field through the public get path, rebuild the device layout, restore.
-    // Lattices are added at set-up time; the single-lattice (large) case never has anything to snapshot.
-    if (dev_weights_newer_) { int r = sync_weights_to_host(); if (r) return r; }
-    std::vector<LatSnap> snaps;
+// Rebuild the device layout after `change` alters its parameters: snapshot every field through the public get path, free,
+// change, allocate, restore.
+int Engine::relayout(const std::function<void()> &change) {
+    struct FieldSnap { uint64_t id; std::string name; int dtype; uint64_t count; std::vector<uint8_t> data; };
+    std::vector<FieldSnap> snaps;
     const bool had_chem = chem_alloc_;
     for (auto &L : lats_) {
-        LatSnap s; s.id = L.id;
         uint32_t cnt = 0; field_count(L.id, &cnt);
         for (uint32_t i = 0; i < cnt; ++i) {
             const char *name; int32_t dt; uint32_t per;
@@ -329,25 +329,24 @@ int Engine::relayout_add(const Lat &nl) {
             if (lookup_field(L, name, &fd)) continue;
             const bool is_chem = fd.kind == FK_NT_FLAGS || fd.kind == FK_NT_T || fd.kind == FK_NT || fd.kind == FK_RC_FLAGS || fd.kind == FK_RC;
             if (is_chem && !had_chem) continue;
-            FieldSnap f; f.name = name; f.dtype = dt; f.count = L.n * per; f.data.resize(std::max<uint64_t>(f.count, 1) * 4);
+            FieldSnap f{L.id, name, dt, L.n * per, {}};
+            f.data.resize(std::max<uint64_t>(f.count, 1) * 4);
             int r = get_field(L.id, name, f.data.data(), f.count, dt);
             if (r) return r;
-            s.fields.push_back(std::move(f));
+            snaps.push_back(std::move(f));
         }
-        snaps.push_back(std::move(s));
     }
     const uint64_t saved_clock = internal_clock;
     free_device();
-    lats_.push_back(nl);
+    change();
     compute_layout();
     int r = alloc_device();
     if (r) return r;
     if (had_chem) { r = ensure_chem(); if (r) return r; }
-    for (auto &s : snaps)
-        for (auto &f : s.fields) {
-            r = set_field(s.id, f.name.c_str(), f.data.data(), f.count, f.dtype);
-            if (r) return r;
-        }
+    for (auto &f : snaps) {
+        r = set_field(f.id, f.name.c_str(), f.data.data(), f.count, f.dtype);
+        if (r) return r;
+    }
     // re-upload preset firing times
     for (auto &L : lats_)
         if (L.is_train && !L.ft_off.empty()) {
@@ -674,41 +673,6 @@ int Engine::set_preset_firing_times(uint64_t id, const uint64_t *offsets, const 
 // ------------------------------------------------------------------------------------------------
 // Node order on a rank: [ghosts below my range, ascending global index | my neurons | ghosts above], so local order == global
 // order and the canonical (ascending presynaptic index) summation order of every row is the one of the unpartitioned lattice.
-int Engine::relayout_keep_fields(const std::function<void()> &change) {
-    // snapshot every field through the public get path, change the layout parameters, rebuild, restore
-    std::vector<LatSnap> snaps;
-    const bool had_chem = chem_alloc_;
-    for (auto &L : lats_) {
-        LatSnap sn; sn.id = L.id;
-        uint32_t cnt = 0; field_count(L.id, &cnt);
-        for (uint32_t i = 0; i < cnt; ++i) {
-            const char *name; int32_t dt; uint32_t per;
-            field_info(L.id, i, &name, &dt, &per);
-            FieldDef fd;
-            if (lookup_field(L, name, &fd)) continue;
-            const bool is_chem = fd.kind == FK_NT_FLAGS || fd.kind == FK_NT_T || fd.kind == FK_NT || fd.kind == FK_RC_FLAGS || fd.kind == FK_RC;
-            if (is_chem && !had_chem) continue;
-            FieldSnap f; f.name = name; f.dtype = dt; f.count = L.n * per; f.data.resize(std::max<uint64_t>(f.count, 1) * 4);
-            int r = get_field(L.id, name, f.data.data(), f.count, dt);
-            if (r) return r;
-            sn.fields.push_back(std::move(f));
-        }
-        snaps.push_back(std::move(sn));
-    }
-    const uint64_t saved_clock = internal_clock;
-    free_device();
-    change();
-    compute_layout();
-    int r = alloc_device();
-    if (r) return r;
-    if (had_chem) { r = ensure_chem(); if (r) return r; }
-    for (auto &sn : snaps)
-        for (auto &f : sn.fields) { r = set_field(sn.id, f.name.c_str(), f.data.data(), f.count, f.dtype); if (r) return r; }
-    internal_clock = saved_clock;
-    graph_dirty_ = true;
-    return SNN_OK;
-}
-
 int Engine::gpart_enable(const std::vector<uint32_t> &remote) {
     if (layout_frozen_) return fail(SNN_UNSUPPORTED, "the graph of a partitioned handle cannot change its reach after the slab was exported");
     const uint64_t cols = lats_[0].cols, g0 = (uint64_t)row0_global * cols, g1 = g0 + n_neurons;
@@ -717,7 +681,7 @@ int Engine::gpart_enable(const std::vector<uint32_t> &remote) {
     (void)g1;
     if (gpart_ && lo == g_lo_ && hi == g_hi_) return SNN_OK;
     for (int d = 0; d < 2; ++d) if (halo_dir_[d].active) return fail(SNN_UNSUPPORTED, "handle already attached as a row strip");
-    int r = relayout_keep_fields([&]() { gpart_ = true; g_lo_ = lo; g_hi_ = hi; });
+    int r = relayout([&]() { gpart_ = true; g_lo_ = lo; g_hi_ = hi; });
     if (r) return r;
     gpeers_.clear();
     gpart_dirty_ = true;
@@ -755,8 +719,13 @@ Engine::GPeerHost *Engine::gpeer(int rank, bool create) {
     return &*gpeers_.insert(it, std::move(g));
 }
 
-int Engine::gpart_wants(int peer, uint32_t *global_idx, uint64_t capacity, uint64_t *n, uint32_t *first_slot) {
+int Engine::check_peer_rank(int peer) {
     if (part_world <= 1 || peer < 0 || peer >= part_world || peer == part_rank) return fail(SNN_INVALID_ARGUMENT, "bad peer rank");
+    return SNN_OK;
+}
+
+int Engine::gpart_wants(int peer, uint32_t *global_idx, uint64_t capacity, uint64_t *n, uint32_t *first_slot) {
+    if (int r = check_peer_rank(peer)) return r;
     if (n) *n = 0;
     if (first_slot) *first_slot = 0;
     if (!gpart_) return SNN_OK;   // a row strip has no gather lists
@@ -776,7 +745,7 @@ int Engine::gpart_wants(int peer, uint32_t *global_idx, uint64_t capacity, uint6
 }
 
 int Engine::gpart_set_exports(int peer, const uint32_t *global_idx, uint64_t n, uint32_t first_slot_at_peer) {
-    if (part_world <= 1 || peer < 0 || peer >= part_world || peer == part_rank) return fail(SNN_INVALID_ARGUMENT, "bad peer rank");
+    if (int r = check_peer_rank(peer)) return r;
     if (n && !global_idx) return fail(SNN_INVALID_ARGUMENT, "null argument");
     if (!gpart_) return fail(SNN_INVALID_ARGUMENT, "not a general-graph partition (set SNN_OPT_GENERAL_PARTITION before the graph on every rank)");
     if (n == 0 && !gpeer(peer, false)) return SNN_OK;
@@ -793,63 +762,30 @@ int Engine::gpart_set_exports(int peer, const uint32_t *global_idx, uint64_t n, 
     return SNN_OK;
 }
 
-int Engine::gpart_attach(int peer, const IpcBlob *blob_in, Engine *local_peer) {
-    if (part_world <= 1 || peer < 0 || peer >= part_world || peer == part_rank) return fail(SNN_INVALID_ARGUMENT, "bad peer rank");
+int Engine::gpart_attach(int peer, const IpcBlob *blob, Engine *local) {
+    if (int r = check_peer_rank(peer)) return r;
     if (!gpart_) return fail(SNN_INVALID_ARGUMENT, "not a general-graph partition (set SNN_OPT_GENERAL_PARTITION before the graph on every rank)");
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
-    GPeerHost *G = gpeer(peer, true);
-    if (G->attached) return fail(SNN_INVALID_ARGUMENT, "peer already attached");
-    IpcBlob blob;
-    if (local_peer) {
-        if (local_peer == this) return fail(SNN_INVALID_ARGUMENT, "bad peer handle");
-        if (local_peer->device != device) {
-            int can = 0;
-            CK(cudaDeviceCanAccessPeer(&can, device, local_peer->device), SNN_GPU_GET_DEVICE_FAILURE);
-            if (!can) return fail(SNN_UNSUPPORTED, "no peer access between the two devices");
-            cudaError_t e = cudaDeviceEnablePeerAccess(local_peer->device, 0);
-            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return cuda_fail(e, SNN_GPU_GET_DEVICE_FAILURE, "cudaDeviceEnablePeerAccess");
-            cudaGetLastError();
-        }
-        int r = local_peer->ipc_export_layout(&blob);
-        if (r) return fail(r, local_peer->last_error);
-        G->slab = local_peer->slab_; G->flags = local_peer->flags_;
-        local_peer->layout_frozen_ = true;
-        local_peers_.push_back(local_peer);
-    } else {
-        blob = *blob_in;
-        if (blob.magic != 0x534E4E42u || blob.version != SNN_B200_ABI_VERSION) return fail(SNN_INVALID_ARGUMENT, "bad ipc blob");
-        CK(cudaIpcOpenMemHandle(&G->slab, blob.slab, cudaIpcMemLazyEnablePeerAccess), SNN_GPU_BUFFER_CREATE_ERROR);
-        CK(cudaIpcOpenMemHandle(&G->flags, blob.flags, cudaIpcMemLazyEnablePeerAccess), SNN_GPU_BUFFER_CREATE_ERROR);
-        G->ipc = true;
-    }
-    if (blob.rank != peer || blob.world != part_world) return fail(SNN_INVALID_ARGUMENT, "ipc blob is not from that rank");
-    if ((blob.chem != 0) != chem_alloc_) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on chemistry");
-    if ((blob.off_act[0] != 0) != (ACT_[0] != nullptr)) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on the neuron model");
-    G->view = blob;
-    G->attached = true;
-    layout_frozen_ = true;
-    // neurotransmitter / receptor type flags of the ghosts that this peer owns (baked into the col words of edges from ghosts)
-    uint64_t cnt = 0; uint32_t slot0 = 0;
-    int r = gpart_wants(peer, nullptr, 0, &cnt, &slot0);
+    const GPeerHost *old = gpeer(peer, false);
+    if (old && old->attached) return fail(SNN_INVALID_ARGUMENT, "peer already attached");
+    GPeerHost G = old ? *old : GPeerHost{};
+    G.rank = peer;
+    int r = map_peer(blob, local, peer, &G.map, &G.view);
     if (r) return r;
-    if (cnt) {
-        std::vector<uint8_t> pf(blob.n_neurons);
-        CK(cudaMemcpy(pf.data(), (const uint8_t *)G->slab + blob.off_flags + blob.own0, blob.n_neurons, cudaMemcpyDefault), SNN_GPU_BUFFER_READ_ERROR);
-        const uint64_t cols = lats_[0].cols, q0 = (uint64_t)snn_partition_begin(rows_global, part_world, peer) * cols;
-        bool changed = false;
-        for (uint64_t k = 0; k < cnt; ++k) {
-            const uint32_t node = slot0 + (uint32_t)k;
-            const uint8_t f = pf[node_to_global(node) - q0];
-            changed |= h_node_flags_[node] != f;
-            h_node_flags_[node] = f;
-        }
-        if (changed) {
-            CK(h2d_sync(node_flags_ + slot0, h_node_flags_.data() + slot0, cnt, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-            flags_cache_valid_ = false;
-            if (dev_weights_newer_) { r = sync_weights_to_host(); if (r) return r; }
-            graph_dirty_ = true;
-        }
+    // the ghosts that this peer owns: slots slot0 .. slot0 + cnt - 1, at the peer's neuron numbers node_to_global(slot) - q0
+    uint64_t cnt = 0; uint32_t slot0 = 0;
+    r = gpart_wants(peer, nullptr, 0, &cnt, &slot0);
+    if (!r && cnt) {
+        const uint64_t q0 = (uint64_t)snn_partition_begin(rows_global, part_world, peer) * lats_[0].cols;
+        std::vector<uint32_t> pick(cnt);
+        for (uint64_t k = 0; k < cnt; ++k) pick[k] = (uint32_t)(node_to_global(slot0 + (uint32_t)k) - q0);
+        r = import_ghost_flags(slot0, (const uint8_t *)G.map.slab + G.view.off_flags + G.view.own0, G.view.n_neurons, pick, false);
     }
+    if (r) { unmap_peer(G.map); return r; }
+    G.attached = true;
+    *gpeer(peer, true) = std::move(G);
+    layout_frozen_ = true;
+    if (local) { local->layout_frozen_ = true; local_peers_.push_back(local); }
     gpart_dirty_ = true;
     return SNN_OK;
 }
@@ -867,13 +803,13 @@ int Engine::gpart_build_device() {
         if (!G.attached) return fail(SNN_INVALID_ARGUMENT, "general-graph partition: rank " + std::to_string(G.rank) + " is not attached");
         GPeer &D = hp[q];
         for (int k = 0; k < 2; ++k) {
-            D.v[k] = (float *)((char *)G.slab + G.view.off_v[k]);
-            D.lft[k] = (int *)((char *)G.slab + G.view.off_lft[k]);
-            D.t[k] = (float *)((char *)G.slab + G.view.off_t[k]);
-            if (ACT_[0]) act[2 * q + k] = (float *)((char *)G.slab + G.view.off_act[k]);
+            D.v[k] = (float *)((char *)G.map.slab + G.view.off_v[k]);
+            D.lft[k] = (int *)((char *)G.map.slab + G.view.off_lft[k]);
+            D.t[k] = (float *)((char *)G.map.slab + G.view.off_t[k]);
+            if (ACT_[0]) act[2 * q + k] = (float *)((char *)G.map.slab + G.view.off_act[k]);
         }
         D.t_stride = G.view.t_stride;
-        D.peer_flag = (unsigned long long *)G.flags + 8 + part_rank;
+        D.peer_flag = (unsigned long long *)G.map.flags + 8 + part_rank;
         D.my_flag = flags_ + 8 + G.rank;
         for (size_t k = 0; k < G.exp_local.size(); ++k) per[G.exp_local[k]].push_back(((uint32_t)q << 28) | (G.peer_slot0 + (uint32_t)k));
     }
@@ -1029,34 +965,10 @@ int Engine::connect_grid(uint64_t id, uint32_t radius, float weight) {
         const uint32_t need = radius * A->cols;
         if (need > A->n && A->n) return fail(SNN_UNSUPPORTED, "strip is thinner than the stencil radius");
         if (need != halo_) {
-            // re-layout with a halo of `radius` rows (snapshot/restore through the field path)
-            if (peer_slab_[0] || peer_slab_[1] || layout_frozen_) return fail(SNN_UNSUPPORTED, "cannot change the stencil after the halo slab was exported");
-            Lat copy = *A;
-            std::vector<LatSnap> unused;
-            // temporarily remove the lattice and add it back with the new halo
-            std::vector<FieldSnap> fields;
-            uint32_t cnt = 0; field_count(id, &cnt);
-            for (uint32_t i = 0; i < cnt; ++i) {
-                const char *name; int32_t dt; uint32_t per;
-                field_info(id, i, &name, &dt, &per);
-                FieldDef fd;
-                if (lookup_field(*A, name, &fd)) continue;
-                const bool is_chem = fd.kind == FK_NT_FLAGS || fd.kind == FK_NT_T || fd.kind == FK_NT || fd.kind == FK_RC_FLAGS || fd.kind == FK_RC;
-                if (is_chem && !chem_alloc_) continue;
-                FieldSnap f; f.name = name; f.dtype = dt; f.count = A->n * per; f.data.resize(std::max<uint64_t>(f.count, 1) * 4);
-                r = get_field(id, name, f.data.data(), f.count, dt);
-                if (r) return r;
-                fields.push_back(std::move(f));
-            }
-            const bool had_chem = chem_alloc_;
-            free_device();
-            halo_ = need;
-            compute_layout();
-            r = alloc_device();
+            // re-layout with a halo of `radius` rows
+            if (layout_frozen_) return fail(SNN_UNSUPPORTED, "cannot change the stencil after the halo slab was exported");
+            r = relayout([&]() { halo_ = need; });
             if (r) return r;
-            if (had_chem) { r = ensure_chem(); if (r) return r; }
-            for (auto &f : fields) { r = set_field(id, f.name.c_str(), f.data.data(), f.count, f.dtype); if (r) return r; }
-            A = B = find(id);
         }
     }
     // the learned weights of every OTHER block live on the device until synced: replacing this block must not discard them
@@ -1134,7 +1046,7 @@ int Engine::finalize_graph() {
     if (!reuse) CK(dev_alloc(&slice_off_, (size_t)n_slices_ + 1), SNN_GPU_BUFFER_CREATE_ERROR);
     // partitioned handles: ghost rows inherit the neurotransmitter type sets of the adjacent owned rows
     if (part_world > 1 && n_neurons && !gpart_) {
-        // (until the neighbour is attached: ipc_attach replaces them with the neighbour's real boundary flags)
+        // (until the neighbour is attached: attach_strip replaces them with the neighbour's real boundary flags)
         for (uint32_t g = 0; g < halo_; ++g) {
             if (part_rank > 0 && !ghost_flags_from_peer_[0]) h_node_flags_[own0_ - halo_ + g] = h_node_flags_[own0_ + (g % std::max<uint64_t>(n_neurons, 1))];
             if (part_rank < part_world - 1 && !ghost_flags_from_peer_[1]) h_node_flags_[ghost_hi0_ + g] = h_node_flags_[own0_ + n_neurons - halo_ + g];
@@ -2071,6 +1983,15 @@ void Engine::wait_local_peers_launched(unsigned long long need, bool second) {
     }
 }
 
+// A per-edge pass of a partitioned handle that reads the neighbours' exports of this timestep's step kernel: it waits for the
+// counter value of the step after mine, and my step kernel of this timestep is in the queue already.
+void Engine::await_step_exports(StepParams &ep) {
+    ep.halo_epoch = halo_epoch_ + 1;
+    if (local_peers_.empty()) return;
+    launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);
+    wait_local_peers_launched(halo_epoch_ + 1, false);
+}
+
 // The step path of a run: which kernel steps the neurons of one timestep.
 enum class StepPath {
     Win,         // window-staged persistent kernel (step_win.cu): radius-1 stencil lattices
@@ -2726,12 +2647,8 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
         if (part_world > 1) {
             // the kernel reads the neighbours' step-s exports: their last_firing_time and current_activity of this step in my
             // ghost slots (see bcm_edge_body for why no second handshake is needed)
-            ep.halo_epoch = halo_epoch_ + 1;
             ep.tf[TFB_ACT_GHOST] = ACT_[out];
-            if (!local_peers_.empty()) {
-                launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);   // my step kernel of this timestep is in the queue
-                wait_local_peers_launched(halo_epoch_ + 1, false);
-            }
+            await_step_exports(ep);
         }
         cudaError_t e = launch_bcm_edges(ep, BcmParams{bcm.decay, bcm.average_scalar, bcm.dt}, stream_);
         if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "launch_bcm_edges");
@@ -2743,11 +2660,7 @@ int Engine::run_step(const RunPlan &pl, LaunchArgs &a, HistStage &hist, uint64_t
         if (pl.rmod_part) {
             // the kernel needs the neighbours' step-s exports (their last_firing_time of this step in my ghost slots)
             for (int d = 0; d < 2; ++d) ep.halo[d].my_flag = halo_dir_[d].my_flag;
-            ep.halo_epoch = halo_epoch_ + 1;
-        }
-        if (pl.rmod_part && !local_peers_.empty()) {
-            launched_pub_.store(halo_epoch_ + 1, std::memory_order_release);   // my step kernel of this timestep is in the queue
-            wait_local_peers_launched(halo_epoch_ + 1, false);
+            await_step_exports(ep);
         }
         cudaError_t e = launch_rstdp_edges(ep, a.rsp, stream_);
         if (pl.rmod_part) launched_pub2_.store(halo_epoch_ + 1, std::memory_order_release);
@@ -2858,6 +2771,8 @@ int Engine::run(uint64_t iterations, float *elapsed_ms, uint64_t *launches, cons
 // ------------------------------------------------------------------------------------------------
 // multi-GPU halo plumbing (CUDA IPC; the caller moves the blobs between ranks)
 // ------------------------------------------------------------------------------------------------
+static constexpr uint32_t kIpcMagic = 0x534E4E42u;   // "SNNB", first word of every IpcBlob
+
 int Engine::ipc_export(IpcBlob *blob) {
     int r = ipc_export_layout(blob);
     if (r) return r;
@@ -2871,7 +2786,7 @@ int Engine::ipc_export(IpcBlob *blob) {
 int Engine::ipc_export_layout(IpcBlob *blob) {
     if (part_world <= 1) return fail(SNN_INVALID_ARGUMENT, "handle is not partitioned");
     memset(blob, 0, sizeof *blob);
-    blob->magic = 0x534E4E42u; blob->version = SNN_B200_ABI_VERSION;
+    blob->magic = kIpcMagic; blob->version = SNN_B200_ABI_VERSION;
     for (int k = 0; k < 2; ++k) {
         blob->off_v[k] = slab_off_v_[k]; blob->off_lft[k] = slab_off_lft_[k]; blob->off_t[k] = slab_off_t_[k];
         blob->off_act[k] = slab_off_act_[k];
@@ -2884,98 +2799,114 @@ int Engine::ipc_export_layout(IpcBlob *blob) {
     return SNN_OK;
 }
 
-int Engine::ipc_attach(int direction, const IpcBlob *blob) {
-    if (part_world <= 1) return fail(SNN_INVALID_ARGUMENT, "handle is not partitioned");
-    if (direction != -1 && direction != 1) return fail(SNN_INVALID_ARGUMENT, "direction must be -1 or +1");
-    if (blob->magic != 0x534E4E42u || blob->version != SNN_B200_ABI_VERSION) return fail(SNN_INVALID_ARGUMENT, "bad ipc blob");
-    CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
-    const int d = direction < 0 ? 0 : 1;
-    if (peer_slab_[d] || halo_dir_[d].active) return fail(SNN_INVALID_ARGUMENT, "direction already attached");
+// Checks a partition peer's layout against mine, then maps its slab and arrival counters: `local` is a handle of this process
+// (addressed directly), else `blob` comes from another process's ipc_export (CUDA IPC).  Nothing is mapped and no peer access
+// is enabled unless every check passes.
+int Engine::map_peer(const IpcBlob *blob, Engine *local, int expect_rank, PeerMap *out, IpcBlob *view) {
+    if (local) {
+        if (local == this) return fail(SNN_INVALID_ARGUMENT, "bad peer handle");
+        int r = local->ipc_export_layout(view);
+        if (r) return fail(r, local->last_error);
+    } else {
+        *view = *blob;
+    }
+    if (view->magic != kIpcMagic || view->version != SNN_B200_ABI_VERSION) return fail(SNN_INVALID_ARGUMENT, "bad ipc blob");
+    if (view->rank != expect_rank || view->world != part_world) return fail(SNN_INVALID_ARGUMENT, "ipc blob is not from that rank");
+    if ((view->chem != 0) != chem_alloc_) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on chemistry");
+    if (!gpart_) {
+        if (view->halo != halo_) return fail(SNN_INVALID_ARGUMENT, "neighbouring strips disagree on halo width");
+        if (halo_ > n_neurons || halo_ > view->n_neurons) return fail(SNN_UNSUPPORTED, "strip thinner than the halo");
+    }
+    if ((view->off_act[0] != 0) != (ACT_[0] != nullptr)) return fail(SNN_INVALID_ARGUMENT, "the ranks disagree on the neuron model");
+    if (local) {
+        if (local->device != device) {
+            int can = 0;
+            CK(cudaDeviceCanAccessPeer(&can, device, local->device), SNN_GPU_GET_DEVICE_FAILURE);
+            if (!can) return fail(SNN_UNSUPPORTED, "no peer access between the two devices");
+            cudaError_t e = cudaDeviceEnablePeerAccess(local->device, 0);
+            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return cuda_fail(e, SNN_GPU_GET_DEVICE_FAILURE, "cudaDeviceEnablePeerAccess");
+            cudaGetLastError();
+        }
+        *out = PeerMap{local->slab_, local->flags_, false};
+        return SNN_OK;
+    }
     void *slab = nullptr, *flags = nullptr;
-    CK(cudaIpcOpenMemHandle(&slab, blob->slab, cudaIpcMemLazyEnablePeerAccess), SNN_GPU_BUFFER_CREATE_ERROR);
-    CK(cudaIpcOpenMemHandle(&flags, blob->flags, cudaIpcMemLazyEnablePeerAccess), SNN_GPU_BUFFER_CREATE_ERROR);
-    peer_slab_[d] = slab; peer_flags_[d] = flags;
-    int r = attach_view(direction, blob, slab, flags);
-    if (r) {
-        cudaIpcCloseMemHandle(slab); cudaIpcCloseMemHandle(flags);
-        peer_slab_[d] = peer_flags_[d] = nullptr;
+    CK(cudaIpcOpenMemHandle(&slab, view->slab, cudaIpcMemLazyEnablePeerAccess), SNN_GPU_BUFFER_CREATE_ERROR);
+    cudaError_t e = cudaIpcOpenMemHandle(&flags, view->flags, cudaIpcMemLazyEnablePeerAccess);
+    if (e != cudaSuccess) {
+        cudaIpcCloseMemHandle(slab);
+        return cuda_fail(e, SNN_GPU_BUFFER_CREATE_ERROR, "cudaIpcOpenMemHandle(flags)");
     }
-    return r;
+    *out = PeerMap{slab, flags, true};
+    return SNN_OK;
 }
 
-// The neighbouring strip lives in THIS process (another handle on the same device, or on a device with peer access): no CUDA
-// IPC, the neighbour's slab and arrival counters are addressed directly.  Both handles must attach each other.  On one device
-// the caller steps the handles from separate host threads and keeps the strips small enough for their step kernels to be
-// resident together (a strip's boundary warps spin on the neighbour's progress).
-int Engine::attach_local(int direction, Engine *peer) {
+// Ghost nodes node0, node0 + 1, ... take the neurotransmitter / receptor type flags of the peer's neurons they mirror (the flags
+// are baked into the col words of edges from ghosts): ghost node0 + k takes byte pick[k] of the `bytes` peer flag bytes at
+// `peer_flags`.  `force` re-encodes the graph even when no flag changes.
+int Engine::import_ghost_flags(uint32_t node0, const uint8_t *peer_flags, uint64_t bytes, const std::vector<uint32_t> &pick, bool force) {
+    std::vector<uint8_t> pf(bytes);
+    CK(cudaMemcpy(pf.data(), peer_flags, bytes, cudaMemcpyDefault), SNN_GPU_BUFFER_READ_ERROR);
+    bool changed = force;
+    for (size_t k = 0; k < pick.size(); ++k) {
+        changed |= h_node_flags_[node0 + k] != pf[pick[k]];
+        h_node_flags_[node0 + k] = pf[pick[k]];
+    }
+    if (!changed) return SNN_OK;
+    CK(h2d_sync(node_flags_ + node0, h_node_flags_.data() + node0, pick.size(), stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    flags_cache_valid_ = false;
+    if (dev_weights_newer_) { int r = sync_weights_to_host(); if (r) return r; }
+    graph_dirty_ = true;
+    return SNN_OK;
+}
+
+// The neighbouring strip lives in another process (`blob`) or in this one (`local`: another handle on the same device, or on a
+// device with peer access).  Both handles must attach each other.  On one device the caller steps in-process strips from separate
+// host threads and keeps the strips small enough for their step kernels to be resident together (a strip's boundary warps spin on
+// the neighbour's progress).
+int Engine::attach_strip(int direction, const IpcBlob *blob, Engine *local) {
     if (part_world <= 1) return fail(SNN_INVALID_ARGUMENT, "handle is not partitioned");
     if (direction != -1 && direction != 1) return fail(SNN_INVALID_ARGUMENT, "direction must be -1 or +1");
-    if (!peer || peer == this) return fail(SNN_INVALID_ARGUMENT, "bad neighbour handle");
+    if (gpart_) return fail(SNN_INVALID_ARGUMENT, "a general-graph partition attaches its peers with gpart_attach");
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
     const int d = direction < 0 ? 0 : 1;
-    if (peer_slab_[d] || halo_dir_[d].active) return fail(SNN_INVALID_ARGUMENT, "direction already attached");
-    if (peer->device != device) {
-        int can = 0;
-        CK(cudaDeviceCanAccessPeer(&can, device, peer->device), SNN_GPU_GET_DEVICE_FAILURE);
-        if (!can) return fail(SNN_UNSUPPORTED, "no peer access between the two devices");
-        cudaError_t e = cudaDeviceEnablePeerAccess(peer->device, 0);
-        if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return cuda_fail(e, SNN_GPU_GET_DEVICE_FAILURE, "cudaDeviceEnablePeerAccess");
-        cudaGetLastError();
-    }
-    IpcBlob blob;
-    int r = peer->ipc_export_layout(&blob);
-    if (r) return fail(r, peer->last_error);
-    r = attach_view(direction, &blob, peer->slab_, peer->flags_);
-    if (!r) {
-        peer->layout_frozen_ = layout_frozen_ = true;   // raw pointers into each other's slabs from now on
-        local_peers_.push_back(peer);
-    }
-    return r;
-}
-
-int Engine::attach_view(int direction, const IpcBlob *blob, void *slab, void *flags) {
-    if (blob->rank != part_rank + direction || blob->world != part_world) return fail(SNN_INVALID_ARGUMENT, "ipc blob is not from the neighbouring rank");
-    if (blob->halo != halo_ || (blob->chem != 0) != chem_alloc_) return fail(SNN_INVALID_ARGUMENT, "neighbouring strips disagree on halo width / chemistry");
-    if (halo_ > n_neurons || halo_ > blob->n_neurons) return fail(SNN_UNSUPPORTED, "strip thinner than the halo");
-    if ((blob->off_act[0] != 0) != (ACT_[0] != nullptr)) return fail(SNN_INVALID_ARGUMENT, "neighbouring strips disagree on the neuron model");
-    const int d = direction < 0 ? 0 : 1;
-    HaloDir &H = halo_dir_[d];
+    if (halo_dir_[d].active) return fail(SNN_INVALID_ARGUMENT, "direction already attached");
+    PeerMap m;
+    IpcBlob v;
+    int r = map_peer(blob, local, part_rank + direction, &m, &v);
+    if (r) return r;
+    HaloDir H;
     memset(&H, 0, sizeof H);
     H.count = halo_;
     // d == 0: my first `halo` neurons go to the upper ghost slots of rank-1; d == 1: my last `halo` neurons go to
     // the lower ghost slots of rank+1
     H.first = d == 0 ? 0 : (uint32_t)n_neurons - halo_;
-    H.peer_node0 = d == 0 ? blob->ghost_hi0 : blob->own0 - blob->halo;
+    H.peer_node0 = d == 0 ? v.ghost_hi0 : v.own0 - v.halo;
     H.my_ghost0 = d == 0 ? own0_ - halo_ : ghost_hi0_;
     for (int k = 0; k < 2; ++k) {
-        H.peer_v[k] = (float *)((char *)slab + blob->off_v[k]);
-        H.peer_lft[k] = (int *)((char *)slab + blob->off_lft[k]);
-        H.peer_t[k] = (float *)((char *)slab + blob->off_t[k]);
-        halo_act_[d][k] = ACT_[0] ? (float *)((char *)slab + blob->off_act[k]) : nullptr;
+        H.peer_v[k] = (float *)((char *)m.slab + v.off_v[k]);
+        H.peer_lft[k] = (int *)((char *)m.slab + v.off_lft[k]);
+        H.peer_t[k] = (float *)((char *)m.slab + v.off_t[k]);
     }
-    H.peer_t_stride = blob->t_stride;
+    H.peer_t_stride = v.t_stride;
     // the neighbour's arrival counter for data coming from me: I am its rank+1 when d == 0 (slot 1), its rank-1 when d == 1 (slot 0)
-    H.peer_flag = (unsigned long long *)flags + (d == 0 ? 1 : 0);
+    H.peer_flag = (unsigned long long *)m.flags + (d == 0 ? 1 : 0);
     H.my_flag = flags_ + d;
     H.peer_flag2 = H.peer_flag + 2;
     H.my_flag2 = H.my_flag + 2;
     H.active = 1;
-    // my ghost rows take the neurotransmitter / receptor type flags of the neighbour's boundary rows (they are baked into the
-    // col words of edges from ghosts): d == 0 reads the LAST halo_ neurons of rank - 1, d == 1 the FIRST halo_ of rank + 1
-    {
-        const uint8_t *peer_f = (const uint8_t *)slab + blob->off_flags + (d == 0 ? blob->own0 + blob->n_neurons - halo_ : blob->own0);
-        std::vector<uint8_t> tmp(halo_);
-        CK(cudaMemcpy(tmp.data(), peer_f, halo_, cudaMemcpyDefault), SNN_GPU_BUFFER_READ_ERROR);
-        bool changed = !ghost_flags_from_peer_[d];
-        for (uint32_t g = 0; g < halo_; ++g) { changed |= h_node_flags_[H.my_ghost0 + g] != tmp[g]; h_node_flags_[H.my_ghost0 + g] = tmp[g]; }
-        ghost_flags_from_peer_[d] = true;
-        if (changed) {
-            CK(h2d_sync(node_flags_ + H.my_ghost0, tmp.data(), halo_, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-            flags_cache_valid_ = false;
-            if (dev_weights_newer_) { int r = sync_weights_to_host(); if (r) return r; }
-            graph_dirty_ = true;
-        }
-    }
+    // my ghost rows mirror the neighbour's boundary rows: d == 0 the LAST halo_ neurons of rank - 1, d == 1 the FIRST halo_ of rank + 1
+    std::vector<uint32_t> pick(halo_);
+    std::iota(pick.begin(), pick.end(), 0u);
+    r = import_ghost_flags(H.my_ghost0, (const uint8_t *)m.slab + v.off_flags + (d == 0 ? v.own0 + v.n_neurons - halo_ : v.own0), halo_,
+                           pick, !ghost_flags_from_peer_[d]);
+    if (r) { unmap_peer(m); return r; }
+    ghost_flags_from_peer_[d] = true;
+    halo_dir_[d] = H;
+    for (int k = 0; k < 2; ++k) halo_act_[d][k] = ACT_[0] ? (float *)((char *)m.slab + v.off_act[k]) : nullptr;
+    strip_map_[d] = m;
+    layout_frozen_ = true;
+    if (local) { local->layout_frozen_ = true; local_peers_.push_back(local); }
     return SNN_OK;
 }
 

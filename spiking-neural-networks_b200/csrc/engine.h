@@ -67,6 +67,11 @@ struct IpcBlob {  // exchanged between neighbouring ranks by the caller (e.g. to
     int32_t rank, world;
 };
 
+struct PeerMap {  // a partition peer's slab and arrival counters as this process addresses them
+    void *slab = nullptr, *flags = nullptr;
+    bool ipc = false;   // opened from CUDA IPC handles (closed by the engine), else the pointers of a handle of this process
+};
+
 class Engine {
 public:
     Engine(int model, int ntk, int rck, int train_kind, int refract, int device);
@@ -146,13 +151,13 @@ public:
 
     // multi-GPU
     int ipc_export(IpcBlob *blob);
-    int ipc_attach(int direction, const IpcBlob *blob);
-    int attach_local(int direction, Engine *peer);   // neighbour handle in the same process (no CUDA IPC)
+    // the attach calls take either the `blob` of another process's ipc_export (CUDA IPC) or a `local` handle of this process
+    int attach_strip(int direction, const IpcBlob *blob, Engine *local);   // row strips: direction -1 = rank-1, +1 = rank+1
     // general-graph partition (contiguous node ranges, in-edges from anywhere): which of `peer`'s nodes this rank reads, which of
     // its own nodes `peer` reads, and the mapping of the peer's arrays
     int gpart_wants(int peer, uint32_t *global_idx, uint64_t capacity, uint64_t *n, uint32_t *first_slot);
     int gpart_set_exports(int peer, const uint32_t *global_idx, uint64_t n, uint32_t first_slot_at_peer);
-    int gpart_attach(int peer, const IpcBlob *blob, Engine *local_peer);
+    int gpart_attach(int peer, const IpcBlob *blob, Engine *local);
     bool is_gpart() const { return gpart_; }
 
     // public knobs (Lattice / LatticeNetwork pub fields, neuron/mod.rs:556-587, 1554-1563)
@@ -234,16 +239,15 @@ private:
     unsigned char *wide_scratch_ = nullptr; size_t wide_scratch_bytes_ = 0;   // parked per-edge terms of the two-pass wide kernels
     unsigned int *multi_barrier_ = nullptr;   // grid-wide arrival counter of the multi-step kernel
     HaloDir halo_dir_[2] = {};
-    void *peer_slab_[2] = {nullptr, nullptr};
-    void *peer_flags_[2] = {nullptr, nullptr};
+    PeerMap strip_map_[2] = {};
     unsigned long long halo_epoch_ = 0;
     // general-graph partition
     struct GPeerHost {
         int rank = -1;
         std::vector<uint32_t> exp_local;   // my local neuron numbers this peer reads (ascending)
         uint32_t peer_slot0 = 0;           // node index in the peer's arrays where they go
-        void *slab = nullptr, *flags = nullptr;
-        bool ipc = false, attached = false;
+        PeerMap map;
+        bool attached = false;
         IpcBlob view{};
     };
     bool gpart_ = false, gpart_dirty_ = true;
@@ -253,9 +257,9 @@ private:
     GPeer *d_gpeers_ = nullptr; uint32_t *d_gexp_off_ = nullptr, *d_gexp_ent_ = nullptr; uint8_t *d_gslice_ = nullptr;
     float **d_gact_ = nullptr;             // BCM Izhikevich: the peers' activity buffers (BcmSlot TFB_GPEER_ACT), else null
     GPeerHost *gpeer(int rank, bool create);
+    int check_peer_rank(int peer);
     int gpart_build_device();
     int gpart_enable(const std::vector<uint32_t> &remote_sorted_unique);
-    int relayout_keep_fields(const std::function<void()> &change);
     int64_t global_to_node(uint64_t g) const;
     uint64_t node_to_global(uint32_t node) const;
     // scratch
@@ -270,18 +274,20 @@ private:
     int refuse_if_graph_history(const char *what);
 
     int ipc_export_layout(IpcBlob *blob);
-    int attach_view(int direction, const IpcBlob *blob, void *slab, void *flags);
-    bool layout_frozen_ = false;
+    int map_peer(const IpcBlob *blob, Engine *local, int expect_rank, PeerMap *out, IpcBlob *view);
+    int import_ghost_flags(uint32_t node0, const uint8_t *peer_flags, uint64_t bytes, const std::vector<uint32_t> &pick, bool force);
+    bool layout_frozen_ = false;   // pointers into or out of my slab exist: its layout must not change
     // in-process neighbours: host-side launch ordering (see wait_local_peers_launched)
     std::vector<Engine *> local_peers_;
     std::atomic<unsigned long long> launched_pub_{0}, launched_pub2_{0};
     void wait_local_peers_launched(unsigned long long need, bool second);
+    void await_step_exports(StepParams &ep);
     int cuda_fail(cudaError_t e, int status, const char *what);
     int ensure_scratch(size_t bytes);
     void free_device();
     int alloc_device();
     int ensure_chem();
-    int relayout_add(const Lat &nl);
+    int relayout(const std::function<void()> &change);
     void compute_layout();
     uint32_t node_off(const Lat &L) const { return (L.is_train ? train0_ : own0_) + (uint32_t)L.off; }
     int n_neuron_lattices() const { int n = 0; for (auto &L : lats_) n += !L.is_train; return n; }

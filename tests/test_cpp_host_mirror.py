@@ -11,31 +11,31 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "spiking-neural-networks_b200")
 SRC = os.path.join(ROOT, "tests", "cpp", "host_mirror.cpp")
-EXE = os.path.join(ROOT, "tests", "cpp", "_build", "host_mirror")
 
 
-def build():
+def build(out_dir):
+    """Compiles the test program into `out_dir` (the repository tree may be read-only)."""
     cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else shutil.which("g++")
     if cxx is None:
         pytest.skip("no host C++ compiler")
     if not os.path.exists(os.path.join(PKG, "libsnn_b200.so")):
         pytest.fail("libsnn_b200.so is not built (python -c 'import __graft_entry__ as g; g.build()')")
-    os.makedirs(os.path.dirname(EXE), exist_ok=True)
-    cmd = [cxx, "-std=c++17", "-O1", "-Wall", "-Wextra", "-Werror", "-I", os.path.join(ROOT, "include"), SRC, "-o", EXE,
+    exe = str(out_dir / "host_mirror")
+    cmd = [cxx, "-std=c++17", "-O1", "-Wall", "-Wextra", "-Werror", "-I", os.path.join(ROOT, "include"), SRC, "-o", exe,
            "-L", PKG, "-lsnn_b200", f"-Wl,-rpath,{PKG}"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    return EXE
+    return exe
 
 
-def test_cpp_mirror_compiles_links_and_has_no_cpu_fallback():
-    exe = build()
+def test_cpp_mirror_compiles_links_and_has_no_cpu_fallback(tmp_path):
+    exe = build(tmp_path)
     r = subprocess.run([exe, "--no-gpu"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stdout + r.stderr
 
 
 @pytest.mark.gpu
-def test_cpp_mirror_replays_reference_integration_tests():
-    exe = build()
+def test_cpp_mirror_replays_reference_integration_tests(tmp_path):
+    exe = build(tmp_path)
     r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "HOST_MIRROR_OK" in r.stdout, r.stdout + r.stderr

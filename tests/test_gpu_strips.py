@@ -149,44 +149,39 @@ def _random_radius_csr(rows, cols, seed, radius, p):
     return SC.dense_to_csr(conn, w)
 
 
-@pytest.mark.parametrize("world", [2, 3, 4])
-@pytest.mark.parametrize("shape,radius,chem,stdp", [((12, 9), 2.5, None, False), ((16, 10), 5.0, "ampa", True), ((14, 7), 30.0, "mixed", True)])
-def test_general_graph_partition_matches_the_oracle(world, shape, radius, chem, stdp):
-    """Contiguous node ranges per rank, random-radius graphs whose edges cross rank boundaries arbitrarily (radius 30 = almost
-    all-to-all: every rank reads nodes of every other rank, also of non-neighbouring ranks): gather-list ghosts, per-neuron
-    export lists, completion counters.  Electrical-only Izhikevich is bit-exact; chemistry + STDP to 1e-4, rasters exact."""
-    rows, cols = shape
+def _configure_general(set_field, each, n, chem, stdp):
+    rng = np.random.default_rng(19)
+    set_field("current_voltage", rng.uniform(-65, 30, n).astype(f32), 1)
+    set_field("b", rng.uniform(0.25, 0.36, n).astype(f32), 1)
+    set_field("gap_conductance", (10 * rng.uniform(0.5, 1.5, n)).astype(f32), 1)
+    set_field("c_m", np.full(n, 4.0, f32), 1)
+    if chem:
+        set_field("neurotransmitters$flags", _nt_flags(n, chem), 3)
+        set_field("receptors$flags", np.ones((n, 3), np.uint32) if chem == "mixed" else _nt_flags(n, chem), 3)
+
+    def opts(be):
+        be.set_option(K.OPT_ELECTRICAL_SYNAPSE, 1)
+        be.set_option(K.OPT_CHEMICAL_SYNAPSE, int(bool(chem)))
+        be.set_option(K.OPT_DO_PLASTICITY, int(stdp), 0)
+        be.set_plasticity(0, 0.05, 0.04, 4.5, 3.0, 0.1)
+    each(opts)
+
+
+def _nt_flags(n, chem):
+    flags = np.zeros((n, 3), np.uint32)
+    flags[:, 0] = 1
+    if chem == "mixed":
+        flags[:, 0] = (np.arange(n) // 5) % 2
+        flags[:, 2] = 1 - flags[:, 0]
+    return flags
+
+
+def _general_matches_the_oracle(parts, rp, pre, w, chem, stdp):
+    """Runs the attached partitions and the CPU oracle side by side and compares state and weights."""
+    rows, cols = parts.rows, parts.cols
     n = rows * cols
-    rp, pre, w = _random_radius_csr(rows, cols, 41, radius, 0.6)
-    parts = LocalStrips(K.MODEL_IZH, rows, cols, world)
-
-    def configure(set_field, each):
-        rng = np.random.default_rng(19)
-        set_field("current_voltage", rng.uniform(-65, 30, n).astype(f32), 1)
-        set_field("b", rng.uniform(0.25, 0.36, n).astype(f32), 1)
-        set_field("gap_conductance", (10 * rng.uniform(0.5, 1.5, n)).astype(f32), 1)
-        set_field("c_m", np.full(n, 4.0, f32), 1)
-        if chem:
-            flags = np.zeros((n, 3), np.uint32)
-            flags[:, 0] = 1
-            if chem == "mixed":
-                flags[:, 0] = (np.arange(n) // 5) % 2
-                flags[:, 2] = 1 - flags[:, 0]
-            set_field("neurotransmitters$flags", flags, 3)
-            set_field("receptors$flags", np.ones((n, 3), np.uint32) if chem == "mixed" else flags, 3)
-
-        def opts(be):
-            be.set_option(K.OPT_ELECTRICAL_SYNAPSE, 1)
-            be.set_option(K.OPT_CHEMICAL_SYNAPSE, int(bool(chem)))
-            be.set_option(K.OPT_DO_PLASTICITY, int(stdp), 0)
-            be.set_plasticity(0, 0.05, 0.04, 4.5, 3.0, 0.1)
-        each(opts)
-
-    configure(lambda nm, a, per: parts.set_field(nm, a, per), parts.each)
-    parts.set_graph_csr(rp, pre, w)
-    parts.attach_general()
     ob = _oracle(rows, cols)
-    configure(lambda nm, a, per: ob.set_field(0, nm, np.asarray(a).reshape(-1)), lambda fn: fn(ob))
+    _configure_general(lambda nm, a, per: ob.set_field(0, nm, np.asarray(a).reshape(-1)), lambda fn: fn(ob), n, chem, stdp)
     ob.connect_csr(0, 0, rp, pre, w)
     names = STATE + (["neurotransmitters$t", "receptors$AMPA$r$kinetics$r"] if chem else [])
     for k in (21, 1, 20):
@@ -205,6 +200,43 @@ def test_general_graph_partition_matches_the_oracle(world, shape, radius, chem, 
     assert (ob.get_field(0, "last_firing_time") >= 0).sum() > n // 4
     if stdp:
         assert np.abs(ow - w).max() > 1e-3
+
+
+@pytest.mark.parametrize("world", [2, 3, 4])
+@pytest.mark.parametrize("shape,radius,chem,stdp", [((12, 9), 2.5, None, False), ((16, 10), 5.0, "ampa", True), ((14, 7), 30.0, "mixed", True)])
+def test_general_graph_partition_matches_the_oracle(world, shape, radius, chem, stdp):
+    """Contiguous node ranges per rank, random-radius graphs whose edges cross rank boundaries arbitrarily (radius 30 = almost
+    all-to-all: every rank reads nodes of every other rank, also of non-neighbouring ranks): gather-list ghosts, per-neuron
+    export lists, completion counters.  Electrical-only Izhikevich is bit-exact; chemistry + STDP to 1e-4, rasters exact."""
+    rows, cols = shape
+    rp, pre, w = _random_radius_csr(rows, cols, 41, radius, 0.6)
+    parts = LocalStrips(K.MODEL_IZH, rows, cols, world)
+    _configure_general(lambda nm, a, per: parts.set_field(nm, a, per), parts.each, rows * cols, chem, stdp)
+    parts.set_graph_csr(rp, pre, w)
+    parts.attach_general()
+    _general_matches_the_oracle(parts, rp, pre, w, chem, stdp)
     if radius >= 30 and world >= 3:   # non-neighbouring ranks exchange too
         idx, _ = parts.strips[0].gpart_wants(world - 1)
         assert idx.size > 0
+
+
+def test_refused_general_graph_attach_leaves_both_handles_unchanged():
+    """An attach that the peer's layout refuses (here: only one rank has chemistry) maps nothing and freezes neither handle: the
+    peer can still allocate its chemical fields, and then the ranks attach and match the oracle."""
+    rows, cols, chem, stdp = 16, 10, "ampa", True
+    n = rows * cols
+    rp, pre, w = _random_radius_csr(rows, cols, 41, 5.0, 0.6)
+    parts = LocalStrips(K.MODEL_IZH, rows, cols, 2)
+    _configure_general(lambda nm, a, per: parts.set_field(nm, a, per), parts.each, n, None, stdp)
+    parts.each(lambda be: be.set_option(K.OPT_CHEMICAL_SYNAPSE, 1))
+    parts.set_graph_csr(rp, pre, w)
+    flags = _nt_flags(n, chem)
+    s0, s1 = parts.strips
+    s0.set_field(0, "neurotransmitters$flags", flags[parts.rows_of(0)].reshape(-1))
+    with pytest.raises(S.SnnError) as ei:
+        s0.gpart_attach_local(1, s1)
+    assert ei.value.status == K.SNN_INVALID_ARGUMENT
+    s1.set_field(0, "neurotransmitters$flags", flags[parts.rows_of(1)].reshape(-1))
+    parts.set_field("receptors$flags", flags, 3)
+    parts.attach_general()
+    _general_matches_the_oracle(parts, rp, pre, w, chem, stdp)
