@@ -320,27 +320,24 @@ int Engine::relayout(const std::function<void()> &change) {
     struct FieldSnap { uint64_t id; std::string name; int dtype; uint64_t count; std::vector<uint8_t> data; };
     std::vector<FieldSnap> snaps;
     const bool had_chem = chem_alloc_;
+    int r = SNN_OK;
     for (auto &L : lats_) {
-        uint32_t cnt = 0; field_count(L.id, &cnt);
-        for (uint32_t i = 0; i < cnt; ++i) {
-            const char *name; int32_t dt; uint32_t per;
-            field_info(L.id, i, &name, &dt, &per);
-            FieldDef fd;
-            if (lookup_field(L, name, &fd)) continue;
+        for_each_field(L, [&](const FieldDef &fd, const char *name) {
             const bool is_chem = fd.kind == FK_NT_FLAGS || fd.kind == FK_NT_T || fd.kind == FK_NT || fd.kind == FK_RC_FLAGS || fd.kind == FK_RC;
-            if (is_chem && !had_chem) continue;
-            FieldSnap f{L.id, name, dt, L.n * per, {}};
+            if (is_chem && !had_chem) return false;
+            FieldSnap f{L.id, name, fd.dtype, L.n * fd.per, {}};
             f.data.resize(std::max<uint64_t>(f.count, 1) * 4);
-            int r = get_field(L.id, name, f.data.data(), f.count, dt);
-            if (r) return r;
-            snaps.push_back(std::move(f));
-        }
+            r = get_field(L.id, name, f.data.data(), f.count, fd.dtype);
+            if (!r) snaps.push_back(std::move(f));
+            return r != SNN_OK;
+        });
+        if (r) return r;
     }
     const uint64_t saved_clock = internal_clock;
     free_device();
     change();
     compute_layout();
-    int r = alloc_device();
+    r = alloc_device();
     if (r) return r;
     if (had_chem) { r = ensure_chem(); if (r) return r; }
     for (auto &f : snaps) {
@@ -362,28 +359,37 @@ int Engine::relayout(const std::function<void()> &change) {
 // ------------------------------------------------------------------------------------------------
 // field directory
 // ------------------------------------------------------------------------------------------------
-static bool field_visible(const FieldDef &fd, int kind_bit, int ntk_, int rck_) {
+static bool field_visible(const FieldDef &fd, int kind_bit, int ntk_) {
     if (!(fd.models & SNN_M(kind_bit))) return false;
     if (fd.kind == FK_NT && fd.aux && !(fd.aux & SNN_M(ntk_))) return false;
-    (void)rck_;
     return true;
+}
+
+// The directory of lattice L in index order: f(fd, name) for every field of this handle's model (or train kind) and kinetics,
+// until f returns true.  Receptor fields are generated per type (fd.name == nullptr); `name` then points into a buffer of this
+// call that the next field overwrites.
+template <class F>
+void Engine::for_each_field(const Lat &L, F &&f) const {
+    const FieldDef *tab = L.is_train ? kTrainFields : kNeuronFields;
+    const int n = L.is_train ? kNumTrainFields : kNumNeuronFields;
+    for (int i = 0; i < n; ++i)
+        if (field_visible(tab[i], L.is_train ? train_kind : model, ntk) && f(tab[i], tab[i].name)) return;
+    if (L.is_train) return;
+    char buf[128];
+    for (int ty = 0; ty < kNT; ++ty)
+        for (const RcFieldDef &rf : kRcFields) {
+            if (rf.nmda_only && ty != SNN_NT_NMDA) continue;
+            if (rf.kinetics_mask && !(rf.kinetics_mask & SNN_M(rck))) continue;
+            snprintf(buf, sizeof buf, "receptors$%s%s", kRcTypeNames[ty], rf.suffix);
+            if (f(FieldDef{nullptr, SNN_F32, 1, FK_RC, rf.slot, ty, kAllModels}, (const char *)buf)) return;
+        }
 }
 
 int Engine::field_count(uint64_t id, uint32_t *count) const {
     const Lat *L = find(id);
     if (!L) return SNN_NET_ID_NOT_FOUND_IN_LATTICES;
     uint32_t c = 0;
-    if (L->is_train) {
-        for (int i = 0; i < kNumTrainFields; ++i) if (field_visible(kTrainFields[i], train_kind, ntk, rck)) c++;
-    } else {
-        for (int i = 0; i < kNumNeuronFields; ++i) if (field_visible(kNeuronFields[i], model, ntk, rck)) c++;
-        for (int ty = 0; ty < kNT; ++ty)
-            for (int i = 0; i < kNumRcFields; ++i) {
-                if (kRcFields[i].nmda_only && ty != SNN_NT_NMDA) continue;
-                if (kRcFields[i].kinetics_mask && !(kRcFields[i].kinetics_mask & SNN_M(rck))) continue;
-                c++;
-            }
-    }
+    for_each_field(*L, [&](const FieldDef &, const char *) { ++c; return false; });
     *count = c;
     return SNN_OK;
 }
@@ -394,56 +400,25 @@ int Engine::field_info(uint64_t id, uint32_t index, const char **name, int32_t *
     const Lat *L = find(id);
     if (!L) return SNN_NET_ID_NOT_FOUND_IN_LATTICES;
     uint32_t c = 0;
-    if (L->is_train) {
-        for (int i = 0; i < kNumTrainFields; ++i)
-            if (field_visible(kTrainFields[i], train_kind, ntk, rck)) {
-                if (c == index) { *name = kTrainFields[i].name; *dtype = kTrainFields[i].dtype; *per = kTrainFields[i].per; return SNN_OK; }
-                c++;
-            }
-    } else {
-        for (int i = 0; i < kNumNeuronFields; ++i)
-            if (field_visible(kNeuronFields[i], model, ntk, rck)) {
-                if (c == index) { *name = kNeuronFields[i].name; *dtype = kNeuronFields[i].dtype; *per = kNeuronFields[i].per; return SNN_OK; }
-                c++;
-            }
-        for (int ty = 0; ty < kNT; ++ty)
-            for (int i = 0; i < kNumRcFields; ++i) {
-                if (kRcFields[i].nmda_only && ty != SNN_NT_NMDA) continue;
-                if (kRcFields[i].kinetics_mask && !(kRcFields[i].kinetics_mask & SNN_M(rck))) continue;
-                if (c == index) {
-                    snprintf(g_name_buf, sizeof g_name_buf, "receptors$%s%s", kRcTypeNames[ty], kRcFields[i].suffix);
-                    *name = g_name_buf; *dtype = SNN_F32; *per = 1;
-                    return SNN_OK;
-                }
-                c++;
-            }
-    }
-    return SNN_INVALID_ARGUMENT;
+    bool found = false;
+    for_each_field(*L, [&](const FieldDef &fd, const char *nm) {
+        if (c++ != index) return false;
+        // a generated receptor name is handed out from this thread's buffer, valid until the next call that returns one
+        *name = fd.name ? fd.name : strcpy(g_name_buf, nm);
+        *dtype = fd.dtype; *per = fd.per;
+        return found = true;
+    });
+    return found ? SNN_OK : SNN_INVALID_ARGUMENT;
 }
 
 int Engine::lookup_field(const Lat &L, const char *name, FieldDef *out) const {
-    if (L.is_train) {
-        for (int i = 0; i < kNumTrainFields; ++i)
-            if (field_visible(kTrainFields[i], train_kind, ntk, rck) && !strcmp(kTrainFields[i].name, name)) { *out = kTrainFields[i]; return SNN_OK; }
-        return SNN_UNKNOWN_FIELD;
-    }
-    for (int i = 0; i < kNumNeuronFields; ++i)
-        if (field_visible(kNeuronFields[i], model, ntk, rck) && !strcmp(kNeuronFields[i].name, name)) { *out = kNeuronFields[i]; return SNN_OK; }
-    if (!strncmp(name, "receptors$", 10)) {
-        for (int ty = 0; ty < kNT; ++ty) {
-            const size_t tl = strlen(kRcTypeNames[ty]);
-            if (strncmp(name + 10, kRcTypeNames[ty], tl)) continue;
-            for (int i = 0; i < kNumRcFields; ++i) {
-                if (kRcFields[i].nmda_only && ty != SNN_NT_NMDA) continue;
-                if (kRcFields[i].kinetics_mask && !(kRcFields[i].kinetics_mask & SNN_M(rck))) continue;
-                if (!strcmp(name + 10 + tl, kRcFields[i].suffix)) {
-                    *out = FieldDef{nullptr, SNN_F32, 1, FK_RC, kRcFields[i].slot, ty, kAllModels};
-                    return SNN_OK;
-                }
-            }
-        }
-    }
-    return SNN_UNKNOWN_FIELD;
+    bool found = false;
+    for_each_field(L, [&](const FieldDef &fd, const char *nm) {
+        if (strcmp(nm, name)) return false;
+        *out = fd;
+        return found = true;
+    });
+    return found ? SNN_OK : SNN_UNKNOWN_FIELD;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -986,7 +961,7 @@ int Engine::connect_grid(uint64_t id, uint32_t radius, float weight) {
     return SNN_OK;
 }
 
-int Engine::materialize_grid(Block &b, const Lat &L) {
+void Engine::materialize_grid(Block &b, const Lat &L) const {
     // host CSR of the Moore stencil (same enumeration order as sell_grid_kernel: ascending flat index)
     const int64_t R = b.radius, rows_g = part_world > 1 ? rows_global : L.rows, cols = L.cols;
     const int64_t r0 = part_world > 1 ? row0_global : 0;
@@ -1006,6 +981,62 @@ int Engine::materialize_grid(Block &b, const Lat &L) {
         }
     b.kind = Block::CSR;
     b.from_grid_radius = b.radius;
+}
+
+// `b` itself, or the host CSR of a stencil block materialised on `tmp`: the block stays a stencil, and with it the device fast
+// path of finalize_graph
+Block &Engine::csr_view(Block &b, const Lat &L, Block &tmp) const {
+    if (b.kind != Block::GRID) return b;
+    tmp = b;
+    materialize_grid(tmp, L);
+    return tmp;
+}
+
+// The row order of the device edge table: for every neuron lattice B (only `into`, if given), every row q and every block into B,
+// f(B, q, A, b, k) with A the presynaptic lattice and k the offset of the block's edges within the row.  Blocks into a lattice
+// follow the node offset of their presynaptic lattice, so that rows stay sorted by node index; each block's edges of the row
+// keep its CSR order.  finalize_graph lays the table out in this order and every map from a host edge to a table element reads
+// it back from here.  A stencil block is visited as its materialised copy.
+template <class F>
+void Engine::for_each_row_segment(F &&f, const Lat *into) {
+    for (const Lat &B : lats_) {
+        if (B.is_train || (into && &B != into)) continue;
+        Block tmp;   // only a lattice's own graph can be a stencil
+        std::vector<std::pair<const Lat *, Block *>> blocks;
+        for (auto &kv : blocks_)
+            if (kv.first.second == B.id) {
+                const Lat *A = find(kv.first.first);
+                if (A) blocks.emplace_back(A, &csr_view(kv.second, B, tmp));
+            }
+        std::sort(blocks.begin(), blocks.end(), [&](auto &x, auto &y) { return node_off(*x.first) < node_off(*y.first); });
+        for (uint64_t q = 0; q < B.n; ++q) {
+            uint64_t k = 0;
+            for (auto &ab : blocks) {
+                Block &b = *ab.second;
+                f(B, q, *ab.first, b, k);
+                k += b.row_ptr[q + 1] - b.row_ptr[q];
+            }
+        }
+    }
+}
+
+static uint32_t stencil_width(uint32_t radius) { return (2 * radius + 1) * (2 * radius + 1) - 1; }
+
+// k-rows of a uniform-width table: whole tiles of the TMA-staged kernel
+static uint64_t uniform_table_krows(uint32_t n_slices, uint32_t width) { return round_up(n_slices, kTmaConsumerWarps) * width; }
+
+// col_ / wgt_ for the table of which the builder writes the first sell_krows_ k-rows.  A uniform-width table (`width` > 0) is
+// allocated to uniform_table_krows; the k-rows past the last slice are padding (col kColPad, weight 0).
+int Engine::alloc_table(uint32_t width) {
+    const uint64_t krows = width ? uniform_table_krows(n_slices_, width) : sell_krows_;
+    CK(dev_alloc(&col_, krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
+    CK(dev_alloc(&wgt_, krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (!width) return SNN_OK;
+    sell_alloc_krows_ = krows;
+    if (krows > sell_krows_) {
+        CK(cudaMemsetAsync(col_ + sell_krows_ * 32, 0xFF, (krows - sell_krows_) * 32 * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+        CK(cudaMemsetAsync(wgt_ + sell_krows_ * 32, 0, (krows - sell_krows_) * 32 * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    }
     return SNN_OK;
 }
 
@@ -1029,9 +1060,7 @@ int Engine::finalize_graph() {
     const uint32_t new_slices = (uint32_t)((n_neurons + 31) / 32);
     bool reuse = false;
     if (blocks_.size() == 1 && blocks_.begin()->second.kind == Block::GRID && col_ && wgt_ && slice_off_ && n_slices_ == new_slices) {
-        const Block &b0 = blocks_.begin()->second;
-        const uint32_t width0 = (2 * b0.radius + 1) * (2 * b0.radius + 1) - 1;
-        reuse = sell_alloc_krows_ == round_up(new_slices, kTmaConsumerWarps) * width0;
+        reuse = sell_alloc_krows_ == uniform_table_krows(new_slices, stencil_width(blocks_.begin()->second.radius));
     }
     if (!reuse) {
         if (slice_off_) cudaFree(slice_off_);
@@ -1060,20 +1089,9 @@ int Engine::finalize_graph() {
     if (n_neuron_lat == 1 && blocks_.size() == 1 && blocks_.begin()->second.kind == Block::GRID &&
         blocks_.begin()->first == std::make_pair(only->id, only->id)) {
         const Block &b = blocks_.begin()->second;
-        const uint32_t width = (2 * b.radius + 1) * (2 * b.radius + 1) - 1;
+        const uint32_t width = stencil_width(b.radius);
         sell_krows_ = (uint64_t)n_slices_ * width;
-        const uint64_t alloc_krows = round_up(n_slices_, kTmaConsumerWarps) * width;  // whole tiles for the TMA kernel
-        if (!reuse) {
-            CK(dev_alloc(&col_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
-            CK(dev_alloc(&wgt_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
-            sell_alloc_krows_ = alloc_krows;
-            // only the slices beyond the last neuron are not written by the generator
-            const uint64_t tail0 = sell_krows_ * 32, tail_n = (alloc_krows - sell_krows_) * 32;
-            if (tail_n) {
-                CK(cudaMemsetAsync(col_ + tail0, 0xFF, tail_n * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-                CK(cudaMemsetAsync(wgt_ + tail0, 0, tail_n * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-            }
-        }
+        if (!reuse) { int r = alloc_table(width); if (r) return r; }
         if (n_neurons == 0) CK(cudaMemsetAsync(slice_off_, 0, 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
         CK(launch_sell_grid(only->rows, only->cols, part_world > 1 ? row0_global : 0, part_world > 1 ? rows_global : only->rows,
                             b.radius, b.weight, own0_, node_flags_, width, slice_off_, col_, wgt_, stream_), SNN_GPU_QUEUE_FAILURE);
@@ -1089,45 +1107,26 @@ int Engine::finalize_graph() {
     for (auto &kv : blocks_)
         if (kv.second.kind == Block::GRID) materialize_grid(kv.second, *find(kv.first.first));
     std::vector<uint64_t> row_ptr(n_neurons + 1, 0);
-    // blocks into each post lattice ordered by the pre lattice's node offset => rows stay sorted by node index
-    std::vector<std::vector<std::pair<const Lat *, const Block *>>> into(lats_.size());
-    for (size_t li = 0; li < lats_.size(); ++li) {
-        if (lats_[li].is_train) continue;
-        for (auto &kv : blocks_)
-            if (kv.first.second == lats_[li].id) {
-                const Lat *A = find(kv.first.first);
-                if (A) into[li].emplace_back(A, &kv.second);
-            }
-        std::sort(into[li].begin(), into[li].end(), [&](auto &x, auto &y) { return node_off(*x.first) < node_off(*y.first); });
-        for (uint64_t q = 0; q < lats_[li].n; ++q) {
-            uint64_t c = 0;
-            for (auto &ab : into[li]) c += ab.second->row_ptr[q + 1] - ab.second->row_ptr[q];
-            row_ptr[lats_[li].off + q + 1] = c;
-        }
-    }
+    for_each_row_segment([&](const Lat &B, uint64_t q, const Lat &, Block &b, uint64_t) {
+        row_ptr[B.off + q + 1] += b.row_ptr[q + 1] - b.row_ptr[q];
+    });
     for (uint64_t i = 0; i < n_neurons; ++i) row_ptr[i + 1] += row_ptr[i];
     const uint64_t nnz = row_ptr[n_neurons];
     std::vector<uint32_t> pre(std::max<uint64_t>(nnz, 1));
     std::vector<float> w(std::max<uint64_t>(nnz, 1));
     const int64_t node_shift = part_world > 1 ? (int64_t)own0_ - (int64_t)row0_global * (only ? only->cols : 0) : 0;
     std::vector<uint64_t> ghost_rows;   // general-graph partition: rows with an in-edge from a ghost
-    for (size_t li = 0; li < lats_.size(); ++li) {
-        if (lats_[li].is_train) continue;
-        for (uint64_t q = 0; q < lats_[li].n; ++q) {
-            uint64_t o = row_ptr[lats_[li].off + q];
-            for (auto &ab : into[li]) {
-                const Block &b = *ab.second;
-                const uint32_t base = node_off(*ab.first);
-                for (uint64_t k = b.row_ptr[q]; k < b.row_ptr[q + 1]; ++k) {
-                    int64_t node = gpart_ ? global_to_node(b.pre[k]) : (part_world > 1 ? (int64_t)b.pre[k] + node_shift : (int64_t)base + b.pre[k]);
-                    if (node < 0 || node >= (int64_t)n_nodes_)
-                        return fail(SNN_UNSUPPORTED, "edge reaches beyond the halo of this strip");
-                    if (gpart_ && (node < (int64_t)own0_ || node >= (int64_t)own0_ + (int64_t)n_neurons)) ghost_rows.push_back(lats_[li].off + q);
-                    pre[o] = (uint32_t)node; w[o] = b.w[k]; ++o;
-                }
-            }
+    bool beyond_halo = false;
+    for_each_row_segment([&](const Lat &B, uint64_t q, const Lat &A, Block &b, uint64_t k) {
+        uint64_t o = row_ptr[B.off + q] + k;
+        for (uint64_t e = b.row_ptr[q]; e < b.row_ptr[q + 1]; ++e, ++o) {
+            int64_t node = gpart_ ? global_to_node(b.pre[e]) : (part_world > 1 ? (int64_t)b.pre[e] + node_shift : (int64_t)node_off(A) + b.pre[e]);
+            if (node < 0 || node >= (int64_t)n_nodes_) { beyond_halo = true; return; }
+            if (gpart_ && (node < (int64_t)own0_ || node >= (int64_t)own0_ + (int64_t)n_neurons)) ghost_rows.push_back(B.off + q);
+            pre[o] = (uint32_t)node; w[o] = b.w[e];
         }
-    }
+    });
+    if (beyond_halo) return fail(SNN_UNSUPPORTED, "edge reaches beyond the halo of this strip");
     std::vector<uint32_t> slice_off(n_slices_ + 1, 0);
     for (uint32_t s = 0; s < n_slices_; ++s) {
         uint64_t mx = 0;
@@ -1141,31 +1140,22 @@ int Engine::finalize_graph() {
     sell_krows_ = slice_off[n_slices_];
     // a materialised stencil (weights came back from the device: STDP, edit_weight) keeps the uniform-width layout of the
     // generator, so the window / TMA step kernels stay eligible after a rebuild
-    uint32_t stencil_width = 0;
+    uint32_t width = 0;
     if (n_neuron_lat == 1 && blocks_.size() == 1 && blocks_.begin()->second.from_grid_radius &&
         blocks_.begin()->first == std::make_pair(only->id, only->id)) {
-        const uint32_t R = blocks_.begin()->second.from_grid_radius;
-        stencil_width = (2 * R + 1) * (2 * R + 1) - 1;
+        width = stencil_width(blocks_.begin()->second.from_grid_radius);
         for (uint32_t s = 0; s < n_slices_; ++s) {
-            if (slice_off[s + 1] - slice_off[s] > stencil_width) { stencil_width = 0; break; }
+            if (slice_off[s + 1] - slice_off[s] > width) { width = 0; break; }
         }
-        if (stencil_width) {
-            for (uint32_t s = 0; s <= n_slices_; ++s) slice_off[s] = s * stencil_width;
-            sell_krows_ = (uint64_t)n_slices_ * stencil_width;
+        if (width) {
+            for (uint32_t s = 0; s <= n_slices_; ++s) slice_off[s] = s * width;
+            sell_krows_ = (uint64_t)n_slices_ * width;
         }
     }
     max_slice_width_ = 0;
     for (uint32_t s = 0; s < n_slices_; ++s) max_slice_width_ = std::max(max_slice_width_, slice_off[s + 1] - slice_off[s]);
-    const uint64_t alloc_krows = stencil_width ? round_up(n_slices_, kTmaConsumerWarps) * stencil_width : sell_krows_;
-    CK(dev_alloc(&col_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
-    CK(dev_alloc(&wgt_, alloc_krows * 32), SNN_GPU_BUFFER_CREATE_ERROR);
-    if (stencil_width) {
-        sell_alloc_krows_ = alloc_krows;
-        if (alloc_krows > sell_krows_) {
-            CK(cudaMemsetAsync(col_ + sell_krows_ * 32, 0xFF, (alloc_krows - sell_krows_) * 32 * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-            CK(cudaMemsetAsync(wgt_ + sell_krows_ * 32, 0, (alloc_krows - sell_krows_) * 32 * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
-        }
-    }
+    int r = alloc_table(width);
+    if (r) return r;
     CK(h2d_sync(slice_off_, slice_off.data(), ((size_t)n_slices_ + 1) * 4, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     uint64_t *d_rp = nullptr; uint32_t *d_pre = nullptr; float *d_w = nullptr;
     CK(dev_alloc(&d_rp, n_neurons + 1), SNN_GPU_BUFFER_CREATE_ERROR);
@@ -1178,7 +1168,7 @@ int Engine::finalize_graph() {
     if (e == cudaSuccess) e = cudaStreamSynchronize(stream_);
     cudaFree(d_rp); cudaFree(d_pre); cudaFree(d_w);
     if (e != cudaSuccess) return cuda_fail(e, SNN_GPU_QUEUE_FAILURE, "sell_from_csr");
-    if (stencil_width) { grid_fast_ = true; uniform_width_ = stencil_width; }
+    if (width) { grid_fast_ = true; uniform_width_ = width; }
     if (gpart_) {
         h_gslice_.assign(n_slices_, 0);
         for (uint64_t row : ghost_rows) h_gslice_[row / 32] |= 1u;
@@ -1271,8 +1261,7 @@ bool Engine::has_reward_lattices() const {
     return false;
 }
 
-// element index (k * 32 + lane) of every edge of block pre_id -> post_id, in the block's CSR order; rows are laid out as
-// finalize_graph wrote them (blocks into a lattice ordered by the presynaptic lattice's node offset)
+// element index (k * 32 + lane) of every edge of block pre_id -> post_id, in the block's CSR order
 int Engine::block_elements(uint64_t pre_id, uint64_t post_id, std::vector<size_t> *elems, Block **blk) {
     Lat *B = find(post_id);
     if (!find(pre_id) || !B || B->is_train) return fail(SNN_INVALID_ARGUMENT, "no such connection block");
@@ -1284,25 +1273,11 @@ int Engine::block_elements(uint64_t pre_id, uint64_t post_id, std::vector<size_t
     std::vector<uint32_t> so((size_t)n_slices_ + 1);
     CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
     CK(cudaMemcpy(so.data(), slice_off_, so.size() * 4, cudaMemcpyDeviceToHost), SNN_GPU_BUFFER_READ_ERROR);
-    Block tmp;
-    const Block *target = &it->second;
-    if (target->kind == Block::GRID) { tmp = *target; materialize_grid(tmp, *B); target = &tmp; }   // single stencil lattice: keep the device fast path
-    std::vector<std::pair<const Lat *, const Block *>> into;
-    for (auto &kv : blocks_)
-        if (kv.first.second == post_id) { const Lat *A = find(kv.first.first); if (A) into.emplace_back(A, &kv.second == &it->second ? target : &kv.second); }
-    std::sort(into.begin(), into.end(), [&](auto &x, auto &y) { return node_off(*x.first) < node_off(*y.first); });
-    elems->reserve(target->pre.size());
-    for (uint64_t q = 0; q < B->n; ++q) {
+    for_each_row_segment([&](const Lat &, uint64_t q, const Lat &A, Block &b, uint64_t k) {
+        if (A.id != pre_id) return;
         const uint64_t row = B->off + q;
-        const uint32_t sl = (uint32_t)(row / 32), lane = (uint32_t)(row % 32);
-        uint32_t k = so[sl];
-        for (auto &ab : into) {
-            const uint64_t len = ab.second->row_ptr[q + 1] - ab.second->row_ptr[q];
-            if (ab.second == target)
-                for (uint64_t e = 0; e < len; ++e) elems->push_back((size_t)(k + e) * 32 + lane);
-            k += (uint32_t)len;
-        }
-    }
+        for (uint64_t i = 0; i < b.row_ptr[q + 1] - b.row_ptr[q]; ++i) elems->push_back((size_t)(so[row / 32] + k + i) * 32 + row % 32);
+    }, B);
     return SNN_OK;
 }
 
@@ -1398,23 +1373,10 @@ int Engine::sync_weights_to_host() {
     }
     for (auto &kv : blocks_)
         if (kv.second.kind == Block::GRID) materialize_grid(kv.second, *find(kv.first.first));
-    // walk every row in the same order finalize_graph wrote it
-    for (auto &L : lats_) {
-        if (L.is_train) continue;
-        std::vector<std::pair<const Lat *, Block *>> into;
-        for (auto &kv : blocks_)
-            if (kv.first.second == L.id) { const Lat *A = find(kv.first.first); if (A) into.emplace_back(A, &kv.second); }
-        std::sort(into.begin(), into.end(), [&](auto &x, auto &y) { return node_off(*x.first) < node_off(*y.first); });
-        for (uint64_t q = 0; q < L.n; ++q) {
-            const uint64_t row = L.off + q;
-            const uint32_t s = (uint32_t)(row / 32), lane = (uint32_t)(row % 32);
-            uint32_t k = so[s];
-            for (auto &ab : into) {
-                Block &b = *ab.second;
-                for (uint64_t e = b.row_ptr[q]; e < b.row_ptr[q + 1]; ++e, ++k) b.w[e] = wg[(size_t)k * 32 + lane];
-            }
-        }
-    }
+    for_each_row_segment([&](const Lat &B, uint64_t q, const Lat &, Block &b, uint64_t k) {
+        const uint64_t row = B.off + q;
+        for (uint64_t i = 0, e = b.row_ptr[q]; e < b.row_ptr[q + 1]; ++i, ++e) b.w[e] = wg[(size_t)(so[row / 32] + k + i) * 32 + row % 32];
+    });
     dev_weights_newer_ = false;
     return SNN_OK;
 }
@@ -1446,17 +1408,8 @@ int Engine::get_connection_csr(uint64_t pre_id, uint64_t post_id, uint64_t *row_
         if (row_ptr) std::fill(row_ptr, row_ptr + n_post + 1, 0);
         return SNN_OK;
     }
-    Block &b = it->second;
-    if (b.kind == Block::GRID) {
-        // materialise on a copy so that the device fast path stays available
-        Block tmp = b;
-        materialize_grid(tmp, *A);
-        if (tmp.pre.size() != nnz) return fail(SNN_SIZE_MISMATCH, "nnz mismatch");
-        if (row_ptr) memcpy(row_ptr, tmp.row_ptr.data(), (n_post + 1) * 8);
-        if (pre) memcpy(pre, tmp.pre.data(), nnz * 4);
-        if (weights) memcpy(weights, tmp.w.data(), nnz * 4);
-        return SNN_OK;
-    }
+    Block tmp;
+    const Block &b = csr_view(it->second, *A, tmp);
     if (b.pre.size() != nnz) return fail(SNN_SIZE_MISMATCH, "nnz mismatch");
     if (row_ptr) memcpy(row_ptr, b.row_ptr.data(), (n_post + 1) * 8);
     if (pre && nnz) memcpy(pre, b.pre.data(), nnz * 4);
@@ -1477,13 +1430,12 @@ int Engine::get_connection_dense(uint64_t pre_id, uint64_t post_id, uint32_t *co
     auto it = blocks_.find({pre_id, post_id});
     if (it == blocks_.end()) return SNN_OK;
     Block tmp;
-    const Block *b = &it->second;
-    if (b->kind == Block::GRID) { tmp = *b; materialize_grid(tmp, *A); b = &tmp; }
+    const Block &b = csr_view(it->second, *A, tmp);
     for (uint64_t q = 0; q < n_post; ++q)
-        for (uint64_t k = b->row_ptr[q]; k < b->row_ptr[q + 1]; ++k) {
-            const uint64_t idx = (uint64_t)b->pre[k] * n_post + q;
+        for (uint64_t k = b.row_ptr[q]; k < b.row_ptr[q + 1]; ++k) {
+            const uint64_t idx = (uint64_t)b.pre[k] * n_post + q;
             if (connections) connections[idx] = 1;
-            if (weights) weights[idx] = b->w[k];
+            if (weights) weights[idx] = b.w[k];
         }
     return SNN_OK;
 }
@@ -2140,28 +2092,21 @@ int Engine::HistStage::plan_graph_history() {
             gp.whole = true;
             gp.h->nnz = e.ghist_nnz_;
         } else if (it != e.blocks_.end()) {
-            // finalize_graph's general path: every block is host CSR; rows hold the blocks into their lattice ordered by the
-            // presynaptic lattice's node offset (sync_weights_to_host walks them the same way)
+            // finalize_graph's general path: every block is host CSR
             if (roff.empty()) {
                 roff.assign(e.n_neurons + 1, 0);
-                for (auto &kv : e.blocks_) {
-                    const Lat *B = e.find(kv.first.second);
-                    for (uint64_t q = 0; q < B->n; ++q) roff[B->off + q + 1] += kv.second.row_ptr[q + 1] - kv.second.row_ptr[q];
-                }
+                e.for_each_row_segment([&](const Lat &B, uint64_t q, const Lat &, Block &b, uint64_t) {
+                    roff[B.off + q + 1] += b.row_ptr[q + 1] - b.row_ptr[q];
+                });
                 for (uint64_t i = 0; i < e.n_neurons; ++i) roff[i + 1] += roff[i];
                 if (roff[e.n_neurons] != e.ghist_nnz_) return e.fail(SNN_GPU_BUFFER_READ_ERROR, "graph history: host and device tables disagree");
             }
-            const Lat *A = e.find(key.first), *B = e.find(key.second);
-            std::vector<const Block *> before;
-            for (auto &kv : e.blocks_)
-                if (kv.first.second == key.second && kv.first != key && e.node_off(*e.find(kv.first.first)) < e.node_off(*A)) before.push_back(&kv.second);
+            const Lat *B = e.find(key.second);
             gp.b = &it->second;
             gp.src.resize(B->n);
-            for (uint64_t q = 0; q < B->n; ++q) {
-                uint64_t o = roff[B->off + q];
-                for (const Block *o_b : before) o += o_b->row_ptr[q + 1] - o_b->row_ptr[q];
-                gp.src[q] = o;
-            }
+            e.for_each_row_segment([&](const Lat &, uint64_t q, const Lat &A, Block &, uint64_t k) {
+                if (A.id == key.first) gp.src[q] = roff[B->off + q] + k;
+            }, B);
             gp.h->nnz = it->second.pre.size();
         } else {
             gp.h->nnz = 0;   // a lattice without an internal graph: empty records

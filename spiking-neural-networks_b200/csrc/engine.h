@@ -291,16 +291,20 @@ private:
     void compute_layout();
     uint32_t node_off(const Lat &L) const { return (L.is_train ? train0_ : own0_) + (uint32_t)L.off; }
     int n_neuron_lattices() const { int n = 0; for (auto &L : lats_) n += !L.is_train; return n; }
+    template <class F> void for_each_field(const Lat &L, F &&f) const;
     int lookup_field(const Lat &L, const char *name, FieldDef *out) const;
     int field_io(Lat &L, const FieldDef &fd, void *data, uint64_t count, bool set);
     int set_bits(uint32_t *words, const uint32_t *host_u32, uint64_t n, uint64_t bit0);
     int get_bits(const uint32_t *words, uint32_t *host_u32, uint64_t n, uint64_t bit0);
+    template <class F> void for_each_row_segment(F &&f, const Lat *into = nullptr);
+    int alloc_table(uint32_t width);
     int finalize_graph();
     int sync_weights_to_host();
     // element index of edge (pre node j -> neuron row) in the sliced-ELL arrays, or -1; the graph must be finalized
     int find_edge(uint64_t row, uint32_t j, int64_t *elem);
     int check_edge_endpoints(uint64_t pre_id, uint64_t post_id, uint64_t pre, uint64_t post, Lat **A, Lat **B);
-    int materialize_grid(Block &b, const Lat &L);
+    void materialize_grid(Block &b, const Lat &L) const;
+    Block &csr_view(Block &b, const Lat &L, Block &tmp) const;
     uint32_t nt_used() const; uint32_t rc_used() const;
     void refresh_flag_cache() const;
     mutable bool flags_cache_valid_ = false;

@@ -1,6 +1,10 @@
 """Boundary behaviour of the C ABI on the device: SoA conversion round trips, graph ingestion, error codes, empty
 lattices.  Mirrors the reference's conversion / edge-case tests (backend/tests/{neuron,neurotransmitter,ligand_gates,
 spike_train}_conversion.rs, size_zero_cases.rs, grid_formation_invariant.rs)."""
+import ctypes as C
+import json
+import os
+
 import numpy as np
 import pytest
 
@@ -67,6 +71,29 @@ def test_field_errors():
     assert lib.snn_lattice_set_field(be.h, b"neurotransmitters$t", p, 9, K.F32) == K.SNN_SIZE_MISMATCH
     assert b"current_voltage" in lib.snn_lattice_last_error(be.h) or b"neurotransmitters" in lib.snn_lattice_last_error(be.h)
     assert lib.snn_lattice_set_option(be.h, 1234, 1) == K.SNN_INVALID_ARGUMENT
+
+
+def test_field_directory_order():
+    """field_info(i) is public by index: the directory of every model x (neurotransmitter, receptor) kinetics lattice and of a
+    network's spike-train lattice of every train kind x neurotransmitter kinetics is the one in golden/field_directory.json
+    (`fields` holds the distinct (name, dtype, per) entries, each directory lists indices into it); index `count` is refused."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "field_directory.json")) as f:
+        golden = json.load(f)
+    entries = [tuple(e) for e in golden["fields"]]
+    name, dt, per = C.c_char_p(), C.c_int32(), C.c_uint32()
+    for key, want in golden["lattice"].items():
+        model, ntk, rck = map(int, key.split())
+        be = CudaLatticeBackend(model, ntk, rck, 2, 3)
+        assert be.fields(0) == [entries[i] for i in want], key
+        assert be.lib.snn_lattice_field_info(be.h, len(want), C.byref(name), C.byref(dt), C.byref(per)) == K.SNN_INVALID_ARGUMENT
+        be.close()
+    for key, want in golden["train"].items():
+        kind, ntk = map(int, key.split())
+        be = CudaNetworkBackend(K.MODEL_IZH, ntk, K.RC_APPROXIMATE, kind)
+        be.add_train_lattice(7, 2, 3)
+        assert be.fields(7) == [entries[i] for i in want], key
+        assert be.lib.snn_network_field_info(be.h, 7, len(want), C.byref(name), C.byref(dt), C.byref(per)) == K.SNN_INVALID_ARGUMENT
+        be.close()
 
 
 def test_graph_ingestion_round_trips():
