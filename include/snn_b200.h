@@ -163,8 +163,11 @@ typedef enum snn_option {
                                          run() first meets the neighbours on the host (4x this bound) before any step is enqueued */
     SNN_OPT_UPDATE_GRAPH_HISTORY = 13,  /* default 0 (per lattice): Graph::update_history of the lattice's own graph (graph/mod.rs:278-284),
                                            one record per step, read with snn_lattice_get_graph_history / snn_network_get_graph_history */
-    SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY = 14  /* default 0 (network-wide): LatticeNetwork::update_connecting_graph_history, one
+    SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY = 14, /* default 0 (network-wide): LatticeNetwork::update_connecting_graph_history, one
                                                      record per step of every connecting block (pre_id != post_id) */
+    SNN_OPT_UPDATE_SPIKE_EVENTS = 15  /* default 0 (per lattice, spike-train lattices included): one record per step of the cells that
+                                         spiked, compacted on the device; read with snn_lattice_get_spike_events /
+                                         snn_network_get_spike_events.  Independent of SNN_OPT_UPDATE_SPIKE_HISTORY */
 } snn_option_t;
 
 /* STDP, backend/src/neuron/plasticity/mod.rs:14-39 (defaults 2, 2, 4.5, 4.5, 0.1) */
@@ -351,6 +354,15 @@ SNN_API int32_t snn_lattice_reset_history(snn_lattice_t *h);
  * records assume one adjacency (edit_weight of an existing edge is allowed; reset_history lifts the restriction). */
 SNN_API int32_t snn_lattice_graph_history_len(snn_lattice_t *h, uint64_t *steps, uint64_t *nnz);
 SNN_API int32_t snn_lattice_get_graph_history(snn_lattice_t *h, float *out, uint64_t capacity_floats);
+/* spike events (SNN_OPT_UPDATE_SPIKE_EVENTS): `steps` records, record k being the cells that spiked in the k-th recorded step (the
+ * same step as row k of the spike history when both are on), `n_events` cell indices in all.  Records ascend by step and indices
+ * ascend inside a record.  Indices are flat cell indices i*cols+j; a row-strip or general-graph partition records the GLOBAL flat
+ * indices of its own rows.  The compaction runs on the device once per history chunk (popcount per raster word, scan, scatter);
+ * only the per-record counts and the events are copied to the host.  Cleared by reset_history (not by reset_timing). */
+SNN_API int32_t snn_lattice_spike_event_count(const snn_lattice_t *h, uint64_t *steps, uint64_t *n_events);
+/* step_ptr: steps + 1 entries (CSR by step: record k is neuron[step_ptr[k] .. step_ptr[k+1])); neuron: up to `capacity` indices,
+ * SNN_SIZE_MISMATCH when n_events exceeds it.  Either pointer may be NULL. */
+SNN_API int32_t snn_lattice_get_spike_events(snn_lattice_t *h, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity);
 
 /* ---- multi-GPU row strips (one process per GPU; plumbing by the caller, e.g. torch.distributed) */
 /* first global row of `rank`'s strip; rank == world gives `rows` */
@@ -500,6 +512,9 @@ SNN_API int32_t snn_network_reset_history(snn_network_t *h);
  * (or without edges) reports steps = nnz = 0.  Same restrictions as the lattice calls (reward-modulated networks: SNN_UNSUPPORTED). */
 SNN_API int32_t snn_network_graph_history_len(snn_network_t *h, uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz);
 SNN_API int32_t snn_network_get_graph_history(snn_network_t *h, uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity_floats);
+/* spike events of lattice `id` (a neuron or spike-train lattice), indices inside that lattice; see the snn_lattice_ calls */
+SNN_API int32_t snn_network_spike_event_count(const snn_network_t *h, uint64_t id, uint64_t *steps, uint64_t *n_events);
+SNN_API int32_t snn_network_get_spike_events(snn_network_t *h, uint64_t id, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity);
 
 #ifdef __cplusplus
 }

@@ -77,6 +77,14 @@ struct GraphHistory {
     std::vector<float> weights;
 };
 
+// Spike events (SNN_OPT_UPDATE_SPIKE_EVENTS): record k holds the flat cell indices that spiked in the k-th recorded step, ascending,
+// in neurons[step_ptr[k] .. step_ptr[k + 1])
+struct SpikeEvents {
+    std::vector<uint64_t> step_ptr{0};
+    std::vector<uint32_t> neurons;
+    std::size_t steps() const { return step_ptr.size() - 1; }
+};
+
 // ----------------------------------------------------------------------------------------------------------------------------
 // Lattice<T, AdjacencyMatrix, GridVoltageHistory, STDP, N>  (neuron/mod.rs:556-1220) on one B200
 // ----------------------------------------------------------------------------------------------------------------------------
@@ -86,6 +94,7 @@ public:
     bool electrical_synapse = true, chemical_synapse = false, do_plasticity = false;
     bool update_grid_history = false, update_spike_history = false, parallel = false;
     bool update_graph_history = false;   // records after each step's plasticity (Lattice::iterate, neuron/mod.rs:973-979)
+    bool update_spike_events = false;    // compacted spike lists next to (or instead of) the dense raster
     STDP plasticity;
 
     Lattice() = default;
@@ -182,6 +191,14 @@ public:
         ck(snn_lattice_get_graph_history(h_, g.weights.data(), g.weights.size()));
         return g;
     }
+    SpikeEvents spike_events() {
+        uint64_t steps = 0, n = 0;
+        ck(snn_lattice_spike_event_count(need(), &steps, &n));
+        SpikeEvents ev;
+        ev.step_ptr.resize(steps + 1); ev.neurons.resize(n);
+        ck(snn_lattice_get_spike_events(h_, ev.step_ptr.data(), ev.neurons.data(), n));
+        return ev;
+    }
 
     snn_lattice_t *handle() { return h_; }
 
@@ -200,6 +217,7 @@ protected:
         ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_GRID_HISTORY, update_grid_history));
         ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_SPIKE_HISTORY, update_spike_history));
         ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_GRAPH_HISTORY, update_graph_history));
+        ck(snn_lattice_set_option(h_, SNN_OPT_UPDATE_SPIKE_EVENTS, update_spike_events));
         ck(snn_lattice_set_option(h_, SNN_OPT_PARALLEL, parallel));
         const snn_stdp_t s{plasticity.a_plus, plasticity.a_minus, plasticity.tau_plus, plasticity.tau_minus, plasticity.dt};
         ck(snn_lattice_set_plasticity(h_, &s));
@@ -322,6 +340,15 @@ public:
         ck(snn_network_get_spike_history(h_, id, v.data(), v.size()));
         return v;
     }
+    // spike events of lattice `id` (SNN_OPT_UPDATE_SPIKE_EVENTS through set_lattice_option), indices inside the lattice
+    SpikeEvents spike_events(std::size_t id) {
+        uint64_t steps = 0, n = 0;
+        ck(snn_network_spike_event_count(h_, id, &steps, &n));
+        SpikeEvents ev;
+        ev.step_ptr.resize(steps + 1); ev.neurons.resize(n);
+        ck(snn_network_get_spike_events(h_, id, ev.step_ptr.data(), ev.neurons.data(), n));
+        return ev;
+    }
     snn_network_t *handle() { return h_; }
 
 protected:
@@ -425,7 +452,7 @@ private:
 // SpikeTrainLattice<N, T, U> on its own (neuron/mod.rs:1290-1428; RunSpikeTrainLattice :1419-1428): a network that holds just this lattice
 class SpikeTrainLattice {
 public:
-    bool update_grid_history = false, update_spike_history = false;
+    bool update_grid_history = false, update_spike_history = false, update_spike_events = false;
     explicit SpikeTrainLattice(snn_spike_train_t kind = SNN_TRAIN_POISSON, std::size_t id = 0) : net_(SNN_MODEL_IZHIKEVICH, kind), id_(id) {}
     // populate(&base_spike_train, num_rows, num_cols), :1321-1341; base = the spike train's fields that differ from Default
     void populate(const std::map<std::string, float> &base_fields, std::size_t rows, std::size_t cols) {
@@ -436,9 +463,11 @@ public:
     void run_lattice(std::size_t iterations) {
         net_.set_lattice_option(id_, SNN_OPT_UPDATE_GRID_HISTORY, update_grid_history);
         net_.set_lattice_option(id_, SNN_OPT_UPDATE_SPIKE_HISTORY, update_spike_history);
+        net_.set_lattice_option(id_, SNN_OPT_UPDATE_SPIKE_EVENTS, update_spike_events);
         net_.run_lattices(iterations);
     }
     std::vector<uint8_t> spike_history() { return net_.spike_history(id_); }
+    SpikeEvents spike_events() { return net_.spike_events(id_); }
 
 private:
     LatticeNetwork net_;

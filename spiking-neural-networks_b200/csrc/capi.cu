@@ -233,6 +233,7 @@ static int32_t engine_set_option(Engine *e, bool have_id, uint64_t id, int32_t o
     case SNN_OPT_UPDATE_EEG_HISTORY: if (!L || L->is_train) break; L->eeg_hist = value != 0; return SNN_OK;
     case SNN_OPT_UPDATE_GRAPH_HISTORY: if (!L || L->is_train) break; L->graph_hist = value != 0; return SNN_OK;
     case SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY: if (L || !e->is_network) break; e->conn_graph_hist = value != 0; return SNN_OK;
+    case SNN_OPT_UPDATE_SPIKE_EVENTS: if (!L) break; L->spike_events = value != 0; return SNN_OK;
     }
     return e->fail(SNN_INVALID_ARGUMENT, "unknown option or missing lattice id");
 }
@@ -256,6 +257,7 @@ static int32_t engine_get_option(const Engine *e, bool have_id, uint64_t id, int
     case SNN_OPT_UPDATE_EEG_HISTORY: if (!L) break; *value = L->eeg_hist; return SNN_OK;
     case SNN_OPT_UPDATE_GRAPH_HISTORY: if (!L) break; *value = L->graph_hist; return SNN_OK;
     case SNN_OPT_UPDATE_CONNECTING_GRAPH_HISTORY: if (L || !e->is_network) break; *value = e->conn_graph_hist; return SNN_OK;
+    case SNN_OPT_UPDATE_SPIKE_EVENTS: if (!L) break; *value = L->spike_events; return SNN_OK;
     }
     return SNN_INVALID_ARGUMENT;
 }
@@ -356,6 +358,14 @@ int32_t snn_lattice_graph_history_len(snn_lattice_t *h, uint64_t *steps, uint64_
 int32_t snn_lattice_get_graph_history(snn_lattice_t *h, float *out, uint64_t capacity_floats) {
     if (!h) return SNN_INVALID_ARGUMENT;
     SNN_TRY return h->e->get_graph_history(kLatticeId, kLatticeId, out, capacity_floats); SNN_CATCH(h)
+}
+int32_t snn_lattice_spike_event_count(const snn_lattice_t *h, uint64_t *steps, uint64_t *n_events) {
+    if (!h || !steps || !n_events) return SNN_INVALID_ARGUMENT;
+    return h->e->spike_event_count(kLatticeId, steps, n_events);
+}
+int32_t snn_lattice_get_spike_events(snn_lattice_t *h, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity) {
+    if (!h) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->get_spike_events(kLatticeId, step_ptr, neuron, capacity); SNN_CATCH(h)
 }
 
 uint32_t snn_lattice_ipc_blob_size(void) { return (uint32_t)sizeof(snn::IpcBlob); }
@@ -610,6 +620,14 @@ int32_t snn_network_graph_history_len(snn_network_t *h, uint64_t pre_id, uint64_
 int32_t snn_network_get_graph_history(snn_network_t *h, uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity_floats) {
     if (!h) return SNN_INVALID_ARGUMENT;
     SNN_TRY return h->e->get_graph_history(pre_id, post_id, out, capacity_floats); SNN_CATCH(h)
+}
+int32_t snn_network_spike_event_count(const snn_network_t *h, uint64_t id, uint64_t *steps, uint64_t *n_events) {
+    if (!h || !steps || !n_events) return SNN_INVALID_ARGUMENT;
+    return h->e->spike_event_count(id, steps, n_events);
+}
+int32_t snn_network_get_spike_events(snn_network_t *h, uint64_t id, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity) {
+    if (!h) return SNN_INVALID_ARGUMENT;
+    SNN_TRY return h->e->get_spike_events(id, step_ptr, neuron, capacity); SNN_CATCH(h)
 }
 
 }  // extern "C"

@@ -409,5 +409,23 @@ cudaError_t launch_transpose_out(const float *src_tm, float *dst_nm, uint64_t n,
 cudaError_t launch_graph_row_offsets(const uint32_t *col, const uint32_t *slice_off, uint32_t n_slices, uint32_t *row_off, cudaStream_t s);
 cudaError_t launch_graph_record(const float *wgt, const uint32_t *slice_off, const uint32_t *row_off, uint32_t n_slices,
                                 uint32_t max_width, float *out, cudaStream_t s);
+// inclusive prefix sum of v[0, n) in place (one CTA: for the short arrays of per-tile or per-row counts)
+cudaError_t launch_scan_u32(uint32_t *v, uint64_t n, cudaStream_t s);
+
+// spike events (spike_events.cu): one lattice's bits [bit0, bit1) of a staged raster whose record s starts at raster + s * stride;
+// words [w0, w0 + nw) hold them.  Its items (one per word and record) start at item0; an event is bit - bit0 + add.
+struct EvSeg {
+    const uint32_t *raster;
+    uint32_t stride, w0, nw, bit0, bit1, add, item0;
+};
+struct EvParams {
+    EvSeg seg[2 * kMaxLattices];   // neuron lattices, then spike-train lattices, in item order
+    uint32_t n_seg, steps, n_items;
+};
+uint32_t ev_tiles(uint32_t n_items);
+// tile_off[0 .. ev_tiles(n_items)]: events before each tile, the chunk's total last
+cudaError_t launch_spike_event_count(const EvParams &p, uint32_t *tile_off, cudaStream_t s);
+// events[0 .. total) in canonical order, rec_off[seg * steps + s] = events before record s of segment seg
+cudaError_t launch_spike_event_scatter(const EvParams &p, const uint32_t *tile_off, uint32_t *events, uint32_t *rec_off, cudaStream_t s);
 
 }  // namespace snn

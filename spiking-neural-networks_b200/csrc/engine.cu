@@ -74,6 +74,7 @@ Engine::~Engine() {
     if (wide_scratch_) cudaFree(wide_scratch_);
     if (scratch_) cudaFree(scratch_);
     if (ghist_row_off_) cudaFree(ghist_row_off_);
+    if (ev_bounce_) cudaFreeHost(ev_bounce_);
     if (ev0_) cudaEventDestroy(ev0_);
     if (ev1_) cudaEventDestroy(ev1_);
     if (stream_) cudaStreamDestroy(stream_);
@@ -1616,7 +1617,10 @@ int Engine::reset_timing() {
 }
 
 int Engine::reset_history() {
-    for (auto &L : lats_) { L.grid_history.clear(); L.spike_history.clear(); L.spike_agg.clear(); L.average_history.clear(); L.eeg_history.clear(); L.hist_len = 0; }
+    for (auto &L : lats_) {
+        L.grid_history.clear(); L.spike_history.clear(); L.spike_agg.clear(); L.average_history.clear(); L.eeg_history.clear(); L.hist_len = 0;
+        L.ev_ptr.clear(); L.ev_neuron.clear();
+    }
     graph_hist_.clear();
     return SNN_OK;
 }
@@ -1702,6 +1706,27 @@ int Engine::get_spike_history(uint64_t id, uint8_t *out, uint64_t capacity) {
     if (!L) return fail(SNN_NET_ID_NOT_FOUND_IN_LATTICES, "Id not present in lattices");
     if (capacity < L->spike_history.size()) return fail(SNN_SIZE_MISMATCH, "history buffer too small");
     if (!L->spike_history.empty()) memcpy(out, L->spike_history.data(), L->spike_history.size());
+    return SNN_OK;
+}
+
+int Engine::spike_event_count(uint64_t id, uint64_t *steps, uint64_t *n_events) const {
+    const Lat *L = find(id);
+    if (!L) return SNN_NET_ID_NOT_FOUND_IN_LATTICES;
+    if (steps) *steps = L->ev_ptr.empty() ? 0 : L->ev_ptr.size() - 1;
+    if (n_events) *n_events = L->ev_neuron.size();
+    return SNN_OK;
+}
+
+// `capacity` bounds the neuron array; step_ptr must hold steps + 1 entries (either pointer may be NULL)
+int Engine::get_spike_events(uint64_t id, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity) {
+    Lat *L = find(id);
+    if (!L) return fail(SNN_NET_ID_NOT_FOUND_IN_LATTICES, "Id not present in lattices");
+    if (neuron && capacity < L->ev_neuron.size()) return fail(SNN_SIZE_MISMATCH, "spike event buffer too small");
+    if (step_ptr) {
+        if (L->ev_ptr.empty()) step_ptr[0] = 0;
+        else memcpy(step_ptr, L->ev_ptr.data(), L->ev_ptr.size() * 8);
+    }
+    if (neuron && !L->ev_neuron.empty()) memcpy(neuron, L->ev_neuron.data(), L->ev_neuron.size() * 4);
     return SNN_OK;
 }
 
@@ -1962,6 +1987,8 @@ struct Engine::RunPlan {
     bool lft_pp = false;                           // last_firing_time is ping-ponged
     // histories: grid (including the grid record the reductions read), its host copy, spikes, train grid / spikes, reductions
     bool want_grid = false, copy_grid = false, want_spk = false, want_tgrid = false, want_tspk = false, want_red = false;
+    // the staged rasters also serve the spike events; copy_*: some lattice of the domain keeps the dense SpikeHistory
+    bool copy_spk = false, copy_tspk = false, want_ev = false;
     bool ghist_on = false;
     std::vector<std::pair<uint64_t, uint64_t>> gh_keys;   // blocks whose graph records this run appends to
     StepPath path = StepPath::General;
@@ -1983,6 +2010,8 @@ struct Engine::LaunchArgs {
     uint64_t launches = 0;
     float total_ms = 0.f;
 };
+
+static constexpr size_t kEvBounceBytes = 4u << 20;
 
 // History staging: chunks of timesteps are recorded on the device and drained to the host between chunks.  Owns the staging
 // buffers of one run().
@@ -2007,7 +2036,15 @@ struct Engine::HistStage {
 
     HistStage(Engine &eng, const RunPlan &plan)
         : e(eng), pl(plan), n_words((eng.n_neurons + 31) / 32), t_words((eng.n_trains + 31) / 32) {}
-    ~HistStage() { cudaFree(grid); cudaFree(spk); cudaFree(tgrid); cudaFree(tspk); cudaFree(red); cudaFree(red_lat); cudaFree(ghist); }
+    // spike events of a chunk: the lattices recorded (segment order of EvParams), per-tile offsets, per-record offsets, the events
+    std::vector<Lat *> ev_lats;
+    uint32_t *ev_tile = nullptr, *ev_rec = nullptr, *ev_buf = nullptr;
+    uint64_t ev_cap = 0;
+
+    ~HistStage() {
+        cudaFree(grid); cudaFree(spk); cudaFree(tgrid); cudaFree(tspk); cudaFree(red); cudaFree(red_lat); cudaFree(ghist);
+        cudaFree(ev_tile); cudaFree(ev_rec); cudaFree(ev_buf);
+    }
     int cuda_fail(cudaError_t x, int status, const char *what) { return e.cuda_fail(x, status, what); }
 
     int init(uint64_t iterations);
@@ -2040,6 +2077,8 @@ struct Engine::HistStage {
     }
     int drain(uint64_t steps);
     int drain_graph();
+    int drain_events(uint64_t steps);
+    int d2h(void *dst, const void *src, size_t bytes);
 };
 
 int Engine::HistStage::init(uint64_t iterations) {
@@ -2068,6 +2107,80 @@ int Engine::HistStage::init(uint64_t iterations) {
         CK(h2d_sync(red_lat, meta.data(), meta.size() * 4, e.stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     }
     if (pl.ghist_on && e.ghist_nnz_) CK(dev_alloc(&ghist, (chunk + 1) * e.ghist_nnz_), SNN_GPU_BUFFER_CREATE_ERROR);
+    if (pl.want_ev) {
+        uint64_t words = 0;
+        for (int dom = 0; dom < 2; ++dom)
+            for (auto &L : e.lats_)
+                if (L.spike_events && L.is_train == (dom == 1)) {
+                    ev_lats.push_back(&L);
+                    if (L.n) words += (L.off + L.n + 31) / 32 - L.off / 32;
+                }
+        CK(dev_alloc(&ev_tile, (uint64_t)ev_tiles((uint32_t)(chunk * words)) + 1), SNN_GPU_BUFFER_CREATE_ERROR);
+        CK(dev_alloc(&ev_rec, chunk * ev_lats.size()), SNN_GPU_BUFFER_CREATE_ERROR);
+        if (!e.ev_bounce_) CK(cudaMallocHost(&e.ev_bounce_, kEvBounceBytes), SNN_GPU_BUFFER_CREATE_ERROR);
+    }
+    return SNN_OK;
+}
+
+// Device -> host through the pinned bounce buffer, on the engine's stream.
+int Engine::HistStage::d2h(void *dst, const void *src, size_t bytes) {
+    for (size_t o = 0; o < bytes; o += kEvBounceBytes) {
+        const size_t b = std::min<size_t>(kEvBounceBytes, bytes - o);
+        CK(cudaMemcpyAsync(e.ev_bounce_, (const char *)src + o, b, cudaMemcpyDeviceToHost, e.stream_), SNN_GPU_BUFFER_READ_ERROR);
+        CK(cudaStreamSynchronize(e.stream_), SNN_GPU_WAIT_ERROR);
+        memcpy((char *)dst + o, e.ev_bounce_, b);
+    }
+    return SNN_OK;
+}
+
+// The chunk's spike events (spike_events.cu): count, scan, size the event buffer from the total, scatter; then only the per-record
+// offsets and the events cross to the host, appended to each lattice's lists.
+int Engine::HistStage::drain_events(uint64_t steps) {
+    EvParams p{};
+    p.steps = (uint32_t)steps;
+    std::vector<Lat *> segs;   // lattice of each segment (lattices without cells have none)
+    uint64_t items = 0;
+    for (Lat *L : ev_lats) {
+        if (!L->n) continue;
+        EvSeg &g = p.seg[p.n_seg++];
+        g.raster = L->is_train ? tspk : spk;
+        g.stride = (uint32_t)(L->is_train ? t_words : n_words);
+        g.bit0 = (uint32_t)L->off; g.bit1 = (uint32_t)(L->off + L->n);
+        g.w0 = g.bit0 / 32; g.nw = (g.bit1 + 31) / 32 - g.w0;
+        // partitions own one lattice: its events are global flat indices of the whole lattice
+        g.add = L->is_train ? 0u : e.row0_global * L->cols;
+        g.item0 = (uint32_t)items;
+        items += steps * g.nw;
+        segs.push_back(L);
+    }
+    p.n_items = (uint32_t)items;
+    const uint32_t tiles = ev_tiles(p.n_items);
+    CK(launch_spike_event_count(p, ev_tile, e.stream_), SNN_GPU_QUEUE_FAILURE);
+    uint32_t total = 0;
+    int r = d2h(&total, ev_tile + tiles, 4);
+    if (r) return r;
+    if (total > ev_cap) {   // grown from the chunk's own total, never sized for the worst case up front
+        const uint64_t cap = std::max<uint64_t>(total, 2 * ev_cap);
+        cudaFree(ev_buf);
+        ev_buf = nullptr; ev_cap = 0;
+        CK(dev_alloc(&ev_buf, cap), SNN_GPU_BUFFER_CREATE_ERROR);
+        ev_cap = cap;
+    }
+    CK(launch_spike_event_scatter(p, ev_tile, ev_buf, ev_rec, e.stream_), SNN_GPU_QUEUE_FAILURE);
+    std::vector<uint32_t> rec((size_t)p.n_seg * steps + 1);
+    if ((r = d2h(rec.data(), ev_rec, (rec.size() - 1) * 4))) return r;
+    rec.back() = total;
+    for (uint32_t k = 0; k < p.n_seg; ++k) {
+        Lat &L = *segs[k];
+        const uint32_t a = rec[(size_t)k * steps], b = rec[(size_t)(k + 1) * steps];
+        const size_t o = L.ev_neuron.size();
+        L.ev_neuron.resize(o + (b - a));
+        if ((r = d2h(L.ev_neuron.data() + o, ev_buf + a, (size_t)(b - a) * 4))) return r;
+        if (L.ev_ptr.empty()) L.ev_ptr.push_back(0);
+        for (uint64_t s = 0; s < steps; ++s) L.ev_ptr.push_back(o + (rec[(size_t)k * steps + s + 1] - a));
+    }
+    for (Lat *L : ev_lats)
+        if (!L->n) { if (L->ev_ptr.empty()) L->ev_ptr.push_back(0); L->ev_ptr.insert(L->ev_ptr.end(), steps, L->ev_neuron.size()); }
     return SNN_OK;
 }
 
@@ -2153,6 +2266,7 @@ int Engine::HistStage::drain_graph() {
 // The records of the chunk's `steps` timesteps, appended to the lattices' host histories.
 int Engine::HistStage::drain(uint64_t steps) {
     if (pl.ghist_on && gh_recs) { int r = drain_graph(); if (r) return r; }
+    if (pl.want_ev) { int r = drain_events(steps); if (r) return r; }
     if (!per_step_bytes) return SNN_OK;
     const uint64_t n_neurons = e.n_neurons, n_trains = e.n_trains;
     std::vector<float> hg, htg; std::vector<uint32_t> hs, hts;
@@ -2180,15 +2294,15 @@ int Engine::HistStage::drain(uint64_t steps) {
             if (!L.grid_hist && !L.spike_hist) L.hist_len += steps;
         }
     }
-    if (pl.want_spk) { hs.resize(steps * n_words); he = cudaMemcpy(hs.data(), spk, hs.size() * 4, cudaMemcpyDeviceToHost); }
+    if (pl.copy_spk) { hs.resize(steps * n_words); he = cudaMemcpy(hs.data(), spk, hs.size() * 4, cudaMemcpyDeviceToHost); }
     if (he == cudaSuccess && pl.want_tgrid) { htg.resize(steps * n_trains); he = cudaMemcpy(htg.data(), tgrid, htg.size() * 4, cudaMemcpyDeviceToHost); }
-    if (he == cudaSuccess && pl.want_tspk) { hts.resize(steps * t_words); he = cudaMemcpy(hts.data(), tspk, hts.size() * 4, cudaMemcpyDeviceToHost); }
+    if (he == cudaSuccess && pl.copy_tspk) { hts.resize(steps * t_words); he = cudaMemcpy(hts.data(), tspk, hts.size() * 4, cudaMemcpyDeviceToHost); }
     if (he != cudaSuccess) return cuda_fail(he, SNN_GPU_BUFFER_READ_ERROR, "history drain");
     // SpikeHistory::aggregate (neuron/mod.rs:335-359): the sum over the chunk's steps is taken on the device from the staged
     // raster; the host only adds one count per neuron and chunk
     std::vector<uint32_t> cnt_n, cnt_t;
     for (int dom = 0; dom < 2 && he == cudaSuccess; ++dom) {
-        const bool on = dom ? pl.want_tspk : pl.want_spk;
+        const bool on = dom ? pl.copy_tspk : pl.copy_spk;
         const uint64_t dn = dom ? n_trains : n_neurons, dw = dom ? t_words : n_words;
         if (!on || dn == 0) continue;
         std::vector<uint32_t> &cnt = dom ? cnt_t : cnt_n;
@@ -2342,8 +2456,13 @@ int Engine::plan_run(RunPlan &pl, LaunchArgs &a) {
     if (gpart_) { r = gpart_build_device(); if (r) return r; }
 
     for (auto &L : lats_) {
-        if (!L.is_train) { pl.spec.stdp |= L.do_plasticity && !L.is_reward; pl.want_grid |= L.grid_hist; pl.want_spk |= L.spike_hist; pl.want_red |= L.avg_hist || L.eeg_hist; }
-        else { pl.want_tgrid |= L.grid_hist; pl.want_tspk |= L.spike_hist; }
+        if (!L.is_train) { pl.spec.stdp |= L.do_plasticity && !L.is_reward; pl.want_grid |= L.grid_hist; pl.copy_spk |= L.spike_hist; pl.want_red |= L.avg_hist || L.eeg_hist; }
+        else { pl.want_tgrid |= L.grid_hist; pl.copy_tspk |= L.spike_hist; }
+        pl.want_ev |= L.spike_events;
+    }
+    for (auto &L : lats_) {
+        const bool stage = L.spike_hist || L.spike_events;
+        (L.is_train ? pl.want_tspk : pl.want_spk) |= stage;
     }
     // AverageVoltageHistory / EEGHistory are reductions of the staged grid record (it stays on the device for them)
     pl.copy_grid = pl.want_grid;

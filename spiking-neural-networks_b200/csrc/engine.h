@@ -26,6 +26,7 @@ struct Lat {
     bool do_plasticity = false, grid_hist = false, spike_hist = false;
     bool avg_hist = false, eeg_hist = false;        // AverageVoltageHistory / EEGHistory (neuron/mod.rs:231-322)
     bool graph_hist = false;                        // update_graph_history: records of this lattice's own graph (graph/mod.rs:278-284)
+    bool spike_events = false;                      // SNN_OPT_UPDATE_SPIKE_EVENTS: compacted (step, cell) spike lists
     float eeg_ref = 0.007f, eeg_dist = 0.8f, eeg_cond = 251.f;   // EEGHistory::default, neuron/mod.rs:243-252
     std::vector<float> average_history, eeg_history;
     snn_stdp_t stdp{2.f, 2.f, 4.5f, 4.5f, 0.1f};  // STDP::default, plasticity/mod.rs:29-39
@@ -39,6 +40,9 @@ struct Lat {
     std::vector<uint8_t> spike_history;
     std::vector<int64_t> spike_agg;                // SpikeHistory::aggregate, accumulated from device-side counts
     uint64_t hist_len = 0;
+    // spike events: record k's cells are ev_neuron[ev_ptr[k] .. ev_ptr[k + 1]) (ev_ptr is empty before the first record)
+    std::vector<uint64_t> ev_ptr;
+    std::vector<uint32_t> ev_neuron;
     std::vector<uint64_t> ft_off;                 // preset firing times (CSR) of a train lattice
     std::vector<float> ft;
 };
@@ -148,6 +152,9 @@ public:
     int graph_history_len(uint64_t pre_id, uint64_t post_id, uint64_t *steps, uint64_t *nnz);
     int get_graph_history(uint64_t pre_id, uint64_t post_id, float *out, uint64_t capacity);
     bool graph_history_nonempty() const;
+    // spike events of one lattice: `steps` records (CSR by step, step_ptr has steps + 1 entries) of `n_events` cell indices
+    int spike_event_count(uint64_t id, uint64_t *steps, uint64_t *n_events) const;
+    int get_spike_events(uint64_t id, uint64_t *step_ptr, uint32_t *neuron, uint64_t capacity);
 
     // multi-GPU
     int ipc_export(IpcBlob *blob);
@@ -272,6 +279,8 @@ private:
     uint64_t ghist_nnz_ = 0;
     bool ghist_off_valid_ = false;
     int refuse_if_graph_history(const char *what);
+    // spike events: pinned bounce buffer of the device-to-host copies (allocated by the first run that records events)
+    void *ev_bounce_ = nullptr;
 
     int ipc_export_layout(IpcBlob *blob);
     int map_peer(const IpcBlob *blob, Engine *local, int expect_rank, PeerMap *out, IpcBlob *view);

@@ -26,7 +26,7 @@ __global__ void __launch_bounds__(256) graph_row_count_kernel(const uint32_t *__
     if (r == 0) row_off[0] = 0;
 }
 
-// inclusive prefix sum of v[0, n) in place, one CTA (once per graph build, not per step)
+// inclusive prefix sum of v[0, n) in place, one CTA (once per graph build, and once per drained chunk of spike events)
 __global__ void __launch_bounds__(1024) graph_row_scan_kernel(uint32_t *v, uint64_t n) {
     __shared__ uint32_t part[1024];
     const uint32_t t = threadIdx.x;
@@ -95,7 +95,12 @@ cudaError_t launch_graph_row_offsets(const uint32_t *col, const uint32_t *slice_
     if (n_slices == 0) return cudaMemsetAsync(row_off, 0, 4, s);
     const uint64_t rows = (uint64_t)n_slices * 32u;
     graph_row_count_kernel<<<(unsigned)((rows + 255u) / 256u), 256, 0, s>>>(col, slice_off, n_slices, row_off);
-    graph_row_scan_kernel<<<1, 1024, 0, s>>>(row_off + 1, rows);
+    cudaError_t e = cudaGetLastError();
+    return e != cudaSuccess ? e : launch_scan_u32(row_off + 1, rows, s);
+}
+
+cudaError_t launch_scan_u32(uint32_t *v, uint64_t n, cudaStream_t s) {
+    graph_row_scan_kernel<<<1, 1024, 0, s>>>(v, n);
     return cudaGetLastError();
 }
 

@@ -6,6 +6,6 @@ from . import _capi
 from ._capi import SnnError, load_library
 from .backend import CudaLatticeBackend, CudaNetworkBackend
 from .lattice import (AverageVoltageHistory, EEGHistory, GraphHistory, GridVoltageHistory, Lattice, LatticeNetwork,
-                      RewardModulatedConnection, RewardModulatedLattice, RewardModulatedLatticeNetwork, SpikeHistory,
-                      SpikeTrainLattice, TraceRSTDP)
+                      RewardModulatedConnection, RewardModulatedLattice, RewardModulatedLatticeNetwork, SpikeEvents,
+                      SpikeHistory, SpikeTrainLattice, TraceRSTDP)
 from .neurons import *  # noqa: F401,F403

@@ -43,7 +43,7 @@ F32, U32, I32 = range(3)
 (OPT_ELECTRICAL_SYNAPSE, OPT_CHEMICAL_SYNAPSE, OPT_DO_PLASTICITY, OPT_UPDATE_GRID_HISTORY, OPT_UPDATE_SPIKE_HISTORY,
  OPT_INTERNAL_CLOCK, OPT_PARALLEL, OPT_RNG_SEED, OPT_UPDATE_AVERAGE_HISTORY, OPT_STEPS_PER_GRAPH,
  OPT_UPDATE_EEG_HISTORY, OPT_HALO_TIMEOUT_MS, OPT_GENERAL_PARTITION, OPT_UPDATE_GRAPH_HISTORY,
- OPT_UPDATE_CONNECTING_GRAPH_HISTORY) = range(15)
+ OPT_UPDATE_CONNECTING_GRAPH_HISTORY, OPT_UPDATE_SPIKE_EVENTS) = range(16)
 
 
 class StdpStruct(C.Structure):
@@ -134,6 +134,8 @@ SIGNATURES = {
     "snn_lattice_reset_history": ([_P], _i32),
     "snn_lattice_graph_history_len": ([_P, C.POINTER(_u64), C.POINTER(_u64)], _i32),
     "snn_lattice_get_graph_history": ([_P, _P, _u64], _i32),
+    "snn_lattice_spike_event_count": ([_P, C.POINTER(_u64), C.POINTER(_u64)], _i32),
+    "snn_lattice_get_spike_events": ([_P, _P, _P, _u64], _i32),
     "snn_partition_begin": ([_u32, _i32, _i32], _u32),
     "snn_lattice_ipc_blob_size": ([], _u32),
     "snn_lattice_ipc_export": ([_P, _P], _i32),
@@ -189,6 +191,8 @@ SIGNATURES = {
     "snn_network_reset_history": ([_P], _i32),
     "snn_network_graph_history_len": ([_P, _u64, _u64, C.POINTER(_u64), C.POINTER(_u64)], _i32),
     "snn_network_get_graph_history": ([_P, _u64, _u64, _P, _u64], _i32),
+    "snn_network_spike_event_count": ([_P, _u64, C.POINTER(_u64), C.POINTER(_u64)], _i32),
+    "snn_network_get_spike_events": ([_P, _u64, _P, _P, _u64], _i32),
 }
 
 _lib = None

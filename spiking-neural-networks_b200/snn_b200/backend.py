@@ -280,6 +280,15 @@ class CudaLatticeBackend(_CudaBase):
         self._ck(self.lib.snn_lattice_get_graph_history(self.h, _ptr(out), out.size))
         return out[:steps.value * nnz.value].reshape(steps.value, nnz.value)
 
+    def spike_events(self, id=0):
+        """Spike events of the lattice: (step_ptr u64[steps + 1], neurons u32[n_events]); record k is
+        neurons[step_ptr[k]:step_ptr[k + 1]], global flat indices on a partitioned handle."""
+        steps, n = C.c_uint64(), C.c_uint64()
+        self._ck(self.lib.snn_lattice_spike_event_count(self.h, C.byref(steps), C.byref(n)))
+        step_ptr, neurons = np.zeros(steps.value + 1, np.uint64), np.zeros(max(n.value, 1), np.uint32)
+        self._ck(self.lib.snn_lattice_get_spike_events(self.h, _ptr(step_ptr), _ptr(neurons), neurons.size))
+        return step_ptr, neurons[:n.value]
+
     # multi-GPU plumbing
     def ipc_export(self) -> bytes:
         buf = C.create_string_buffer(self.lib.snn_lattice_ipc_blob_size())
@@ -495,3 +504,11 @@ class CudaNetworkBackend(_CudaBase):
         out = np.zeros(max(steps.value * nnz.value, 1), np.float32)
         self._ck(self.lib.snn_network_get_graph_history(self.h, pre_id, post_id, _ptr(out), out.size))
         return out[:steps.value * nnz.value].reshape(steps.value, nnz.value)
+
+    def spike_events(self, id):
+        """Spike events of lattice `id`: (step_ptr u64[steps + 1], neurons u32[n_events]), indices inside the lattice."""
+        steps, n = C.c_uint64(), C.c_uint64()
+        self._ck(self.lib.snn_network_spike_event_count(self.h, id, C.byref(steps), C.byref(n)))
+        step_ptr, neurons = np.zeros(steps.value + 1, np.uint64), np.zeros(max(n.value, 1), np.uint32)
+        self._ck(self.lib.snn_network_get_spike_events(self.h, id, _ptr(step_ptr), _ptr(neurons), neurons.size))
+        return step_ptr, neurons[:n.value]

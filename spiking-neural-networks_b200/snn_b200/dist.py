@@ -10,6 +10,7 @@ from __future__ import annotations
 
 from . import _capi as K
 from .backend import CudaLatticeBackend
+from .lattice import SpikeEvents
 
 
 def partition_rows(rows: int, world: int, rank: int):
@@ -24,6 +25,33 @@ def exchange_blobs(blob: bytes, rank: int, world: int, group=None):
     blobs = [None] * world
     dist.all_gather_object(blobs, blob, group=group)
     return (blobs[rank - 1] if rank > 0 else None), (blobs[rank + 1] if rank < world - 1 else None)
+
+
+def merge_spike_events(parts, rows, cols):
+    """One SpikeEvents of the whole lattice from every rank's (step_ptr, neurons), in rank order: record k is the ranks' records k
+    one after the other.  Ranks own contiguous rows in rank order, so that is already ascending global order."""
+    import numpy as np
+    steps = {p[0].size - 1 for p in parts}
+    if len(steps) != 1:
+        raise ValueError(f"the ranks hold different numbers of spike-event records: {sorted(steps)}")
+    steps = steps.pop()
+    counts = np.stack([np.diff(p[0].astype(np.int64)) for p in parts])   # ranks x steps
+    step_ptr = np.zeros(steps + 1, np.uint64)
+    step_ptr[1:] = np.cumsum(counts.sum(axis=0))
+    step_of = np.concatenate([np.repeat(np.arange(steps), c) for c in counts]) if steps else np.zeros(0, np.int64)
+    neurons = np.concatenate([p[1] for p in parts]) if parts else np.zeros(0, np.uint32)
+    order = np.argsort(step_of, kind="stable")   # stable: the ranks stay in rank order inside a step
+    return SpikeEvents(step_ptr, neurons[order], rows, cols)
+
+
+def gather_spike_events(be, rank, world, group=None):
+    """torch.distributed: every rank's spike events of a row-strip or general-graph partition, merged as merge_spike_events does
+    (one all_gather_object); returns the whole lattice's SpikeEvents on every rank."""
+    import torch.distributed as dist
+    parts = [None] * world
+    dist.all_gather_object(parts, (be.spike_events(), be.shape()), group=group)
+    rows, cols = sum(p[1][0] for p in parts), parts[0][1][1]
+    return merge_spike_events([p[0] for p in parts], rows, cols)
 
 
 class StripLattice:
@@ -147,6 +175,10 @@ class LocalStrips:
             t.join()
         if errs:
             raise errs[0]
+
+    def spike_events(self):
+        """The whole lattice's spike events (SNN_OPT_UPDATE_SPIKE_EVENTS on every strip), the ranks' lists merged step by step."""
+        return merge_spike_events([be.spike_events() for be in self.strips], self.rows, self.cols)
 
     def graph_csr(self):
         """Whole-lattice CSR (global presynaptic indices) assembled from the strips."""

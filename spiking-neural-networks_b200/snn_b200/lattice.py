@@ -88,6 +88,34 @@ class SpikeHistory(GridVoltageHistory):
         return self._o._be.spike_aggregate(self._o._bid).reshape(self._o.rows, self._o.cols)
 
 
+class SpikeEvents:
+    """Spike events of one lattice (update_spike_events): record k holds the flat cell indices i*cols+j that spiked in the k-th
+    recorded step, ascending, in `neurons[step_ptr[k]:step_ptr[k + 1]]`.  The same data as the dense SpikeHistory raster, without
+    the steps x n grid: the compaction runs on the device and only the events reach the host."""
+
+    def __init__(self, step_ptr, neurons, rows, cols):
+        self.step_ptr = np.asarray(step_ptr, np.uint64)
+        self.neurons = np.asarray(neurons, np.uint32)
+        self.rows, self.cols = rows, cols
+
+    @property
+    def steps(self):
+        return self.step_ptr.size - 1
+
+    def _step_of_event(self):
+        return np.repeat(np.arange(self.steps, dtype=np.int64), np.diff(self.step_ptr.astype(np.int64)))
+
+    def pairs(self):
+        """(n_events, 2) int64 array of (step, flat index): np.nonzero of the dense raster, in the same order."""
+        return np.stack([self._step_of_event(), self.neurons.astype(np.int64)], axis=1)
+
+    def dense(self):
+        """The events expanded to the layout of spike_history.history: steps x rows x cols booleans."""
+        out = np.zeros((self.steps, self.rows * self.cols), bool)
+        out[self._step_of_event(), self.neurons.astype(np.int64)] = True
+        return out.reshape(self.steps, self.rows, self.cols)
+
+
 class AverageVoltageHistory(GridVoltageHistory):
     """neuron/mod.rs:303-322: `.history[step]` = mean membrane voltage of the lattice."""
     option = K.OPT_UPDATE_AVERAGE_HISTORY
@@ -161,8 +189,15 @@ class _CellLattice:
         self.cols = 0
         self.update_grid_history = False
         self.update_spike_history = False
+        self.update_spike_events = False
         self.grid_history = GridVoltageHistory(self)
         self.spike_history = SpikeHistory(self)
+
+    @property
+    def spike_events(self):
+        """The recorded spike events (SpikeEvents); cleared by spike_history.reset() / reset_history, not by reset_timing."""
+        step_ptr, neurons = self._be.spike_events(self._bid)
+        return SpikeEvents(step_ptr, neurons, self.rows, self.cols)
 
     # ---- field level (fast path) --------------------------------------------------------------
     @property
@@ -484,6 +519,7 @@ class Lattice(_CellLattice):
             be.set_eeg_parameters(i, gh.reference_voltage, gh.distance, gh.conductivity)
         be.set_option(gh.option, self.update_grid_history, i)
         be.set_option(K.OPT_UPDATE_SPIKE_HISTORY, self.update_spike_history, i)
+        _push_flag(self, be, K.OPT_UPDATE_SPIKE_EVENTS, self.update_spike_events, i)
         _push_flag(self, be, K.OPT_UPDATE_GRAPH_HISTORY, self.update_graph_history, i)
         p = self.plasticity
         if isinstance(p, BCM):   # Lattice<BCMIzhikevichNeuron, ..., BCM, ...>
@@ -687,6 +723,7 @@ class SpikeTrainLattice(_CellLattice):
             return
         self._be.set_option(K.OPT_UPDATE_GRID_HISTORY, self.update_grid_history, self._bid)
         self._be.set_option(K.OPT_UPDATE_SPIKE_HISTORY, self.update_spike_history, self._bid)
+        _push_flag(self, self._be, K.OPT_UPDATE_SPIKE_EVENTS, self.update_spike_events, self._bid)
         self._be.run(iterations)
 
 
@@ -873,6 +910,7 @@ class LatticeNetwork:
         for st in self._spike_train_lattices.values():
             self._be.set_option(K.OPT_UPDATE_GRID_HISTORY, st.update_grid_history, st.get_id())
             self._be.set_option(K.OPT_UPDATE_SPIKE_HISTORY, st.update_spike_history, st.get_id())
+            _push_flag(st, self._be, K.OPT_UPDATE_SPIKE_EVENTS, st.update_spike_events, st.get_id())
         self._be.run(iterations)
 
 
@@ -1048,6 +1086,7 @@ class RewardModulatedLatticeNetwork(LatticeNetwork):
         for st in self._spike_train_lattices.values():
             self._be.set_option(K.OPT_UPDATE_GRID_HISTORY, st.update_grid_history, st.get_id())
             self._be.set_option(K.OPT_UPDATE_SPIKE_HISTORY, st.update_spike_history, st.get_id())
+            _push_flag(st, self._be, K.OPT_UPDATE_SPIKE_EVENTS, st.update_spike_events, st.get_id())
 
     def run_lattices(self, iterations: int):
         """RunNetwork::run_lattices (neuron/mod.rs:5411-5426): no reward signal."""
