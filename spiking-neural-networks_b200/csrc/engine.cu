@@ -1969,13 +1969,13 @@ void Engine::await_step_exports(StepParams &ep) {
     wait_local_peers_launched(halo_epoch_ + 1, false);
 }
 
-// The step path of a run: which kernel steps the neurons of one timestep.
-enum class StepPath {
-    Win,         // window-staged persistent kernel (step_win.cu): radius-1 stencil lattices
-    Tma,         // TMA-staged persistent kernel (step_tma.cu): other uniform-width stencil lattices
-    Wide,        // one CTA per slice (step_wide.cu): wide rows
-    WideSplit,   // two passes, per-edge terms then ordered sums (step_wide.cu): very wide rows
-    General      // one thread per neuron (kernels.cu)
+// The step path of a run: which kernel steps the neurons of one timestep.  The values are those SNN_OPT_STEP_PATH reports.
+enum class StepPath : uint32_t {
+    General = 1,     // one thread per neuron (kernels.cu)
+    Wide = 2,        // one CTA per slice (step_wide.cu): wide rows
+    WideSplit = 3,   // two passes, per-edge terms then ordered sums (step_wide.cu): very wide rows
+    Tma = 4,         // TMA-staged persistent kernel (step_tma.cu): other uniform-width stencil lattices
+    Win = 5          // window-staged persistent kernel (step_win.cu): radius-1 stencil lattices
 };
 
 // Decisions fixed for a whole run(), taken once by plan_run.
@@ -2549,6 +2549,7 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
         pl.multi = launch_step_multi(a.sp, a.tp, probe, pl.spec, pl.path == StepPath::Wide, device, true, stream_) == cudaSuccess;
         cudaGetLastError();
     }
+    last_step_path = (uint32_t)pl.path + (pl.multi ? 16u : 0u);
     return SNN_OK;
 }
 

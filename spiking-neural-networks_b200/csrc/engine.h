@@ -178,6 +178,7 @@ public:
     uint64_t train_draws = 0;       // Philox counter word: one per spike-train step of this handle, never reset (reset_timing
                                     // restarts the clocks, not the random stream: the reference draws from thread_rng)
     uint32_t steps_per_graph = 0;
+    uint32_t last_step_path = 0;        // SNN_OPT_STEP_PATH: step path of the last run, path + 16 * multi (0: nothing run yet)
     bool force_gpart = false;           // SNN_OPT_GENERAL_PARTITION: CSR graphs of a partitioned handle always use gather-list ghosts
     uint64_t halo_timeout_ms = 30000;   // multi-GPU: how long a step may wait for a neighbouring strip before SNN_GPU_WAIT_ERROR
     std::string last_error;

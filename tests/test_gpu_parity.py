@@ -17,7 +17,8 @@ f32 = np.float32
 
 @pytest.fixture(autouse=True, params=["auto", "tma", "tma_l1"])
 def kernel_path(request, monkeypatch):
-    """Every parity test runs three times: with the automatic kernel choice (general step_kernel for small lattices), with
+    """Every parity test runs three times: with the automatic kernel choice (for small lattices the cooperative multi-step
+    step_multi_kernel, in its 16-CTA cluster variant up to 320 slices), with
     the TMA-staged persistent kernels forced wherever they are eligible (stencil graphs: the window-staged step_win_kernel
     for radius 1, the L1-gather step_tma_kernel for larger radii), and with the window kernel disabled so that
     step_tma_kernel also serves radius 1 — all three are held to the same bar."""
