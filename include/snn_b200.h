@@ -168,11 +168,14 @@ typedef enum snn_option {
     SNN_OPT_UPDATE_SPIKE_EVENTS = 15, /* default 0 (per lattice, spike-train lattices included): one record per step of the cells that
                                          spiked, compacted on the device; read with snn_lattice_get_spike_events /
                                          snn_network_get_spike_events.  Independent of SNN_OPT_UPDATE_SPIKE_HISTORY */
-    SNN_OPT_STEP_PATH = 16            /* read-only: the step path of the handle's last run / run_timed / run_with_rewards, path + 16 * multi.
+    SNN_OPT_STEP_PATH = 16,           /* read-only: the step path of the handle's last run / run_timed / run_with_rewards, path + 16 * multi.
                                          path: 0 nothing run yet, 1 general (one thread per neuron), 2 wide (one CTA per slice),
                                          3 wide split (per-edge terms pass, then ordered sums), 4 TMA-staged persistent kernel,
                                          5 window-staged persistent kernel (radius-1 stencils).  multi: 1 when whole chunks of
                                          timesteps ran in one cooperative launch (SNN_OPT_STEPS_PER_GRAPH) */
+    SNN_OPT_UNIFORM_TILES = 17        /* read-only: of the 256-neuron tiles of the handle's last run on the window-staged kernel, those
+                                         whose neurons all have the bit patterns of the tile's first neuron in every parameter the step
+                                         reads (these tiles read one copy of them instead of one per neuron); 0 on every other path */
 } snn_option_t;
 
 /* STDP, backend/src/neuron/plasticity/mod.rs:14-39 (defaults 2, 2, 4.5, 4.5, 0.1) */

@@ -256,7 +256,17 @@ struct WinLayout {
     uint32_t lrows, trows, tslots;   // window rows kept for last_firing_time / t, neurotransmitter type slots
     uint32_t o_vwin, o_lwin, o_twin, o_spk, o_flags, o_col, o_wgt;
     uint32_t o_f[F_NA_CUR];          // 0xFFFFFFFF = not read by this model
+    // rows (some tile reads its parameter row): the state fields first, then the row, then the parameters, so that a stage without
+    // per-neuron parameters ends at uni_end; without rows every field in slot order and no row (o_row = 0xFFFFFFFF)
+    uint32_t o_row;                  // the tile's parameter row (copied from the tile table, see win_field_param)
+    uint32_t uni_end;                // first byte after the part every tile fills (state fields and the row; multiple of 16)
     uint32_t fixed_end;              // first byte after the compile-time part (multiple of 128)
+    // the tile row, in 32-bit words: [0] 1 = every neuron of the tile has the first one's parameters (bit patterns), then the
+    // first neuron's parameters: r_f[slot] for the model's, [r_nt + NtSlot * kNT + type] for the neurotransmitters',
+    // [r_rc + (RcSlot - RCF_K1) * kNT + type] for the receptors' (words of kinetics this run does not read stay 0)
+    uint32_t r_f[F_NA_CUR];
+    uint32_t r_nt, r_rc;
+    uint32_t row_bytes;              // multiple of 16
 };
 
 // fields the step of `model` reads (must mirror neuron_step, step_body.cuh)
@@ -290,7 +300,21 @@ __host__ __device__ constexpr bool win_field_read(int model, bool ntrel, int slo
     }
 }
 
-__host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool ntrel, bool stdp) {
+// State among the fields win_field_read lists: neuron_step reads them through src.state<SLOT>() or writes them back.  The
+// others are parameters, read through src.f<SLOT>() only; with the neurotransmitter parameters (src.nt()) and the receptor
+// parameters (src.rc(): every receptor field but RCF_R, which is state and read through src.rc_state()) they are what a tile
+// whose neurons all share them takes from its tile row instead of from per-neuron streams.  WinSrc asserts both lists.
+__host__ __device__ constexpr bool win_field_state(int slot) {
+    switch (slot) {
+    case F_W: case F_REFR: case F_M: case F_H: case F_N: case F_AVG_ACT: case F_CUR_ACT: case F_NSPK: case F_FRCLK: return true;
+    default: return false;
+    }
+}
+__host__ __device__ constexpr bool win_field_param(int model, bool ntrel, int slot) {
+    return win_field_read(model, ntrel, slot) && !win_field_state(slot);
+}
+
+__host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool ntrel, bool stdp, bool rows) {
     WinLayout L{};
     uint32_t off = 0;
     L.lrows = stdp ? 3u : 1u;
@@ -304,16 +328,32 @@ __host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool nt
     L.o_flags = off; off += kWinTile;
     L.o_col = off; off += kWinEdgeBytes;
     L.o_wgt = off; off += kWinEdgeBytes;
+    uint32_t w = 1;
     for (int s = 0; s < F_NA_CUR; ++s) {
-        if (win_field_read(model, ntrel, s)) { L.o_f[s] = off; off += kWinTile * 4u; }
-        else L.o_f[s] = 0xFFFFFFFFu;
+        L.o_f[s] = 0xFFFFFFFFu;
+        L.r_f[s] = 0;
+        if (win_field_read(model, ntrel, s) && (win_field_state(s) || !rows)) { L.o_f[s] = off; off += kWinTile * 4u; }
+        if (win_field_param(model, ntrel, s)) L.r_f[s] = w++;
     }
+    L.r_nt = w; if (ntrel) w += NTF_COUNT * kNT;
+    L.r_rc = w; if (ntrel) w += (RCF_MG - RCF_K1 + 1) * kNT;
+    L.row_bytes = (w * 4u + 15u) & ~15u;
+    L.o_row = 0xFFFFFFFFu;
+    if (rows) {
+        L.o_row = off; off += L.row_bytes;
+        L.uni_end = off;
+        off = (off + 127u) & ~127u;
+        for (int s = 0; s < F_NA_CUR; ++s)
+            if (win_field_param(model, ntrel, s)) { L.o_f[s] = off; off += kWinTile * 4u; }
+    }
+    if (!rows) L.uni_end = off;
     L.fixed_end = off;
     return L;
 }
 
 struct WinParams {
-    uint32_t n_tiles, n_streams, stage_bytes, stages, fixed_tx_bytes;
+    uint32_t n_tiles, n_streams, stage_bytes, stages;
+    uint32_t n_state;             // streams [0, n_state) go to every tile, [n_state, n_streams) (parameters) to non-uniform tiles only
     uint32_t node_cap;            // elements allocated per node array (window copies are clamped to [0, node_cap))
     uint32_t cols;
     uint32_t lft_copy;            // copy last_firing_time windows at all (STDP or ping-ponged lft)
@@ -322,13 +362,35 @@ struct WinParams {
     TmaStream st[kMaxTmaStreams]; // per-tile contiguous operands (src + tile * bytes_per_tile)
     uint32_t o_nt[NTF_COUNT][kNT];   // run-time part of the stage layout: per-type chemical parameters
     uint32_t o_rc[RCF_COUNT][kNT];
+    // tile rows [n_tiles][row_words] (WinLayout::r_f ...), copied into every stage by the stream n_state - 1; nullptr: no tile is
+    // uniform (no row is copied, the stage layout is win_layout(..., rows = false))
+    const uint32_t *tile_par;
+    uint32_t row_words;
+    // first_lo + first_hi, and stages % consumer groups != 0, for the kernels that read tile rows: held in registers as values
+    // (as the kernel without rows holds them) they made those kernels spill
+    uint32_t first_end, ring_check;
 };
 
 // groups of 8 consumer warps per CTA (register budget: 65536 / ((groups * 8 + 1) * 32))
 // models with wide operand sets (Hodgkin-Huxley, three neurotransmitter types): fewer, fatter stages
-__host__ __device__ constexpr int win_groups(int model, int chemg) { return (model == SNN_MODEL_HODGKIN_HUXLEY || chemg == 3) ? 2 : 3; }
+// mixed: the kernel for lattices with both uniform and streaming tiles, which carries both step variants (with 3 groups and 72
+// registers, the variants of AdEx and simple LIF with chemistry and STDP spilled)
+__host__ __device__ constexpr int win_groups(int model, int chemg, bool mixed) {
+    return (mixed || model == SNN_MODEL_HODGKIN_HUXLEY || chemg == 3) ? 2 : 3;
+}
 
 cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const StepSpec &spec, unsigned grid, cudaStream_t s);
+
+// Tile rows of the window kernel: per kWinTile tile of [0, n_neurons), word 0 = 1 when every valid neuron of the tile has the
+// bit pattern of the tile's first neuron in every src[k] (compared as 32-bit words: -0.0 != +0.0, a NaN equals only its own
+// payload), word word[k] = the first neuron's src[k].  The other words are left as they are; *n_mixed += tiles with word 0 = 0.
+constexpr int kWinMaxPar = 48;
+struct TileParSrc {
+    const uint32_t *src[kWinMaxPar];   // indexed by local neuron number
+    uint32_t word[kWinMaxPar];
+    uint32_t n_par, row_words, n_neurons, n_tiles;
+};
+cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *n_mixed, cudaStream_t s);
 
 // ---- kernel launchers (kernels.cu) ------------------------------------------------------------
 cudaError_t launch_step(const StepParams &p, const StepSpec &spec, cudaStream_t s);

@@ -173,6 +173,7 @@ void Engine::free_device() {
     for (auto &p : TF_) fr(p);
     fr(ft_off_); fr(ft_); fr(d_lat_);
     fr(slice_off_); fr(col_); fr(wgt_);
+    fr(tile_par_); tile_par_bytes_ = 0; tile_par_dirty_ = true;
     free_reward_arrays();
     chem_alloc_ = false;
     graph_dirty_ = true;
@@ -286,6 +287,7 @@ int Engine::ensure_chem() {
     }
     CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
     chem_alloc_ = true;
+    tile_par_dirty_ = true;
     return SNN_OK;
 }
 
@@ -470,6 +472,7 @@ int Engine::field_io(Lat &L, const FieldDef &fd, void *data, uint64_t count, boo
         CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
         return SNN_OK;
     };
+    if (set && (fd.kind == FK_NEURON_DEV || fd.kind == FK_NT || fd.kind == FK_RC)) tile_par_dirty_ = true;
     switch (fd.kind) {
     case FK_NEURON_DEV:
         return plain(F_[fd.slot] + L.off, n);
@@ -600,6 +603,7 @@ int Engine::fill_field(uint64_t id, const char *name, uint32_t bits, int dtype) 
     if (dtype != fd.dtype) return fail(SNN_DTYPE_MISMATCH, std::string("dtype mismatch for field: ") + name);
     if (L->n == 0) return SNN_OK;
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
+    tile_par_dirty_ = true;
     // fast device-side fills for the plain arrays; everything else goes through the host path
     uint32_t *dev = nullptr;
     switch (fd.kind) {
@@ -1596,6 +1600,7 @@ int Engine::set_dt(float dt) {
             CK(fill_f32(TF_[TF_DT] + L.off, dt, L.n, stream_), SNN_GPU_QUEUE_FAILURE);
         } else {
             CK(fill_f32(F_[F_DT] + L.off, dt, L.n, stream_), SNN_GPU_QUEUE_FAILURE);
+            tile_par_dirty_ = true;
             L.stdp.dt = dt;
             if (L.is_reward) L.rstdp.dt = dt;   // RewardModulatedLattice::set_dt, neuron/mod.rs:2867-2870
         }
@@ -1857,24 +1862,73 @@ bool Engine::build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp,
     return true;
 }
 
-// Operand streams of the window-staged kernel (step_win.cu): radius-1 stencil lattices.  false = not eligible.
-bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid) {
+// Operand streams of the window-staged kernel (step_win.cu): radius-1 stencil lattices.
+//
+// Parameters (win_field_param, and the chemical ones the run reads) are the same in whole blocks of neurons in the common
+// case (Lattice::populate copies one neuron into every cell): a tile whose neurons all share the first one's bit patterns
+// takes them from its tile row (one copy of at most a few hundred bytes) instead of from one 1 KB stream per parameter.
+// When no tile streams its parameters the stage has no room for them, and the ring gets deeper.
+int Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid, bool *eligible) {
+    *eligible = false;
     memset(&wp, 0xFF, sizeof wp);
-    if (!grid_fast_ || uniform_width_ != kWinWidth || n_neurons == 0) return false;
-    if (mode == 0) return false;
+    if (!grid_fast_ || uniform_width_ != kWinWidth || n_neurons == 0) return SNN_OK;
+    if (mode == 0) return SNN_OK;
     // tiny lattices are launch-latency bound: the persistent kernel only pays off with at least a few tiles per SM
-    if (mode < 2 && n_neurons < 64 * 1024) return false;
+    if (mode < 2 && n_neurons < 64 * 1024) return SNN_OK;
     uint32_t cols = 0;
     for (auto &L : lats_) if (!L.is_train) cols = L.cols;
-    if (cols == 0) return false;
-    const WinLayout L = win_layout(model, chemg, ntrel, stdp);
-    uint32_t off = L.fixed_end, n = 0, tx = 0;
+    if (cols == 0) return SNN_OK;
+    // the layout with rows; the one without (every parameter streamed) is chosen below when no tile is uniform
+    const WinLayout L = win_layout(model, chemg, ntrel, stdp, true);
+    wp.n_tiles = (uint32_t)((n_neurons + kWinTile - 1) / kWinTile);
+    // the parameters: array (per local neuron), word of the tile row, and where a non-uniform tile's stream of it goes
+    // (the model's at compile-time offsets, the chemical ones at offsets assigned after the state part of the stage)
+    TileParSrc tp{};
+    uint32_t par_off[kWinMaxPar] = {}, *par_rt[kWinMaxPar] = {};
+    auto par = [&](const float *src, uint32_t word, uint32_t smem_off, uint32_t *rt) {
+        if (tp.n_par < (uint32_t)kWinMaxPar) {
+            tp.src[tp.n_par] = (const uint32_t *)src; tp.word[tp.n_par] = word;
+            par_off[tp.n_par] = smem_off; par_rt[tp.n_par] = rt;
+        }
+        ++tp.n_par;
+    };
+    for (int sl = 0; sl < F_NA_CUR; ++sl) {
+        if (L.o_f[sl] == 0xFFFFFFFFu) continue;
+        if (!F_[sl]) return SNN_OK;
+        if (win_field_param(model, ntrel, sl)) par(F_[sl], L.r_f[sl], L.o_f[sl], nullptr);
+    }
+    const uint32_t ntu = ntrel ? nt_used() : 0u, rcu = ntrel ? rc_used() : 0u;
+    for (int ty = 0; ty < kNT; ++ty) {
+        auto nt = [&](int sl) { par(NT_[sl] + (size_t)ty * node_cap_ + own0_, L.r_nt + sl * kNT + ty, 0u, &wp.o_nt[sl][ty]); };
+        auto rc = [&](int sl) { par(RC_[sl] + (size_t)ty * neuron_cap_, L.r_rc + (sl - RCF_K1) * kNT + ty, 0u, &wp.o_rc[sl][ty]); };
+        if (ntu & (1u << ty)) {
+            nt(NTF_TMAX);
+            if (ntk != SNN_NT_DISCRETE_SPIKE) nt(NTF_P1);
+            if (ntk == SNN_NT_DESTEXHE) nt(NTF_P2);
+        }
+        if (rcu & (1u << ty)) {
+            rc(RCF_G);
+            rc(RCF_E);
+            if (rck != SNN_RC_APPROXIMATE) { rc(RCF_K1); rc(RCF_K2); }
+            if (ty == SNN_NT_NMDA) rc(RCF_MG);
+        }
+    }
+    if (tp.n_par > (uint32_t)kWinMaxPar) return SNN_OK;
+    tp.row_words = L.row_bytes / 4u;
+    tp.n_neurons = (uint32_t)n_neurons;
+    tp.n_tiles = wp.n_tiles;
+    const int r = refresh_tile_params(tp);
+    if (r) return r;
+    const uint32_t mixed = tile_par_mixed_;
+    const bool rows = mixed < wp.n_tiles;
+    const WinLayout L0 = win_layout(model, chemg, ntrel, stdp, false);
+
+    uint32_t off = !rows ? L0.fixed_end : (mixed ? L.fixed_end : L.uni_end), n = 0;
     auto add_at = [&](const void *src, uint32_t bytes_per_tile, uint32_t smem_off) {
         if (n >= (uint32_t)kMaxTmaStreams) { n = kMaxTmaStreams + 1; return; }
         wp.st[n].src = (const unsigned char *)src;
         wp.st[n].bytes_per_tile = bytes_per_tile;
         wp.st[n].smem_off = smem_off;
-        tx += bytes_per_tile;
         ++n;
     };
     auto add = [&](const void *src, uint32_t bytes_per_tile) -> uint32_t {
@@ -1884,16 +1938,13 @@ bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, b
         return o;
     };
     const uint32_t fb = kWinTile * 4;
-    if (ntrel) add_at(node_flags_ + own0_, kWinTile, L.o_flags);
-    add_at(col_, kWinEdgeBytes, L.o_col);
-    add_at(wgt_, kWinEdgeBytes, L.o_wgt);
-    for (int sl = 0; sl < F_NA_CUR; ++sl)
-        if (L.o_f[sl] != 0xFFFFFFFFu) {
-            if (!F_[sl]) return false;
-            add_at(F_[sl], fb, L.o_f[sl]);
-        }
-    if (ntrel) {
-        const uint32_t ntu = nt_used(), rcu = rc_used();
+    if (!rows) {
+        // no tile is uniform: every operand streamed, in slot order (no row, no parameter region of its own)
+        if (ntrel) add_at(node_flags_ + own0_, kWinTile, L0.o_flags);
+        add_at(col_, kWinEdgeBytes, L0.o_col);
+        add_at(wgt_, kWinEdgeBytes, L0.o_wgt);
+        for (int sl = 0; sl < F_NA_CUR; ++sl)
+            if (L0.o_f[sl] != 0xFFFFFFFFu) add_at(F_[sl], fb, L0.o_f[sl]);
         for (int ty = 0; ty < kNT; ++ty) {
             if (ntu & (1u << ty)) {
                 wp.o_nt[NTF_TMAX][ty] = add(NT_[NTF_TMAX] + (size_t)ty * node_cap_ + own0_, fb);
@@ -1911,12 +1962,31 @@ bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, b
                 if (ty == SNN_NT_NMDA) wp.o_rc[RCF_MG][ty] = add(RC_[RCF_MG] + (size_t)ty * neuron_cap_, fb);
             }
         }
+        wp.tile_par = nullptr;
+        wp.n_state = n;
+    } else {
+        // every tile: flags, edges, state
+        if (ntrel) add_at(node_flags_ + own0_, kWinTile, L.o_flags);
+        add_at(col_, kWinEdgeBytes, L.o_col);
+        add_at(wgt_, kWinEdgeBytes, L.o_wgt);
+        for (int sl = 0; sl < F_NA_CUR; ++sl)
+            if (L.o_f[sl] != 0xFFFFFFFFu && win_field_state(sl)) add_at(F_[sl], fb, L.o_f[sl]);
+        for (int ty = 0; ty < kNT; ++ty)
+            if (rcu & (1u << ty)) wp.o_rc[RCF_R][ty] = add(RC_[RCF_R] + (size_t)ty * neuron_cap_, fb);
+        wp.tile_par = tile_par_;
+        add_at(tile_par_, L.row_bytes, L.o_row);
+        wp.n_state = n;
+        // non-uniform tiles: the parameters
+        if (mixed)
+            for (uint32_t k = 0; k < tp.n_par; ++k) {
+                if (par_rt[k]) *par_rt[k] = add(tp.src[k], fb);
+                else add_at(tp.src[k], fb, par_off[k]);
+            }
     }
-    if (n > (uint32_t)kMaxTmaStreams) return false;
+    wp.row_words = tp.row_words;
+    if (n > (uint32_t)kMaxTmaStreams) return SNN_OK;
     wp.n_streams = n;
-    wp.stage_bytes = off;
-    wp.fixed_tx_bytes = tx;
-    wp.n_tiles = (uint32_t)((n_neurons + kWinTile - 1) / kWinTile);
+    wp.stage_bytes = (uint32_t)round_up(off, 16);
     wp.node_cap = (uint32_t)node_cap_;
     wp.cols = cols;
     wp.lft_copy = (stdp || lft_pp) ? 1u : 0u;
@@ -1931,16 +2001,39 @@ bool Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, b
         wp.bnd_lo = wp.first_lo; wp.bnd_hi = wp.first_hi;
         if (wp.first_lo + wp.first_hi > wp.n_tiles) wp.first_lo = wp.first_hi = 0;   // a strip of a few rows: every tile is a boundary tile
     }
-    const uint32_t G = (uint32_t)win_groups(model, chemg);
-    uint32_t stages = (224u * 1024u) / (off + 16u);
+    wp.first_end = wp.first_lo + wp.first_hi;
+    const uint32_t G = (uint32_t)win_groups(model, chemg, rows && mixed);
+    uint32_t stages = (224u * 1024u) / (wp.stage_bytes + 16u);
     stages = std::min<uint32_t>(stages, 8);
-    if (stages < G) return false;   // the consumer groups need a stage each
+    if (stages < G) return SNN_OK;   // the consumer groups need a stage each
     wp.stages = stages;
+    wp.ring_check = stages % G != 0u ? 1u : 0u;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     *grid = (unsigned)std::min<uint64_t>((wp.n_tiles + G - 1) / G, (uint64_t)sms);
     if (*grid == 0) *grid = 1;
-    return true;
+    *eligible = true;
+    return SNN_OK;
+}
+
+int Engine::refresh_tile_params(const TileParSrc &a) {
+    if (!tile_par_dirty_ && memcmp(&a, &tile_par_key_, sizeof a) == 0) return SNN_OK;
+    const size_t bytes = (size_t)a.n_tiles * a.row_words * 4u;
+    if (bytes + 16u > tile_par_bytes_) {
+        if (tile_par_) cudaFree(tile_par_);
+        tile_par_ = nullptr; tile_par_bytes_ = 0;
+        CK(cudaMalloc((void **)&tile_par_, bytes + 16u), SNN_GPU_BUFFER_CREATE_ERROR);
+        tile_par_bytes_ = bytes + 16u;
+    }
+    // the count of non-uniform tiles sits after the rows
+    unsigned int *d_mixed = (unsigned int *)((char *)tile_par_ + bytes);
+    CK(cudaMemsetAsync(tile_par_, 0, bytes + 16u, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
+    CK(launch_tile_params(a, tile_par_, d_mixed, stream_), SNN_GPU_QUEUE_FAILURE);
+    CK(cudaMemcpyAsync(&tile_par_mixed_, d_mixed, 4, cudaMemcpyDeviceToHost, stream_), SNN_GPU_BUFFER_READ_ERROR);
+    CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
+    tile_par_key_ = a;
+    tile_par_dirty_ = false;
+    return SNN_OK;
 }
 
 // Partition handles of ONE process (attach_local / gpart_attach_local) are stepped from one host thread each, and their kernels
@@ -2507,7 +2600,13 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
     const char *tma_env = getenv("SNN_B200_TMA"), *win_env = getenv("SNN_B200_WIN");
     const int tma_mode = tma_env ? atoi(tma_env) : 1;
     const int win_mode = (win_env && atoi(win_env) == 0) ? 0 : tma_mode;
-    if (!pl.spec.net && build_win_params(a.win, pl.spec.chemg, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, win_mode, &pl.grid)) {
+    bool win = false;
+    if (!pl.spec.net) {
+        const int r = build_win_params(a.win, pl.spec.chemg, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, win_mode, &pl.grid, &win);
+        if (r) return r;
+    }
+    last_uniform_tiles = win ? a.win.n_tiles - tile_par_mixed_ : 0u;
+    if (win) {
         pl.path = StepPath::Win;
     } else if (!pl.spec.net && build_tma_params(a.tma, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, tma_mode, &pl.grid)) {
         pl.path = StepPath::Tma;

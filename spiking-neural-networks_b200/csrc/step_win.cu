@@ -15,6 +15,8 @@
 // The col words are still read and used (the window is selected by comparing the presynaptic index against the
 // tile's bounds), so any per-edge weight / type content of the sliced-ELL table keeps working; only the index
 // pattern must be the radius-1 stencil that set_graph_grid generates.
+#include <type_traits>
+
 #include "step_body.cuh"
 #include "tma_util.cuh"
 
@@ -43,13 +45,15 @@ __device__ __forceinline__ float lds_f32_rt(uint32_t addr) {
     return v;
 }
 
-template <int MODEL, int CHEMG, bool NTREL, bool STDP>
+// UNI: every neuron of the tile has the parameters of its first one (WinLayout::o_row): f<>(), nt() and rc() read that row
+// ROWS: the stage has a row (win_layout(..., rows = true))
+template <int MODEL, int CHEMG, bool NTREL, bool STDP, bool ROWS, bool UNI>
 struct WinSrc {
     static constexpr bool kEarlyLoads = false;   // operands sit in shared memory: read them where they are used
     static constexpr bool kCheapEdges = false;
     static constexpr bool kWide = false;
     static constexpr uint32_t kWidth = kWinWidth;
-    static __host__ __device__ constexpr WinLayout lay() { return win_layout(MODEL, CHEMG, NTREL, STDP); }
+    static __host__ __device__ constexpr WinLayout lay() { return win_layout(MODEL, CHEMG, NTREL, STDP, ROWS); }
 
     const StepParams &p;
     const WinParams &wp;
@@ -60,13 +64,17 @@ struct WinSrc {
     uint32_t d0, d1, d2;        // shared address of V[node 0] as seen through the upper / middle / lower window (mod 2^32)
     uint32_t k0g, lane;         // first k-row of this warp's slice in the global edge arrays
     uint32_t tid;               // neuron within the tile
+    uint32_t row;               // shared address of this stage's tile row
 
     template <int SLOT> __device__ __forceinline__ float f() const {
-        constexpr uint32_t o = lay().o_f[SLOT];
-        static_assert(o != 0xFFFFFFFFu, "field is not staged for this model (win_field_read)");
-        return lds_f32<o>(me);
+        static_assert(win_field_param(MODEL, NTREL, SLOT), "not a parameter of this model (win_field_read, win_field_state)");
+        if constexpr (UNI) return lds_f32<lay().r_f[SLOT] * 4u>(row);
+        else return lds_f32<lay().o_f[SLOT]>(me);
     }
-    template <int SLOT> __device__ __forceinline__ float state() const { return f<SLOT>(); }
+    template <int SLOT> __device__ __forceinline__ float state() const {
+        static_assert(win_field_read(MODEL, NTREL, SLOT) && win_field_state(SLOT), "not a state field of this model (win_field_state)");
+        return lds_f32<lay().o_f[SLOT]>(me);
+    }
     __device__ __forceinline__ float v() const { return lds_f32<lay().o_vwin + kWinRowBytes>(own); }
     __device__ __forceinline__ int lft() const {
         return (int)lds_u32<lay().o_lwin + (lay().lrows == 3 ? kWinRowBytes : 0u)>(own);
@@ -80,9 +88,16 @@ struct WinSrc {
         const uint32_t q = (CHEMG == 1) ? 0u : (uint32_t)ty;
         return lds_f32_rt(own + o + (q * tr + (tr == 3 ? 1u : 0u)) * kWinRowBytes);
     }
-    __device__ __forceinline__ float nt(int slot, int ty) const { return lds_f32_rt(me + wp.o_nt[slot][ty]); }
-    __device__ __forceinline__ float rc(int slot, int ty) const { return lds_f32_rt(me + wp.o_rc[slot][ty]); }
-    __device__ __forceinline__ float rc_state(int slot, int ty) const { return rc(slot, ty); }
+    // slot and ty are constants after neuron_step's loops unroll: the row offsets fold into the loads
+    __device__ __forceinline__ float nt(int slot, int ty) const {
+        if constexpr (UNI) return lds_f32_rt(row + (lay().r_nt + (uint32_t)(slot * kNT + ty)) * 4u);
+        else return lds_f32_rt(me + wp.o_nt[slot][ty]);
+    }
+    __device__ __forceinline__ float rc(int slot, int ty) const {
+        if constexpr (UNI) return lds_f32_rt(row + (lay().r_rc + (uint32_t)((slot - RCF_K1) * kNT + ty)) * 4u);
+        else return lds_f32_rt(me + wp.o_rc[slot][ty]);
+    }
+    __device__ __forceinline__ float rc_state(int slot, int ty) const { return lds_f32_rt(me + wp.o_rc[slot][ty]); }
     __device__ __forceinline__ uint32_t width() const { return kWinWidth; }
     __device__ __forceinline__ uint32_t col(uint32_t kk) const { return lds_u32<lay().o_col>(edge + kk * 128u); }
     __device__ __forceinline__ float wgt(uint32_t kk) const { return lds_f32<lay().o_wgt>(edge + kk * 128u); }
@@ -117,8 +132,9 @@ struct WinSrc {
 // the previous step left in L2 is what this step reads first).  Row strips: the tiles that import ghosts / export boundary rows
 // go FIRST, so a strip's exports of step s leave at the start of step s and its neighbour — which needs them at the start of its
 // step s + 1 — finds them long arrived: the NVLink store / fence / flag latency (~10 us) is off the critical path of every step.
+template <bool ROWS>
 __device__ __forceinline__ uint32_t win_tile_of(const StepParams &p, const WinParams &wp, uint32_t seq) {
-    const uint32_t nb = wp.first_lo + wp.first_hi;
+    const uint32_t nb = ROWS ? wp.first_end : wp.first_lo + wp.first_hi;
     if (seq < wp.first_lo) return seq;
     if (seq < nb) return wp.n_tiles - 1u - (seq - wp.first_lo);
     const uint32_t k = seq - nb, n_int = wp.n_tiles - nb;
@@ -128,11 +144,19 @@ __device__ __forceinline__ uint32_t win_tile_of(const StepParams &p, const WinPa
 constexpr int kWinProducers = 4;   // producer warps per CTA; together they issue the copies of every tile
 template <int G> constexpr int win_threads() { return (G * 8 + kWinProducers) * 32; }
 
-template <int MODEL, int CHEMG, bool NTREL, bool STDP, int G>
+// Which tiles read their parameter row (WinParams::tile_par).  Each case is its own kernel: compiled with both step variants, the
+// kernel's code doubles and its registers are allocated over both, which cost 2-8 % on lattices whose tiles all stream (measured on
+// one B200 at 1000 W: 1000 x 1000 LIF + STDP 23.6 -> 25.5 us per step, Hodgkin-Huxley 2048 x 2048 317 -> 323 us).  kRowsNone has
+// the stage layout, stream order and loop code of the kernel before tile rows (win_layout(..., rows = false)); kRowsSome runs with
+// two consumer groups (win_groups).
+enum WinRows : int { kRowsNone = 0, kRowsAll = 1, kRowsSome = 2 };
+
+template <int MODEL, int CHEMG, bool NTREL, bool STDP, int G, int ROWS>
 __global__ void __launch_bounds__(win_threads<G>(), 1)
 step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ WinParams wp) {
     extern __shared__ __align__(128) unsigned char smem[];
-    constexpr WinLayout L = win_layout(MODEL, CHEMG, NTREL, STDP);
+    constexpr bool R = ROWS != kRowsNone;
+    constexpr WinLayout L = win_layout(MODEL, CHEMG, NTREL, STDP, R);
     const uint32_t S = wp.stages;
     uint64_t *full = reinterpret_cast<uint64_t *>(smem + (size_t)S * wp.stage_bytes);
     uint64_t *empty = full + S;
@@ -174,15 +198,25 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
         // last_firing_time, 2..: t slots)
         const uint32_t idx = q + kWinProducers * lane;
         const bool is_stream = idx < wp.n_streams;
+        const bool is_par = is_stream && idx >= wp.n_state;   // a parameter stream: non-uniform tiles only
         const uint32_t wv = idx - wp.n_streams, arr = wv / 3u, r = wv - arr * 3u;
         bool is_win = !is_stream && arr < 2u + n_t;
         if (is_win && arr == 1u) is_win = lft_on && (L.lrows == 3 || r == 1u);
         if (is_win && arr >= 2u) is_win = (L.trows == 3 || r == 1u);
         TmaStream my{nullptr, 0u, 0u};
         if (is_stream) my = wp.st[idx];
+        // uniform flag of the next tile, loaded one tile ahead (its L2 latency overlaps the empty-barrier wait and the copies of
+        // the tile before); only needed when some tiles are uniform and others stream their parameters
+        constexpr bool flags_needed = ROWS == kRowsSome;
+        auto uniform_of = [&](uint32_t seq) -> uint32_t {
+            return (flags_needed && seq < wp.n_tiles) ? __ldg(wp.tile_par + (size_t)win_tile_of<R>(p, wp, seq) * wp.row_words) : 0u;
+        };
+        uint32_t uni_next = uniform_of(blockIdx.x);
         uint32_t s = 0, ph = 0;
         for (uint32_t tile_seq = blockIdx.x; tile_seq < wp.n_tiles; tile_seq += gridDim.x) {
-            const uint32_t tile = win_tile_of(p, wp, tile_seq);
+            const uint32_t tile = win_tile_of<R>(p, wp, tile_seq);
+            const bool uni = uni_next != 0u;
+            uni_next = uniform_of(tile_seq + gridDim.x);
             mbar_wait_backoff(&empty[s], ph ^ 1u);   // the whole warp probes: no divergent lane-0 loop with 31 lanes parked at a reconvergence barrier
             const uint32_t ts = tile * kWinTile;   // first local neuron of the tile
             // multi-GPU: ghost rows are written by the neighbouring GPU over NVLink; they must have landed before TMA reads
@@ -200,7 +234,7 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
             unsigned char *dst = smem + (size_t)s * wp.stage_bytes;
             const void *src = nullptr;
             uint32_t bytes = 0;
-            if (is_stream) {
+            if (is_stream && !(is_par && uni)) {
                 src = my.src + (size_t)tile * my.bytes_per_tile;
                 dst += my.smem_off;
                 bytes = my.bytes_per_tile;
@@ -243,7 +277,7 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
     const uint32_t smem_s = smem_u32(smem);
     uint32_t s = g % S, ph = (g / S) & 1u;
     for (uint32_t tile_seq = blockIdx.x + g * gridDim.x; tile_seq < wp.n_tiles; tile_seq += G * gridDim.x) {
-        const uint32_t tile = win_tile_of(p, wp, tile_seq);
+        const uint32_t tile = win_tile_of<R>(p, wp, tile_seq);
         const uint32_t warp_global = tile * 8u + wg;
         const uint32_t ln = warp_global * 32u + lane;
         const bool active = warp_global * 32u < p.n_neurons;
@@ -257,7 +291,7 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
         // "round k - 1 is still landing" (two phases apart).  Bulk copies of different stages complete out of order, so
         // first make sure that round k - 1 of this stage has been consumed (the empty barrier; a producer that issued this
         // warp's previous tile has already seen round k - 2 consumed, so this wait is unambiguous), then wait for the data.
-        if (S % G != 0u) mbar_wait(&empty[s], ph ^ 1u);
+        if (R ? wp.ring_check != 0u : S % G != 0u) mbar_wait(&empty[s], ph ^ 1u);
         mbar_wait(&full[s], ph);
         if (active) {
             const uint32_t ts_node = p.own0 + tile * kWinTile;
@@ -269,10 +303,16 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
             const uint32_t d2 = st + 2u * kWinRowBytes - (uint32_t)(a2 & ~3) * 4u;
             // this neuron inside a row-relative window: node (ts_node + tid) sits (ts_node + tid - floor4(a1)) elements in
             const uint32_t own = st + ((uint32_t)((int32_t)ts_node - (a1 & ~3)) + tid) * 4u;
-            const WinSrc<MODEL, CHEMG, NTREL, STDP> src{p, wp, st + tid * 4u, own, st + (wg * kWinWidth * 32u + lane) * 4u,
-                                                         ts_node ? ts_node - 1u : 0u, ts_node + kWinTile, d0, d1, d2,
-                                                         warp_global * kWinWidth, lane, tid};
-            neuron_step<MODEL, CHEMG, NTREL, STDP, false>(p, src, warp_global, lane, ln, lnc, valid, export_lo, export_hi);
+            auto step = [&](auto uni) {
+                const WinSrc<MODEL, CHEMG, NTREL, STDP, R, decltype(uni)::value> src{
+                    p, wp, st + tid * 4u, own, st + (wg * kWinWidth * 32u + lane) * 4u, ts_node ? ts_node - 1u : 0u, ts_node + kWinTile,
+                    d0, d1, d2, warp_global * kWinWidth, lane, tid, st + L.o_row};
+                neuron_step<MODEL, CHEMG, NTREL, STDP, false>(p, src, warp_global, lane, ln, lnc, valid, export_lo, export_hi);
+            };
+            if constexpr (ROWS == kRowsNone) step(std::false_type{});
+            else if constexpr (ROWS == kRowsAll) step(std::true_type{});
+            else if (lds_u32<L.o_row>(st) != 0u) step(std::true_type{});   // CTA-uniform
+            else step(std::false_type{});
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty[s]);
@@ -298,13 +338,41 @@ cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const Step
         if constexpr (K::NET) {
             return cudaErrorInvalidValue;   // single lattices only
         } else {
-            constexpr int G = win_groups(K::MODEL, K::CHEMG);
-            auto kern = step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G>;
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            return launch_pdl(pdl_ok(p), kern, dim3(grid), dim3(win_threads<G>()), smem, s, p, wp);
+            constexpr int G = win_groups(K::MODEL, K::CHEMG, false), GM = win_groups(K::MODEL, K::CHEMG, true);
+            auto launch = [&](auto kern, int threads) {
+                cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                if (e != cudaSuccess) return e;
+                return launch_pdl(pdl_ok(p), kern, dim3(grid), dim3(threads), smem, s, p, wp);
+            };
+            if (wp.tile_par == nullptr) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsNone>, win_threads<G>());
+            if (wp.n_streams == wp.n_state) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsAll>, win_threads<G>());
+            return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, GM, kRowsSome>, win_threads<GM>());
         }
     });
+}
+
+// one CTA per tile, one thread per neuron (see TileParSrc)
+__global__ void __launch_bounds__(kWinTile) tile_params_kernel(const __grid_constant__ TileParSrc a, uint32_t *rows, unsigned int *n_mixed) {
+    const uint32_t tile = blockIdx.x, ts = tile * kWinTile;
+    const bool valid = ts + threadIdx.x < a.n_neurons;
+    uint32_t *row = rows + (size_t)tile * a.row_words;
+    bool same = true;
+    for (uint32_t k = 0; k < a.n_par; ++k) {
+        const uint32_t first = __ldg(a.src[k] + ts);
+        if (valid) same = same && __ldg(a.src[k] + ts + threadIdx.x) == first;
+        if (threadIdx.x == 0) row[a.word[k]] = first;
+    }
+    const bool uni = __syncthreads_and(same) != 0;
+    if (threadIdx.x == 0) {
+        row[0] = uni ? 1u : 0u;
+        if (!uni) atomicAdd(n_mixed, 1u);
+    }
+}
+
+cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *n_mixed, cudaStream_t s) {
+    if (a.n_tiles == 0) return cudaSuccess;
+    tile_params_kernel<<<a.n_tiles, kWinTile, 0, s>>>(a, rows, n_mixed);
+    return cudaGetLastError();
 }
 
 }  // namespace snn
