@@ -173,9 +173,13 @@ typedef enum snn_option {
                                          3 wide split (per-edge terms pass, then ordered sums), 4 TMA-staged persistent kernel,
                                          5 window-staged persistent kernel (radius-1 stencils).  multi: 1 when whole chunks of
                                          timesteps ran in one cooperative launch (SNN_OPT_STEPS_PER_GRAPH) */
-    SNN_OPT_UNIFORM_TILES = 17        /* read-only: of the 256-neuron tiles of the handle's last run on the window-staged kernel, those
+    SNN_OPT_UNIFORM_TILES = 17,       /* read-only: of the 256-neuron tiles of the handle's last run on the window-staged kernel, those
                                          whose neurons all have the bit patterns of the tile's first neuron in every parameter the step
                                          reads (these tiles read one copy of them instead of one per neuron); 0 on every other path */
+    SNN_OPT_STENCIL_TILES = 18        /* read-only: of the 256-neuron tiles of the handle's last run on the window-staged kernel, those
+                                         that derived their in-edge indices from the radius-1 stencil instead of reading the edge table's
+                                         index words: every tile when every tile reads its parameter row and every index word of the table
+                                         is the stencil's, bit for bit (type bits included); else 0, as on every other path */
 } snn_option_t;
 
 /* STDP, backend/src/neuron/plasticity/mod.rs:14-39 (defaults 2, 2, 4.5, 4.5, 0.1) */

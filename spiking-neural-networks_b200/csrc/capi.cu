@@ -249,6 +249,7 @@ static int32_t engine_get_option(const Engine *e, bool have_id, uint64_t id, int
     case SNN_OPT_STEPS_PER_GRAPH: *value = e->steps_per_graph; return SNN_OK;
     case SNN_OPT_STEP_PATH: *value = e->last_step_path; return SNN_OK;
     case SNN_OPT_UNIFORM_TILES: *value = e->last_uniform_tiles; return SNN_OK;
+    case SNN_OPT_STENCIL_TILES: *value = e->last_stencil_tiles; return SNN_OK;
     case SNN_OPT_HALO_TIMEOUT_MS: *value = (int64_t)e->halo_timeout_ms; return SNN_OK;
     case SNN_OPT_GENERAL_PARTITION: *value = e->force_gpart || e->is_gpart(); return SNN_OK;
     case SNN_OPT_INTERNAL_CLOCK: *value = (int64_t)((L && L->is_train) ? L->clock : e->internal_clock); return SNN_OK;

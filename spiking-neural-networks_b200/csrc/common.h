@@ -50,6 +50,40 @@ constexpr uint32_t kColNtShift = 28;
 constexpr uint32_t kColTrainBit = 0x80000000u;
 constexpr uint64_t kMaxNodes = 0x0FFFFFFEull;
 
+// device code unrolls the loop that follows (host compilers do not know the pragma)
+#ifdef __CUDA_ARCH__
+#define SNN_UNROLL _Pragma("unroll")
+#else
+#define SNN_UNROLL
+#endif
+
+// The col words of one row of a radius-1 Moore stencil table, as sell_grid_kernel writes them: slot k holds the k-th in-bounds
+// neighbour of local neuron ln in ascending node index, OR'd with `nt` << kColNtShift (the generator passes 0 and stamps each
+// neighbour's own release bits); the slots past the last neighbour, and every slot of a lane ln >= n, hold kColPad.  The lattice
+// has rows_global rows of `cols` cells; local neuron 0 is the first cell of row row0_global and has node index own0.
+__host__ __device__ __forceinline__ void stencil_cols(uint32_t ln, uint32_t n, uint32_t cols, uint32_t row0_global, uint32_t rows_global,
+                                                      uint32_t own0, uint32_t nt, uint32_t (&c)[8]) {
+    const bool valid = ln < n;
+    const uint32_t r = valid ? ln / cols : 0u, x = valid ? ln - r * cols : 0u;
+    const bool up = r + row0_global > 0u, dn = r + row0_global + 1u < rows_global, lf = x > 0u, rt = x + 1u < cols;
+    const uint32_t me = own0 + ln, hi = nt << kColNtShift;
+    uint32_t k = 0;
+SNN_UNROLL
+    for (int u = 0; u < 8; ++u) c[u] = kColPad;
+    // candidate q: three in the row above, the two side neighbours, three in the row below; it can only fill slots u <= q
+SNN_UNROLL
+    for (int q = 0; q < 8; ++q) {
+        const int dr = q < 3 ? -1 : (q < 5 ? 0 : 1);
+        const int dc = q < 3 ? q - 1 : (q < 5 ? 2 * q - 7 : q - 6);
+        const bool ok = valid && (dr < 0 ? up : (dr > 0 ? dn : true)) && (dc < 0 ? lf : (dc > 0 ? rt : true));
+        const uint32_t w = (me + (uint32_t)dr * cols + (uint32_t)dc) | hi;
+SNN_UNROLL
+        for (int u = 0; u <= q; ++u)
+            if (ok && k == (uint32_t)u) c[u] = w;
+        k += ok ? 1u : 0u;
+    }
+}
+
 // ---- per-neuron device field slots (index into StepParams::f) ---------------------------------
 enum NeuronSlot : int {
     F_GAP = 0, F_DT, F_CM, F_VTH, F_VRESET, F_REFR, F_TREF, F_LEAK, F_INTEG, F_EL, F_GL, F_TAUM,
@@ -254,15 +288,15 @@ constexpr uint32_t kWinEdgeBytes = 8 * kWinWidth * 32 * 4;  // col (or weight) b
 
 struct WinLayout {
     uint32_t lrows, trows, tslots;   // window rows kept for last_firing_time / t, neurotransmitter type slots
-    uint32_t o_vwin, o_lwin, o_twin, o_spk, o_flags, o_col, o_wgt;
+    uint32_t o_vwin, o_lwin, o_twin, o_spk, o_flags, o_wgt;
+    uint32_t o_col;                  // 0xFFFFFFFF = stencil: every tile's col words are those of stencil_cols, none staged
     uint32_t o_f[F_NA_CUR];          // 0xFFFFFFFF = not read by this model
     // rows (some tile reads its parameter row): the state fields first, then the row, then the parameters, so that a stage without
     // per-neuron parameters ends at uni_end; without rows every field in slot order and no row (o_row = 0xFFFFFFFF)
     uint32_t o_row;                  // the tile's parameter row (copied from the tile table, see win_field_param)
     uint32_t uni_end;                // first byte after the part every tile fills (state fields and the row; multiple of 16)
     uint32_t fixed_end;              // first byte after the compile-time part (multiple of 128)
-    // the tile row, in 32-bit words: [0] 1 = every neuron of the tile has the first one's parameters (bit patterns), then the
-    // first neuron's parameters: r_f[slot] for the model's, [r_nt + NtSlot * kNT + type] for the neurotransmitters',
+    // the tile row, in 32-bit words: [0] flags (kTileUniform, kTileStencil, kTileFullShift), then the first neuron's parameters: r_f[slot] for the model's, [r_nt + NtSlot * kNT + type] for the neurotransmitters',
     // [r_rc + (RcSlot - RCF_K1) * kNT + type] for the receptors' (words of kinetics this run does not read stay 0)
     uint32_t r_f[F_NA_CUR];
     uint32_t r_nt, r_rc;
@@ -314,7 +348,12 @@ __host__ __device__ constexpr bool win_field_param(int model, bool ntrel, int sl
     return win_field_read(model, ntrel, slot) && !win_field_state(slot);
 }
 
-__host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool ntrel, bool stdp, bool rows) {
+// word 0 of a tile row (WinLayout): every neuron of the tile has the first one's parameters (bit patterns); every col word of the
+// tile is that of stencil_cols for the lattice-wide release mask WinParams::stencil_nt; bit kTileFullShift + w: warp w of the
+// tile is full (32 valid lanes with 8 in-edges each)
+constexpr uint32_t kTileUniform = 1u, kTileStencil = 2u, kTileFullShift = 8;
+
+__host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool ntrel, bool stdp, bool rows, bool stencil) {
     WinLayout L{};
     uint32_t off = 0;
     L.lrows = stdp ? 3u : 1u;
@@ -326,7 +365,8 @@ __host__ __device__ constexpr WinLayout win_layout(int model, int chemg, bool nt
     off = (off + 127u) & ~127u;
     L.o_spk = off; off += 128u;
     L.o_flags = off; off += kWinTile;
-    L.o_col = off; off += kWinEdgeBytes;
+    L.o_col = 0xFFFFFFFFu;
+    if (!stencil) { L.o_col = off; off += kWinEdgeBytes; }
     L.o_wgt = off; off += kWinEdgeBytes;
     uint32_t w = 1;
     for (int s = 0; s < F_NA_CUR; ++s) {
@@ -369,6 +409,10 @@ struct WinParams {
     // first_lo + first_hi, and stages % consumer groups != 0, for the kernels that read tile rows: held in registers as values
     // (as the kernel without rows holds them) they made those kernels spill
     uint32_t first_end, ring_check;
+    // every tile is a stencil tile (kTileStencil) and reads its parameter row: the kernel without col words (win_layout(...,
+    // stencil = true)), with the release mask of every node and the rows of the lattice that stencil_cols needs for the border
+    // warps
+    uint32_t stencil, stencil_nt, row0_global, rows_global;
 };
 
 // groups of 8 consumer warps per CTA (register budget: 65536 / ((groups * 8 + 1) * 32))
@@ -381,16 +425,20 @@ __host__ __device__ constexpr int win_groups(int model, int chemg, bool mixed) {
 
 cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const StepSpec &spec, unsigned grid, cudaStream_t s);
 
-// Tile rows of the window kernel: per kWinTile tile of [0, n_neurons), word 0 = 1 when every valid neuron of the tile has the
-// bit pattern of the tile's first neuron in every src[k] (compared as 32-bit words: -0.0 != +0.0, a NaN equals only its own
-// payload), word word[k] = the first neuron's src[k].  The other words are left as they are; *n_mixed += tiles with word 0 = 0.
+// Tile rows of the window kernel: per kWinTile tile of [0, n_neurons), word 0 has kTileUniform when every valid neuron of the
+// tile has the bit pattern of the tile's first neuron in every src[k] (compared as 32-bit words: -0.0 != +0.0, a NaN equals only
+// its own payload), kTileStencil when the tile's 8 x 8 x 32 words of the uniform-width table `col` equal those of stencil_cols
+// (cols, row0_global, rows_global, own0, stencil_nt) bit for bit, and the tile's full warps; word word[k] = the first neuron's
+// src[k].  The other words are left as they are.  counts[0] += tiles without kTileUniform, counts[1] += tiles without kTileStencil.
 constexpr int kWinMaxPar = 48;
 struct TileParSrc {
     const uint32_t *src[kWinMaxPar];   // indexed by local neuron number
     uint32_t word[kWinMaxPar];
     uint32_t n_par, row_words, n_neurons, n_tiles;
+    const uint32_t *col;
+    uint32_t cols, row0_global, rows_global, own0, stencil_nt;
 };
-cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *n_mixed, cudaStream_t s);
+cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *counts, cudaStream_t s);
 
 // ---- kernel launchers (kernels.cu) ------------------------------------------------------------
 cudaError_t launch_step(const StepParams &p, const StepSpec &spec, cudaStream_t s);

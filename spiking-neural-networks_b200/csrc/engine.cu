@@ -1057,6 +1057,7 @@ uint32_t Engine::rc_used() const { refresh_flag_cache(); return rc_used_; }
 
 int Engine::finalize_graph() {
     if (!graph_dirty_) return SNN_OK;
+    tile_par_dirty_ = true;     // the col table is written below: the window kernel checks its stencil tiles again
     ghist_off_valid_ = false;   // the canonical order of the new table is counted again by the next run that records it
     free_reward_arrays();   // a rebuilt graph starts from TraceRSTDP::default traces
     CK(cudaSetDevice(device), SNN_GPU_GET_DEVICE_FAILURE);
@@ -1875,11 +1876,11 @@ int Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bo
     if (mode == 0) return SNN_OK;
     // tiny lattices are launch-latency bound: the persistent kernel only pays off with at least a few tiles per SM
     if (mode < 2 && n_neurons < 64 * 1024) return SNN_OK;
-    uint32_t cols = 0;
-    for (auto &L : lats_) if (!L.is_train) cols = L.cols;
+    uint32_t cols = 0, lat_rows = 0;
+    for (auto &L : lats_) if (!L.is_train) { cols = L.cols; lat_rows = L.rows; }
     if (cols == 0) return SNN_OK;
     // the layout with rows; the one without (every parameter streamed) is chosen below when no tile is uniform
-    const WinLayout L = win_layout(model, chemg, ntrel, stdp, true);
+    const WinLayout L = win_layout(model, chemg, ntrel, stdp, true, false);
     wp.n_tiles = (uint32_t)((n_neurons + kWinTile - 1) / kWinTile);
     // the parameters: array (per local neuron), word of the tile row, and where a non-uniform tile's stream of it goes
     // (the model's at compile-time offsets, the chemical ones at offsets assigned after the state part of the stage)
@@ -1917,13 +1918,28 @@ int Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bo
     tp.row_words = L.row_bytes / 4u;
     tp.n_neurons = (uint32_t)n_neurons;
     tp.n_tiles = wp.n_tiles;
+    // the stencil the tiles are checked against: the one sell_grid_kernel writes for this lattice (or strip), every node
+    // releasing the union of the release types (a node that releases fewer makes its neighbours' tiles differ)
+    tp.col = col_;
+    tp.cols = cols;
+    tp.row0_global = part_world > 1 ? row0_global : 0u;
+    tp.rows_global = part_world > 1 ? rows_global : lat_rows;
+    tp.own0 = (uint32_t)own0_;
+    tp.stencil_nt = nt_used();
     const int r = refresh_tile_params(tp);
     if (r) return r;
-    const uint32_t mixed = tile_par_mixed_;
+    const uint32_t mixed = tile_par_counts_[0];
     const bool rows = mixed < wp.n_tiles;
-    const WinLayout L0 = win_layout(model, chemg, ntrel, stdp, false);
+    // a stage without col words when every tile is a stencil tile and reads its row.  Not for lattices whose tiles stream their
+    // parameters: a variant for them (the row staged for its full-warp mask) measured 5 % slower on Hodgkin-Huxley (DESIGN.md §3)
+    wp.stencil = rows && !mixed && tile_par_counts_[1] == 0u ? 1u : 0u;
+    wp.stencil_nt = tp.stencil_nt;
+    wp.row0_global = tp.row0_global;
+    wp.rows_global = tp.rows_global;
+    const WinLayout L0 = win_layout(model, chemg, ntrel, stdp, false, false);
+    const WinLayout L1 = win_layout(model, chemg, ntrel, stdp, true, wp.stencil != 0u);
 
-    uint32_t off = !rows ? L0.fixed_end : (mixed ? L.fixed_end : L.uni_end), n = 0;
+    uint32_t off = !rows ? L0.fixed_end : (mixed ? L.fixed_end : L1.uni_end), n = 0;
     auto add_at = [&](const void *src, uint32_t bytes_per_tile, uint32_t smem_off) {
         if (n >= (uint32_t)kMaxTmaStreams) { n = kMaxTmaStreams + 1; return; }
         wp.st[n].src = (const unsigned char *)src;
@@ -1965,16 +1981,16 @@ int Engine::build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bo
         wp.tile_par = nullptr;
         wp.n_state = n;
     } else {
-        // every tile: flags, edges, state
-        if (ntrel) add_at(node_flags_ + own0_, kWinTile, L.o_flags);
-        add_at(col_, kWinEdgeBytes, L.o_col);
-        add_at(wgt_, kWinEdgeBytes, L.o_wgt);
+        // every tile: flags, edges (the weights only, on stencil stages), state
+        if (ntrel) add_at(node_flags_ + own0_, kWinTile, L1.o_flags);
+        if (!wp.stencil) add_at(col_, kWinEdgeBytes, L1.o_col);
+        add_at(wgt_, kWinEdgeBytes, L1.o_wgt);
         for (int sl = 0; sl < F_NA_CUR; ++sl)
-            if (L.o_f[sl] != 0xFFFFFFFFu && win_field_state(sl)) add_at(F_[sl], fb, L.o_f[sl]);
+            if (L1.o_f[sl] != 0xFFFFFFFFu && win_field_state(sl)) add_at(F_[sl], fb, L1.o_f[sl]);
         for (int ty = 0; ty < kNT; ++ty)
             if (rcu & (1u << ty)) wp.o_rc[RCF_R][ty] = add(RC_[RCF_R] + (size_t)ty * neuron_cap_, fb);
         wp.tile_par = tile_par_;
-        add_at(tile_par_, L.row_bytes, L.o_row);
+        add_at(tile_par_, L1.row_bytes, L1.o_row);
         wp.n_state = n;
         // non-uniform tiles: the parameters
         if (mixed)
@@ -2025,13 +2041,13 @@ int Engine::refresh_tile_params(const TileParSrc &a) {
         CK(cudaMalloc((void **)&tile_par_, bytes + 16u), SNN_GPU_BUFFER_CREATE_ERROR);
         tile_par_bytes_ = bytes + 16u;
     }
-    // the count of non-uniform tiles sits after the rows
+    // the counts of non-uniform and of non-stencil tiles sit after the rows
     unsigned int *d_mixed = (unsigned int *)((char *)tile_par_ + bytes);
     CK(cudaMemsetAsync(tile_par_, 0, bytes + 16u, stream_), SNN_GPU_BUFFER_WRITE_ERROR);
     CK(launch_tile_params(a, tile_par_, d_mixed, stream_), SNN_GPU_QUEUE_FAILURE);
-    CK(cudaMemcpyAsync(&tile_par_mixed_, d_mixed, 4, cudaMemcpyDeviceToHost, stream_), SNN_GPU_BUFFER_READ_ERROR);
+    CK(cudaMemcpyAsync(tile_par_counts_, d_mixed, sizeof tile_par_counts_, cudaMemcpyDeviceToHost, stream_), SNN_GPU_BUFFER_READ_ERROR);
     CK(cudaStreamSynchronize(stream_), SNN_GPU_WAIT_ERROR);
-    tile_par_key_ = a;
+    memcpy(&tile_par_key_, &a, sizeof a);   // compared bytewise above, padding included (build_win_params zeroes it)
     tile_par_dirty_ = false;
     return SNN_OK;
 }
@@ -2605,7 +2621,8 @@ int Engine::plan_step_path(RunPlan &pl, LaunchArgs &a) {
         const int r = build_win_params(a.win, pl.spec.chemg, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, win_mode, &pl.grid, &win);
         if (r) return r;
     }
-    last_uniform_tiles = win ? a.win.n_tiles - tile_par_mixed_ : 0u;
+    last_uniform_tiles = win ? a.win.n_tiles - tile_par_counts_[0] : 0u;
+    last_stencil_tiles = win && a.win.stencil ? a.win.n_tiles : 0u;
     if (win) {
         pl.path = StepPath::Win;
     } else if (!pl.spec.net && build_tma_params(a.tma, pl.spec.ntrel, pl.spec.stdp, pl.lft_pp, tma_mode, &pl.grid)) {

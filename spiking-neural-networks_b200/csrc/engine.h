@@ -180,6 +180,8 @@ public:
     uint32_t steps_per_graph = 0;
     uint32_t last_step_path = 0;        // SNN_OPT_STEP_PATH: step path of the last run, path + 16 * multi (0: nothing run yet)
     uint32_t last_uniform_tiles = 0;    // SNN_OPT_UNIFORM_TILES: window-kernel tiles of the last run that read their parameter row
+    uint32_t last_stencil_tiles = 0;    // SNN_OPT_STENCIL_TILES: window-kernel tiles of the last run that took their in-edge
+                                        // indices from the stencil instead of the col table
     bool force_gpart = false;           // SNN_OPT_GENERAL_PARTITION: CSR graphs of a partitioned handle always use gather-list ghosts
     uint64_t halo_timeout_ms = 30000;   // multi-GPU: how long a step may wait for a neighbouring strip before SNN_GPU_WAIT_ERROR
     std::string last_error;
@@ -327,12 +329,13 @@ private:
     bool build_tma_params(TmaParams &tp, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid);
     // *eligible = false: the window kernel does not take this configuration (the status is that of the tile-row build)
     int build_win_params(WinParams &wp, int chemg, bool ntrel, bool stdp, bool lft_pp, int mode, unsigned *grid, bool *eligible);
-    // window kernel: the tile rows (TileParSrc) and the number of tiles among them that are not uniform.  Rebuilt when a
-    // parameter array was written or moved since (tile_par_dirty_), or when a run reads another set of arrays.
+    // window kernel: the tile rows (TileParSrc) and the numbers of tiles among them that are not uniform / not stencil tiles.
+    // Rebuilt when a parameter array was written or moved, or the col table rewritten, since (tile_par_dirty_), or when a run
+    // reads another set of arrays.
     uint32_t *tile_par_ = nullptr; size_t tile_par_bytes_ = 0;
     bool tile_par_dirty_ = true;
     TileParSrc tile_par_key_{};
-    uint32_t tile_par_mixed_ = 0;
+    uint32_t tile_par_counts_[2] = {0, 0};
     int refresh_tile_params(const TileParSrc &a);
 
     // run(), phase by phase (engine.cu)

@@ -576,11 +576,23 @@ __global__ void sell_grid_kernel(uint32_t rows_local, uint32_t cols, uint32_t ro
         if ((uint64_t)(warp_global + 1) * 32u >= n) slice_off[warp_global + 1] = (warp_global + 1) * width;
     }
     const uint64_t ln = (uint64_t)warp_global * 32u + lane;
+    const size_t base = (size_t)warp_global * width * 32u + lane;
+    if (radius == 1u) {
+        // the window step kernel checks its tiles against the same function (tile_params_kernel)
+        uint32_t c[8];
+        stencil_cols((uint32_t)ln, (uint32_t)n, cols, row0_global, rows_global, own0, 0u, c);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const bool pad = c[k] == kColPad;
+            col[base + (size_t)k * 32u] = pad ? kColPad : c[k] | ((uint32_t)(node_flags[c[k]] & 0x7u) << kColNtShift);
+            wgt[base + (size_t)k * 32u] = pad ? 0.f : weight;
+        }
+        return;
+    }
     const bool valid = ln < n;
     const int64_t r = valid ? (int64_t)(ln / cols) + row0_global : 0, c0 = valid ? (int64_t)(ln % cols) : 0;
     const int R = (int)radius;
     uint32_t k = 0;
-    const size_t base = (size_t)warp_global * width * 32u + lane;
     if (valid) {
         for (int dr = -R; dr <= R; ++dr)
             for (int dc = -R; dc <= R; ++dc) {

@@ -211,6 +211,7 @@ struct GlobalSrc {
     static constexpr bool kCheapEdges = false;
     static constexpr bool kWide = false;
     static constexpr uint32_t kWidth = 0;   // slice width known at run time only
+    static constexpr bool kStencil = false;  // col words come from the table (gather_edges8)
     const StepParams &p;
     uint32_t lnc;   // clamped local neuron number
     uint32_t i;     // node index
@@ -379,7 +380,9 @@ __device__ __forceinline__ void stdp_chunk8_staged(const StepParams &p, const SR
 // FULL (warp-uniform): no lane of the warp has a padding slot and, with a single neurotransmitter type, every
 // presynaptic neuron releases it — the per-edge validity / type tests and the in-edge counters fold away.  The
 // accumulation order and every rounding are those of gather_edges (a skipped `+ 0` term of a padding slot is exact).
-template <int CHEMG, bool STDP, bool FULL, bool FULLT, class SRC>
+// STEN (with FULL): a full warp of a stencil tile (WinSrc): slot u is node i + stencil_off(u), every presynaptic node releases
+// stencil_nt(), and c[] only answers validity tests (every slot holds an edge).
+template <int CHEMG, bool STDP, bool FULL, bool FULLT, bool STEN, class SRC>
 __device__ __forceinline__ void gather_edges8_body(const StepParams &p, const SRC &src, uint32_t i, float v, float gap, int lft_me,
                                                    bool post_trig, int li, uint32_t ty0, const uint32_t (&c)[8], EdgeAcc &A) {
     constexpr int U = 8;
@@ -390,7 +393,8 @@ __device__ __forceinline__ void gather_edges8_body(const StepParams &p, const SR
     typename SRC::Handle h[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
-        j[u] = (FULL || c[u] != kColPad) ? (c[u] & kColIdxMask) : i;
+        if constexpr (STEN) j[u] = i + src.stencil_off(u);
+        else j[u] = (FULL || c[u] != kColPad) ? (c[u] & kColIdxMask) : i;
         // a full row of a generated radius-1 stencil lists its presynaptic neurons in ascending order: three in the row
         // above, the two side neighbours, three in the row below
         h[u] = FULL ? src.gh_row(u < 3 ? 0 : (u < 5 ? 1 : 2), j[u]) : src.gh(j[u]);   // u folds after unrolling
@@ -414,7 +418,8 @@ __device__ __forceinline__ void gather_edges8_body(const StepParams &p, const SR
     } else if (CHEMG == 3) {
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-            const uint32_t m = (FULL || c[u] != kColPad) ? (c[u] >> kColNtShift) : 0u;
+            uint32_t m = (FULL || c[u] != kColPad) ? (c[u] >> kColNtShift) : 0u;
+            if constexpr (STEN) m = src.stencil_nt();
 #pragma unroll
             for (int ty = 0; ty < kNT; ++ty) tj[u][ty] = (FULLT || (m & (1u << ty))) ? src.gt(h[u], ty) : 0.f;
         }
@@ -442,7 +447,8 @@ __device__ __forceinline__ void gather_edges8_body(const StepParams &p, const SR
 #pragma unroll
                 for (int ty = 0; ty < kNT; ++ty) A.acc_t[ty] = A.acc_t[ty] + tj[u][ty] * wu;
             } else {
-                const uint32_t m = ok ? (c[u] >> kColNtShift) : 0u;
+                uint32_t m = ok ? (c[u] >> kColNtShift) : 0u;
+                if constexpr (STEN) m = src.stencil_nt();
 #pragma unroll
                 for (int ty = 0; ty < kNT; ++ty) {
                     const bool has = (m >> ty) & 1u;
@@ -468,8 +474,23 @@ template <int CHEMG, bool STDP, class SRC>
 __device__ __forceinline__ void gather_edges8(const StepParams &p, const SRC &src, uint32_t i, float v, float gap, int lft_me,
                                               bool post_trig, int li, uint32_t ty0, EdgeAcc &A) {
     uint32_t c[8];
+    if constexpr (SRC::kStencil) {
+        // FULL needs, with one neurotransmitter type, that every presynaptic node releases it: uniform over the launch here
+        const uint32_t nt = src.stencil_nt();
+        if (src.stencil_full() && (CHEMG != 1 || ((nt >> ty0) & 1u))) {
 #pragma unroll
-    for (int u = 0; u < 8; ++u) c[u] = src.col(u);
+            for (int u = 0; u < 8; ++u) c[u] = 0u;
+            A.fast8 = true;
+            A.fast8t = CHEMG == 3 && nt == 7u;
+            if (CHEMG == 3 && A.fast8t) gather_edges8_body<CHEMG, STDP, true, true, true>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
+            else gather_edges8_body<CHEMG, STDP, true, false, true>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
+            return;
+        }
+        src.stencil_cols(c);   // border warps
+    } else {
+#pragma unroll
+        for (int u = 0; u < 8; ++u) c[u] = src.col(u);
+    }
     // sliced-ELL rows keep their valid entries first (sell_grid_kernel / sell_from_csr_kernel pad at the end), so a valid
     // last slot means a full row
     bool lane_full = c[7] != kColPad;
@@ -478,9 +499,9 @@ __device__ __forceinline__ void gather_edges8(const StepParams &p, const SRC &sr
     A.fast8 = __all_sync(0xffffffffu, lane_full);
     A.fast8t = false;
     if (CHEMG == 3) A.fast8t = A.fast8 && __all_sync(0xffffffffu, ((all >> kColNtShift) & 7u) == 7u);
-    if (CHEMG == 3 && A.fast8t) gather_edges8_body<CHEMG, STDP, true, true>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
-    else if (A.fast8) gather_edges8_body<CHEMG, STDP, true, false>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
-    else gather_edges8_body<CHEMG, STDP, false, false>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
+    if (CHEMG == 3 && A.fast8t) gather_edges8_body<CHEMG, STDP, true, true, false>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
+    else if (A.fast8) gather_edges8_body<CHEMG, STDP, true, false, false>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
+    else gather_edges8_body<CHEMG, STDP, false, false, false>(p, src, i, v, gap, lft_me, post_trig, li, ty0, c, A);
 }
 
 // CHEMG: 0 = no chemical gather, 1 = exactly one neurotransmitter type in the whole node array (type index ty0),

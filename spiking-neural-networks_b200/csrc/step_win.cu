@@ -12,9 +12,11 @@
 // common.h), and HBM latency is hidden by the depth of the stage ring instead of by warp occupancy.
 //
 // CTA = G groups of 8 consumer warps + kWinProducers producer warps; tile n of the CTA goes to group n % G and stage n % S.
-// The col words are still read and used (the window is selected by comparing the presynaptic index against the
-// tile's bounds), so any per-edge weight / type content of the sliced-ELL table keeps working; only the index
-// pattern must be the radius-1 stencil that set_graph_grid generates.
+// The col words are read and used (the window is selected by comparing the presynaptic index against the tile's bounds),
+// so any per-edge weight / type content of the sliced-ELL table keeps working; only the index pattern must be the
+// radius-1 stencil that set_graph_grid generates.  When tile_params_kernel has found every col word of every tile equal
+// to stencil_cols (STEN), the col words are not staged at all: full warps derive their neighbours from their own index,
+// border warps compute the words with stencil_cols, and both run the same arithmetic on them as the kernel that reads them.
 #include <type_traits>
 
 #include "step_body.cuh"
@@ -47,13 +49,16 @@ __device__ __forceinline__ float lds_f32_rt(uint32_t addr) {
 
 // UNI: every neuron of the tile has the parameters of its first one (WinLayout::o_row): f<>(), nt() and rc() read that row
 // ROWS: the stage has a row (win_layout(..., rows = true))
-template <int MODEL, int CHEMG, bool NTREL, bool STDP, bool ROWS, bool UNI>
+// STEN: every tile is a stencil tile (kTileStencil): no col words in the stage (gather_edges8 asks stencil_full() instead)
+template <int MODEL, int CHEMG, bool NTREL, bool STDP, bool ROWS, bool UNI, bool STEN>
 struct WinSrc {
     static constexpr bool kEarlyLoads = false;   // operands sit in shared memory: read them where they are used
     static constexpr bool kCheapEdges = false;
     static constexpr bool kWide = false;
+    static constexpr bool kStencil = STEN;
+    static_assert(!STEN || ROWS, "the full-warp mask of a stencil tile is in its tile row");
     static constexpr uint32_t kWidth = kWinWidth;
-    static __host__ __device__ constexpr WinLayout lay() { return win_layout(MODEL, CHEMG, NTREL, STDP, ROWS); }
+    static __host__ __device__ constexpr WinLayout lay() { return win_layout(MODEL, CHEMG, NTREL, STDP, ROWS, STEN); }
 
     const StepParams &p;
     const WinParams &wp;
@@ -99,7 +104,20 @@ struct WinSrc {
     }
     __device__ __forceinline__ float rc_state(int slot, int ty) const { return lds_f32_rt(me + wp.o_rc[slot][ty]); }
     __device__ __forceinline__ uint32_t width() const { return kWinWidth; }
-    __device__ __forceinline__ uint32_t col(uint32_t kk) const { return lds_u32<lay().o_col>(edge + kk * 128u); }
+    __device__ __forceinline__ uint32_t col(uint32_t kk) const {
+        static_assert(!STEN, "a stencil stage has no col words");
+        return lds_u32<lay().o_col>(edge + kk * 128u);
+    }
+    // STEN: this warp is full (warp-uniform; from the tile row), the lattice-wide release mask, the node index offset of slot u
+    // of a full row, and the col words of this lane (border warps)
+    __device__ __forceinline__ bool stencil_full() const { return (lds_u32<0>(row) >> (kTileFullShift + (tid >> 5))) & 1u; }
+    __device__ __forceinline__ uint32_t stencil_nt() const { return wp.stencil_nt; }
+    __device__ __forceinline__ uint32_t stencil_off(int u) const {
+        return u < 3 ? (uint32_t)(u - 1) - wp.cols : (u < 5 ? (uint32_t)(2 * u - 7) : wp.cols + (uint32_t)(u - 6));
+    }
+    __device__ __forceinline__ void stencil_cols(uint32_t (&c)[8]) const {
+        snn::stencil_cols(k0g * 4u + lane, p.n_neurons, wp.cols, wp.row0_global, wp.rows_global, p.own0, wp.stencil_nt, c);
+    }
     __device__ __forceinline__ float wgt(uint32_t kk) const { return lds_f32<lay().o_wgt>(edge + kk * 128u); }
     __device__ __forceinline__ float *wgt_ptr(uint32_t kk) const { return p.wgt + (size_t)(k0g + kk) * 32u + lane; }
     // STDP: the new weight goes to the stage (this step's gather reads it from there) and to HBM
@@ -151,12 +169,14 @@ template <int G> constexpr int win_threads() { return (G * 8 + kWinProducers) * 
 // two consumer groups (win_groups).
 enum WinRows : int { kRowsNone = 0, kRowsAll = 1, kRowsSome = 2 };
 
-template <int MODEL, int CHEMG, bool NTREL, bool STDP, int G, int ROWS>
+// STEN (kRowsAll only): every tile is a stencil tile, see WinSrc
+template <int MODEL, int CHEMG, bool NTREL, bool STDP, int G, int ROWS, bool STEN>
 __global__ void __launch_bounds__(win_threads<G>(), 1)
 step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ WinParams wp) {
     extern __shared__ __align__(128) unsigned char smem[];
     constexpr bool R = ROWS != kRowsNone;
-    constexpr WinLayout L = win_layout(MODEL, CHEMG, NTREL, STDP, R);
+    static_assert(!STEN || ROWS == kRowsAll, "stencil stages are built for lattices whose tiles all read their rows");
+    constexpr WinLayout L = win_layout(MODEL, CHEMG, NTREL, STDP, R, STEN);
     const uint32_t S = wp.stages;
     uint64_t *full = reinterpret_cast<uint64_t *>(smem + (size_t)S * wp.stage_bytes);
     uint64_t *empty = full + S;
@@ -209,7 +229,7 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
         // the tile before); only needed when some tiles are uniform and others stream their parameters
         constexpr bool flags_needed = ROWS == kRowsSome;
         auto uniform_of = [&](uint32_t seq) -> uint32_t {
-            return (flags_needed && seq < wp.n_tiles) ? __ldg(wp.tile_par + (size_t)win_tile_of<R>(p, wp, seq) * wp.row_words) : 0u;
+            return (flags_needed && seq < wp.n_tiles) ? __ldg(wp.tile_par + (size_t)win_tile_of<R>(p, wp, seq) * wp.row_words) & kTileUniform : 0u;
         };
         uint32_t uni_next = uniform_of(blockIdx.x);
         uint32_t s = 0, ph = 0;
@@ -304,14 +324,14 @@ step_win_kernel(const __grid_constant__ StepParams p, const __grid_constant__ Wi
             // this neuron inside a row-relative window: node (ts_node + tid) sits (ts_node + tid - floor4(a1)) elements in
             const uint32_t own = st + ((uint32_t)((int32_t)ts_node - (a1 & ~3)) + tid) * 4u;
             auto step = [&](auto uni) {
-                const WinSrc<MODEL, CHEMG, NTREL, STDP, R, decltype(uni)::value> src{
+                const WinSrc<MODEL, CHEMG, NTREL, STDP, R, decltype(uni)::value, STEN> src{
                     p, wp, st + tid * 4u, own, st + (wg * kWinWidth * 32u + lane) * 4u, ts_node ? ts_node - 1u : 0u, ts_node + kWinTile,
                     d0, d1, d2, warp_global * kWinWidth, lane, tid, st + L.o_row};
                 neuron_step<MODEL, CHEMG, NTREL, STDP, false>(p, src, warp_global, lane, ln, lnc, valid, export_lo, export_hi);
             };
             if constexpr (ROWS == kRowsNone) step(std::false_type{});
             else if constexpr (ROWS == kRowsAll) step(std::true_type{});
-            else if (lds_u32<L.o_row>(st) != 0u) step(std::true_type{});   // CTA-uniform
+            else if (lds_u32<L.o_row>(st) & kTileUniform) step(std::true_type{});   // CTA-uniform
             else step(std::false_type{});
         }
         __syncwarp();
@@ -344,34 +364,51 @@ cudaError_t launch_step_win(const StepParams &p, const WinParams &wp, const Step
                 if (e != cudaSuccess) return e;
                 return launch_pdl(pdl_ok(p), kern, dim3(grid), dim3(threads), smem, s, p, wp);
             };
-            if (wp.tile_par == nullptr) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsNone>, win_threads<G>());
-            if (wp.n_streams == wp.n_state) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsAll>, win_threads<G>());
-            return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, GM, kRowsSome>, win_threads<GM>());
+            if (wp.tile_par == nullptr) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsNone, false>, win_threads<G>());
+            if (wp.n_streams == wp.n_state) {
+                if (wp.stencil) return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsAll, true>, win_threads<G>());
+                return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, G, kRowsAll, false>, win_threads<G>());
+            }
+            return launch(step_win_kernel<K::MODEL, K::CHEMG, K::NTREL, K::STDP, GM, kRowsSome, false>, win_threads<GM>());
         }
     });
 }
 
-// one CTA per tile, one thread per neuron (see TileParSrc)
-__global__ void __launch_bounds__(kWinTile) tile_params_kernel(const __grid_constant__ TileParSrc a, uint32_t *rows, unsigned int *n_mixed) {
-    const uint32_t tile = blockIdx.x, ts = tile * kWinTile;
-    const bool valid = ts + threadIdx.x < a.n_neurons;
+// one CTA per tile, one thread per neuron (see TileParSrc); thread t checks lane t % 32 of the tile's warp t / 32 in the table
+__global__ void __launch_bounds__(kWinTile) tile_params_kernel(const __grid_constant__ TileParSrc a, uint32_t *rows, unsigned int *counts) {
+    __shared__ uint32_t full_warps;
+    const uint32_t tile = blockIdx.x, ts = tile * kWinTile, ln = ts + threadIdx.x;
+    const bool valid = ln < a.n_neurons;
     uint32_t *row = rows + (size_t)tile * a.row_words;
+    if (threadIdx.x == 0) full_warps = 0u;
     bool same = true;
     for (uint32_t k = 0; k < a.n_par; ++k) {
         const uint32_t first = __ldg(a.src[k] + ts);
         if (valid) same = same && __ldg(a.src[k] + ts + threadIdx.x) == first;
         if (threadIdx.x == 0) row[a.word[k]] = first;
     }
+    uint32_t c[8];
+    stencil_cols(ln, a.n_neurons, a.cols, a.row0_global, a.rows_global, a.own0, a.stencil_nt, c);
+    // the slices of a uniform-width table: warp w's k-row u at ((tile * 8 + w) * 8 + u) * 32 (allocated for whole tiles)
+    const uint32_t *cw = a.col + ((size_t)(ln >> 5) * kWinWidth) * 32u + (threadIdx.x & 31u);
+    bool sten = true;
+#pragma unroll
+    for (int u = 0; u < 8; ++u) sten = sten && __ldg(cw + u * 32) == c[u];
+    const bool full = __all_sync(0xffffffffu, c[7] != kColPad);
+    __syncthreads();
+    if (full && (threadIdx.x & 31u) == 0u) atomicOr(&full_warps, 1u << (threadIdx.x >> 5));
     const bool uni = __syncthreads_and(same) != 0;
+    const bool all_sten = __syncthreads_and(sten) != 0;
     if (threadIdx.x == 0) {
-        row[0] = uni ? 1u : 0u;
-        if (!uni) atomicAdd(n_mixed, 1u);
+        row[0] = (uni ? kTileUniform : 0u) | (all_sten ? kTileStencil : 0u) | full_warps << kTileFullShift;
+        if (!uni) atomicAdd(counts, 1u);
+        if (!all_sten) atomicAdd(counts + 1, 1u);
     }
 }
 
-cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *n_mixed, cudaStream_t s) {
+cudaError_t launch_tile_params(const TileParSrc &a, uint32_t *rows, unsigned int *counts, cudaStream_t s) {
     if (a.n_tiles == 0) return cudaSuccess;
-    tile_params_kernel<<<a.n_tiles, kWinTile, 0, s>>>(a, rows, n_mixed);
+    tile_params_kernel<<<a.n_tiles, kWinTile, 0, s>>>(a, rows, counts);
     return cudaGetLastError();
 }
 

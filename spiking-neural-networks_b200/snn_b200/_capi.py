@@ -43,9 +43,10 @@ F32, U32, I32 = range(3)
 (OPT_ELECTRICAL_SYNAPSE, OPT_CHEMICAL_SYNAPSE, OPT_DO_PLASTICITY, OPT_UPDATE_GRID_HISTORY, OPT_UPDATE_SPIKE_HISTORY,
  OPT_INTERNAL_CLOCK, OPT_PARALLEL, OPT_RNG_SEED, OPT_UPDATE_AVERAGE_HISTORY, OPT_STEPS_PER_GRAPH,
  OPT_UPDATE_EEG_HISTORY, OPT_HALO_TIMEOUT_MS, OPT_GENERAL_PARTITION, OPT_UPDATE_GRAPH_HISTORY,
- OPT_UPDATE_CONNECTING_GRAPH_HISTORY, OPT_UPDATE_SPIKE_EVENTS, OPT_STEP_PATH, OPT_UNIFORM_TILES) = range(18)
+ OPT_UPDATE_CONNECTING_GRAPH_HISTORY, OPT_UPDATE_SPIKE_EVENTS, OPT_STEP_PATH, OPT_UNIFORM_TILES, OPT_STENCIL_TILES) = range(19)
 # OPT_STEP_PATH (read-only): path + STEP_PATH_MULTI * multi of the last run
 # OPT_UNIFORM_TILES (read-only): window-kernel tiles of the last run whose neurons share every parameter (read from one tile row)
+# OPT_STENCIL_TILES (read-only): window-kernel tiles of the last run that derived their in-edge indices from the stencil
 STEP_PATH_NONE, STEP_PATH_GENERAL, STEP_PATH_WIDE, STEP_PATH_WIDE_SPLIT, STEP_PATH_TMA, STEP_PATH_WIN = range(6)
 STEP_PATH_MULTI = 16
 
